@@ -7,7 +7,10 @@ one STEP evaluates R independent hyper-parameter sets (restarts, seeded log-norm
 reference's initial values) for all 49 bins in one launch of the K6 kernel.
 metric = "NLML+grad evals/sec across bins", one eval = one full 49-bin NLML+gradient.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes the last timed step's nlml and gradient (rank 0) as DIR/nlml.npy and DIR/grad.npy, so that two
+builds can be compared output for output: the inputs depend only on the arguments.
 
 N > 1 (torchrun, one rank per GPU): bins/restarts shard across ranks with no data-path
 collective; every rank runs the same per-GPU batch (weak scaling); value = all ranks' evals /
@@ -58,6 +61,25 @@ def make_thetas(R, seed):
     rng = np.random.default_rng(seed)
     th = np.exp(0.3 * rng.standard_normal((R * NBINS, 2 * DIM + 3)))
     return np.ascontiguousarray(th), np.full(R * NBINS, 1e-3)
+
+
+DUMP_ROWS = 1 << 18  # problems kept by --dump-outputs: nlml + grad of 2^18 problems are 31.5 MB of float64
+
+
+def dump_outputs(out_dir, nlml, grad):
+    """nlml [nprob] and grad [nprob, 2d+4] (float64 tensors, as gpr_batched_nlml_grad returns them) -> out_dir/nlml.npy and
+    out_dir/grad.npy.  A step of more than DUMP_ROWS problems is cut to a seeded sample of DUMP_ROWS problems in increasing
+    order, the same on every run with the same --restarts."""
+    import torch
+
+    n = nlml.shape[0]
+    if n > DUMP_ROWS:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+        idx = torch.from_numpy(idx).to(nlml.device)
+        nlml, grad = nlml[idx], grad[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "nlml.npy"), nlml.cpu().numpy())
+    np.save(os.path.join(out_dir, "grad.npy"), grad.cpu().numpy())
 
 
 def config(R, extra=None):
@@ -208,6 +230,7 @@ class Ctx:
         if not torch.cuda.is_available():
             raise SystemExit("bench.py: no CUDA device; the product path has no CPU fallback")
         torch.cuda.set_device(self.local)
+        torch.manual_seed(self.rank)  # the potrf / covariance legs draw their inputs from torch: the same on every run
         self.dev = torch.device("cuda", self.local)
         if self.world > 1:
             dist.init_process_group("nccl", device_id=self.dev)
@@ -563,6 +586,8 @@ def run_mine(args):
     clocks = sampler.stop()
     assert h.sync() == 0
     assert bool(torch.isfinite(nlml).all()) and bool(torch.isfinite(grad).all())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, nlml, grad)
     sec = cx.max_over_ranks(sec)
     value = world * R * args.steps / sec
     kernel_sec = sec / args.steps  # one K6 launch per step
@@ -667,7 +692,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--cpu-potrf", action="store_true", help="reference arm: add the LAPACK dpotrf line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's nlml / grad to DIR/*.npy")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs applies to the GPU arm")
     if args.impl == "reference":
         run_reference(args)
     else:

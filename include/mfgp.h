@@ -85,6 +85,30 @@ int mfgp_gpr_batched_nlml_grad(mfgp_handle* h, const double* X, int N, int d, co
                                long ldy, int ycols, int B, const double* theta, const double* noise,
                                double* nlml, double* grad, int* info);
 
+/* Cached posterior of B independent exact GPs (GPflow model.posterior() with PrecomputeCacheType.TENSOR): factor once,
+ * predict many times.  X [N, d+1] is shared.  Problem b uses theta[b, 2d+3], noise[b] and the RHS columns
+ * Y[:, c : c + P] with c = (b * P) % ycols (row stride ldy; requires ycols % P == 0).  P = 1, ycols = #bins gives the
+ * per-bin convention of mfgp_gpr_batched_nlml_grad (b = r * bins + p); B = 1, P = ycols gives MultiFidelityGPModel.
+ *  - Snapshot: the posterior owns device copies of X, theta and noise and the factors W = L^-1 [B][N][ld] and
+ *    a = W Y [B][N][round_up(P, 2)]; later changes to the caller's buffers do not reach it.
+ *  - Memory: plain cudaMalloc on the handle's device (not the per-call pool, not the mfgp_workspace arena).  The posterior
+ *    belongs to that device, not to the handle: any handle on the same device may predict with it, and it may be
+ *    destroyed before or after the handle that created it.
+ *  - info [B] or NULL.  With info, a non-PD problem is that problem's status (1-based pivot in info[b]), it predicts NaN,
+ *    *out is set and the call returns the first failure's pivot like the other batched calls.  Without info, a non-PD
+ *    problem makes the call return its pivot with *out = NULL.  Creation always synchronises (it decides what is returned).
+ *  - Cost: the blocked batched factorisation (K1 -> potrf -> trtri -> a = W Y), chunked over B by free memory.
+ * mfgp_gpr_posterior_predict: mean [B, Ns, P], var [B, Ns] (the same for every column, like mfgp_gpr_predict); host or
+ * device pointers, async mode as for every call.  N <= 64, d <= 16, P <= 64 run ONE fused kernel for all problems and
+ * points (gpr_posterior_predict_kernel); anything larger the blocked route (K1, cov_diag, two batched GEMMs), chunked over
+ * B.  A point's result does not depend on the other points or problems of the call. */
+typedef struct mfgp_gpr_posterior mfgp_gpr_posterior;
+int mfgp_gpr_posterior_create(mfgp_handle* h, const double* X, int N, int d, const double* Y, long ldy, int ycols, int P,
+                              int B, const double* theta, const double* noise, int* info, mfgp_gpr_posterior** out);
+int mfgp_gpr_posterior_predict(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns,
+                               double* mean, double* var);
+int mfgp_gpr_posterior_destroy(mfgp_gpr_posterior* post);
+
 /* Training loop on the device (SURVEY 8(f) rank 1): the Adam branch of MultiFidelityGPModel.optimize (mfgpflow/linear.py:
  * 190-221: loss = -log_marginal_likelihood, tape.gradient w.r.t. the UNCONSTRAINED variables, Keras Adam, noise fixed) for
  * B independent per-bin GPs, nsteps steps without a host round trip.  Per step: theta = softplus(u) -> K6 NLML + gradient

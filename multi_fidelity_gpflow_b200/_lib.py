@@ -50,6 +50,9 @@ def _load():
         "mfgp_gpr_predict": ([vp, vp, vp, i, i, i, vp, i, vp, d, vp, vp], i),
         "mfgp_gpr_batched_nlml_grad": ([vp, vp, i, i, vp, l, i, i, vp, vp, vp, vp, vp], i),
         "mfgp_gpr_batched_adam": ([vp, vp, i, i, vp, l, i, i, vp, vp, vp, vp, vp, d, d, d, i, i, vp, vp, vp], i),
+        "mfgp_gpr_posterior_create": ([vp, vp, i, i, vp, l, i, i, i, vp, vp, vp, C.POINTER(vp)], i),
+        "mfgp_gpr_posterior_predict": ([vp, vp, vp, i, vp, vp], i),
+        "mfgp_gpr_posterior_destroy": ([vp], i),
         "mfgp_graph_nparams": ([i, i], i),
         "mfgp_graph_cov": ([vp, vp, i, i, i, vp, vp, l], i),
         "mfgp_graph_cov_diag": ([vp, vp, i, i, i, vp, vp], i),
@@ -83,6 +86,7 @@ EXPORTED_SYMBOLS = [
     "mfgp_version", "mfgp_create", "mfgp_destroy", "mfgp_set_stream", "mfgp_reset_stream", "mfgp_set_async", "mfgp_sync",
     "mfgp_last_error", "mfgp_sm_count", "mfgp_cov", "mfgp_cov_diag", "mfgp_cov_grad", "mfgp_gpr_nlml", "mfgp_gpr_nlml_grad",
     "mfgp_gpr_predict", "mfgp_gpr_batched_nlml_grad", "mfgp_gpr_batched_adam",
+    "mfgp_gpr_posterior_create", "mfgp_gpr_posterior_predict", "mfgp_gpr_posterior_destroy",
     "mfgp_graph_nparams", "mfgp_graph_cov", "mfgp_graph_cov_diag", "mfgp_graph_gpr_nlml_grad", "mfgp_svgp_elbo_grad", "mfgp_svgp_elbo_grad_v", "mfgp_svgp_predict", "mfgp_svgp_adam",
     "mfgp_svgp_flat_size", "mfgp_svgp_constrain", "mfgp_svgp_elbo_grad_flat", "mfgp_svgp_adam_update", "mfgp_gemm",
     "mfgp_potrf", "mfgp_potrf_inv", "mfgp_tall_skinny_update", "mfgp_peer_store", "mfgp_graph_mem_trim", "mfgp_workspace", "mfgp_fp64_peak",
@@ -311,6 +315,22 @@ class Handle:
             self._check(rc, "mfgp_gpr_batched_nlml_grad")
         return nlml, grad
 
+    def gpr_posterior(self, X, Y, thetas, noises, P=1, info=None):
+        """Factor B = thetas.shape[0] exact GPs once (include/mfgp.h: mfgp_gpr_posterior_create) and return a
+        GprPosterior whose predict() reuses the factors.  Y is [N, ycols]; problem b uses columns
+        Y[:, c : c + P] with c = (b * P) % ycols.  A non-positive Cholesky pivot raises NotPositiveDefiniteError unless a
+        per-problem `info` array (int32 [B]) is passed: then info[b] holds problem b's pivot (0 = ok) and it predicts NaN."""
+        X, Y, thetas, noises = as_f64(X), as_f64(Y), as_f64(thetas), as_f64(noises)
+        N, d = X.shape[0], X.shape[1] - 1
+        ycols = ldy = Y.shape[1]
+        B = thetas.shape[0]
+        out = C.c_void_p()
+        rc = _lib.mfgp_gpr_posterior_create(self._h, _ptr(X), N, d, _ptr(Y), ldy, ycols, int(P), B, _ptr(thetas),
+                                            _ptr(noises), _ptr(info), C.byref(out))
+        if not (rc > 0 and info is not None):
+            self._check(rc, "mfgp_gpr_posterior_create")
+        return GprPosterior(self, out, B, N, d, int(P))
+
     def svgp_adam(self, X, Y, L, M, P, has_W, u, m, v, mask, lr_t, beta1, beta2, eps=1e-7, scale=1.0, kl_mult=1.0,
                   hetero=False, jitter=1e-6, lik_lower=1e-6, masked=False, lik_per_output=False):
         """len(lr_t) full-batch Adam steps on the device; u, m, v (flat layout of include/mfgp.h) are updated in place.
@@ -470,6 +490,40 @@ class Handle:
         out = C.c_double(0.0)
         self._check(_lib.mfgp_fp64_peak(self._h, kind, iters, C.byref(out)), "mfgp_fp64_peak")
         return out.value
+
+
+class GprPosterior:
+    """Device-resident factors of B exact GPs (W = L^-1, a = W Y) made by Handle.gpr_posterior: a snapshot of the
+    hyper-parameters and data at creation.  predict() returns mean [B, Ns, P] and var [B, Ns]."""
+
+    def __init__(self, handle, ptr, B, N, d, P):
+        self.handle, self._p = handle, ptr
+        self.B, self.N, self.d, self.P = B, N, d, P
+
+    def predict(self, Xs, mean=None, var=None):
+        """Host arrays or device tensors; mean / var (optional outputs) may be device tensors (zero-copy)."""
+        if not self._p:
+            raise ValueError("GprPosterior is closed")
+        Xs = as_f64(Xs)
+        Ns = Xs.shape[0]
+        if Xs.shape[1] != self.d + 1:
+            raise ValueError(f"Xs must have {self.d + 1} columns")
+        mean = np.empty((self.B, Ns, self.P)) if mean is None else mean
+        var = np.empty((self.B, Ns)) if var is None else var
+        self.handle._check(_lib.mfgp_gpr_posterior_predict(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean), _ptr(var)),
+                           "mfgp_gpr_posterior_predict")
+        return mean, var
+
+    def close(self):
+        if getattr(self, "_p", None):
+            _lib.mfgp_gpr_posterior_destroy(self._p)
+            self._p = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 _default = {}

@@ -339,6 +339,133 @@ int mfgp_gpr_batched_nlml_grad(mfgp_handle* h, const double* X, int N, int d, co
 }
 
 // ---------------------------------------------------------------------------------------------
+// Cached posterior (include/mfgp.h).  One cudaMalloc block holds the device copies of X, theta, noise and the factors;
+// it belongs to the device, not to the handle that created it.
+}  // extern "C"
+
+struct mfgp_gpr_posterior {
+    int device;
+    GprPosteriorData q;
+    void* mem;
+};
+
+namespace {
+// Problems whose factorisation failed: NaN on the diagonal of W and in a (real columns), so both predict routes give NaN.
+__global__ void posterior_poison_kernel(const int* __restrict__ info, int B, int N, long ld, int P, int Pp, double* __restrict__ W,
+                                        double* __restrict__ a) {
+    const double qnan = __longlong_as_double(0x7ff8000000000000ll);
+    for (long b = blockIdx.x; b < B; b += gridDim.x) {
+        if (!info[b]) continue;
+        for (int i = threadIdx.x; i < N; i += blockDim.x) W[b * N * ld + (long)i * ld + i] = qnan;
+        for (long i = threadIdx.x; i < (long)N * Pp; i += blockDim.x)
+            if (i % Pp < P) a[b * N * Pp + i] = qnan;
+    }
+}
+}  // namespace
+
+extern "C" {
+
+int mfgp_gpr_posterior_create(mfgp_handle* h, const double* X, int N, int d, const double* Y, long ldy, int ycols, int P,
+                              int B, const double* theta, const double* noise, int* info, mfgp_gpr_posterior** out) {
+    CHECK_H(h);
+    if (out) *out = nullptr;
+    if (!out || !X || !Y || !theta || !noise || N < 1 || d < 1 || d > MFGP_MAX_D || P < 1 || B < 1 || ycols < P ||
+        ycols % P != 0 || ldy < ycols)
+        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_gpr_posterior_create: bad argument (ycols must be a multiple of P)");
+    cudaSetDevice(h->device);
+    const int np = 2 * d + 3, Pp = (int)round_up(P, 2);
+    const long ld = round_up(N, 2);
+    size_t tot = 0;
+    auto carve = [&](size_t count) {
+        const size_t o = tot;
+        tot += (count * sizeof(double) + 255) & ~(size_t)255;
+        return o;
+    };
+    const size_t oX = carve((size_t)N * (d + 1)), oT = carve((size_t)B * np), oN = carve(B),
+                 oW = carve((size_t)B * N * ld), oA = carve((size_t)B * N * Pp);
+    void* mem = nullptr;
+    CUDA_TRY(h, cudaMalloc(&mem, tot));
+    char* base = static_cast<char*>(mem);
+    double *dX = reinterpret_cast<double*>(base + oX), *dT = reinterpret_cast<double*>(base + oT),
+           *dN = reinterpret_cast<double*>(base + oN), *dW = reinterpret_cast<double*>(base + oW),
+           *dA = reinterpret_cast<double*>(base + oA);
+    const int rc = [&]() -> int {
+        Scope sc(h);
+        cudaStream_t s = h->stream;
+        CUDA_TRY(h, cudaMemcpyAsync(dX, X, (size_t)N * (d + 1) * sizeof(double), cudaMemcpyDefault, s));
+        CUDA_TRY(h, cudaMemcpyAsync(dT, theta, (size_t)B * np * sizeof(double), cudaMemcpyDefault, s));
+        CUDA_TRY(h, cudaMemcpyAsync(dN, noise, (size_t)B * sizeof(double), cudaMemcpyDefault, s));
+        const double* dY = sc.in(Y, (size_t)N * ldy);
+        int* di = info ? sc.out(info, B, true) : sc.alloc<int>(B, true);
+        if (!sc.ok) return sc.finish();
+        // the blocked batched route of mfgp_gpr_batched_nlml_grad, chunked so that its workspaces fit comfortably
+        size_t freeb = 0, totb = 0;
+        cudaMemGetInfo(&freeb, &totb);
+        const size_t per = ((size_t)3 * N * ld + (size_t)chol_dinv_count(N, 1) + (size_t)2 * N * Pp + N) * sizeof(double);
+        long chunk = (long)((freeb / 2) / per);
+        if (chunk < 1) chunk = 1;
+        if (chunk > 16384) chunk = 16384;
+        for (long b0 = 0; b0 < B; b0 += chunk) {
+            const int nb = (int)((B - b0) < chunk ? (B - b0) : chunk);
+            Scope inner(h);
+            GprFactor f;
+            MFGP_TRY(gpr_factor(h, inner, dX, dY, ldy, P, (int)b0, ycols, N, d, P, nb, dT + b0 * np, dN + b0, di + b0, f, true));
+            if (!inner.ok) return inner.finish();
+            CUDA_TRY(h, cudaMemcpyAsync(dW + b0 * N * ld, f.W, (size_t)nb * N * ld * sizeof(double), cudaMemcpyDeviceToDevice, s));
+            CUDA_TRY(h, cudaMemcpyAsync(dA + b0 * N * Pp, f.a, (size_t)nb * N * Pp * sizeof(double), cudaMemcpyDeviceToDevice, s));
+        }
+        posterior_poison_kernel<<<(unsigned)(B < 4096 ? B : 4096), 128, 0, s>>>(di, B, N, ld, P, Pp, dW, dA);
+        sc.host_out = true;  // always synchronise: the factorisation status decides what the call returns
+        return sc.finish();
+    }();
+    if (rc < 0 || (rc > 0 && !info)) {
+        cudaFree(mem);
+        return rc;
+    }
+    auto* post = new mfgp_gpr_posterior();
+    post->device = h->device;
+    post->mem = mem;
+    post->q = GprPosteriorData{N, d, P, Pp, B, ld, dX, dT, dN, dW, dA};
+    *out = post;
+    return rc;
+}
+
+int mfgp_gpr_posterior_predict(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns, double* mean,
+                               double* var) {
+    CHECK_H(h);
+    if (!post || !Xs || !mean || !var || Ns < 0) return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_gpr_posterior_predict: bad argument");
+    if (post->device != h->device)
+        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_gpr_posterior_predict: the posterior lives on device %d, the handle on %d",
+                         post->device, h->device);
+    if (Ns == 0) return 0;
+    cudaSetDevice(h->device);
+    const GprPosteriorData& q = post->q;
+    Scope sc(h);
+    const double* dXs = sc.in(Xs, (size_t)Ns * (q.d + 1));
+    double* dm = sc.out(mean, (size_t)q.B * Ns * q.P);
+    double* dv = sc.out(var, (size_t)q.B * Ns);
+    if (!sc.ok) return sc.finish();
+    if (gpr_posterior_fused_ok(q.N, q.d, q.P)) {
+        if (gpr_posterior_predict_fused(h->stream, q, dXs, Ns, dm, dv))
+            return mfgp_fail(h, MFGP_ERR_CUDA, "gpr_posterior_predict_kernel launch failed");
+    } else {
+        MFGP_TRY(gpr_posterior_predict_blocked(h, q, dXs, Ns, dm, dv));
+    }
+    return sc.finish();
+}
+
+int mfgp_gpr_posterior_destroy(mfgp_gpr_posterior* post) {
+    if (!post) return 0;
+    int prev = 0;
+    cudaGetDevice(&prev);
+    cudaSetDevice(post->device);
+    const cudaError_t e = cudaFree(post->mem);
+    cudaSetDevice(prev);
+    delete post;
+    return e == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+}
+
+// ---------------------------------------------------------------------------------------------
 int mfgp_cov_grad(mfgp_handle* h, const double* X, int N, int d, const double* theta, const double* G, long ldg, double scale,
                   double* out) {
     CHECK_H(h);

@@ -53,25 +53,29 @@ __global__ void nlml_kernel(const double* __restrict__ a, int N, int Pp, int P, 
     if (threadIdx.x == 0) out[b] = 0.5 * q + P * ld + 0.5 * (double)N * P * LOG2PI;
 }
 
-// var[j] = kss[j] - sum_i As[i][j]^2
+// var[b][j] = kss[b][j] - sum_i As[b][i][j]^2  (problem b = blockIdx.y; As stride strideA, kss / var stride Ns)
 __global__ void predict_var_kernel(const double* __restrict__ As, int N, int Ns, long ld, const double* __restrict__ kss,
-                                   double* __restrict__ var) {
+                                   double* __restrict__ var, long strideA) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= Ns) return;
+    const long b = blockIdx.y;
+    As += b * strideA;
     double s = 0.0;
     for (int i = 0; i < N; ++i) {
         const double v = As[(long)i * ld + j];
         s = fma(v, v, s);
     }
-    var[j] = kss[j] - s;
+    var[b * Ns + j] = kss[b * Ns + j] - s;
 }
+
+}  // namespace
 
 using Factor = GprFactor;
 
 // Assemble + factor + invert + a = W Y for `batch` problems.  theta_d/noise_d are device arrays.
-int factor(mfgp_handle* h, Scope& sc, const double* X, const double* Y, long ldy, int per_batch_cols, int b_off,
-           int ycols, int N, int d, int P, int batch, const double* theta_d, const double* noise_d, int* info_vec, Factor& f,
-           bool want_W = true) {
+int gpr_factor(mfgp_handle* h, Scope& sc, const double* X, const double* Y, long ldy, int per_batch_cols, int b_off,
+               int ycols, int N, int d, int P, int batch, const double* theta_d, const double* noise_d, int* info_vec,
+               Factor& f, bool want_W) {
     MFGP_TRY(gpr_factor_alloc(h, sc, N, P, batch, f, want_W));
     CovArgs c{};
     c.Xa = X; c.Na = N; c.Xb = X; c.Nb = N; c.d = d;
@@ -83,8 +87,6 @@ int factor(mfgp_handle* h, Scope& sc, const double* X, const double* Y, long ldy
     if (launch_cov(h->stream, c)) return mfgp_fail(h, MFGP_ERR_CUDA, "cov launch failed");
     return gpr_factor_from_K(h, Y, ldy, per_batch_cols, b_off, ycols, N, P, batch, info_vec, f);
 }
-
-}  // namespace
 
 int gpr_factor_alloc(mfgp_handle* h, Scope& sc, int N, int P, int batch, GprFactor& f, bool want_W) {
     f.ld = round_up(N, 2);
@@ -204,7 +206,7 @@ int gpr_nlml_grad_device(mfgp_handle* h, Scope& sc, const double* X, const doubl
                          double* nlml_d, double* grad_d, int* info_vec) {
     cudaStream_t s = h->stream;
     Factor f;
-    MFGP_TRY(factor(h, sc, X, Y, ldy, per_batch_cols, b_off, ycols, N, d, P, batch, theta_d, noise_d, info_vec, f, grad_d != nullptr));
+    MFGP_TRY(gpr_factor(h, sc, X, Y, ldy, per_batch_cols, b_off, ycols, N, d, P, batch, theta_d, noise_d, info_vec, f, grad_d != nullptr));
     gpr_nlml_from_factor(h, f, N, P, batch, nlml_d);
     if (!grad_d) return 0;
     MFGP_TRY(gpr_build_G(h, sc, N, P, batch, f));
@@ -234,7 +236,7 @@ int gpr_predict_device(mfgp_handle* h, Scope& sc, const double* X, const double*
     // flops) for as long as Ns < N: measured at N = 16 384 (scripts/predict_once.py) 61 + 0.0098 Ns ms against
     // 100 + 0.0077 Ns ms for W + one full-rate GEMM.
     const bool want_W = Ns > N;
-    MFGP_TRY(factor(h, sc, X, Y, P, 0, 0, 0, N, d, P, 1, theta_d, noise_d, nullptr, f, want_W));
+    MFGP_TRY(gpr_factor(h, sc, X, Y, P, 0, 0, 0, N, d, P, 1, theta_d, noise_d, nullptr, f, want_W));
     const long lds = round_up(Ns, 2);
     double* Ks = sc.alloc<double>((size_t)N * lds);
     double* As = sc.alloc<double>((size_t)N * lds);
@@ -259,7 +261,7 @@ int gpr_predict_device(mfgp_handle* h, Scope& sc, const double* X, const double*
     } else {
         MFGP_TRY(gpr_forward_subst(h, f, N, 1, Ks, As, Ns, lds, 0));
     }
-    predict_var_kernel<<<(Ns + 127) / 128, 128, 0, s>>>(As, N, Ns, lds, kss, var_d);
+    predict_var_kernel<<<(Ns + 127) / 128, 128, 0, s>>>(As, N, Ns, lds, kss, var_d, 0);
     GemmArgs m;  // mean = As^T a
     m.transA = true; m.transB = false;
     m.M = Ns; m.N = P; m.K = N;
@@ -267,5 +269,55 @@ int gpr_predict_device(mfgp_handle* h, Scope& sc, const double* X, const double*
     m.B = f.a; m.ldb = f.Pp;
     m.C = mean_d; m.ldc = P;
     if (launch_gemm(s, m)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (mean) failed");
+    return 0;
+}
+
+// Cached-posterior prediction for any N, d, P: per chunk of problems  K_s = K(X, Xs) (K1, batched rectangular), k_ss,
+// A_s = W K_s, var = k_ss - colsum(A_s^2), mean = A_s^T a.  Chunked so that K_s and A_s of a chunk take at most half of
+// the free device memory.
+int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
+                                  double* var) {
+    cudaStream_t s = h->stream;
+    const int np = 2 * q.d + 3, N = q.N;
+    const long lds = round_up(Ns, 2);
+    size_t freeb = 0, totb = 0;
+    cudaMemGetInfo(&freeb, &totb);
+    const size_t per = ((size_t)2 * N * lds + Ns) * sizeof(double);
+    long chunk = (long)((freeb / 2) / per);
+    if (chunk < 1) chunk = 1;
+    if (chunk > 16384) chunk = 16384;  // grid z of the batched kernels
+    for (long b0 = 0; b0 < q.B; b0 += chunk) {
+        const int nb = (int)((q.B - b0) < chunk ? (q.B - b0) : chunk);
+        Scope inner(h);
+        double* Ks = inner.alloc<double>((size_t)nb * N * lds);
+        double* As = inner.alloc<double>((size_t)nb * N * lds);
+        double* kss = inner.alloc<double>((size_t)nb * Ns);
+        if (!inner.ok) return inner.finish();
+        const double* th = q.theta + b0 * np;
+        CovArgs c{};
+        c.Xa = q.X; c.Na = N; c.Xb = Xs; c.Nb = Ns; c.d = q.d;
+        c.theta = th; c.theta_stride = np;
+        c.K = Ks; c.ldk = lds; c.strideK = (long)N * lds;
+        c.batch = nb;
+        if (launch_cov(s, c)) return mfgp_fail(h, MFGP_ERR_CUDA, "cov launch failed");
+        if (launch_cov_diag(s, Xs, Ns, q.d, th, np, kss, Ns, nb)) return mfgp_fail(h, MFGP_ERR_CUDA, "cov_diag failed");
+        GemmArgs g;  // A_s = W K_s
+        g.M = N; g.N = Ns; g.K = N;
+        g.A = q.W + b0 * N * q.ld; g.lda = q.ld; g.strideA = (long)N * q.ld;
+        g.B = Ks; g.ldb = lds; g.strideB = (long)N * lds;
+        g.C = As; g.ldc = lds; g.strideC = (long)N * lds;
+        g.batch = nb;
+        g.krange = KR_HI_I;
+        if (launch_gemm(s, g)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (As) failed");
+        predict_var_kernel<<<dim3((Ns + 127) / 128, nb), 128, 0, s>>>(As, N, Ns, lds, kss, var + b0 * Ns, (long)N * lds);
+        GemmArgs m;  // mean = A_s^T a
+        m.transA = true;
+        m.M = Ns; m.N = q.P; m.K = N;
+        m.A = As; m.lda = lds; m.strideA = (long)N * lds;
+        m.B = q.a + b0 * N * q.Pp; m.ldb = q.Pp; m.strideB = (long)N * q.Pp;
+        m.C = mean + b0 * Ns * q.P; m.ldc = q.P; m.strideC = (long)Ns * q.P;
+        m.batch = nb;
+        if (launch_gemm(s, m)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (mean) failed");
+    }
     return 0;
 }

@@ -30,3 +30,31 @@ int gpr_forward_subst(mfgp_handle* h, const GprFactor& f, int N, int batch, doub
 void gpr_nlml_from_factor(mfgp_handle* h, const GprFactor& f, int N, int P, int batch, double* nlml_d);
 // ... and f.G (lower tiles) <- alpha alpha^T - P K^-1.
 int gpr_build_G(mfgp_handle* h, Scope& sc, int N, int P, int batch, GprFactor& f);
+// Assemble (K1 + noise) -> factor -> (want_W) W = L^-1 -> a = W Y for `batch` problems, RHS columns as in
+// gpr_nlml_grad_device.  theta_d [batch, 2d+3] and noise_d [batch] are device arrays; buffers come from `sc`.
+int gpr_factor(mfgp_handle* h, Scope& sc, const double* X, const double* Y, long ldy, int per_batch_cols, int b_off,
+               int ycols, int N, int d, int P, int batch, const double* theta_d, const double* noise_d, int* info_vec,
+               GprFactor& f, bool want_W = true);
+
+// Cached posterior of B exact GPs that share X (mfgp_gpr_posterior_* in include/mfgp.h).  The storage format both predict
+// routes read; every pointer is device memory owned by the posterior.
+//   W [B][N][ld]  W = L^-1 of K + noise I: lower triangle; zero above the diagonal and in the padding column (ld even)
+//   a [B][N][Pp]  a = W Y (Pp = round_up(P, 2), padding column zero)
+// A problem whose factorisation failed holds NaN on the diagonal of W and in all of a, so both routes predict NaN for it.
+struct GprPosteriorData {
+    int N, d, P, Pp, B;
+    long ld;
+    const double* X;      // [N, d+1]
+    const double* theta;  // [B, 2d+3]
+    const double* noise;  // [B]
+    const double* W;
+    const double* a;
+};
+// mean [B][Ns][P], var [B][Ns]; all device pointers.
+// Fused route (gpr_posterior.cu): one kernel, N <= 64, d <= 16, P <= 64 (gpr_posterior_fused_ok).
+bool gpr_posterior_fused_ok(int N, int d, int P);
+int gpr_posterior_predict_fused(cudaStream_t s, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
+                                double* var);
+// Blocked route (gpr.cu): any size, built from K1 / cov_diag / the batched GEMM, chunked over problems.
+int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
+                                  double* var);

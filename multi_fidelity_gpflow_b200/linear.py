@@ -77,6 +77,15 @@ class MultiFidelityGPModel:
         mean, var = self.predict_f(Xnew)
         return mean, var + float(self.likelihood.variance.numpy())
 
+    def posterior(self):
+        """Cached posterior at the current parameters (GPflow's model.posterior(), PrecomputeCacheType.TENSOR): the
+        factorisation is done once here and reused by every predict_f / predict_y of the returned object; later training
+        does not change it.  predict_f keeps the reference's behaviour of factoring on every call."""
+        X, Y = self.data
+        theta, noise = self._theta_noise()
+        post = self.handle.gpr_posterior(X, Y, np.ascontiguousarray(theta)[None, :], np.array([noise]), P=Y.shape[1])
+        return MultiFidelityGPPosterior(post, noise)
+
     # ---- training loops (linear.py:190-234) ----------------------------------------------------
     def optimize(self, max_iters=1000, learning_rate=0.01, use_adam=True, unfix_noise_after=500, verbose=True):
         self.loss_history = []
@@ -105,3 +114,24 @@ class MultiFidelityGPModel:
             vs = self.trainable_variables
             opt.minimize(lambda: self.value_and_grad(vs), vs, options={"maxiter": max_iters})
         return self
+
+
+class MultiFidelityGPPosterior:
+    """What MultiFidelityGPModel.posterior returns: predict_f / predict_y with the model's shapes, from cached factors."""
+
+    def __init__(self, post, noise):
+        self._post = post
+        self.noise = float(noise)
+
+    def predict_f(self, Xnew, full_cov=False, full_output_cov=False):
+        if full_cov or full_output_cov:
+            raise NotImplementedError("the reference only calls predict_f(Xnew) (marginal variances)")
+        mean, var = self._post.predict(np.ascontiguousarray(Xnew, dtype=np.float64))
+        return mean[0], np.tile(var[0][:, None], (1, mean.shape[2]))  # same variance in every output column
+
+    def predict_y(self, Xnew):
+        mean, var = self.predict_f(Xnew)
+        return mean, var + self.noise
+
+    def close(self):
+        self._post.close()

@@ -99,3 +99,48 @@ class MultiBinMFGP:
             mu, s2 = self.handle.gpr_predict(self.X, np.ascontiguousarray(self.Y[:, p:p + 1]), Xnew, th[p], self.noise)
             mean[:, p], var[:, p] = mu[:, 0], s2
         return mean, var
+
+    def posterior(self, restarts="best"):
+        """Cached posterior of the bins at the current hyper-parameters (a snapshot: later training does not change it).
+        restarts="best": each bin at its best restart, predict_f(Xnew) -> [N*, P] (equal to predict_f);
+        "all": every (restart, bin), predict_f -> [R, N*, P], NaN for a restart whose covariance is not positive
+        definite.  One cached factorisation per problem b = r * P + p; every prediction is one library call."""
+        if restarts == "best":
+            th = self.best_thetas()
+            post = self.handle.gpr_posterior(self.X, self.Y, np.ascontiguousarray(th), np.full(self.P, self.noise))
+            return MultiBinPosterior(post, np.full(self.P, self.noise), None)
+        if restarts == "all":
+            B = self.R * self.P
+            info = np.zeros(B, dtype=np.int32)
+            post = self.handle.gpr_posterior(self.X, self.Y, np.ascontiguousarray(self.thetas.reshape(B, -1)),
+                                             np.full(B, self.noise), info=info)
+            return MultiBinPosterior(post, np.full(B, self.noise).reshape(self.R, self.P), info.reshape(self.R, self.P))
+        raise ValueError('restarts must be "best" or "all"')
+
+
+class MultiBinPosterior:
+    """What MultiBinMFGP.posterior returns: predictions of every bin (and restart) from factors kept on the device."""
+
+    def __init__(self, post, noises, failed):
+        self._post = post
+        self.noises = noises  # [P] ("best") or [R, P] ("all")
+        self.failed = failed  # [R, P] first failing pivot per (restart, bin) at creation, 0 = ok; None for "best"
+
+    def predict_f(self, Xnew):
+        """Mean and variance [N*, P] ("best") or [R, N*, P] ("all")."""
+        mean, var = self._post.predict(np.ascontiguousarray(Xnew, dtype=np.float64))  # [B, N*, 1], [B, N*]
+        P = self.noises.shape[-1]
+        mean = mean[:, :, 0].reshape(-1, P, mean.shape[1])
+        var = var.reshape(-1, P, var.shape[1])
+        mean, var = np.swapaxes(mean, 1, 2), np.swapaxes(var, 1, 2)  # [R, N*, P]
+        if self.noises.ndim == 1:
+            return np.ascontiguousarray(mean[0]), np.ascontiguousarray(var[0])
+        return mean, var
+
+    def predict_y(self, Xnew):
+        """predict_f plus each problem's likelihood noise on the variance."""
+        mean, var = self.predict_f(Xnew)
+        return mean, var + (self.noises if self.noises.ndim == 1 else self.noises[:, None, :])
+
+    def close(self):
+        self._post.close()

@@ -107,6 +107,16 @@ int mfgp_gpr_posterior_create(mfgp_handle* h, const double* X, int N, int d, con
                               int B, const double* theta, const double* noise, int* info, mfgp_gpr_posterior** out);
 int mfgp_gpr_posterior_predict(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns,
                                double* mean, double* var);
+/* mfgp_gpr_posterior_predict_grad: mean [B, Ns, P] and var [B, Ns] as mfgp_gpr_posterior_predict, and their gradients
+ * with respect to the d continuous coordinates of each test point, dmean [B, Ns, P, d] = d mean / d Xs[s, j] and
+ * dvar [B, Ns, d] = d var / d Xs[s, j] (the fidelity column has no gradient: it enters the kernel only through equality
+ * masks).  All four outputs are required.  A test row with fidelity not in {0, 1} has zero gradients; a problem whose
+ * factorisation failed gives NaN in all four.  Pointers, async mode, the device check and Ns == 0 as for _predict.  The
+ * fused route (N <= 64, d <= 16, P <= 64) is one kernel, gpr_posterior_predict_grad_kernel; the blocked route adds
+ * beta = K^-1 K_s and alpha = W^T a (two batched GEMMs) and posterior_dx_kernel to the _predict pipeline.  A point's
+ * results do not depend on the other points or problems of the call. */
+int mfgp_gpr_posterior_predict_grad(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns,
+                                    double* mean, double* var, double* dmean, double* dvar);
 int mfgp_gpr_posterior_destroy(mfgp_gpr_posterior* post);
 
 /* Training loop on the device (SURVEY 8(f) rank 1): the Adam branch of MultiFidelityGPModel.optimize (mfgpflow/linear.py:

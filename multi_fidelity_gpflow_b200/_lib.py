@@ -52,6 +52,7 @@ def _load():
         "mfgp_gpr_batched_adam": ([vp, vp, i, i, vp, l, i, i, vp, vp, vp, vp, vp, d, d, d, i, i, vp, vp, vp], i),
         "mfgp_gpr_posterior_create": ([vp, vp, i, i, vp, l, i, i, i, vp, vp, vp, C.POINTER(vp)], i),
         "mfgp_gpr_posterior_predict": ([vp, vp, vp, i, vp, vp], i),
+        "mfgp_gpr_posterior_predict_grad": ([vp, vp, vp, i, vp, vp, vp, vp], i),
         "mfgp_gpr_posterior_destroy": ([vp], i),
         "mfgp_graph_nparams": ([i, i], i),
         "mfgp_graph_cov": ([vp, vp, i, i, i, vp, vp, l], i),
@@ -86,7 +87,8 @@ EXPORTED_SYMBOLS = [
     "mfgp_version", "mfgp_create", "mfgp_destroy", "mfgp_set_stream", "mfgp_reset_stream", "mfgp_set_async", "mfgp_sync",
     "mfgp_last_error", "mfgp_sm_count", "mfgp_cov", "mfgp_cov_diag", "mfgp_cov_grad", "mfgp_gpr_nlml", "mfgp_gpr_nlml_grad",
     "mfgp_gpr_predict", "mfgp_gpr_batched_nlml_grad", "mfgp_gpr_batched_adam",
-    "mfgp_gpr_posterior_create", "mfgp_gpr_posterior_predict", "mfgp_gpr_posterior_destroy",
+    "mfgp_gpr_posterior_create", "mfgp_gpr_posterior_predict", "mfgp_gpr_posterior_predict_grad",
+    "mfgp_gpr_posterior_destroy",
     "mfgp_graph_nparams", "mfgp_graph_cov", "mfgp_graph_cov_diag", "mfgp_graph_gpr_nlml_grad", "mfgp_svgp_elbo_grad", "mfgp_svgp_elbo_grad_v", "mfgp_svgp_predict", "mfgp_svgp_adam",
     "mfgp_svgp_flat_size", "mfgp_svgp_constrain", "mfgp_svgp_elbo_grad_flat", "mfgp_svgp_adam_update", "mfgp_gemm",
     "mfgp_potrf", "mfgp_potrf_inv", "mfgp_tall_skinny_update", "mfgp_peer_store", "mfgp_graph_mem_trim", "mfgp_workspace", "mfgp_fp64_peak",
@@ -513,6 +515,23 @@ class GprPosterior:
         self.handle._check(_lib.mfgp_gpr_posterior_predict(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean), _ptr(var)),
                            "mfgp_gpr_posterior_predict")
         return mean, var
+
+    def predict_grad(self, Xs, mean=None, var=None, dmean=None, dvar=None):
+        """predict() plus the gradients with respect to the d continuous coordinates of each test point:
+        (mean [B, Ns, P], var [B, Ns], dmean [B, Ns, P, d], dvar [B, Ns, d]).  Host arrays or device tensors."""
+        if not self._p:
+            raise ValueError("GprPosterior is closed")
+        Xs = as_f64(Xs)
+        Ns = Xs.shape[0]
+        if Xs.shape[1] != self.d + 1:
+            raise ValueError(f"Xs must have {self.d + 1} columns")
+        mean = np.empty((self.B, Ns, self.P)) if mean is None else mean
+        var = np.empty((self.B, Ns)) if var is None else var
+        dmean = np.empty((self.B, Ns, self.P, self.d)) if dmean is None else dmean
+        dvar = np.empty((self.B, Ns, self.d)) if dvar is None else dvar
+        self.handle._check(_lib.mfgp_gpr_posterior_predict_grad(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean), _ptr(var),
+                                                                _ptr(dmean), _ptr(dvar)), "mfgp_gpr_posterior_predict_grad")
+        return mean, var, dmean, dvar
 
     def close(self):
         if getattr(self, "_p", None):

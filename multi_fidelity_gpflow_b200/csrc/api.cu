@@ -430,13 +430,17 @@ int mfgp_gpr_posterior_create(mfgp_handle* h, const double* X, int N, int d, con
     return rc;
 }
 
-int mfgp_gpr_posterior_predict(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns, double* mean,
-                               double* var) {
+}  // extern "C"
+
+namespace {
+// mfgp_gpr_posterior_predict and _predict_grad: one body, the gradients when dmean != NULL.
+int posterior_predict(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns, double* mean, double* var,
+                      double* dmean, double* dvar, const char* name) {
     CHECK_H(h);
-    if (!post || !Xs || !mean || !var || Ns < 0) return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_gpr_posterior_predict: bad argument");
+    if (!post || !Xs || !mean || !var || Ns < 0) return mfgp_fail(h, MFGP_ERR_ARG, "%s: bad argument", name);
     if (post->device != h->device)
-        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_gpr_posterior_predict: the posterior lives on device %d, the handle on %d",
-                         post->device, h->device);
+        return mfgp_fail(h, MFGP_ERR_ARG, "%s: the posterior lives on device %d, the handle on %d", name, post->device,
+                         h->device);
     if (Ns == 0) return 0;
     cudaSetDevice(h->device);
     const GprPosteriorData& q = post->q;
@@ -444,14 +448,33 @@ int mfgp_gpr_posterior_predict(mfgp_handle* h, const mfgp_gpr_posterior* post, c
     const double* dXs = sc.in(Xs, (size_t)Ns * (q.d + 1));
     double* dm = sc.out(mean, (size_t)q.B * Ns * q.P);
     double* dv = sc.out(var, (size_t)q.B * Ns);
+    double* ddm = dmean ? sc.out(dmean, (size_t)q.B * Ns * q.P * q.d) : nullptr;
+    double* ddv = dmean ? sc.out(dvar, (size_t)q.B * Ns * q.d) : nullptr;
     if (!sc.ok) return sc.finish();
     if (gpr_posterior_fused_ok(q.N, q.d, q.P)) {
-        if (gpr_posterior_predict_fused(h->stream, q, dXs, Ns, dm, dv))
-            return mfgp_fail(h, MFGP_ERR_CUDA, "gpr_posterior_predict_kernel launch failed");
+        if (gpr_posterior_predict_fused(h->stream, q, dXs, Ns, dm, dv, ddm, ddv))
+            return mfgp_fail(h, MFGP_ERR_CUDA, "%s: fused kernel launch failed", name);
     } else {
-        MFGP_TRY(gpr_posterior_predict_blocked(h, q, dXs, Ns, dm, dv));
+        MFGP_TRY(gpr_posterior_predict_blocked(h, q, dXs, Ns, dm, dv, ddm, ddv));
     }
     return sc.finish();
+}
+}  // namespace
+
+extern "C" {
+
+int mfgp_gpr_posterior_predict(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns, double* mean,
+                               double* var) {
+    return posterior_predict(h, post, Xs, Ns, mean, var, nullptr, nullptr, "mfgp_gpr_posterior_predict");
+}
+
+int mfgp_gpr_posterior_predict_grad(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns, double* mean,
+                                    double* var, double* dmean, double* dvar) {
+    if (!dmean || !dvar) {
+        CHECK_H(h);
+        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_gpr_posterior_predict_grad: bad argument (dmean and dvar are required)");
+    }
+    return posterior_predict(h, post, Xs, Ns, mean, var, dmean, dvar, "mfgp_gpr_posterior_predict_grad");
 }
 
 int mfgp_gpr_posterior_destroy(mfgp_gpr_posterior* post) {

@@ -274,15 +274,16 @@ int gpr_predict_device(mfgp_handle* h, Scope& sc, const double* X, const double*
 
 // Cached-posterior prediction for any N, d, P: per chunk of problems  K_s = K(X, Xs) (K1, batched rectangular), k_ss,
 // A_s = W K_s, var = k_ss - colsum(A_s^2), mean = A_s^T a.  Chunked so that K_s and A_s of a chunk take at most half of
-// the free device memory.
+// the free device memory.  With dmean / dvar the chunk goes on from the same A_s: beta = W^T A_s = K^-1 K_s (into the
+// K_s buffer, which is free by then), alpha = W^T a, and posterior_dx_kernel contracts dK_s/dx* with both.
 int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
-                                  double* var) {
+                                  double* var, double* dmean, double* dvar) {
     cudaStream_t s = h->stream;
     const int np = 2 * q.d + 3, N = q.N;
     const long lds = round_up(Ns, 2);
     size_t freeb = 0, totb = 0;
     cudaMemGetInfo(&freeb, &totb);
-    const size_t per = ((size_t)2 * N * lds + Ns) * sizeof(double);
+    const size_t per = ((size_t)2 * N * lds + Ns + (dmean ? (size_t)N * q.Pp : 0)) * sizeof(double);
     long chunk = (long)((freeb / 2) / per);
     if (chunk < 1) chunk = 1;
     if (chunk > 16384) chunk = 16384;  // grid z of the batched kernels
@@ -292,6 +293,7 @@ int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, con
         double* Ks = inner.alloc<double>((size_t)nb * N * lds);
         double* As = inner.alloc<double>((size_t)nb * N * lds);
         double* kss = inner.alloc<double>((size_t)nb * Ns);
+        double* alpha = dmean ? inner.alloc<double>((size_t)nb * N * q.Pp) : nullptr;
         if (!inner.ok) return inner.finish();
         const double* th = q.theta + b0 * np;
         CovArgs c{};
@@ -318,6 +320,29 @@ int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, con
         m.C = mean + b0 * Ns * q.P; m.ldc = q.P; m.strideC = (long)Ns * q.P;
         m.batch = nb;
         if (launch_gemm(s, m)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (mean) failed");
+        if (!dmean) continue;
+        GemmArgs bt;  // beta = W^T A_s, into the K_s buffer
+        bt.transA = true;
+        bt.M = N; bt.N = Ns; bt.K = N;
+        bt.A = g.A; bt.lda = q.ld; bt.strideA = g.strideA;
+        bt.B = As; bt.ldb = lds; bt.strideB = (long)N * lds;
+        bt.C = Ks; bt.ldc = lds; bt.strideC = (long)N * lds;
+        bt.batch = nb;
+        bt.krange = KR_LO_I;
+        if (launch_gemm(s, bt)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (beta) failed");
+        GemmArgs at;  // alpha = W^T a
+        at.transA = true;
+        at.M = N; at.N = q.Pp; at.K = N;
+        at.A = g.A; at.lda = q.ld; at.strideA = g.strideA;
+        at.B = m.B; at.ldb = q.Pp; at.strideB = m.strideB;
+        at.C = alpha; at.ldc = q.Pp; at.strideC = (long)N * q.Pp;
+        at.batch = nb;
+        at.krange = KR_LO_I;
+        if (launch_gemm(s, at)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (alpha) failed");
+        GprPosteriorData qc = q;
+        qc.theta = th;
+        if (launch_posterior_dx(s, qc, nb, Xs, Ns, alpha, Ks, lds, dmean + b0 * Ns * q.P * q.d, dvar + b0 * Ns * q.d))
+            return mfgp_fail(h, MFGP_ERR_CUDA, "posterior_dx_kernel launch failed");
     }
     return 0;
 }

@@ -11,6 +11,17 @@
 //                    (k-step 2i + e <-> n = 8i + 2t + e), so V feeds the next product without a transpose; DFMA below 8
 // Every value of a test point is computed by the lanes of its own row from its own inputs: no cross-point reduction and
 // no atomics, so a result does not depend on which other points or problems share the call.
+//
+// gpr_posterior_predict_grad_kernel (mfgp_gpr_posterior_predict_grad) adds d mean / dx* and d var / dx* on the same
+// decomposition.  K_s is built in its two parts kL and kD in predict's A-fragment layout, so V, var and mean are
+// computed the same way predict computes them.  Two quad shuffles per tile and part then move kL and kD to
+// the C-fragment order (slot k of lane (g, t) is n = 8(k/2) + 2t + (k&1)), where beta = W^T V = K^-1 k_s, which DMMA
+// returns in the C layout, holds the same n: the dvar sum is lane-local.  W is staged as predict stages it (for V) and
+// once more transposed with permuted columns (for beta), which keeps both B-fragment loads free of bank conflicts, and
+// alpha = W^T a is formed once per CTA in shared memory.  Per
+// coordinate j:  gk_n = dk_n/dx*_j = -kL_n (u*_j - u_nj) / ls_Lj - kD_n (w*_j - w_nj) / ls_dj  (differences, never the
+// expanded form), dvar_j = -2 sum_n beta_n gk_n (lane-local, then the quad), dmean_pj = sum_n alpha_np gk_n (DMMA with
+// gk as the A fragment for P >= 8, DFMA below).
 #include <cmath>
 
 #include "gpr.cuh"
@@ -40,6 +51,8 @@ struct FusedArgs {
     int gpc;  // 8-point groups per CTA
     double* mean;
     double* var;
+    double* dmean;  // grad kernel only: [B][Ns][P][d]
+    double* dvar;   //                   [B][Ns][d]
 };
 
 // Shared-memory pitches (doubles).  W rows: WP = NP + 4 (= 4 or 12 mod 16) puts the B-fragment loads W[8i+g][4k+t] of a
@@ -55,6 +68,17 @@ size_t fused_smem_bytes(int NT, int d, int P) {
     return sizeof(double) * ((size_t)NP * w_pitch(NP) + (size_t)NP * a_pitch(P) + (size_t)(2 * d + 4) * NP +
                              (size_t)PW * 8 * rec_len(d));
 }
+// grad kernel: a second copy of W (transposed), alpha next to a, and the 2d inverse lengthscales
+size_t fused_grad_smem_bytes(int NT, int d, int P) {
+    const int NP = 8 * NT;
+    return fused_smem_bytes(NT, d, P) + sizeof(double) * ((size_t)NP * w_pitch(NP) + (size_t)NP * a_pitch(P) + 2 * d);
+}
+
+// C-fragment order of the training index used by the grad kernel after V: slot 4k + t (k-step k, lane t) holds
+// n = 8(k/2) + 2t + (k&1), and back.
+__host__ __device__ constexpr int perm_n(int slot) { return 8 * (slot >> 3) + 2 * (slot & 3) + ((slot >> 2) & 1); }
+__host__ __device__ constexpr int perm_slot(int n) { return 8 * (n >> 3) + 4 * (n & 1) + ((n >> 1) & 3); }
+__host__ __device__ constexpr int slot_off(int k) { return 8 * (k >> 1) + (k & 1); }  // n - 2t of slot k
 
 // Scaled coordinates and flags of one point, as the covariance kernel K1 prepares them (cov_prescale_kernel): dead rows
 // (fidelity not exactly 0 or 1) get zero coordinates and s = h = 0, so their covariance with anything is exactly 0.
@@ -220,13 +244,371 @@ __global__ void __launch_bounds__(PW * 32) gpr_posterior_predict_kernel(FusedArg
 }
 
 template <int NT>
+__global__ void __launch_bounds__(PW * 32) gpr_posterior_predict_grad_kernel(FusedArgs p) {
+    constexpr int NP = 8 * NT, WP = w_pitch(NP);
+    extern __shared__ __align__(16) double sm[];
+    __shared__ __align__(16) double etab[512];
+    const GprPosteriorData& q = p.q;
+    const int N = q.N, d = q.d, P = q.P, AP = a_pitch(P), S1 = rec_len(d);
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
+    const long b = blockIdx.y;
+    const double* __restrict__ th = q.theta + b * (2 * d + 3);
+    double* Ws = sm;                            // [NP][WP]  W, as gpr_posterior_predict_kernel stages it
+    double* Wt = Ws + NP * WP;                  // [NP][WP]  Wt[c][slot] = W[perm_n(slot)][c]
+    double* As = Wt + NP * WP;                  // [NP][AP]  a
+    double* Al = As + NP * AP;                  // [NP][AP]  alpha = W^T a
+    double* Xt = Al + NP * AP;                  // [2d+4][NP]  training points, k-major
+    double* Il = Xt + (2 * d + 4) * NP;         // [2d]  -1/ls_L, -1/ls_delta
+    double* Xw = Il + 2 * d + warp * 8 * S1;    // [8][S1]  this warp's test points
+    fexp512_table_fill(etab, tid, blockDim.x);
+    const double hlL = 0.5 * log(th[1 + d]), hlD = 0.5 * log(th[2 + 2 * d]);
+
+    // ---- stage the problem: W twice (lower triangle, zero elsewhere), a, scaled training inputs; then alpha = W^T a
+    {
+        const double* __restrict__ Wg = q.W + b * N * q.ld;
+        for (int idx = tid; idx < NP * NP; idx += blockDim.x) {
+            const int r = idx / NP, c = idx - r * NP, m = perm_n(c);
+            Ws[r * WP + c] = (r < N && c <= r) ? Wg[(long)r * q.ld + c] : 0.0;
+            Wt[r * WP + c] = (m < N && r <= m) ? Wg[(long)m * q.ld + r] : 0.0;
+        }
+        const double* __restrict__ ag = q.a + b * N * q.Pp;
+        for (int idx = tid; idx < NP * AP; idx += blockDim.x) {
+            const int r = idx / AP, c = idx - r * AP;
+            As[idx] = (r < N && c < P) ? ag[(long)r * q.Pp + c] : 0.0;
+        }
+        for (int n = tid; n < NP; n += blockDim.x) prescale_point(q.X + (long)n * (d + 1), n < N, d, th, hlL, hlD, Xt + n, NP);
+        for (int k = tid; k < d; k += blockDim.x) {
+            Il[k] = -1.0 / th[1 + k];
+            Il[d + k] = -1.0 / th[2 + d + k];
+        }
+    }
+    __syncthreads();
+    for (int idx = tid; idx < NP * AP; idx += blockDim.x) {
+        const int r = idx / AP, c = idx - r * AP;
+        double s = 0.0;
+        if (r < N && c < P)
+            for (int m = r; m < N; ++m) s = fma(Wt[r * WP + perm_slot(m)], As[m * AP + c], s);
+        Al[idx] = s;
+    }
+    __syncthreads();
+    const double rho = th[0], vL = th[1 + d], vD = th[2 + 2 * d];
+    const double kss_hf = __dadd_rn(__dmul_rn(vL, __dmul_rn(rho, rho)), vD);
+
+    for (int grp = warp; grp < p.gpc; grp += PW) {
+        const long pt0 = ((long)blockIdx.x * p.gpc + grp) * 8;
+        if (pt0 >= p.Ns) break;
+        if (lane < 8) {
+            const long pt = pt0 + lane;
+            const bool exists = pt < p.Ns;
+            double* rec = Xw + lane * S1;
+            prescale_point(p.Xs + (exists ? pt : 0) * (d + 1), exists, d, th, hlL, hlD, rec, 1);
+            rec[2 * d + 4] = rec[2 * d + 3] != 0.0 ? kss_hf : (rec[2 * d + 2] != 0.0 ? vL : 0.0);
+        }
+        __syncwarp();
+        const double* xg = Xw + g * S1;
+        const double sg = xg[2 * d + 2], hg = xg[2 * d + 3];
+        const bool anyh = __any_sync(0xffffffffu, hg != 0.0);
+
+        // ---- the two parts of K_s^T in predict's A-fragment layout: kL[k], kD[k] at n = 4k + t
+        double kL[2 * NT], kD[2 * NT];
+        {
+            const double* xe = Xt + 2 * d * NP + t;
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) kL[k] = xe[4 * k] + xg[2 * d];
+            for (int c = 0; c < d; ++c) {
+                const double xc = xg[c];
+                const double* xr = Xt + c * NP + t;
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k) kL[k] = fma(xr[4 * k], xc, kL[k]);
+            }
+            const double* sr = Xt + (2 * d + 2) * NP + t;
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) kL[k] = fexp512(kL[k], etab) * (sr[4 * k] * sg);
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) kD[k] = 0.0;
+            if (anyh) {
+                const double* xf = Xt + (2 * d + 1) * NP + t;
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k) kD[k] = xf[4 * k] + xg[2 * d + 1];
+                for (int c = 0; c < d; ++c) {
+                    const double xc = xg[d + c];
+                    const double* xr = Xt + (d + c) * NP + t;
+#pragma unroll
+                    for (int k = 0; k < 2 * NT; ++k) kD[k] = fma(xr[4 * k], xc, kD[k]);
+                }
+                const double* hr = Xt + (2 * d + 3) * NP + t;
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k) kD[k] = hr[4 * k] * hg != 0.0 ? fexp512(kD[k], etab) : 0.0;
+            }
+        }
+
+        // ---- V^T = K_s^T W^T over the lower-triangular tiles: v[i][e] = V^T[g][8i + 2t + e]
+        double v[NT][2];
+        {
+            double ks[2 * NT];
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) ks[k] = __dadd_rn(kL[k], kD[k]);  // predict's K_s, not contracted
+#pragma unroll
+            for (int i = 0; i < NT; ++i) {
+                v[i][0] = v[i][1] = 0.0;
+                const double* wr = Ws + (8 * i + g) * WP + t;
+#pragma unroll
+                for (int k = 0; k <= 2 * i + 1; ++k) dmma(v[i][0], v[i][1], ks[k], wr[4 * k]);
+            }
+        }
+
+        // ---- var = k_ss - sum_n V^2, mean = V^T a  (as gpr_posterior_predict_kernel)
+        double ss = 0.0;
+#pragma unroll
+        for (int i = 0; i < NT; ++i) ss = fma(v[i][1], v[i][1], fma(v[i][0], v[i][0], ss));
+        ss = quad_sum(ss);
+        const long ptg = pt0 + g;
+        const bool live = ptg < p.Ns;
+        if (t == 0 && live) p.var[b * p.Ns + ptg] = xg[2 * d + 4] - ss;
+        double* mrow = p.mean + (b * p.Ns + ptg) * P;
+        if (P >= 8) {
+            for (int j = 0; j < (P + 7) / 8; ++j) {
+                double c0 = 0.0, c1 = 0.0;
+                const double* ar = As + (2 * t) * AP + 8 * j + g;
+#pragma unroll
+                for (int i = 0; i < NT; ++i) {
+                    dmma(c0, c1, v[i][0], ar[(8 * i) * AP]);
+                    dmma(c0, c1, v[i][1], ar[(8 * i + 1) * AP]);
+                }
+                const int col = 8 * j + 2 * t;
+                if (live) {
+                    if (col < P) mrow[col] = c0;
+                    if (col + 1 < P) mrow[col + 1] = c1;
+                }
+            }
+        } else {
+            for (int c = 0; c < P; ++c) {
+                const double* ar = As + (2 * t) * AP + c;
+                double m = 0.0;
+#pragma unroll
+                for (int i = 0; i < NT; ++i) m = fma(v[i][1], ar[(8 * i + 1) * AP], fma(v[i][0], ar[(8 * i) * AP], m));
+                m = quad_sum(m);
+                if (t == 0 && live) mrow[c] = m;
+            }
+        }
+
+        // ---- kL, kD to the C-fragment order: slot 2i + e of lane t <- n = 8i + 2t + e, which lane (2t + e) & 3 of the
+        //      quad holds in slot 2i + t / 2
+        {
+            const int src0 = (lane & ~3) | ((2 * t) & 3), src1 = (lane & ~3) | ((2 * t + 1) & 3);
+            const bool hi = t >= 2;
+#pragma unroll
+            for (int i = 0; i < NT; ++i) {
+                const double a0 = __shfl_sync(0xffffffffu, kL[2 * i], src0), b0 = __shfl_sync(0xffffffffu, kL[2 * i + 1], src0);
+                const double a1 = __shfl_sync(0xffffffffu, kL[2 * i], src1), b1 = __shfl_sync(0xffffffffu, kL[2 * i + 1], src1);
+                kL[2 * i] = hi ? b0 : a0;
+                kL[2 * i + 1] = hi ? b1 : a1;
+            }
+            if (anyh) {
+#pragma unroll
+                for (int i = 0; i < NT; ++i) {
+                    const double a0 = __shfl_sync(0xffffffffu, kD[2 * i], src0), b0 = __shfl_sync(0xffffffffu, kD[2 * i + 1], src0);
+                    const double a1 = __shfl_sync(0xffffffffu, kD[2 * i], src1), b1 = __shfl_sync(0xffffffffu, kD[2 * i + 1], src1);
+                    kD[2 * i] = hi ? b0 : a0;
+                    kD[2 * i + 1] = hi ? b1 : a1;
+                }
+            }
+        }
+
+        // ---- beta^T = V^T W over the tiles m >= n: be[2i + e] = beta[8i + 2t + e], the n of kL[2i + e] / kD[2i + e]
+        double be[2 * NT];
+#pragma unroll
+        for (int i = 0; i < NT; ++i) {
+            double c0 = 0.0, c1 = 0.0;
+            const double* wr = Wt + (8 * i + g) * WP + t;
+#pragma unroll
+            for (int i2 = i; i2 < NT; ++i2) {
+                dmma(c0, c1, v[i2][0], wr[8 * i2]);
+                dmma(c0, c1, v[i2][1], wr[8 * i2 + 4]);
+            }
+            be[2 * i] = c0;
+            be[2 * i + 1] = c1;
+        }
+
+        // ---- per coordinate j: gk = dk_s/dx*_j, dvar_j = -2 beta . gk, dmean_:j = alpha^T gk
+        double* dmrow = p.dmean + (b * p.Ns + ptg) * P * d;
+        for (int j = 0; j < d; ++j) {
+            double gk[2 * NT];
+            {
+                const double uj = xg[j], cL = Il[j];
+                const double* ur = Xt + j * NP + 2 * t;
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k) gk[k] = kL[k] * (uj - ur[slot_off(k)]) * cL;
+                if (anyh) {
+                    const double wj = xg[d + j], cD = Il[d + j];
+                    const double* wr = Xt + (d + j) * NP + 2 * t;
+#pragma unroll
+                    for (int k = 0; k < 2 * NT; ++k) gk[k] = fma(kD[k] * (wj - wr[slot_off(k)]), cD, gk[k]);
+                }
+            }
+            double sv = 0.0;
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) sv = fma(be[k], gk[k], sv);
+            sv = quad_sum(sv);
+            if (t == 0 && live) p.dvar[(b * p.Ns + ptg) * d + j] = -2.0 * sv;
+            if (P >= 8) {
+                for (int jj = 0; jj < (P + 7) / 8; ++jj) {
+                    double c0 = 0.0, c1 = 0.0;
+                    const double* ar = Al + (2 * t) * AP + 8 * jj + g;
+#pragma unroll
+                    for (int i = 0; i < NT; ++i) {
+                        dmma(c0, c1, gk[2 * i], ar[(8 * i) * AP]);
+                        dmma(c0, c1, gk[2 * i + 1], ar[(8 * i + 1) * AP]);
+                    }
+                    const int col = 8 * jj + 2 * t;
+                    if (live) {
+                        if (col < P) dmrow[col * d + j] = c0;
+                        if (col + 1 < P) dmrow[(col + 1) * d + j] = c1;
+                    }
+                }
+            } else {
+                for (int c = 0; c < P; ++c) {
+                    const double* ar = Al + (2 * t) * AP + c;
+                    double m = 0.0;
+#pragma unroll
+                    for (int i = 0; i < NT; ++i)
+                        m = fma(gk[2 * i + 1], ar[(8 * i + 1) * AP], fma(gk[2 * i], ar[(8 * i) * AP], m));
+                    m = quad_sum(m);
+                    if (t == 0 && live) dmrow[c * d + j] = m;
+                }
+            }
+        }
+        __syncwarp();
+    }
+}
+
+// Input gradient of the blocked route (launch_posterior_dx): one CTA per (tile of TS test points, chunk of PC columns,
+// problem), walking the training points in tiles of TN.  Per tile it evaluates kL and kD from the scaled inputs (as K5
+// recomputes dK: nothing N x Ns is stored), forms G[j][s][n] = dk_sn/dx_sj in shared memory and adds G alpha (thread =
+// (point, column)) and G beta (thread = (point, coordinate)) to accumulators in shared memory.  Each sum runs over n in
+// a fixed order and involves only its own test point: no atomics, no cross-point reduction.
+constexpr int DX_TS = 8, DX_PC = 32, DX_TN = 16, DX_THREADS = DX_TS * DX_PC;
+
+size_t posterior_dx_smem_bytes(int d) {
+    const int R = 2 * d + 4;
+    return sizeof(double) * ((size_t)DX_TS * R + (size_t)R * DX_TN + 2 * DX_TS * DX_TN + (size_t)d * DX_TS * DX_TN +
+                             DX_TN * DX_PC + DX_TN * DX_TS + (size_t)DX_TS * d * DX_PC + (size_t)DX_TS * d + 2 * d);
+}
+
+__global__ void __launch_bounds__(DX_THREADS) posterior_dx_kernel(GprPosteriorData q, const double* __restrict__ Xs, int Ns,
+                                                                const double* __restrict__ alpha,
+                                                                const double* __restrict__ beta, long ldb,
+                                                                double* __restrict__ dmean, double* __restrict__ dvar) {
+    extern __shared__ __align__(16) double sm[];
+    const int N = q.N, d = q.d, P = q.P, R = 2 * d + 4, tid = threadIdx.x;
+    const long b = blockIdx.z;
+    const int s0 = blockIdx.x * DX_TS, p0 = blockIdx.y * DX_PC;
+    const bool want_var = blockIdx.y == 0;
+    const double* __restrict__ th = q.theta + b * (2 * d + 3);
+    double* xs = sm;                       // [TS][R]   test points
+    double* xn = xs + DX_TS * R;           // [R][TN]   training points of the tile
+    double* kl = xn + R * DX_TN;           // [TS][TN]
+    double* kd = kl + DX_TS * DX_TN;       // [TS][TN]
+    double* G = kd + DX_TS * DX_TN;        // [d][TS][TN]
+    double* al = G + d * DX_TS * DX_TN;    // [TN][PC]
+    double* be = al + DX_TN * DX_PC;       // [TN][TS]
+    double* acc = be + DX_TN * DX_TS;      // [TS][d][PC]
+    double* dv = acc + DX_TS * d * DX_PC;  // [TS][d]
+    double* il = dv + DX_TS * d;           // [2d]  -1/ls_L, -1/ls_delta
+    const double hlL = 0.5 * log(th[1 + d]), hlD = 0.5 * log(th[2 + 2 * d]), vL = th[1 + d], vD = th[2 + 2 * d];
+    if (tid < DX_TS) prescale_point(Xs + (long)(s0 + tid < Ns ? s0 + tid : 0) * (d + 1), s0 + tid < Ns, d, th, hlL, hlD,
+                                    xs + tid * R, 1);
+    for (int k = tid; k < d; k += DX_THREADS) {
+        il[k] = -1.0 / th[1 + k];
+        il[d + k] = -1.0 / th[2 + d + k];
+    }
+    for (int i = tid; i < DX_TS * d * DX_PC; i += DX_THREADS) acc[i] = 0.0;
+    for (int i = tid; i < DX_TS * d; i += DX_THREADS) dv[i] = 0.0;
+    const double* __restrict__ ab = alpha + b * N * q.Pp;
+    const double* __restrict__ bb = beta + b * N * ldb;
+    const int ts = tid / DX_PC, tp = tid % DX_PC;
+
+    for (int n0 = 0; n0 < N; n0 += DX_TN) {
+        if (tid < DX_TN) prescale_point(q.X + (long)(n0 + tid < N ? n0 + tid : 0) * (d + 1), n0 + tid < N, d, th, hlL, hlD,
+                                        xn + tid, DX_TN);
+        for (int i = tid; i < DX_TN * DX_PC; i += DX_THREADS) {
+            const int n = n0 + i / DX_PC, c = p0 + i % DX_PC;
+            al[i] = (n < N && c < P) ? ab[(long)n * q.Pp + c] : 0.0;
+        }
+        for (int i = tid; i < DX_TN * DX_TS; i += DX_THREADS) {
+            const int n = n0 + i / DX_TS, c = s0 + i % DX_TS;
+            be[i] = (n < N && c < Ns) ? bb[(long)n * ldb + c] : 0.0;
+        }
+        __syncthreads();
+        for (int i = tid; i < DX_TS * DX_TN; i += DX_THREADS) {
+            const int si = i / DX_TN, n = i % DX_TN;
+            const double* x = xs + si * R;
+            double rL = 0.0, rD = 0.0;
+            for (int c = 0; c < d; ++c) {
+                const double eL = x[c] - xn[c * DX_TN + n], eD = x[d + c] - xn[(d + c) * DX_TN + n];
+                rL = fma(eL, eL, rL);
+                rD = fma(eD, eD, rD);
+            }
+            kl[i] = (x[2 * d + 2] * xn[(2 * d + 2) * DX_TN + n]) * (vL * exp(-0.5 * rL));
+            kd[i] = x[2 * d + 3] * xn[(2 * d + 3) * DX_TN + n] != 0.0 ? vD * exp(-0.5 * rD) : 0.0;
+        }
+        __syncthreads();
+        for (int i = tid; i < d * DX_TS * DX_TN; i += DX_THREADS) {
+            const int j = i / (DX_TS * DX_TN), si = (i / DX_TN) % DX_TS, n = i % DX_TN, sn = si * DX_TN + n;
+            const double* x = xs + si * R;
+            G[i] = fma(kd[sn] * (x[d + j] - xn[(d + j) * DX_TN + n]), il[d + j], kl[sn] * (x[j] - xn[j * DX_TN + n]) * il[j]);
+        }
+        __syncthreads();
+        for (int j = 0; j < d; ++j) {
+            const double* gr = G + (j * DX_TS + ts) * DX_TN;
+            double a = 0.0;
+#pragma unroll
+            for (int n = 0; n < DX_TN; ++n) a = fma(gr[n], al[n * DX_PC + tp], a);
+            acc[(ts * d + j) * DX_PC + tp] += a;
+        }
+        if (want_var)
+            for (int i = tid; i < DX_TS * d; i += DX_THREADS) {
+                const int si = i / d, j = i % d;
+                const double* gr = G + (j * DX_TS + si) * DX_TN;
+                double a = 0.0;
+#pragma unroll
+                for (int n = 0; n < DX_TN; ++n) a = fma(gr[n], be[n * DX_TS + si], a);
+                dv[i] += a;
+            }
+        __syncthreads();
+    }
+    for (int i = tid; i < DX_TS * DX_PC * d; i += DX_THREADS) {
+        const int si = i / (DX_PC * d), r = i % (DX_PC * d), c = r / d, j = r % d;
+        if (s0 + si < Ns && p0 + c < P) dmean[((b * Ns + s0 + si) * P + p0 + c) * d + j] = acc[(si * d + j) * DX_PC + c];
+    }
+    if (want_var)
+        for (int i = tid; i < DX_TS * d; i += DX_THREADS)
+            if (s0 + i / d < Ns) dvar[(b * Ns + s0) * d + i] = -2.0 * dv[i];
+}
+
+template <int NT, bool GRAD>
 int launch_fused(cudaStream_t s, const FusedArgs& a, int B, size_t smem) {
     static SmemOptIn optin;
-    if (!optin.ensure(gpr_posterior_predict_kernel<NT>, smem)) return -2;
+    void (*kern)(FusedArgs) = GRAD ? gpr_posterior_predict_grad_kernel<NT> : gpr_posterior_predict_kernel<NT>;
+    if (!optin.ensure(kern, smem)) return -2;
     const long G = (a.Ns + 7) / 8;
     dim3 grid((unsigned)((G + a.gpc - 1) / a.gpc), (unsigned)B);
-    gpr_posterior_predict_kernel<NT><<<grid, PW * 32, smem, s>>>(a);
+    kern<<<grid, PW * 32, smem, s>>>(a);
     return cudaGetLastError() == cudaSuccess ? 0 : -2;
+}
+
+template <bool GRAD>
+int launch_fused_nt(int NT, cudaStream_t s, const FusedArgs& a, int B, size_t smem) {
+    switch (NT) {
+        case 1: return launch_fused<1, GRAD>(s, a, B, smem);
+        case 2: return launch_fused<2, GRAD>(s, a, B, smem);
+        case 3: return launch_fused<3, GRAD>(s, a, B, smem);
+        case 4: return launch_fused<4, GRAD>(s, a, B, smem);
+        case 5: return launch_fused<5, GRAD>(s, a, B, smem);
+        case 6: return launch_fused<6, GRAD>(s, a, B, smem);
+        case 7: return launch_fused<7, GRAD>(s, a, B, smem);
+        default: return launch_fused<8, GRAD>(s, a, B, smem);
+    }
 }
 
 }  // namespace
@@ -236,11 +618,12 @@ bool gpr_posterior_fused_ok(int N, int d, int P) {
 }
 
 int gpr_posterior_predict_fused(cudaStream_t s, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
-                                double* var) {
+                                double* var, double* dmean, double* dvar) {
     if (!gpr_posterior_fused_ok(q.N, q.d, q.P)) return -1;
     if (Ns <= 0 || q.B <= 0) return 0;
+    const bool grad = dmean != nullptr;
     const int NT = (q.N + 7) / 8;
-    const size_t smem = fused_smem_bytes(NT, q.d, q.P);
+    const size_t smem = grad ? fused_grad_smem_bytes(NT, q.d, q.P) : fused_smem_bytes(NT, q.d, q.P);
     // 8-point groups per CTA: enough CTAs for ~8 per SM, and no more than 256 groups so that a CTA's staging of W and a
     // (read once per CTA) stays small against its arithmetic.  The split never changes a result (see the file comment).
     const long G = (Ns + 7) / 8;
@@ -262,18 +645,22 @@ int gpr_posterior_predict_fused(cudaStream_t s, const GprPosteriorData& q, const
         a.Xs = Xs; a.Ns = Ns; a.gpc = (int)gpc;
         a.mean = mean + (long)b0 * Ns * q.P;
         a.var = var + (long)b0 * Ns;
-        int rc = 0;
-        switch (NT) {
-            case 1: rc = launch_fused<1>(s, a, nb, smem); break;
-            case 2: rc = launch_fused<2>(s, a, nb, smem); break;
-            case 3: rc = launch_fused<3>(s, a, nb, smem); break;
-            case 4: rc = launch_fused<4>(s, a, nb, smem); break;
-            case 5: rc = launch_fused<5>(s, a, nb, smem); break;
-            case 6: rc = launch_fused<6>(s, a, nb, smem); break;
-            case 7: rc = launch_fused<7>(s, a, nb, smem); break;
-            default: rc = launch_fused<8>(s, a, nb, smem); break;
+        if (grad) {
+            a.dmean = dmean + (long)b0 * Ns * q.P * q.d;
+            a.dvar = dvar + (long)b0 * Ns * q.d;
         }
+        const int rc = grad ? launch_fused_nt<true>(NT, s, a, nb, smem) : launch_fused_nt<false>(NT, s, a, nb, smem);
         if (rc) return rc;
     }
     return 0;
+}
+
+int launch_posterior_dx(cudaStream_t s, const GprPosteriorData& q, int nb, const double* Xs, int Ns, const double* alpha,
+                        const double* beta, long ldb, double* dmean, double* dvar) {
+    static SmemOptIn optin;
+    const size_t smem = posterior_dx_smem_bytes(q.d);
+    if (!optin.ensure(posterior_dx_kernel, smem)) return -2;
+    dim3 grid((unsigned)((Ns + DX_TS - 1) / DX_TS), (unsigned)((q.P + DX_PC - 1) / DX_PC), (unsigned)nb);
+    posterior_dx_kernel<<<grid, DX_THREADS, smem, s>>>(q, Xs, Ns, alpha, beta, ldb, dmean, dvar);
+    return cudaGetLastError() == cudaSuccess ? 0 : -2;
 }

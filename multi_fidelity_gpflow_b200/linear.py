@@ -133,5 +133,17 @@ class MultiFidelityGPPosterior:
         mean, var = self.predict_f(Xnew)
         return mean, var + self.noise
 
+    def predict_f_grad(self, Xnew):
+        """predict_f and its gradient with respect to Xnew: mean [N*, P], var [N*, P], dmean_dx [N*, P, d+1] and
+        dvar_dx [N*, P, d+1] (d value[s, p] / d Xnew[s, j]).  The last (fidelity) column is exactly 0, as
+        tape.gradient gives it in the reference; predict_y has the same gradient."""
+        mean, var, dmean, dvar = self._post.predict_grad(np.ascontiguousarray(Xnew, dtype=np.float64))
+        P = mean.shape[2]
+        dm = np.zeros(dmean.shape[1:3] + (dmean.shape[3] + 1,))
+        dm[..., :-1] = dmean[0]
+        dv = np.zeros_like(dm)
+        dv[..., :-1] = dvar[0][:, None, :]
+        return mean[0], np.tile(var[0][:, None], (1, P)), dm, dv
+
     def close(self):
         self._post.close()

@@ -137,6 +137,23 @@ class MultiBinPosterior:
             return np.ascontiguousarray(mean[0]), np.ascontiguousarray(var[0])
         return mean, var
 
+    def predict_f_grad(self, Xnew):
+        """predict_f and its gradient with respect to Xnew: mean, var [N*, P] and dmean_dx, dvar_dx [N*, P, d+1] ("best"),
+        or the same with a leading restart axis R ("all"; NaN for a failed restart).  The last (fidelity) column of the
+        gradients is exactly 0, as tape.gradient gives it in the reference."""
+        mean, var, dmean, dvar = self._post.predict_grad(np.ascontiguousarray(Xnew, dtype=np.float64))
+        P = self.noises.shape[-1]
+        B, Ns, _, d = dmean.shape
+        pad = lambda g: np.concatenate([g, np.zeros(g.shape[:-1] + (1,))], axis=-1)
+        mean = np.swapaxes(mean[:, :, 0].reshape(-1, P, Ns), 1, 2)  # [R, N*, P], problem b = r * P + p
+        var = np.swapaxes(var.reshape(-1, P, Ns), 1, 2)
+        dmean = pad(np.swapaxes(dmean[:, :, 0, :].reshape(-1, P, Ns, d), 1, 2))  # [R, N*, P, d+1]
+        dvar = pad(np.swapaxes(dvar.reshape(-1, P, Ns, d), 1, 2))
+        out = (mean, var, dmean, dvar)
+        if self.noises.ndim == 1:
+            return tuple(np.ascontiguousarray(a[0]) for a in out)
+        return tuple(np.ascontiguousarray(a) for a in out)
+
     def predict_y(self, Xnew):
         """predict_f plus each problem's likelihood noise on the variance."""
         mean, var = self.predict_f(Xnew)

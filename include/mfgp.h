@@ -192,6 +192,30 @@ int mfgp_svgp_predict(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* Xs
                       const double* Z, const double* theta, const double* W, const double* q_mu,
                       const double* q_sqrt, double* mean, double* var);
 
+/* Cached SVGP posterior (GPflow SVGP.posterior()): factor the inducing covariances of the L latents once, then predict
+ * every latent in one launch, with the results of mfgp_svgp_predict.
+ *  - cfg supplies L, M, P, d and jitter as for mfgp_svgp_predict; B and the likelihood fields are ignored.  W [P, L] or
+ *    NULL (SeparateIndependent, L == P).  Only the lower triangle of q_sqrt [L, M, M] is read; q_mu is [M, L].
+ *  - Snapshot: the posterior owns device copies of Z, theta, W, q_mu, Wm = Lm^-1 of K_l(Z,Z) + jitter I and
+ *    Lq = tril(q_sqrt) (the factors mfgp_svgp_predict computes); later changes to the caller's buffers do not reach it.
+ *  - Memory: one plain cudaMalloc block on the handle's device, owned by the device (not the handle): any handle on that
+ *    device may predict with it, and it outlives the handle that created it.  Free it with mfgp_svgp_posterior_destroy.
+ *  - Status: creation always synchronises.  Without info a non-positive-definite latent makes the call return its pivot
+ *    (> 0) with *out = NULL.  With info [L] (host or device) info[l] holds latent l's pivot (0 = ok), the call returns the
+ *    first pivot and the posterior exists: latent l predicts NaN, so with W every output reads NaN (NaN * 0 = NaN).
+ * mfgp_svgp_posterior_predict: mean [Ns, P], var [Ns, P] as mfgp_svgp_predict; host or device pointers, async mode, Ns == 0
+ * returns at once, and the handle must be on the posterior's device.  M <= 64 and d <= 16 run one sm_100a kernel
+ * (svgp_posterior_predict_kernel: V = Wm K_s and U = Lq^T V on DMMA) plus the mix when W is given; anything larger runs
+ * the second half of mfgp_svgp_predict (K1, cov_diag, two batched GEMMs, col_reduce, mix) chunked over Ns.  A point's
+ * result does not depend on the other points of the call. */
+typedef struct mfgp_svgp_posterior mfgp_svgp_posterior;
+int mfgp_svgp_posterior_create(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* Z, const double* theta,
+                               const double* W, const double* q_mu, const double* q_sqrt, int* info,
+                               mfgp_svgp_posterior** out);
+int mfgp_svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns,
+                                double* mean, double* var);
+int mfgp_svgp_posterior_destroy(mfgp_svgp_posterior* post);
+
 /* Training loop on the device for the SVGP models (SURVEY 8(f) rank 1): the optimize() loops of mfgpflow/singlebin_svgp.py:
  * 64-97 and mfgpflow/linear_svgp.py:153-203 -- full-batch, Keras Adam (+ CosineDecay folded into lr_t, see
  * mfgp_gpr_batched_adam), loss = -ELBO + (kl_mult - 1) KL -- nsteps steps without a host round trip.

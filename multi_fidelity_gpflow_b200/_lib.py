@@ -61,6 +61,9 @@ def _load():
         "mfgp_svgp_elbo_grad": ([vp, vp, vp, vp, vp, vp, vp, vp, vp, d, vp, vp, vp, vp, vp, vp, vp, vp], i),
         "mfgp_svgp_elbo_grad_v": ([vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp], i),
         "mfgp_svgp_predict": ([vp, vp, vp, i, vp, vp, vp, vp, vp, vp, vp], i),
+        "mfgp_svgp_posterior_create": ([vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(vp)], i),
+        "mfgp_svgp_posterior_predict": ([vp, vp, vp, i, vp, vp], i),
+        "mfgp_svgp_posterior_destroy": ([vp], i),
         "mfgp_svgp_adam": ([vp, vp, vp, vp, i, vp, vp, vp, vp, vp, d, d, d, i, vp, vp], i),
         "mfgp_svgp_flat_size": ([vp, i], l),
         "mfgp_svgp_constrain": ([vp, vp, i, vp, vp], i),
@@ -89,7 +92,8 @@ EXPORTED_SYMBOLS = [
     "mfgp_gpr_predict", "mfgp_gpr_batched_nlml_grad", "mfgp_gpr_batched_adam",
     "mfgp_gpr_posterior_create", "mfgp_gpr_posterior_predict", "mfgp_gpr_posterior_predict_grad",
     "mfgp_gpr_posterior_destroy",
-    "mfgp_graph_nparams", "mfgp_graph_cov", "mfgp_graph_cov_diag", "mfgp_graph_gpr_nlml_grad", "mfgp_svgp_elbo_grad", "mfgp_svgp_elbo_grad_v", "mfgp_svgp_predict", "mfgp_svgp_adam",
+    "mfgp_graph_nparams", "mfgp_graph_cov", "mfgp_graph_cov_diag", "mfgp_graph_gpr_nlml_grad", "mfgp_svgp_elbo_grad", "mfgp_svgp_elbo_grad_v", "mfgp_svgp_predict",
+    "mfgp_svgp_posterior_create", "mfgp_svgp_posterior_predict", "mfgp_svgp_posterior_destroy", "mfgp_svgp_adam",
     "mfgp_svgp_flat_size", "mfgp_svgp_constrain", "mfgp_svgp_elbo_grad_flat", "mfgp_svgp_adam_update", "mfgp_gemm",
     "mfgp_potrf", "mfgp_potrf_inv", "mfgp_tall_skinny_update", "mfgp_peer_store", "mfgp_graph_mem_trim", "mfgp_workspace", "mfgp_fp64_peak",
 ]
@@ -437,6 +441,24 @@ class Handle:
         self._check(rc, "mfgp_svgp_predict")
         return mean, var
 
+    def svgp_posterior(self, Z, thetas, W, q_mu, q_sqrt, jitter=1e-6, info=None):
+        """Factor the inducing covariances of the L = q_mu.shape[1] latents once (include/mfgp.h:
+        mfgp_svgp_posterior_create) and return an SvgpPosterior whose predict() gives what svgp_predict gives for the same
+        arguments.  W [P, L] or None (P = L).  A non-positive Cholesky pivot raises NotPositiveDefiniteError unless a
+        per-latent `info` array (int32 [L]) is passed: then info[l] holds latent l's pivot (0 = ok) and it predicts NaN."""
+        Z, thetas, q_mu, q_sqrt = map(as_f64, (Z, thetas, q_mu, q_sqrt))
+        W = None if W is None else as_f64(W)
+        M, L = q_mu.shape
+        d = Z.shape[1] - 1
+        P = L if W is None else W.shape[0]
+        cfg = SvgpCfg(L, M, P, 0, d, 0, 1.0, 1.0, float(jitter), 0.0, 0, 0)
+        out = C.c_void_p()
+        rc = _lib.mfgp_svgp_posterior_create(self._h, C.byref(cfg), _ptr(Z), _ptr(thetas), _ptr(W), _ptr(q_mu), _ptr(q_sqrt),
+                                             _ptr(info), C.byref(out))
+        if not (rc > 0 and info is not None):
+            self._check(rc, "mfgp_svgp_posterior_create")
+        return SvgpPosterior(self, out, L, M, P, d)
+
     # -- building blocks -------------------------------------------------------------------------
     def cov_grad(self, X, theta, G, scale=1.0):
         """scale * sum_ij G_ij dK_ij/dtheta (lower triangle of the symmetric G, off-diagonal twice) and, last, scale * trace(G)."""
@@ -536,6 +558,40 @@ class GprPosterior:
     def close(self):
         if getattr(self, "_p", None):
             _lib.mfgp_gpr_posterior_destroy(self._p)
+            self._p = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class SvgpPosterior:
+    """Device-resident factors of an SVGP (Wm = Lm^-1, tril(q_sqrt), q_mu, W) made by Handle.svgp_posterior: a snapshot of
+    the parameters at creation.  predict() returns mean [Ns, P] and var [Ns, P], as Handle.svgp_predict."""
+
+    def __init__(self, handle, ptr, L, M, P, d):
+        self.handle, self._p = handle, ptr
+        self.L, self.M, self.P, self.d = L, M, P, d
+
+    def predict(self, Xs, mean=None, var=None):
+        """Host arrays or device tensors; mean / var (optional outputs) may be device tensors (zero-copy)."""
+        if not self._p:
+            raise ValueError("SvgpPosterior is closed")
+        Xs = as_f64(Xs)
+        Ns = Xs.shape[0]
+        if Xs.shape[1] != self.d + 1:
+            raise ValueError(f"Xs must have {self.d + 1} columns")
+        mean = np.empty((Ns, self.P)) if mean is None else mean
+        var = np.empty((Ns, self.P)) if var is None else var
+        self.handle._check(_lib.mfgp_svgp_posterior_predict(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean), _ptr(var)),
+                           "mfgp_svgp_posterior_predict")
+        return mean, var
+
+    def close(self):
+        if getattr(self, "_p", None):
+            _lib.mfgp_svgp_posterior_destroy(self._p)
             self._p = None
 
     def __del__(self):

@@ -489,6 +489,121 @@ int mfgp_gpr_posterior_destroy(mfgp_gpr_posterior* post) {
 }
 
 // ---------------------------------------------------------------------------------------------
+// Cached SVGP posterior (include/mfgp.h): the memory model of mfgp_gpr_posterior, the factors of svgp_factor.
+}  // extern "C"
+
+struct mfgp_svgp_posterior {
+    int device;
+    SvgpPosteriorData q;
+    void* mem;
+};
+
+extern "C" {
+
+int mfgp_svgp_posterior_create(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* Z, const double* theta,
+                               const double* W, const double* q_mu, const double* q_sqrt, int* info,
+                               mfgp_svgp_posterior** out) {
+    CHECK_H(h);
+    if (out) *out = nullptr;
+    if (!out || !cfg || !Z || !theta || !q_mu || !q_sqrt)
+        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_posterior_create: NULL argument");
+    const int L = cfg->L, M = cfg->M, P = cfg->P, d = cfg->d;
+    if (L < 1 || M < 1 || P < 1 || d < 1 || d > MFGP_MAX_D || (!W && L != P))
+        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_posterior_create: bad configuration");
+    cudaSetDevice(h->device);
+    const int np = 2 * d + 3;
+    const long ld = round_up(M, 2);
+    size_t tot = 0;
+    auto carve = [&](size_t count) {
+        const size_t o = tot;
+        tot += (count * sizeof(double) + 255) & ~(size_t)255;
+        return o;
+    };
+    const size_t oZ = carve((size_t)M * (d + 1)), oT = carve((size_t)L * np), oW = carve(W ? (size_t)P * L : 0),
+                 oWm = carve((size_t)L * M * ld), oLq = carve((size_t)L * M * ld), oQ = carve((size_t)M * L);
+    void* mem = nullptr;
+    CUDA_TRY(h, cudaMalloc(&mem, tot));
+    char* base = static_cast<char*>(mem);
+    double *dZ = reinterpret_cast<double*>(base + oZ), *dT = reinterpret_cast<double*>(base + oT),
+           *dW = W ? reinterpret_cast<double*>(base + oW) : nullptr, *dWm = reinterpret_cast<double*>(base + oWm),
+           *dLq = reinterpret_cast<double*>(base + oLq), *dQ = reinterpret_cast<double*>(base + oQ);
+    const int rc = [&]() -> int {
+        Scope sc(h);
+        cudaStream_t s = h->stream;
+        CUDA_TRY(h, cudaMemcpyAsync(dZ, Z, (size_t)M * (d + 1) * sizeof(double), cudaMemcpyDefault, s));
+        CUDA_TRY(h, cudaMemcpyAsync(dT, theta, (size_t)L * np * sizeof(double), cudaMemcpyDefault, s));
+        if (W) CUDA_TRY(h, cudaMemcpyAsync(dW, W, (size_t)P * L * sizeof(double), cudaMemcpyDefault, s));
+        CUDA_TRY(h, cudaMemcpyAsync(dQ, q_mu, (size_t)M * L * sizeof(double), cudaMemcpyDefault, s));
+        const double* dqs = sc.in(q_sqrt, (size_t)L * M * M);
+        int* di = info ? sc.out(info, L, true) : sc.alloc<int>(L, true);
+        if (!sc.ok) return sc.finish();
+        Fwd f{};
+        f.Wm = dWm;
+        f.Lq = dLq;
+        f.ldM = ld;
+        f.sMM = (long)M * ld;
+        MFGP_TRY(svgp_factor(h, sc, L, M, d, cfg->jitter, dZ, dT, dqs, di, f));
+        // a failed latent: NaN on the diagonal of Wm (P = 0: q_mu is left as it is); it reaches every output of the latent
+        posterior_poison_kernel<<<(unsigned)(L < 4096 ? L : 4096), 128, 0, s>>>(di, L, M, ld, 0, 1, dWm, nullptr);
+        sc.host_out = true;  // always synchronise: the factorisation status decides what the call returns
+        return sc.finish();
+    }();
+    if (rc < 0 || (rc > 0 && !info)) {
+        cudaFree(mem);
+        return rc;
+    }
+    auto* post = new mfgp_svgp_posterior();
+    post->device = h->device;
+    post->mem = mem;
+    post->q = SvgpPosteriorData{L, M, P, d, ld, dZ, dT, dW, dWm, dLq, dQ};
+    *out = post;
+    return rc;
+}
+
+int mfgp_svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns, double* mean,
+                                double* var) {
+    CHECK_H(h);
+    if (!post || !Xs || !mean || !var || Ns < 0) return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_posterior_predict: bad argument");
+    if (post->device != h->device)
+        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_posterior_predict: the posterior lives on device %d, the handle on %d",
+                         post->device, h->device);
+    if (Ns == 0) return 0;
+    cudaSetDevice(h->device);
+    const SvgpPosteriorData& q = post->q;
+    Scope sc(h);
+    const double* dXs = sc.in(Xs, (size_t)Ns * (q.d + 1));
+    double* dm = sc.out(mean, (size_t)Ns * q.P);
+    double* dv = sc.out(var, (size_t)Ns * q.P);
+    if (!sc.ok) return sc.finish();
+    if (svgp_posterior_fused_ok(q.L, q.M, q.d)) {
+        if (!q.W) {
+            if (svgp_posterior_predict_fused(h->stream, q, dXs, Ns, dm, dv, 1, q.P))
+                return mfgp_fail(h, MFGP_ERR_CUDA, "mfgp_svgp_posterior_predict: fused kernel launch failed");
+        } else {
+            double* g = sc.alloc<double>((size_t)2 * q.L * Ns);  // latent marginals [L][Ns], mean then var
+            if (!sc.ok) return sc.finish();
+            if (svgp_posterior_predict_fused(h->stream, q, dXs, Ns, g, g + (size_t)q.L * Ns, Ns, 1) ||
+                launch_svgp_mix(h->stream, g, g + (size_t)q.L * Ns, q.L, Ns, q.P, q.W, dm, dv))
+                return mfgp_fail(h, MFGP_ERR_CUDA, "mfgp_svgp_posterior_predict: fused kernel launch failed");
+        }
+    } else {
+        MFGP_TRY(svgp_posterior_predict_blocked(h, q, dXs, Ns, dm, dv));
+    }
+    return sc.finish();
+}
+
+int mfgp_svgp_posterior_destroy(mfgp_svgp_posterior* post) {
+    if (!post) return 0;
+    int prev = 0;
+    cudaGetDevice(&prev);
+    cudaSetDevice(post->device);
+    const cudaError_t e = cudaFree(post->mem);
+    cudaSetDevice(prev);
+    delete post;
+    return e == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+}
+
+// ---------------------------------------------------------------------------------------------
 int mfgp_cov_grad(mfgp_handle* h, const double* X, int N, int d, const double* theta, const double* G, long ldg, double scale,
                   double* out) {
     CHECK_H(h);

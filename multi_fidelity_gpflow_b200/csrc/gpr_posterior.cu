@@ -27,6 +27,7 @@
 #include "gpr.cuh"
 #include "gpr_small.cuh"
 #include "mathx.cuh"
+#include "svgp.cuh"
 
 namespace {
 
@@ -482,6 +483,152 @@ __global__ void __launch_bounds__(PW * 32) gpr_posterior_predict_grad_kernel(Fus
     }
 }
 
+// svgp_posterior_predict_kernel (mfgp_svgp_posterior_predict): the same decomposition with the inducing points Z in the
+// place of X, one latent per blockIdx.y.  V = Wm K_s as predict's V = W K_s; U = Lq^T V as the grad kernel's
+// beta = W^T V, from Lq staged transposed with permuted columns, so U lands in the C-fragment layout and sum U^2 is
+// lane-local.  var = k_ss - sum V^2 + sum U^2, mean = V^T q_mu (predict's DFMA path for P = 1).
+struct SvgpFusedArgs {
+    SvgpPosteriorData q;
+    const double* Xs;
+    int Ns;
+    int gpc;  // 8-point groups per CTA
+    double* mean;
+    double* var;
+    long ls, ns;  // output of (latent l, point n) at l * ls + n * ns
+};
+
+size_t svgp_fused_smem_bytes(int NT, int d) {
+    const int NP = 8 * NT;
+    return sizeof(double) * (2 * (size_t)NP * w_pitch(NP) + NP + (size_t)(2 * d + 4) * NP + (size_t)PW * 8 * rec_len(d));
+}
+
+template <int NT>
+__global__ void __launch_bounds__(PW * 32) svgp_posterior_predict_kernel(SvgpFusedArgs p) {
+    constexpr int NP = 8 * NT, WP = w_pitch(NP);
+    extern __shared__ __align__(16) double sm[];
+    __shared__ __align__(16) double etab[512];
+    const SvgpPosteriorData& q = p.q;
+    const int M = q.M, d = q.d, S1 = rec_len(d);
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
+    const long l = blockIdx.y;
+    const double* __restrict__ th = q.theta + l * (2 * d + 3);
+    double* Ws = sm;                                  // [NP][WP]  Wm, as gpr_posterior_predict_kernel stages W
+    double* Lt = Ws + NP * WP;                        // [NP][WP]  Lt[c][slot] = Lq[perm_n(slot)][c]
+    double* Qs = Lt + NP * WP;                        // [NP]      q_mu[:, l]
+    double* Xt = Qs + NP;                             // [2d+4][NP]  inducing points, k-major
+    double* Xw = Xt + (2 * d + 4) * NP + warp * 8 * S1;  // [8][S1]  this warp's test points
+    fexp512_table_fill(etab, tid, blockDim.x);
+    const double hlL = 0.5 * log(th[1 + d]), hlD = 0.5 * log(th[2 + 2 * d]);
+
+    // ---- stage the latent: Wm and Lq^T (lower triangles; zero elsewhere), q_mu, scaled inducing points
+    {
+        const double* __restrict__ Wg = q.Wm + l * M * q.ld;
+        const double* __restrict__ Lg = q.Lq + l * M * q.ld;
+        for (int idx = tid; idx < NP * NP; idx += blockDim.x) {
+            const int r = idx / NP, c = idx - r * NP, m = perm_n(c);
+            Ws[r * WP + c] = (r < M && c <= r) ? Wg[(long)r * q.ld + c] : 0.0;
+            Lt[r * WP + c] = (m < M && r <= m) ? Lg[(long)m * q.ld + r] : 0.0;
+        }
+        for (int m = tid; m < NP; m += blockDim.x) Qs[m] = m < M ? q.q_mu[(long)m * q.L + l] : 0.0;
+        for (int n = tid; n < NP; n += blockDim.x) prescale_point(q.Z + (long)n * (d + 1), n < M, d, th, hlL, hlD, Xt + n, NP);
+    }
+    __syncthreads();
+    const double rho = th[0], vL = th[1 + d], vD = th[2 + 2 * d];
+    const double kss_hf = __dadd_rn(__dmul_rn(vL, __dmul_rn(rho, rho)), vD);  // K_diag at fidelity 1, as cov_diag_kernel
+
+    for (int grp = warp; grp < p.gpc; grp += PW) {
+        const long pt0 = ((long)blockIdx.x * p.gpc + grp) * 8;
+        if (pt0 >= p.Ns) break;
+        // ---- this group's 8 test points (padding points beyond Ns are dead: K_s = 0, never stored)
+        if (lane < 8) {
+            const long pt = pt0 + lane;
+            const bool exists = pt < p.Ns;
+            double* rec = Xw + lane * S1;
+            prescale_point(p.Xs + (exists ? pt : 0) * (d + 1), exists, d, th, hlL, hlD, rec, 1);
+            rec[2 * d + 4] = rec[2 * d + 3] != 0.0 ? kss_hf : (rec[2 * d + 2] != 0.0 ? vL : 0.0);
+        }
+        __syncwarp();
+        const double* xg = Xw + g * S1;
+        const double sg = xg[2 * d + 2], hg = xg[2 * d + 3];
+
+        // ---- K_s^T fragment: ks[k] = k(z_m, xs_g), m = 4k + t
+        double ks[2 * NT];
+        {
+            double e[2 * NT];
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) e[k] = Xt[2 * d * NP + 4 * k + t] + xg[2 * d];
+            for (int c = 0; c < d; ++c) {
+                const double xc = xg[c];
+                const double* xr = Xt + c * NP + t;
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k) e[k] = fma(xr[4 * k], xc, e[k]);
+            }
+            const double* sr = Xt + (2 * d + 2) * NP + t;
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) ks[k] = fexp512(e[k], etab) * (sr[4 * k] * sg);
+            if (__any_sync(0xffffffffu, hg != 0.0)) {  // some HF test point: discrepancy GP on the HF x HF pairs
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k) e[k] = Xt[(2 * d + 1) * NP + 4 * k + t] + xg[2 * d + 1];
+                for (int c = 0; c < d; ++c) {
+                    const double xc = xg[d + c];
+                    const double* xr = Xt + (d + c) * NP + t;
+#pragma unroll
+                    for (int k = 0; k < 2 * NT; ++k) e[k] = fma(xr[4 * k], xc, e[k]);
+                }
+                const double* hr = Xt + (2 * d + 3) * NP + t;
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k)
+                    if (hr[4 * k] * hg != 0.0) ks[k] += fexp512(e[k], etab);
+            }
+        }
+
+        // ---- V^T = K_s^T Wm^T over the lower-triangular tiles: v[i][e] = V^T[g][8i + 2t + e]
+        double v[NT][2];
+#pragma unroll
+        for (int i = 0; i < NT; ++i) {
+            v[i][0] = v[i][1] = 0.0;
+            const double* wr = Ws + (8 * i + g) * WP + t;
+#pragma unroll
+            for (int k = 0; k <= 2 * i + 1; ++k) dmma(v[i][0], v[i][1], ks[k], wr[4 * k]);
+        }
+
+        // ---- sum V^2, and sum U^2 with U^T = V^T Lq over the tiles m >= n (U never leaves the accumulators)
+        double ss = 0.0;
+#pragma unroll
+        for (int i = 0; i < NT; ++i) ss = fma(v[i][1], v[i][1], fma(v[i][0], v[i][0], ss));
+        double su = 0.0;
+#pragma unroll
+        for (int i = 0; i < NT; ++i) {
+            double c0 = 0.0, c1 = 0.0;
+            const double* lr = Lt + (8 * i + g) * WP + t;
+#pragma unroll
+            for (int i2 = i; i2 < NT; ++i2) {
+                dmma(c0, c1, v[i2][0], lr[8 * i2]);
+                dmma(c0, c1, v[i2][1], lr[8 * i2 + 4]);
+            }
+            su = fma(c1, c1, fma(c0, c0, su));
+        }
+        ss = quad_sum(ss);
+        su = quad_sum(su);
+
+        // ---- mean = V^T q_mu
+        double m = 0.0;
+        {
+            const double* qr = Qs + 2 * t;
+#pragma unroll
+            for (int i = 0; i < NT; ++i) m = fma(v[i][1], qr[8 * i + 1], fma(v[i][0], qr[8 * i], m));
+        }
+        m = quad_sum(m);
+        const long ptg = pt0 + g;
+        if (t == 0 && ptg < p.Ns) {
+            const long o = l * p.ls + ptg * p.ns;
+            p.mean[o] = m;
+            p.var[o] = xg[2 * d + 4] - ss + su;
+        }
+        __syncwarp();  // the group's records are read by every lane before lanes 0-7 overwrite them
+    }
+}
+
 // Input gradient of the blocked route (launch_posterior_dx): one CTA per (tile of TS test points, chunk of PC columns,
 // problem), walking the training points in tiles of TN.  Per tile it evaluates kL and kD from the scaled inputs (as K5
 // recomputes dK: nothing N x Ns is stored), forms G[j][s][n] = dk_sn/dx_sj in shared memory and adds G alpha (thread =
@@ -611,6 +758,16 @@ int launch_fused_nt(int NT, cudaStream_t s, const FusedArgs& a, int B, size_t sm
     }
 }
 
+template <int NT>
+int launch_svgp_fused(cudaStream_t s, const SvgpFusedArgs& a, size_t smem) {
+    static SmemOptIn optin;
+    if (!optin.ensure(svgp_posterior_predict_kernel<NT>, smem)) return -2;
+    const long G = (a.Ns + 7) / 8;
+    dim3 grid((unsigned)((G + a.gpc - 1) / a.gpc), (unsigned)a.q.L);
+    svgp_posterior_predict_kernel<NT><<<grid, PW * 32, smem, s>>>(a);
+    return cudaGetLastError() == cudaSuccess ? 0 : -2;
+}
+
 }  // namespace
 
 bool gpr_posterior_fused_ok(int N, int d, int P) {
@@ -663,4 +820,34 @@ int launch_posterior_dx(cudaStream_t s, const GprPosteriorData& q, int nb, const
     dim3 grid((unsigned)((Ns + DX_TS - 1) / DX_TS), (unsigned)((q.P + DX_PC - 1) / DX_PC), (unsigned)nb);
     posterior_dx_kernel<<<grid, DX_THREADS, smem, s>>>(q, Xs, Ns, alpha, beta, ldb, dmean, dvar);
     return cudaGetLastError() == cudaSuccess ? 0 : -2;
+}
+
+bool svgp_posterior_fused_ok(int L, int M, int d) {
+    return L >= 1 && L <= 65535 && M >= 1 && M <= MFGP_SMALL_MAX_N && d >= 1 && d <= MFGP_SMALL_MAX_D;
+}
+
+int svgp_posterior_predict_fused(cudaStream_t s, const SvgpPosteriorData& q, const double* Xs, int Ns, double* mean,
+                                 double* var, long ls, long ns) {
+    if (!svgp_posterior_fused_ok(q.L, q.M, q.d)) return -1;
+    if (Ns <= 0) return 0;
+    const int NT = (q.M + 7) / 8;
+    const size_t smem = svgp_fused_smem_bytes(NT, q.d);
+    // 8-point groups per CTA as gpr_posterior_predict_fused chooses them (at most 256: chunks of <= 2048 points)
+    const long G = (Ns + 7) / 8;
+    const long target = (long)mfgp_current_dev_info().sms * 8;
+    long gpc = (G * q.L + target - 1) / target;
+    if (gpc > 256) gpc = 256;
+    if (gpc > G) gpc = G;
+    if (gpc < 1) gpc = 1;
+    SvgpFusedArgs a{q, Xs, Ns, (int)gpc, mean, var, ls, ns};
+    switch (NT) {
+        case 1: return launch_svgp_fused<1>(s, a, smem);
+        case 2: return launch_svgp_fused<2>(s, a, smem);
+        case 3: return launch_svgp_fused<3>(s, a, smem);
+        case 4: return launch_svgp_fused<4>(s, a, smem);
+        case 5: return launch_svgp_fused<5>(s, a, smem);
+        case 6: return launch_svgp_fused<6>(s, a, smem);
+        case 7: return launch_svgp_fused<7>(s, a, smem);
+        default: return launch_svgp_fused<8>(s, a, smem);
+    }
 }

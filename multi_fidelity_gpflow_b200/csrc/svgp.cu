@@ -331,30 +331,15 @@ __global__ void finalize_kernel(const double* __restrict__ part, int nblocks, co
 
 inline dim3 g2(long total, int L) { return dim3((unsigned)((total + 255) / 256 > 4096 ? 4096 : (total + 255) / 256), L); }
 
-struct Fwd {
-    double *Kmm, *Wm, *S, *dinv, *logd, *Kmn, *A, *C, *Lq, *knn, *g_mean, *g_var;
-    long ldM, ldB, sMM, sMB;
-};
+}  // namespace
 
-int svgp_forward(mfgp_handle* h, Scope& sc, int L, int M, int B, int d, double jitter, const double* X,
-                 const double* Z, const double* theta, const double* q_mu, const double* q_sqrt, Fwd& f) {
+int svgp_factor(mfgp_handle* h, Scope& sc, int L, int M, int d, double jitter, const double* Z, const double* theta,
+                const double* q_sqrt, int* info_vec, Fwd& f) {
     cudaStream_t s = h->stream;
-    f.ldM = round_up(M, 2);
-    f.ldB = round_up(B, 2);
-    f.sMM = (long)M * f.ldM;
-    f.sMB = (long)M * f.ldB;
     f.Kmm = sc.alloc<double>((size_t)L * f.sMM);
-    f.Wm = sc.alloc<double>((size_t)L * f.sMM);
     f.S = sc.alloc<double>((size_t)L * f.sMM);
     f.dinv = sc.alloc<double>((size_t)chol_dinv_count(M, L));
     f.logd = sc.alloc<double>((size_t)L * M);
-    f.Kmn = sc.alloc<double>((size_t)L * f.sMB);
-    f.A = sc.alloc<double>((size_t)L * f.sMB);
-    f.C = sc.alloc<double>((size_t)L * f.sMB);
-    f.Lq = sc.alloc<double>((size_t)L * f.sMM);
-    f.knn = sc.alloc<double>((size_t)L * B);
-    f.g_mean = sc.alloc<double>((size_t)L * B);
-    f.g_var = sc.alloc<double>((size_t)L * B);
     if (!sc.ok) return MFGP_ERR_CUDA;
 
     CovArgs c{};
@@ -364,6 +349,28 @@ int svgp_forward(mfgp_handle* h, Scope& sc, int L, int M, int B, int d, double j
     c.symmetric = 1; c.mirror = 0; c.diag_add = jitter;
     c.batch = L;
     if (launch_cov(s, c)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp: cov(Z,Z) failed");
+    CholArgs ch{};
+    ch.A = f.Kmm; ch.N = M; ch.lda = f.ldM; ch.strideA = f.sMM; ch.batch = L;
+    ch.dinv = f.dinv; ch.logd = f.logd; ch.d_info = h->d_info; ch.aux = h->aux_stream; ch.ev = h->ev; ch.info_vec = info_vec;
+    if (launch_potrf(s, ch)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp: potrf failed");
+    if (launch_trtri(s, ch, f.Wm, f.ldM, f.sMM, f.S)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp: trtri failed");
+    tril_copy_kernel<<<g2(f.sMM, L), 256, 0, s>>>(q_sqrt, M, f.ldM, f.Lq);
+    return 0;
+}
+
+int svgp_conditional(mfgp_handle* h, Scope& sc, int L, int M, int B, int d, const double* X, const double* Z,
+                     const double* theta, const double* q_mu, Fwd& f) {
+    cudaStream_t s = h->stream;
+    f.ldB = round_up(B, 2);
+    f.sMB = (long)M * f.ldB;
+    f.Kmn = sc.alloc<double>((size_t)L * f.sMB);
+    f.A = sc.alloc<double>((size_t)L * f.sMB);
+    f.C = sc.alloc<double>((size_t)L * f.sMB);
+    f.knn = sc.alloc<double>((size_t)L * B);
+    f.g_mean = sc.alloc<double>((size_t)L * B);
+    f.g_var = sc.alloc<double>((size_t)L * B);
+    if (!sc.ok) return MFGP_ERR_CUDA;
+
     CovArgs cn{};
     cn.Xa = Z; cn.Na = M; cn.Xb = X; cn.Nb = B; cn.d = d;
     cn.theta = theta; cn.theta_stride = 2 * d + 3;
@@ -371,14 +378,6 @@ int svgp_forward(mfgp_handle* h, Scope& sc, int L, int M, int B, int d, double j
     cn.batch = L;
     if (launch_cov(s, cn)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp: cov(Z,X) failed");
     if (launch_cov_diag(s, X, B, d, theta, 2 * d + 3, f.knn, B, L)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp: cov_diag failed");
-
-    CholArgs ch{};
-    ch.A = f.Kmm; ch.N = M; ch.lda = f.ldM; ch.strideA = f.sMM; ch.batch = L;
-    ch.dinv = f.dinv; ch.logd = f.logd; ch.d_info = h->d_info; ch.aux = h->aux_stream; ch.ev = h->ev; ch.info_vec = nullptr;
-    if (launch_potrf(s, ch)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp: potrf failed");
-    if (launch_trtri(s, ch, f.Wm, f.ldM, f.sMM, f.S)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp: trtri failed");
-
-    tril_copy_kernel<<<g2(f.sMM, L), 256, 0, s>>>(q_sqrt, M, f.ldM, f.Lq);
 
     GemmArgs a;  // A = Wm Kmn
     a.M = M; a.N = B; a.K = M;
@@ -397,6 +396,52 @@ int svgp_forward(mfgp_handle* h, Scope& sc, int L, int M, int B, int d, double j
     if (launch_gemm(s, cc)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp: gemm C failed");
     col_reduce_kernel<<<dim3((B + 127) / 128, L), 128, 0, s>>>(f.A, f.C, M, B, f.ldB, q_mu, L, f.knn, f.g_mean, f.g_var);
     return 0;
+}
+
+int launch_svgp_mix(cudaStream_t s, const double* g_mean, const double* g_var, int L, int B, int P, const double* W,
+                    double* mean, double* var) {
+    const int nblk = (int)(((long)B * P + 255) / 256);
+    mix_ve_kernel<<<nblk, 256, 0, s>>>(1, g_mean, g_var, L, B, P, W, nullptr, 0, 0, nullptr, 0, 1.0, nullptr, nullptr,
+                                       nullptr, nullptr, mean, var);
+    return cudaGetLastError() == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+}
+
+// Cached-posterior prediction for any M, d: per chunk of test points svgp_conditional from the cached Wm and Lq, then the
+// mix.  Chunked so that the chunk's Kmn, A and C take at most half of the free device memory.  The same kernels on the
+// same factors as mfgp_svgp_predict.
+int svgp_posterior_predict_blocked(mfgp_handle* h, const SvgpPosteriorData& q, const double* Xs, int Ns, double* mean,
+                                   double* var) {
+    size_t freeb = 0, totb = 0;
+    cudaMemGetInfo(&freeb, &totb);
+    const size_t per = ((size_t)3 * q.L * q.M + (size_t)3 * q.L) * sizeof(double);
+    long chunk = (long)((freeb / 2) / per);
+    if (chunk < 2) chunk = 2;
+    for (long n0 = 0; n0 < Ns; n0 += chunk) {
+        const int nb = (int)((Ns - n0) < chunk ? (Ns - n0) : chunk);
+        Scope inner(h);
+        Fwd f{};
+        f.Wm = const_cast<double*>(q.Wm);  // read only: svgp_conditional does not write the factors
+        f.Lq = const_cast<double*>(q.Lq);
+        f.ldM = q.ld;
+        f.sMM = (long)q.M * q.ld;
+        MFGP_TRY(svgp_conditional(h, inner, q.L, q.M, nb, q.d, Xs + n0 * (q.d + 1), q.Z, q.theta, q.q_mu, f));
+        if (launch_svgp_mix(h->stream, f.g_mean, f.g_var, q.L, nb, q.P, q.W, mean + n0 * q.P, var + n0 * q.P))
+            return mfgp_fail(h, MFGP_ERR_CUDA, "svgp posterior: mix launch failed");
+    }
+    return 0;
+}
+
+namespace {
+
+int svgp_forward(mfgp_handle* h, Scope& sc, int L, int M, int B, int d, double jitter, const double* X,
+                 const double* Z, const double* theta, const double* q_mu, const double* q_sqrt, Fwd& f) {
+    f.ldM = round_up(M, 2);
+    f.sMM = (long)M * f.ldM;
+    f.Wm = sc.alloc<double>((size_t)L * f.sMM);
+    f.Lq = sc.alloc<double>((size_t)L * f.sMM);
+    if (!sc.ok) return MFGP_ERR_CUDA;
+    MFGP_TRY(svgp_factor(h, sc, L, M, d, jitter, Z, theta, q_sqrt, nullptr, f));
+    return svgp_conditional(h, sc, L, M, B, d, X, Z, theta, q_mu, f);
 }
 
 }  // namespace
@@ -603,9 +648,8 @@ int mfgp_svgp_predict(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* Xs
     if (!sc.ok) return sc.finish();
     Fwd f;
     MFGP_TRY(svgp_forward(h, sc, L, M, Ns, d, cfg->jitter, dX, dZ, dth, dqm, dqs, f));
-    const int nblk = (int)(((long)Ns * P + 255) / 256);
-    mix_ve_kernel<<<nblk, 256, 0, s>>>(1, f.g_mean, f.g_var, L, Ns, P, dW, nullptr, 0, 0, nullptr, 0, 1.0, nullptr, nullptr,
-                                       nullptr, nullptr, dmean, dvar);
+    if (launch_svgp_mix(s, f.g_mean, f.g_var, L, Ns, P, dW, dmean, dvar))
+        return mfgp_fail(h, MFGP_ERR_CUDA, "mfgp_svgp_predict: mix launch failed");
     return sc.finish();
 }
 

@@ -222,6 +222,14 @@ class SVGPBase:
         return self.handle.svgp_predict(Xnew, self.Z.numpy(), self._thetas(d), self._W(), self.q_mu.numpy(),
                                         np.tril(self.q_sqrt.numpy()))
 
+    def posterior(self):
+        """SVGPPosterior: the inducing covariances factored once at the current parameters (a snapshot of Z, the
+        kernels, W, q_mu and tril(q_sqrt)); its predict_f gives what predict_f gives, without factoring on every call."""
+        Z = self.Z.numpy()
+        d = Z.shape[1] - 1
+        return SVGPPosterior(self.handle.svgp_posterior(Z, self._thetas(d), self._W(), self.q_mu.numpy(),
+                                                        np.tril(self.q_sqrt.numpy())))
+
     # ---- checkpoint (pickle of gpflow.utilities.parameter_dict-style names) ------------------------
     def save_model(self, filename):
         with open(filename, "wb") as f:
@@ -231,3 +239,15 @@ class SVGPBase:
         with open(filename, "rb") as f:
             multiple_assign(self, pickle.load(f))
         return self
+
+
+class SVGPPosterior:
+    """What SVGPBase.posterior() returns: predict_f(Xnew) -> mean, var [N*, P] from the cached factors."""
+
+    def __init__(self, post):
+        self.post = post
+
+    def predict_f(self, Xnew, full_cov=False, full_output_cov=False):
+        if full_cov or full_output_cov:
+            raise NotImplementedError("the reference only calls predict_f(Xnew) (marginal variances)")
+        return self.post.predict(_lib.as_f64(Xnew))

@@ -516,22 +516,49 @@ class Handle:
         return out.value
 
 
-class GprPosterior:
+class _Posterior:
+    """A device-resident posterior owned by this object: freed by close() or when the object is collected."""
+
+    _destroy = None  # the C-ABI destroy function of the subclass's posterior type
+
+    def __init__(self, handle, ptr):
+        self.handle, self._p = handle, ptr
+
+    def _xs(self, Xs):
+        """Xs as float64 [Ns, d+1], after checking that the posterior is open."""
+        if not self._p:
+            raise ValueError(f"{type(self).__name__} is closed")
+        Xs = as_f64(Xs)
+        if Xs.shape[1] != self.d + 1:
+            raise ValueError(f"Xs must have {self.d + 1} columns")
+        return Xs
+
+    def close(self):
+        if getattr(self, "_p", None):
+            type(self)._destroy(self._p)
+            self._p = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class GprPosterior(_Posterior):
     """Device-resident factors of B exact GPs (W = L^-1, a = W Y) made by Handle.gpr_posterior: a snapshot of the
     hyper-parameters and data at creation.  predict() returns mean [B, Ns, P] and var [B, Ns]."""
 
+    _destroy = _lib.mfgp_gpr_posterior_destroy
+
     def __init__(self, handle, ptr, B, N, d, P):
-        self.handle, self._p = handle, ptr
+        super().__init__(handle, ptr)
         self.B, self.N, self.d, self.P = B, N, d, P
 
     def predict(self, Xs, mean=None, var=None):
         """Host arrays or device tensors; mean / var (optional outputs) may be device tensors (zero-copy)."""
-        if not self._p:
-            raise ValueError("GprPosterior is closed")
-        Xs = as_f64(Xs)
+        Xs = self._xs(Xs)
         Ns = Xs.shape[0]
-        if Xs.shape[1] != self.d + 1:
-            raise ValueError(f"Xs must have {self.d + 1} columns")
         mean = np.empty((self.B, Ns, self.P)) if mean is None else mean
         var = np.empty((self.B, Ns)) if var is None else var
         self.handle._check(_lib.mfgp_gpr_posterior_predict(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean), _ptr(var)),
@@ -541,12 +568,8 @@ class GprPosterior:
     def predict_grad(self, Xs, mean=None, var=None, dmean=None, dvar=None):
         """predict() plus the gradients with respect to the d continuous coordinates of each test point:
         (mean [B, Ns, P], var [B, Ns], dmean [B, Ns, P, d], dvar [B, Ns, d]).  Host arrays or device tensors."""
-        if not self._p:
-            raise ValueError("GprPosterior is closed")
-        Xs = as_f64(Xs)
+        Xs = self._xs(Xs)
         Ns = Xs.shape[0]
-        if Xs.shape[1] != self.d + 1:
-            raise ValueError(f"Xs must have {self.d + 1} columns")
         mean = np.empty((self.B, Ns, self.P)) if mean is None else mean
         var = np.empty((self.B, Ns)) if var is None else var
         dmean = np.empty((self.B, Ns, self.P, self.d)) if dmean is None else dmean
@@ -555,50 +578,26 @@ class GprPosterior:
                                                                 _ptr(dmean), _ptr(dvar)), "mfgp_gpr_posterior_predict_grad")
         return mean, var, dmean, dvar
 
-    def close(self):
-        if getattr(self, "_p", None):
-            _lib.mfgp_gpr_posterior_destroy(self._p)
-            self._p = None
 
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-
-class SvgpPosterior:
+class SvgpPosterior(_Posterior):
     """Device-resident factors of an SVGP (Wm = Lm^-1, tril(q_sqrt), q_mu, W) made by Handle.svgp_posterior: a snapshot of
     the parameters at creation.  predict() returns mean [Ns, P] and var [Ns, P], as Handle.svgp_predict."""
 
+    _destroy = _lib.mfgp_svgp_posterior_destroy
+
     def __init__(self, handle, ptr, L, M, P, d):
-        self.handle, self._p = handle, ptr
+        super().__init__(handle, ptr)
         self.L, self.M, self.P, self.d = L, M, P, d
 
     def predict(self, Xs, mean=None, var=None):
         """Host arrays or device tensors; mean / var (optional outputs) may be device tensors (zero-copy)."""
-        if not self._p:
-            raise ValueError("SvgpPosterior is closed")
-        Xs = as_f64(Xs)
+        Xs = self._xs(Xs)
         Ns = Xs.shape[0]
-        if Xs.shape[1] != self.d + 1:
-            raise ValueError(f"Xs must have {self.d + 1} columns")
         mean = np.empty((Ns, self.P)) if mean is None else mean
         var = np.empty((Ns, self.P)) if var is None else var
         self.handle._check(_lib.mfgp_svgp_posterior_predict(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean), _ptr(var)),
                            "mfgp_svgp_posterior_predict")
         return mean, var
-
-    def close(self):
-        if getattr(self, "_p", None):
-            _lib.mfgp_svgp_posterior_destroy(self._p)
-            self._p = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
 
 _default = {}

@@ -10,6 +10,7 @@
 #include "gemm.cuh"
 #include "gpr.cuh"
 #include "gpr_small.cuh"
+#include "mathx.cuh"
 #include "svgp.cuh"
 
 #define CHECK_H(h) \
@@ -320,12 +321,8 @@ int mfgp_gpr_batched_nlml_grad(mfgp_handle* h, const double* X, int N, int d, co
             return mfgp_fail(h, MFGP_ERR_CUDA, "gpr_small launch failed");
     } else {
         // blocked path, chunked so that 3 N^2 workspaces per problem fit comfortably
-        size_t freeb = 0, totb = 0;
-        cudaMemGetInfo(&freeb, &totb);
-        const size_t per = (size_t)3 * N * round_up(N, 2) * 8 + (size_t)chol_dinv_count(N, 1) * 8;
-        long chunk = (long)((freeb / 2) / per);
-        if (chunk < 1) chunk = 1;
-        if (chunk > 16384) chunk = 16384;
+        const long chunk =
+            chunk_by_free_memory((size_t)3 * N * round_up(N, 2) * 8 + (size_t)chol_dinv_count(N, 1) * 8, 1, 16384);
         for (long b0 = 0; b0 < B; b0 += chunk) {
             const int nb = (int)((B - b0) < chunk ? (B - b0) : chunk);
             Scope inner(h);
@@ -339,17 +336,72 @@ int mfgp_gpr_batched_nlml_grad(mfgp_handle* h, const double* X, int N, int d, co
 }
 
 // ---------------------------------------------------------------------------------------------
-// Cached posterior (include/mfgp.h).  One cudaMalloc block holds the device copies of X, theta, noise and the factors;
-// it belongs to the device, not to the handle that created it.
+// Cached posteriors (include/mfgp.h).  One cudaMalloc block holds the device copies of the inputs and the factors; it
+// belongs to the device, not to the handle that created it.
 }  // extern "C"
 
-struct mfgp_gpr_posterior {
+struct PosteriorMem {
     int device;
-    GprPosteriorData q;
     void* mem;
+};
+struct mfgp_gpr_posterior {
+    PosteriorMem m;
+    GprPosteriorData q;
+};
+struct mfgp_svgp_posterior {
+    PosteriorMem m;
+    SvgpPosteriorData q;
 };
 
 namespace {
+// Offsets of consecutive arrays of doubles in one block, each 256-byte aligned: add() every array, allocate tot bytes,
+// then at() gives each array's address.
+struct Carve {
+    size_t tot = 0;
+    size_t add(size_t count) {
+        const size_t o = tot;
+        tot += (count * sizeof(double) + 255) & ~(size_t)255;
+        return o;
+    }
+    static double* at(void* mem, size_t off) { return reinterpret_cast<double*>(static_cast<char*>(mem) + off); }
+};
+
+// The end of a create call: the block is freed when the call fails (rc < 0, or a failed factorisation without an info
+// array to report it in); otherwise *out becomes a new posterior that owns it.
+template <class Post, class Data>
+int publish_posterior(mfgp_handle* h, int rc, const int* info, void* mem, const Data& q, Post** out) {
+    if (rc < 0 || (rc > 0 && !info)) {
+        cudaFree(mem);
+        return rc;
+    }
+    *out = new Post{{h->device, mem}, q};
+    return rc;
+}
+
+// The checks every predict call of a posterior starts with.  Returns 1 when there is work, else what the call returns
+// (0 for Ns == 0, or the error code).  Makes the handle's device current.
+template <class Post>
+int posterior_predict_prologue(mfgp_handle* h, const Post* post, const double* Xs, int Ns, const double* mean,
+                               const double* var, const char* name) {
+    CHECK_H(h);
+    if (!post || !Xs || !mean || !var || Ns < 0) return mfgp_fail(h, MFGP_ERR_ARG, "%s: bad argument", name);
+    if (post->m.device != h->device)
+        return mfgp_fail(h, MFGP_ERR_ARG, "%s: the posterior lives on device %d, the handle on %d", name, post->m.device,
+                         h->device);
+    if (Ns == 0) return 0;
+    cudaSetDevice(h->device);
+    return 1;
+}
+
+int free_posterior_mem(const PosteriorMem& m) {
+    int prev = 0;
+    cudaGetDevice(&prev);
+    cudaSetDevice(m.device);
+    const cudaError_t e = cudaFree(m.mem);
+    cudaSetDevice(prev);
+    return e == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+}
+
 // Problems whose factorisation failed: NaN on the diagonal of W and in a (real columns), so both predict routes give NaN.
 __global__ void posterior_poison_kernel(const int* __restrict__ info, int B, int N, long ld, int P, int Pp, double* __restrict__ W,
                                         double* __restrict__ a) {
@@ -375,20 +427,13 @@ int mfgp_gpr_posterior_create(mfgp_handle* h, const double* X, int N, int d, con
     cudaSetDevice(h->device);
     const int np = 2 * d + 3, Pp = (int)round_up(P, 2);
     const long ld = round_up(N, 2);
-    size_t tot = 0;
-    auto carve = [&](size_t count) {
-        const size_t o = tot;
-        tot += (count * sizeof(double) + 255) & ~(size_t)255;
-        return o;
-    };
-    const size_t oX = carve((size_t)N * (d + 1)), oT = carve((size_t)B * np), oN = carve(B),
-                 oW = carve((size_t)B * N * ld), oA = carve((size_t)B * N * Pp);
+    Carve c;
+    const size_t oX = c.add((size_t)N * (d + 1)), oT = c.add((size_t)B * np), oN = c.add(B), oW = c.add((size_t)B * N * ld),
+                 oA = c.add((size_t)B * N * Pp);
     void* mem = nullptr;
-    CUDA_TRY(h, cudaMalloc(&mem, tot));
-    char* base = static_cast<char*>(mem);
-    double *dX = reinterpret_cast<double*>(base + oX), *dT = reinterpret_cast<double*>(base + oT),
-           *dN = reinterpret_cast<double*>(base + oN), *dW = reinterpret_cast<double*>(base + oW),
-           *dA = reinterpret_cast<double*>(base + oA);
+    CUDA_TRY(h, cudaMalloc(&mem, c.tot));
+    double *dX = Carve::at(mem, oX), *dT = Carve::at(mem, oT), *dN = Carve::at(mem, oN), *dW = Carve::at(mem, oW),
+           *dA = Carve::at(mem, oA);
     const int rc = [&]() -> int {
         Scope sc(h);
         cudaStream_t s = h->stream;
@@ -399,12 +444,8 @@ int mfgp_gpr_posterior_create(mfgp_handle* h, const double* X, int N, int d, con
         int* di = info ? sc.out(info, B, true) : sc.alloc<int>(B, true);
         if (!sc.ok) return sc.finish();
         // the blocked batched route of mfgp_gpr_batched_nlml_grad, chunked so that its workspaces fit comfortably
-        size_t freeb = 0, totb = 0;
-        cudaMemGetInfo(&freeb, &totb);
         const size_t per = ((size_t)3 * N * ld + (size_t)chol_dinv_count(N, 1) + (size_t)2 * N * Pp + N) * sizeof(double);
-        long chunk = (long)((freeb / 2) / per);
-        if (chunk < 1) chunk = 1;
-        if (chunk > 16384) chunk = 16384;
+        const long chunk = chunk_by_free_memory(per, 1, 16384);
         for (long b0 = 0; b0 < B; b0 += chunk) {
             const int nb = (int)((B - b0) < chunk ? (B - b0) : chunk);
             Scope inner(h);
@@ -418,16 +459,7 @@ int mfgp_gpr_posterior_create(mfgp_handle* h, const double* X, int N, int d, con
         sc.host_out = true;  // always synchronise: the factorisation status decides what the call returns
         return sc.finish();
     }();
-    if (rc < 0 || (rc > 0 && !info)) {
-        cudaFree(mem);
-        return rc;
-    }
-    auto* post = new mfgp_gpr_posterior();
-    post->device = h->device;
-    post->mem = mem;
-    post->q = GprPosteriorData{N, d, P, Pp, B, ld, dX, dT, dN, dW, dA};
-    *out = post;
-    return rc;
+    return publish_posterior(h, rc, info, mem, GprPosteriorData{N, d, P, Pp, B, ld, dX, dT, dN, dW, dA}, out);
 }
 
 }  // extern "C"
@@ -436,13 +468,7 @@ namespace {
 // mfgp_gpr_posterior_predict and _predict_grad: one body, the gradients when dmean != NULL.
 int posterior_predict(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns, double* mean, double* var,
                       double* dmean, double* dvar, const char* name) {
-    CHECK_H(h);
-    if (!post || !Xs || !mean || !var || Ns < 0) return mfgp_fail(h, MFGP_ERR_ARG, "%s: bad argument", name);
-    if (post->device != h->device)
-        return mfgp_fail(h, MFGP_ERR_ARG, "%s: the posterior lives on device %d, the handle on %d", name, post->device,
-                         h->device);
-    if (Ns == 0) return 0;
-    cudaSetDevice(h->device);
+    if (const int rc = posterior_predict_prologue(h, post, Xs, Ns, mean, var, name); rc <= 0) return rc;
     const GprPosteriorData& q = post->q;
     Scope sc(h);
     const double* dXs = sc.in(Xs, (size_t)Ns * (q.d + 1));
@@ -479,27 +505,13 @@ int mfgp_gpr_posterior_predict_grad(mfgp_handle* h, const mfgp_gpr_posterior* po
 
 int mfgp_gpr_posterior_destroy(mfgp_gpr_posterior* post) {
     if (!post) return 0;
-    int prev = 0;
-    cudaGetDevice(&prev);
-    cudaSetDevice(post->device);
-    const cudaError_t e = cudaFree(post->mem);
-    cudaSetDevice(prev);
+    const int rc = free_posterior_mem(post->m);
     delete post;
-    return e == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+    return rc;
 }
 
 // ---------------------------------------------------------------------------------------------
 // Cached SVGP posterior (include/mfgp.h): the memory model of mfgp_gpr_posterior, the factors of svgp_factor.
-}  // extern "C"
-
-struct mfgp_svgp_posterior {
-    int device;
-    SvgpPosteriorData q;
-    void* mem;
-};
-
-extern "C" {
-
 int mfgp_svgp_posterior_create(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* Z, const double* theta,
                                const double* W, const double* q_mu, const double* q_sqrt, int* info,
                                mfgp_svgp_posterior** out) {
@@ -513,20 +525,13 @@ int mfgp_svgp_posterior_create(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const d
     cudaSetDevice(h->device);
     const int np = 2 * d + 3;
     const long ld = round_up(M, 2);
-    size_t tot = 0;
-    auto carve = [&](size_t count) {
-        const size_t o = tot;
-        tot += (count * sizeof(double) + 255) & ~(size_t)255;
-        return o;
-    };
-    const size_t oZ = carve((size_t)M * (d + 1)), oT = carve((size_t)L * np), oW = carve(W ? (size_t)P * L : 0),
-                 oWm = carve((size_t)L * M * ld), oLq = carve((size_t)L * M * ld), oQ = carve((size_t)M * L);
+    Carve c;
+    const size_t oZ = c.add((size_t)M * (d + 1)), oT = c.add((size_t)L * np), oW = c.add(W ? (size_t)P * L : 0),
+                 oWm = c.add((size_t)L * M * ld), oLq = c.add((size_t)L * M * ld), oQ = c.add((size_t)M * L);
     void* mem = nullptr;
-    CUDA_TRY(h, cudaMalloc(&mem, tot));
-    char* base = static_cast<char*>(mem);
-    double *dZ = reinterpret_cast<double*>(base + oZ), *dT = reinterpret_cast<double*>(base + oT),
-           *dW = W ? reinterpret_cast<double*>(base + oW) : nullptr, *dWm = reinterpret_cast<double*>(base + oWm),
-           *dLq = reinterpret_cast<double*>(base + oLq), *dQ = reinterpret_cast<double*>(base + oQ);
+    CUDA_TRY(h, cudaMalloc(&mem, c.tot));
+    double *dZ = Carve::at(mem, oZ), *dT = Carve::at(mem, oT), *dW = W ? Carve::at(mem, oW) : nullptr,
+           *dWm = Carve::at(mem, oWm), *dLq = Carve::at(mem, oLq), *dQ = Carve::at(mem, oQ);
     const int rc = [&]() -> int {
         Scope sc(h);
         cudaStream_t s = h->stream;
@@ -548,27 +553,13 @@ int mfgp_svgp_posterior_create(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const d
         sc.host_out = true;  // always synchronise: the factorisation status decides what the call returns
         return sc.finish();
     }();
-    if (rc < 0 || (rc > 0 && !info)) {
-        cudaFree(mem);
-        return rc;
-    }
-    auto* post = new mfgp_svgp_posterior();
-    post->device = h->device;
-    post->mem = mem;
-    post->q = SvgpPosteriorData{L, M, P, d, ld, dZ, dT, dW, dWm, dLq, dQ};
-    *out = post;
-    return rc;
+    return publish_posterior(h, rc, info, mem, SvgpPosteriorData{L, M, P, d, ld, dZ, dT, dW, dWm, dLq, dQ}, out);
 }
 
 int mfgp_svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns, double* mean,
                                 double* var) {
-    CHECK_H(h);
-    if (!post || !Xs || !mean || !var || Ns < 0) return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_posterior_predict: bad argument");
-    if (post->device != h->device)
-        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_posterior_predict: the posterior lives on device %d, the handle on %d",
-                         post->device, h->device);
-    if (Ns == 0) return 0;
-    cudaSetDevice(h->device);
+    if (const int rc = posterior_predict_prologue(h, post, Xs, Ns, mean, var, "mfgp_svgp_posterior_predict"); rc <= 0)
+        return rc;
     const SvgpPosteriorData& q = post->q;
     Scope sc(h);
     const double* dXs = sc.in(Xs, (size_t)Ns * (q.d + 1));
@@ -594,13 +585,9 @@ int mfgp_svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post,
 
 int mfgp_svgp_posterior_destroy(mfgp_svgp_posterior* post) {
     if (!post) return 0;
-    int prev = 0;
-    cudaGetDevice(&prev);
-    cudaSetDevice(post->device);
-    const cudaError_t e = cudaFree(post->mem);
-    cudaSetDevice(prev);
+    const int rc = free_posterior_mem(post->m);
     delete post;
-    return e == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+    return rc;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -929,10 +916,7 @@ __global__ void __launch_bounds__(256) dmma_peak_kernel(double* out, int iters) 
     const double a = 1.0 + 1e-9 * threadIdx.x, b = 1e-9;
     for (int it = 0; it < iters; ++it) {
 #pragma unroll
-        for (int i = 0; i < 16; ++i)
-            asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                         : "+d"(c[i][0]), "+d"(c[i][1])
-                         : "d"(a), "d"(b));
+        for (int i = 0; i < 16; ++i) dmma(c[i][0], c[i][1], a, b);
     }
     double s = 0.0;
 #pragma unroll
@@ -955,10 +939,7 @@ __global__ void __launch_bounds__(256) dmix_peak_kernel(double* out, int iters) 
 #pragma unroll
         for (int r = 0; r < 4; ++r) {
 #pragma unroll
-            for (int i = 0; i < 2; ++i)
-                asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                             : "+d"(c[2 * r + i][0]), "+d"(c[2 * r + i][1])
-                             : "d"(am), "d"(bm));
+            for (int i = 0; i < 2; ++i) dmma(c[2 * r + i][0], c[2 * r + i][1], am, bm);
 #pragma unroll
             for (int i = 0; i < 16; ++i) a[i] = fma(a[i], x, y);
         }

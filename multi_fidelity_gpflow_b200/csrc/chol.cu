@@ -16,6 +16,7 @@
 #include <cstdlib>
 
 #include "gemm.cuh"
+#include "mathx.cuh"
 
 namespace {
 
@@ -35,11 +36,6 @@ struct DiagArgs {
 };
 
 // ---- DMMA tile helpers (same swizzled 8x8-tile layout as gpr_small_v4.cu) ---------------------------
-__device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                 : "+d"(c0), "+d"(c1)
-                 : "d"(a), "d"(b));
-}
 __device__ __forceinline__ int tslot(int i, int j) { return i * (i + 1) / 2 + j; }  // i >= j
 __device__ __forceinline__ int tile_off(int r, int c) { return r * 8 + ((((c >> 1) ^ (r & 2))) << 1) + (c & 1); }
 

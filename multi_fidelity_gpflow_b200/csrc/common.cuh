@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include <chrono>
+#include <climits>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstdio>
@@ -260,3 +261,14 @@ struct Scope {
 };
 
 __host__ __device__ inline long round_up(long x, long m) { return (x + m - 1) / m * m; }
+
+// Items per chunk of a chunked call: as many as take at most half of the free device memory at per_item bytes each,
+// clamped to [lo, hi].
+inline long chunk_by_free_memory(size_t per_item, long lo, long hi) {
+    size_t freeb = 0, totb = 0;
+    cudaMemGetInfo(&freeb, &totb);
+    long chunk = (long)((freeb / 2) / per_item);
+    if (chunk < lo) chunk = lo;
+    if (chunk > hi) chunk = hi;
+    return chunk;
+}

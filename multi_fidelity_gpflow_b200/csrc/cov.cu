@@ -747,12 +747,6 @@ __global__ void __launch_bounds__(256, SYM ? 2 : 3) cov_stream_kernel(CovStreamA
 // Panel rows are padded to 68 doubles in shared memory so that the 8-byte fragment loads (address t * 68 + g) of a
 // half-warp fall into 16 different bank pairs.
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void dmma_acc(double& c0, double& c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                 : "+d"(c0), "+d"(c1)
-                 : "d"(a), "d"(b));
-}
-
 constexpr int COV_PS = 68;  // shared-memory pitch of a panel row (doubles)
 
 // acc[mi][ni][2] += sum over the d coordinate rows starting at row `c0` + the two augmented columns built from row `hrow`
@@ -779,7 +773,7 @@ __device__ __forceinline__ void tile_dmma(const double* __restrict__ Ar, const d
 #pragma unroll
         for (int mi = 0; mi < 2; ++mi)
 #pragma unroll
-            for (int ni = 0; ni < 4; ++ni) dmma_acc(acc[mi][ni][0], acc[mi][ni][1], a[mi], b[ni]);
+            for (int ni = 0; ni < 4; ++ni) dmma(acc[mi][ni][0], acc[mi][ni][1], a[mi], b[ni]);
     };
     if constexpr (D > 0) {
         constexpr int KS = (D + 2 + 3) / 4;

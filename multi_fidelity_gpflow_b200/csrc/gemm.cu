@@ -24,6 +24,8 @@
 #include <cstdint>
 #include <cstdlib>
 
+#include "mathx.cuh"
+
 namespace {
 
 constexpr int BK = 16;
@@ -41,11 +43,6 @@ __device__ __forceinline__ double lds64(uint32_t addr) {
     double v;
     asm volatile("ld.shared.f64 %0, [%1];\n" : "=d"(v) : "r"(addr));
     return v;
-}
-__device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                 : "+d"(c0), "+d"(c1)
-                 : "d"(a), "d"(b));
 }
 
 // ---- TMA / mbarrier primitives -------------------------------------------------------------------

@@ -281,12 +281,8 @@ int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, con
     cudaStream_t s = h->stream;
     const int np = 2 * q.d + 3, N = q.N;
     const long lds = round_up(Ns, 2);
-    size_t freeb = 0, totb = 0;
-    cudaMemGetInfo(&freeb, &totb);
     const size_t per = ((size_t)2 * N * lds + Ns + (dmean ? (size_t)N * q.Pp : 0)) * sizeof(double);
-    long chunk = (long)((freeb / 2) / per);
-    if (chunk < 1) chunk = 1;
-    if (chunk > 16384) chunk = 16384;  // grid z of the batched kernels
+    const long chunk = chunk_by_free_memory(per, 1, 16384);  // 16384: grid z of the batched kernels
     for (long b0 = 0; b0 < q.B; b0 += chunk) {
         const int nb = (int)((q.B - b0) < chunk ? (q.B - b0) : chunk);
         Scope inner(h);

@@ -52,14 +52,14 @@ struct GprPosteriorData {
 };
 // mean [B][Ns][P], var [B][Ns]; with dmean [B][Ns][P][d] and dvar [B][Ns][d] (both or neither) also the gradients with
 // respect to the d continuous coordinates of each test point (mfgp_gpr_posterior_predict_grad).  All device pointers.
-// Fused route (gpr_posterior.cu): one kernel, N <= 64, d <= 16, P <= 64 (gpr_posterior_fused_ok).
+// Fused route (posterior.cu): one kernel, N <= 64, d <= 16, P <= 64 (gpr_posterior_fused_ok).
 bool gpr_posterior_fused_ok(int N, int d, int P);
 int gpr_posterior_predict_fused(cudaStream_t s, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
                                 double* var, double* dmean = nullptr, double* dvar = nullptr);
 // Blocked route (gpr.cu): any size, built from K1 / cov_diag / the batched GEMM, chunked over problems.
 int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
                                   double* var, double* dmean = nullptr, double* dvar = nullptr);
-// The input-gradient contraction of the blocked route (gpr_posterior.cu) for nb problems of q (theta from q.theta):
+// The input-gradient contraction of the blocked route (posterior.cu) for nb problems of q (theta from q.theta):
 // dmean[b][s][p][j] = sum_n alpha[b][n][p] dk_sn/dx_sj, dvar[b][s][j] = -2 sum_n beta[b][n][s] dk_sn/dx_sj, with
 // alpha [nb][N][q.Pp] = W^T a and beta [nb][N][ldb] = K^-1 K_s.
 int launch_posterior_dx(cudaStream_t s, const GprPosteriorData& q, int nb, const double* Xs, int Ns, const double* alpha,

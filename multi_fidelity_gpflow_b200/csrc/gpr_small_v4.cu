@@ -54,16 +54,6 @@ __device__ __forceinline__ double warp_sum(double v) {
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
-__device__ __forceinline__ double quad_sum(double v) {  // sum over the 4 lanes that share g
-    v += __shfl_xor_sync(0xffffffffu, v, 1);
-    v += __shfl_xor_sync(0xffffffffu, v, 2);
-    return v;
-}
-__device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                 : "+d"(c0), "+d"(c1)
-                 : "d"(a), "d"(b));
-}
 // element offset (doubles) inside a 64-double tile: 16-byte chunks of a row XOR-swizzled by (row & 2)
 __host__ __device__ __forceinline__ constexpr int tile_off(int r, int c) {
     return r * 8 + ((((c >> 1) ^ (r & 2))) << 1) + (c & 1);

@@ -1,5 +1,18 @@
-// mathx.cuh -- branch-free fp64 exp for the SE-kernel exponent (arguments <= ~0).
+// mathx.cuh -- branch-free fp64 exp for the SE-kernel exponent (arguments <= ~0), and the FP64 tensor-core warp primitives.
 #pragma once
+
+// One mma.sync.m8n8k4.f64 (SASS: DMMA.8x8x4): C[8x8] += A[8x4] B[4x8].  Lane (g, t) = (lane / 4, lane % 4) holds
+// A[g][t], B[t][g] and C[g][2t], C[g][2t + 1].
+__device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b) {
+    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
+                 : "+d"(c0), "+d"(c1)
+                 : "d"(a), "d"(b));
+}
+__device__ __forceinline__ double quad_sum(double v) {  // sum over the 4 lanes that share g
+    v += __shfl_xor_sync(0xffffffffu, v, 1);
+    v += __shfl_xor_sync(0xffffffffu, v, 2);
+    return v;
+}
 
 // Round-to-nearest range reduction, degree-13 Taylor/Horner on |r| <= ln2/2 (truncation 4e-18), exponent spliced
 // into the high word.  Arguments below -700 are clamped (result ~1e-304 instead of a denormal / 0).

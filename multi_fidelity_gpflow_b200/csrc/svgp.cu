@@ -411,11 +411,7 @@ int launch_svgp_mix(cudaStream_t s, const double* g_mean, const double* g_var, i
 // same factors as mfgp_svgp_predict.
 int svgp_posterior_predict_blocked(mfgp_handle* h, const SvgpPosteriorData& q, const double* Xs, int Ns, double* mean,
                                    double* var) {
-    size_t freeb = 0, totb = 0;
-    cudaMemGetInfo(&freeb, &totb);
-    const size_t per = ((size_t)3 * q.L * q.M + (size_t)3 * q.L) * sizeof(double);
-    long chunk = (long)((freeb / 2) / per);
-    if (chunk < 2) chunk = 2;
+    const long chunk = chunk_by_free_memory(((size_t)3 * q.L * q.M + (size_t)3 * q.L) * sizeof(double), 2, LONG_MAX);
     for (long n0 = 0; n0 < Ns; n0 += chunk) {
         const int nb = (int)((Ns - n0) < chunk ? (Ns - n0) : chunk);
         Scope inner(h);

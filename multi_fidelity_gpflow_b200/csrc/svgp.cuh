@@ -37,7 +37,7 @@ struct SvgpPosteriorData {
     const double* Lq;
     const double* q_mu;
 };
-// Fused route (gpr_posterior.cu): one kernel for M <= 64, d <= 16.  Writes the latent marginals of point n and latent l
+// Fused route (posterior.cu): one kernel for M <= 64, d <= 16.  Writes the latent marginals of point n and latent l
 // to mean[l * ls + n * ns] and var[l * ls + n * ns]: (ls, ns) = (1, P) is the [Ns][P] output itself when W == NULL,
 // (Ns, 1) the [L][Ns] input of launch_svgp_mix.
 bool svgp_posterior_fused_ok(int L, int M, int d);

@@ -327,7 +327,7 @@ int mfgp_gpr_batched_nlml_grad(mfgp_handle* h, const double* X, int N, int d, co
             const int nb = (int)((B - b0) < chunk ? (B - b0) : chunk);
             Scope inner(h);
             int rc = gpr_nlml_grad_device(h, inner, dX, dY, ldy, 1, (int)b0, ycols, N, d, 1, nb, dth + b0 * (2 * d + 3),
-                                          dnz + b0, dn + b0, dg ? dg + b0 * (2 * d + 4) : nullptr, di ? di + b0 : nullptr);
+                                          dnz + b0, dn + b0, dg ? dg + b0 * (2 * d + 4) : nullptr, di ? di + b0 : nullptr, B);
             if (rc) return rc;
             if (!inner.ok) return inner.finish();
         }
@@ -450,7 +450,8 @@ int mfgp_gpr_posterior_create(mfgp_handle* h, const double* X, int N, int d, con
             const int nb = (int)((B - b0) < chunk ? (B - b0) : chunk);
             Scope inner(h);
             GprFactor f;
-            MFGP_TRY(gpr_factor(h, inner, dX, dY, ldy, P, (int)b0, ycols, N, d, P, nb, dT + b0 * np, dN + b0, di + b0, f, true));
+            MFGP_TRY(gpr_factor(h, inner, dX, dY, ldy, P, (int)b0, ycols, N, d, P, nb, dT + b0 * np, dN + b0, di + b0, f, true,
+                               B));
             if (!inner.ok) return inner.finish();
             CUDA_TRY(h, cudaMemcpyAsync(dW + b0 * N * ld, f.W, (size_t)nb * N * ld * sizeof(double), cudaMemcpyDeviceToDevice, s));
             CUDA_TRY(h, cudaMemcpyAsync(dA + b0 * N * Pp, f.a, (size_t)nb * N * Pp * sizeof(double), cudaMemcpyDeviceToDevice, s));

@@ -999,7 +999,7 @@ int launch_cov(cudaStream_t s, const CovArgs& a) {
     const long ntiles = a.symmetric ? (long)TI * (TI + 1) / 2 : (long)TI * TJ;
     const int vec_ok = aligned16(a.K) && (a.ldk % 2 == 0) && (a.strideK % 2 == 0);
     static const int stream_min = [] { const char* e = getenv("MFGP_COV_STREAM_MIN_TILES"); return e ? atoi(e) : 1024; }();
-    if (ntiles * a.batch >= stream_min) return launch_cov_stream(s, a, TI, TJ, ntiles, vec_ok);
+    if (ntiles * (a.route_batch > 0 ? a.route_batch : a.batch) >= stream_min) return launch_cov_stream(s, a, TI, TJ, ntiles, vec_ok);
     const size_t smem = tile_smem_bytes(a.d);
     static SmemOptIn optin;
     if (!optin.ensure(cov_kernel, tile_smem_bytes(MFGP_MAX_D))) return -2;

@@ -21,6 +21,9 @@ struct CovArgs {
     double diag_add;                // added on global i == j (symmetric only)
     const double* diag_add_vec;     // optional per-batch value (overrides diag_add)
     int batch;
+    // problem count that picks the kernel (streaming or tiled; their results differ in the last bits): the whole call's
+    // count when a call is chunked over problems, so that a problem's result does not depend on its chunk.  0: batch
+    long route_batch;
 };
 int launch_cov(cudaStream_t s, const CovArgs& a);
 int launch_cov_diag(cudaStream_t s, const double* X, int N, int d, const double* theta, long theta_stride,

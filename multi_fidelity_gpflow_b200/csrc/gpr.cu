@@ -75,7 +75,7 @@ using Factor = GprFactor;
 // Assemble + factor + invert + a = W Y for `batch` problems.  theta_d/noise_d are device arrays.
 int gpr_factor(mfgp_handle* h, Scope& sc, const double* X, const double* Y, long ldy, int per_batch_cols, int b_off,
                int ycols, int N, int d, int P, int batch, const double* theta_d, const double* noise_d, int* info_vec,
-               Factor& f, bool want_W) {
+               Factor& f, bool want_W, long route_batch) {
     MFGP_TRY(gpr_factor_alloc(h, sc, N, P, batch, f, want_W));
     CovArgs c{};
     c.Xa = X; c.Na = N; c.Xb = X; c.Nb = N; c.d = d;
@@ -83,7 +83,7 @@ int gpr_factor(mfgp_handle* h, Scope& sc, const double* X, const double* Y, long
     c.K = f.K; c.ldk = f.ld; c.strideK = f.strideM;
     c.symmetric = 1; c.mirror = 0;
     c.diag_add = 0.0; c.diag_add_vec = noise_d;
-    c.batch = batch;
+    c.batch = batch; c.route_batch = route_batch;
     if (launch_cov(h->stream, c)) return mfgp_fail(h, MFGP_ERR_CUDA, "cov launch failed");
     return gpr_factor_from_K(h, Y, ldy, per_batch_cols, b_off, ycols, N, P, batch, info_vec, f);
 }
@@ -203,10 +203,11 @@ int gpr_build_G(mfgp_handle* h, Scope& sc, int N, int P, int batch, GprFactor& f
 
 int gpr_nlml_grad_device(mfgp_handle* h, Scope& sc, const double* X, const double* Y, long ldy, int per_batch_cols,
                          int b_off, int ycols, int N, int d, int P, int batch, const double* theta_d, const double* noise_d,
-                         double* nlml_d, double* grad_d, int* info_vec) {
+                         double* nlml_d, double* grad_d, int* info_vec, long route_batch) {
     cudaStream_t s = h->stream;
     Factor f;
-    MFGP_TRY(gpr_factor(h, sc, X, Y, ldy, per_batch_cols, b_off, ycols, N, d, P, batch, theta_d, noise_d, info_vec, f, grad_d != nullptr));
+    MFGP_TRY(gpr_factor(h, sc, X, Y, ldy, per_batch_cols, b_off, ycols, N, d, P, batch, theta_d, noise_d, info_vec, f, grad_d != nullptr,
+                        route_batch));
     gpr_nlml_from_factor(h, f, N, P, batch, nlml_d);
     if (!grad_d) return 0;
     MFGP_TRY(gpr_build_G(h, sc, N, P, batch, f));
@@ -296,7 +297,7 @@ int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, con
         c.Xa = q.X; c.Na = N; c.Xb = Xs; c.Nb = Ns; c.d = q.d;
         c.theta = th; c.theta_stride = np;
         c.K = Ks; c.ldk = lds; c.strideK = (long)N * lds;
-        c.batch = nb;
+        c.batch = nb; c.route_batch = q.B;
         if (launch_cov(s, c)) return mfgp_fail(h, MFGP_ERR_CUDA, "cov launch failed");
         if (launch_cov_diag(s, Xs, Ns, q.d, th, np, kss, Ns, nb)) return mfgp_fail(h, MFGP_ERR_CUDA, "cov_diag failed");
         GemmArgs g;  // A_s = W K_s

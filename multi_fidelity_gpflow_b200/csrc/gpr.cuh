@@ -6,7 +6,7 @@
 // ldy; ycols == 0: c = 0), theta_d[b, 2d+3], noise_d[b].  nlml_d [batch]; grad_d [batch, 2d+4] or nullptr.
 int gpr_nlml_grad_device(mfgp_handle* h, Scope& sc, const double* X, const double* Y, long ldy, int per_batch_cols,
                          int b_off, int ycols, int N, int d, int P, int batch, const double* theta_d, const double* noise_d,
-                         double* nlml_d, double* grad_d, int* info_vec);
+                         double* nlml_d, double* grad_d, int* info_vec, long route_batch = 0);
 int gpr_predict_device(mfgp_handle* h, Scope& sc, const double* X, const double* Y, int N, int d, int P,
                        const double* Xs, int Ns, const double* theta_d, const double* noise_d, double* mean_d,
                        double* var_d);
@@ -31,10 +31,11 @@ void gpr_nlml_from_factor(mfgp_handle* h, const GprFactor& f, int N, int P, int 
 // ... and f.G (lower tiles) <- alpha alpha^T - P K^-1.
 int gpr_build_G(mfgp_handle* h, Scope& sc, int N, int P, int batch, GprFactor& f);
 // Assemble (K1 + noise) -> factor -> (want_W) W = L^-1 -> a = W Y for `batch` problems, RHS columns as in
-// gpr_nlml_grad_device.  theta_d [batch, 2d+3] and noise_d [batch] are device arrays; buffers come from `sc`.
+// gpr_nlml_grad_device.  theta_d [batch, 2d+3] and noise_d [batch] are device arrays; buffers come from `sc`.  A call
+// chunked over problems passes its whole problem count as route_batch (CovArgs::route_batch).
 int gpr_factor(mfgp_handle* h, Scope& sc, const double* X, const double* Y, long ldy, int per_batch_cols, int b_off,
                int ycols, int N, int d, int P, int batch, const double* theta_d, const double* noise_d, int* info_vec,
-               GprFactor& f, bool want_W = true);
+               GprFactor& f, bool want_W = true, long route_batch = 0);
 
 // Cached posterior of B exact GPs that share X (mfgp_gpr_posterior_* in include/mfgp.h).  The storage format both predict
 // routes read; every pointer is device memory owned by the posterior.

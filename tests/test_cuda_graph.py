@@ -19,7 +19,7 @@ def h():
     return _lib.Handle(0)
 
 
-@pytest.mark.parametrize("m,d,N", [(1, 2, 30), (2, 3, 40), (3, 5, 150), (2, 10, 333)])
+@pytest.mark.parametrize("m,d,N", [(1, 2, 30), (2, 3, 40), (3, 5, 150), (2, 10, 333), (2, 32, 70)])
 def test_graph_cov_and_diag(h, m, d, N):
     rng = np.random.default_rng(m * 100 + d)
     X, _, gth = graph_problem(rng, N=N, d=d, m=m)
@@ -32,7 +32,7 @@ def test_graph_cov_and_diag(h, m, d, N):
     np.testing.assert_allclose(h.graph_cov_diag(X, m, gth), onp.graph_K_diag(X, gth, m), rtol=1e-14)
 
 
-@pytest.mark.parametrize("m,d,N,P", [(1, 2, 30, 1), (2, 3, 40, 2), (3, 5, 150, 4), (2, 6, 300, 1)])
+@pytest.mark.parametrize("m,d,N,P", [(1, 2, 30, 1), (2, 3, 40, 2), (3, 5, 150, 4), (2, 6, 300, 1), (2, 32, 80, 2)])
 def test_graph_gpr_nlml_grad(h, m, d, N, P):
     """Value 1e-9, gradient 1e-7 (north-star tolerances) against the torch oracle, which follows TensorFlow's semantics
     for the (asymmetric) graph covariance: lower-triangle Cholesky, symmetrised sensitivity, all N^2 entries."""

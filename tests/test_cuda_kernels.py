@@ -30,7 +30,8 @@ def rand_X(rng, n, d, frac_h=0.3, shuffle=True):
 
 
 # ------------------------------------------------------------------------------------ K1 cov
-@pytest.mark.parametrize("N,N2,d", [(53, 10, 5), (1, 1, 1), (64, 64, 3), (65, 129, 10), (300, 1164, 10), (200, 77, 16)])
+@pytest.mark.parametrize("N,N2,d", [(53, 10, 5), (1, 1, 1), (64, 64, 3), (65, 129, 10), (300, 1164, 10), (200, 77, 16),
+                                    (65, 129, 17), (70, 90, 32)])
 def test_cov_rect(h, N, N2, d):
     rng = np.random.default_rng(N * 1000 + N2)
     X, X2, th = rand_X(rng, N, d), rand_X(rng, N2, d), rand_theta(rng, d)
@@ -264,7 +265,8 @@ def test_batched_identity_sum_equals_shared_and_G1(h):
     assert abs(nlml.sum() - shared) / abs(shared) < 1e-10
 
 
-@pytest.mark.parametrize("N,d,frac", [(1, 1, 0.0), (2, 3, 1.0), (17, 2, 0.5), (64, 16, 0.3), (33, 7, 0.0)])
+@pytest.mark.parametrize("N,d,frac", [(1, 1, 0.0), (2, 3, 1.0), (17, 2, 0.5), (64, 16, 0.3), (33, 7, 0.0),
+                                      (64, 17, 0.3), (20, 32, 0.5)])  # d > 16: the blocked route
 def test_batched_small_edge_shapes(h, N, d, frac):
     rng = np.random.default_rng(N)
     X = rand_X(rng, N, d, frac)
@@ -341,10 +343,11 @@ def test_cov_streaming_kernel_full_size_properties(h):
     np.testing.assert_allclose(got, ref, rtol=1e-12, atol=1e-12)
 
 
-@pytest.mark.parametrize("d", [5, 7, 10])
+@pytest.mark.parametrize("d", [5, 7, 10, 17, 32])
 def test_cov_streaming_kernel_vs_oracle(h, d):
     """The streaming K1 path (taken from 1024 tiles on) element by element against the oracle: d = 5 and 10 are the compiled-in
-    dimensions, d = 7 the run-time one; ragged sizes, shuffled fidelities, rho != 1."""
+    dimensions, d = 7, 17 and 32 run-time ones (32 = MFGP_MAX_D, the largest shared-memory footprint); ragged sizes,
+    shuffled fidelities, rho != 1."""
     rng = np.random.default_rng(40 + d)
     X, X2, th = rand_X(rng, 2101, d), rand_X(rng, 2075, d), rand_theta(rng, d)
     np.testing.assert_allclose(h.cov(X, X2, th), onp.mf_K(X, X2, th), rtol=1e-12, atol=1e-14)
@@ -373,7 +376,7 @@ def test_cov_streaming_kernel_far_points_underflow(h):
     assert np.delete(K2.ravel(), i * K2.shape[1] + j).max() < 1e-300
 
 
-@pytest.mark.parametrize("N,d", [(53, 5), (130, 3), (700, 10)])
+@pytest.mark.parametrize("N,d", [(53, 5), (130, 3), (700, 10), (53, 17), (130, 32)])
 def test_cov_grad_contraction_vs_autograd(h, N, d):
     """mfgp_cov_grad: sum_ij G_ij dK_ij/dtheta for a symmetric G given by its lower triangle (the backward pass of K)."""
     import torch

@@ -13,7 +13,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("MFGP_LIB_PATH") or os.path.join(_HERE, "libmfgp.so")  # override: kernel-variant experiments only
+LIB_PATH = os.path.join(_HERE, "libmfgp.so")
 
 
 class MFGPError(RuntimeError):

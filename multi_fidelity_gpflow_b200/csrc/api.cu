@@ -1,7 +1,6 @@
 // api.cu -- extern "C" entry points of libmfgp.so (see include/mfgp.h for the contract).
 #include <cuda_runtime.h>
 
-#include <cstdlib>
 #include <vector>
 
 #include "chol.cuh"
@@ -34,11 +33,10 @@ int mfgp_create(int device, mfgp_handle** out) {
     cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking);
     {
         // the panel chain of potrf runs on the aux stream next to the trailing update's thousands of CTAs: highest priority,
-        // so that its few CTAs are scheduled first (MFGP_AUX_PRIORITY=0 restores the default for A/B timing)
+        // so that its few CTAs are scheduled first
         int lo = 0, hi = 0;
         cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        const char* e = getenv("MFGP_AUX_PRIORITY");
-        cudaStreamCreateWithPriority(&h->aux_stream, cudaStreamNonBlocking, (e && e[0] == '0') ? lo : hi);
+        cudaStreamCreateWithPriority(&h->aux_stream, cudaStreamNonBlocking, hi);
     }
     cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking);
     for (auto& e : h->ev) cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
@@ -185,8 +183,7 @@ static int gpr_common(mfgp_handle* h, const double* X, const double* Y, int N, i
     double* dn = sc.out(nlml, 1);
     double* dg = grad ? sc.out(grad, 2 * d + 4) : nullptr;
     if (!sc.ok) return sc.finish();
-    static const bool small_ok = [] { const char* e = getenv("MFGP_SHARED_SMALL"); return !(e && e[0] == '0'); }();
-    if (small_ok && N <= MFGP_SMALL_MAX_N && d <= MFGP_SMALL_MAX_D && P <= 8192) {
+    if (N <= MFGP_SMALL_MAX_N && d <= MFGP_SMALL_MAX_D && P <= 8192) {
         const int np = 2 * d + 3;
         double* th = sc.alloc<double>((size_t)P * np);
         double* nz = sc.alloc<double>(P);
@@ -298,10 +295,9 @@ int mfgp_gpr_batched_nlml_grad(mfgp_handle* h, const double* X, int N, int d, co
     cudaSetDevice(h->device);
     if (B == 0) return 0;
     {
-        static const bool pipe = [] { const char* e = getenv("MFGP_BATCH_PIPELINE"); return !(e && e[0] == '0'); }();
         const bool host_io = !mfgp_is_device_ptr(theta) && !mfgp_is_device_ptr(noise) && !mfgp_is_device_ptr(nlml) &&
                              (!grad || !mfgp_is_device_ptr(grad)) && (!info || !mfgp_is_device_ptr(info));
-        if (pipe && host_io && N <= MFGP_SMALL_MAX_N && d <= MFGP_SMALL_MAX_D && B >= 16L * h->sm_count * 12)
+        if (host_io && N <= MFGP_SMALL_MAX_N && d <= MFGP_SMALL_MAX_D && B >= 16L * h->sm_count * 12)
             return batched_small_pipelined(h, X, N, d, Y, ldy, ycols, B, theta, noise, nlml, grad, info);
     }
     Scope sc(h);

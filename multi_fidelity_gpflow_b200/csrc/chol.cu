@@ -13,8 +13,6 @@
 #include "chol.cuh"
 #include "common.cuh"
 
-#include <cstdlib>
-
 #include "gemm.cuh"
 #include "mathx.cuh"
 
@@ -44,11 +42,8 @@ constexpr int DTRI = DT * (DT + 1) / 2;     // 136 lower tiles
 // Warps of the diagonal-block kernel.  The kernel is latency bound (ncu, round 1: one warp per scheduler issues an
 // instruction every 6 cycles; 23 % of them are address arithmetic), so more warps per scheduler shorten it directly:
 // measured (profiles/r02_potrf_diag_warps.log) with 4 / 8 / 16 warps: potrf_inv of a 1024 block 924 / 802 / 792 us, potrf
-// N = 8192 19.2 / 20.3 / 20.3 TFLOP/s, N = 16 384 29.1 / 29.5 / 29.5 (cuSOLVER 29.5).  MFGP_DIAG_WARPS overrides at build time.
-#ifndef MFGP_DIAG_WARPS
-#define MFGP_DIAG_WARPS 8
-#endif
-constexpr int DIAG_WARPS = MFGP_DIAG_WARPS;
+// N = 8192 19.2 / 20.3 / 20.3 TFLOP/s, N = 16 384 29.1 / 29.5 / 29.5 (cuSOLVER 29.5).
+constexpr int DIAG_WARPS = 8;
 constexpr int DIAG_THREADS = 32 * DIAG_WARPS;
 
 // One CTA factors a 128x128 diagonal block on the FP64 tensor path and inverts the factor:
@@ -313,19 +308,13 @@ int launch_potrf(cudaStream_t s, const CholArgs& a) {
     // outer block: the trailing update is a rank-OB GEMM (OB / 128 panels of 128 columns); wider = fewer read-modify-write
     // passes over the trailing matrix and longer DMMA main loops per tile, at the price of more skinny inner updates on
     // the panel stream.  Measured on B200 (scripts/potrf_once.py): see DESIGN.md section 5.
-    static const int OB_env = [] {
-        const char* e = getenv("MFGP_POTRF_OB");
-        int v = e ? atoi(e) : 0;
-        return v < NB ? 0 : (v / NB) * NB;
-    }();
     // measured with the TMA-fed GEMM (profiles/r02_potrf_outer_block.log): N = 8192: 128 -> 18.0, 256 -> 19.2, 384 -> 18.6 TFLOP/s;
     // N = 16 384: 256 -> 27.7, 384 -> 28.6, 512 -> 29.0, 768 -> 28.9; N = 32 768: 512 -> 32.6, 768 -> 33.2, 1024 -> 33.4
-    const int OB = OB_env ? OB_env : (N <= 12288 ? 2 * NB : (N <= 24576 ? 4 * NB : 8 * NB));
+    const int OB = N <= 12288 ? 2 * NB : (N <= 24576 ? 4 * NB : 8 * NB);
     // Look-ahead: the latency-bound chain  diag -> panel -> inner update -> diag -> panel  runs on the aux stream and
     // overlaps the FP64-bound trailing update of the previous outer step; the main stream hands over the next
     // OB columns early.
-    static const int la_min = [] { const char* e = getenv("MFGP_POTRF_LA_MIN"); return e ? atoi(e) : 0; }();  // experiments
-    const bool la = a.aux != nullptr && a.ev != nullptr && N > 2 * OB && N > la_min;
+    const bool la = a.aux != nullptr && a.ev != nullptr && N > 2 * OB;
     cudaStream_t sp = la ? a.aux : s;
     if (la) {
         cudaEventRecord(a.ev[0], s);

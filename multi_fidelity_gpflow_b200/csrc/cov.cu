@@ -19,7 +19,6 @@
 #include "mathx.cuh"
 
 #include <cstdio>
-#include <cstdlib>
 
 namespace {
 
@@ -962,15 +961,13 @@ static int launch_cov_stream(cudaStream_t s, const CovArgs& a, int TI, int TJ, l
     const bool sym = a.symmetric != 0;
     // The tensor-path variant pays off when d + 2 fills whole k4 steps: measured at N = 32 768 (profiles/r02_cov_stream_variants.log)
     // d = 10: 2.49 ms against 2.58 ms for the DFMA kernel; d = 5 (K' = 7 padded to 8): 2.19 against 2.08; run-time d = 7: 2.67 / 2.47.
-    static const bool rect_dmma = [] { const char* e = getenv("MFGP_COV_RECT_DMMA"); return !(e && e[0] == '0'); }();  // experiments
-    const bool dm = !sym && rect_dmma && a.d == 10;
+    const bool dm = !sym && a.d == 10;
     const size_t smem = (size_t)(4 * S * (dm ? COV_PS : T) + (sym ? 8 * 32 * 18 : 0)) * sizeof(double);
     const int slots = sym ? 2 : 3;  // resident CTAs per SM (launch bounds of the two variants)
 
     // contiguous chunks of tiles per CTA; measured at N = 32 768: 8 chunks per resident CTA slot / <= 64 tiles 3930 GB/s,
     // 32 / <= 16 tiles 4057 GB/s (shorter tail, better balance between the two dies)
-    static const int cps = [] { const char* e = getenv("MFGP_COV_CHUNKS_PER_SLOT"); return e ? atoi(e) : 32; }();
-    static const int per_max = [] { const char* e = getenv("MFGP_COV_PER_MAX"); return e ? atoi(e) : 16; }();
+    constexpr int cps = 32, per_max = 16;
     long per = (q.total + (long)sms * slots * cps - 1) / ((long)sms * slots * cps);
     if (per < 1) per = 1;
     if (per > per_max) per = per_max;
@@ -982,10 +979,9 @@ static int launch_cov_stream(cudaStream_t s, const CovArgs& a, int TI, int TJ, l
         if (ok) kernel<<<(unsigned)grid, 256, smem, s>>>(q);
     };
     // the reference's data sets have d = 5 (HBS2021) and d = 10 (Goku): those dimensions are compiled in
-    static SmemOptIn o5s, o5r, o10s, o10r, o0s, o0r, o10d;
-    if (dm) go(cov_stream_rect_kernel<10>, o10d);
-    else if (a.d == 5) sym ? go(cov_stream_kernel<5, true>, o5s) : go(cov_stream_kernel<5, false>, o5r);
-    else if (a.d == 10) sym ? go(cov_stream_kernel<10, true>, o10s) : go(cov_stream_kernel<10, false>, o10r);
+    static SmemOptIn o5s, o5r, o10s, o10r, o0s, o0r;
+    if (a.d == 5) sym ? go(cov_stream_kernel<5, true>, o5s) : go(cov_stream_kernel<5, false>, o5r);
+    else if (a.d == 10) sym ? go(cov_stream_kernel<10, true>, o10s) : go(cov_stream_rect_kernel<10>, o10r);
     else sym ? go(cov_stream_kernel<0, true>, o0s) : go(cov_stream_kernel<0, false>, o0r);
     ok = ok && cudaGetLastError() == cudaSuccess;
     mfgp_ws_free(ws, s);
@@ -998,7 +994,7 @@ int launch_cov(cudaStream_t s, const CovArgs& a) {
     const int TI = (a.Na + COV_TILE - 1) / COV_TILE, TJ = (a.Nb + COV_TILE - 1) / COV_TILE;
     const long ntiles = a.symmetric ? (long)TI * (TI + 1) / 2 : (long)TI * TJ;
     const int vec_ok = aligned16(a.K) && (a.ldk % 2 == 0) && (a.strideK % 2 == 0);
-    static const int stream_min = [] { const char* e = getenv("MFGP_COV_STREAM_MIN_TILES"); return e ? atoi(e) : 1024; }();
+    constexpr long stream_min = 1024;
     if (ntiles * (a.route_batch > 0 ? a.route_batch : a.batch) >= stream_min) return launch_cov_stream(s, a, TI, TJ, ntiles, vec_ok);
     const size_t smem = tile_smem_bytes(a.d);
     static SmemOptIn optin;

@@ -22,7 +22,6 @@
 #include <cuda.h>  // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint, libcuda is not linked)
 
 #include <cstdint>
-#include <cstdlib>
 
 #include "mathx.cuh"
 
@@ -352,9 +351,7 @@ int launch_gemm(cudaStream_t s, const GemmArgs& a) {
     // tile config: 0 = 128x128 (1 CTA/SM; the only one safe for the in-place panel solve), 1 = 64x64,
     // 2 = 128x64 (2 CTAs/SM: one CTA's prologue/epilogue hides behind the other's main loop) -- the default.
     int cfg;
-    static const int cfg_env = [] { const char* e = getenv("MFGP_GEMM_CFG"); return e ? atoi(e) : -1; }();  // experiments only
     if (a.small_tiles >= 0) cfg = a.small_tiles;
-    else if (cfg_env >= 0) cfg = cfg_env;
     else {
         // 64x64 tiles when the grid would be small, or when 128-row tiles would pad M by > 12 % more than 64-row tiles do:
         // M = 300 (the SVGP inducing-point count) is 384 in 128-row tiles but 320 in 64-row tiles -- measured on the Goku

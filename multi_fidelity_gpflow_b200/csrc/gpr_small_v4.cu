@@ -36,17 +36,10 @@ namespace {
 // One CTA per SM; its warp count (= problems in flight per SM) is chosen at launch: as many as shared memory allows,
 // at most 12 (168 registers per thread).  One 12-warp CTA measured 8 % faster than 3 x 4 or 2 x 6 warps.
 constexpr int MAX_WPC = 12;
-// MFGP_V4_COOP_DIAG=1 selects a cooperative (shuffle-based) factorisation of the 8x8 diagonal tiles: 128 instead of 212
-// FP64-pipe instructions per tile, but 6 shuffles on the critical path of each of its 8 steps.  Measured: 766 k evals/s against
-// 790 k for the redundant per-lane version, so the default stays 0 (both pass the parity suite, same checksums).
+// The 8x8 diagonal tiles are factored per lane: a cooperative, shuffle-based factorisation measured 766 k against 790 k evals/s.
 // Tiles assembled per loop iteration (2 * n independent exp chains per lane).  Measured: 2 -> 791 k, 4 -> 783 k, 7 -> 760 k
 // evals/s: more chains only add register pressure at the 168-register cap.
-#ifndef MFGP_V4_TILES_PER_ITER
-#define MFGP_V4_TILES_PER_ITER 2
-#endif
-#ifndef MFGP_V4_COOP_DIAG
-#define MFGP_V4_COOP_DIAG 0
-#endif
+constexpr int TILES_PER_ITER = 2;
 constexpr double LOG2PI = 1.8378770664093454835606594728112;
 
 __device__ __forceinline__ double warp_sum(double v) {
@@ -194,7 +187,7 @@ __global__ void __launch_bounds__(MAX_WPC * 32, 1) gpr_small_v4_kernel(SmallArgs
 
         // ---- 1: covariance tiles --------------------------------------------------------------------
         {
-            constexpr int TPI = MFGP_V4_TILES_PER_ITER;  // tiles per iteration = 2 * TPI independent exp chains per lane
+            constexpr int TPI = TILES_PER_ITER;  // tiles per iteration = 2 * TPI independent exp chains per lane
             int i = 0, j = 0;
 #pragma unroll 1
             for (int s = 0; s < NTRI; s += TPI) {
@@ -278,65 +271,6 @@ __global__ void __launch_bounds__(MAX_WPC * 32, 1) gpr_small_v4_kernel(SmallArgs
                         acc[u][0] = c.x - acc[u][0];
                         acc[u][1] = c.y - acc[u][1];
                     }
-#if MFGP_V4_COOP_DIAG
-                // Diagonal tile, cooperatively in its C-fragment layout (lane (g, t) owns A[g][2t], A[g][2t+1] of the SYMMETRIC
-                // tile): right-looking 8-step Cholesky with the pivot / row / column values fetched by shuffles, and the inverse
-                // built alongside by forward elimination on an identity tile.  128 FP64-pipe instructions per tile instead of the
-                // 212 of the redundant per-lane factorisation, and the tile never leaves the registers.
-                __syncwarp();
-#pragma unroll
-                for (int u = 1; u < NT; ++u)
-                    if (u < cnt) *reinterpret_cast<double2*>(pk + u * 64 + cst) = make_double2(acc[u][0], acc[u][1]);
-                __syncwarp();
-#pragma unroll
-                for (int u = 1; u < NT; ++u)  // K-major fragments of the raw panel tiles (acc reused as storage)
-                    if (u < cnt) {
-                        acc[u][0] = pk[u * 64 + km0];
-                        acc[u][1] = pk[u * 64 + km1];
-                    }
-                {
-                    double a0 = acc[0][0], a1 = acc[0][1];
-                    double b0 = (g == 2 * t) ? 1.0 : 0.0, b1 = (g == 2 * t + 1) ? 1.0 : 0.0;
-                    double prod = 1.0;
-                    int hiv[8], hmin = 0x7fffffff, hmax = 0;
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) {
-                        const double aj = (j & 1) ? a1 : a0;  // the element of column j this lane may own
-                        const double piv = __shfl_sync(0xffffffffu, aj, j * 4 + (j >> 1));
-                        const double rv = __shfl_sync(0xffffffffu, aj, (lane & ~3) | (j >> 1));   // A[g][j]
-                        const double c0 = __shfl_sync(0xffffffffu, a0, j * 4 + t);               // A[j][2t]   = A[2t][j]
-                        const double c1 = __shfl_sync(0xffffffffu, a1, j * 4 + t);               // A[j][2t+1] = A[2t+1][j]
-                        const double r0 = __shfl_sync(0xffffffffu, b0, j * 4 + t);               // row j of the inverse so far
-                        const double r1 = __shfl_sync(0xffffffffu, b1, j * 4 + t);
-                        hiv[j] = __double2hiint(piv);
-                        hmin = min(hmin, hiv[j]);
-                        hmax = max(hmax, hiv[j]);
-                        prod *= piv;
-                        const double ri = frsqrt(piv);
-                        const double lg = rv * ri, lc0 = c0 * ri, lc1 = c1 * ri;
-                        a0 = fma(-lg, lc0, a0);  // rows / columns <= j turn into don't-care values that only feed each other
-                        a1 = fma(-lg, lc1, a1);
-                        const double s0 = r0 * ri, s1 = r1 * ri;
-                        const double le = (g > j) ? lg : 0.0;
-                        b0 = (g == j) ? s0 : fma(-le, s0, b0);
-                        b1 = (g == j) ? s1 : fma(-le, s1, b1);
-                    }
-                    if (hmin <= 0 || hmax >= 0x7ff00000) {  // a pivot <= 0 (or denormal), inf or NaN: report the first one
-                        if (!bad) {
-#pragma unroll
-                            for (int j = 7; j >= 0; --j)
-                                if (hiv[j] <= 0 || hiv[j] >= 0x7ff00000) bad = 8 * kb + j + 1;
-                        }
-                        prod = nan("");
-                    }
-                    {
-                        const int ph = __double2hiint(prod);
-                        lexp += ((ph >> 20) & 0x7ff) - 1023;
-                        lmant *= __hiloint2double((ph & 0x800fffff) | 0x3ff00000, __double2loint(prod));
-                    }
-                    *reinterpret_cast<double2*>(pk + cst) = make_double2(b0, b1);  // the diagonal slot keeps inv(L_kk)
-                }
-#else
                 __syncwarp();
 #pragma unroll
                 for (int u = 0; u < NT; ++u)
@@ -406,7 +340,6 @@ __global__ void __launch_bounds__(MAX_WPC * 32, 1) gpr_small_v4_kernel(SmallArgs
                         for (int i = 0; i < 8; ++i) pk[tile_off(i, c)] = w[i];
                     }
                 }
-#endif
                 __syncwarp();
                 // panel: L_ik = A_ik inv(L_kk)^T
                 {

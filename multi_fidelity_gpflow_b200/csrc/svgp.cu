@@ -18,8 +18,6 @@
 // Every O(M^2 B) / O(M^3) product is a DMMA GEMM (gemm.cu); the rest are streaming kernels.
 #include "svgp.cuh"
 
-#include <cstdlib>
-
 #include "chol.cuh"
 #include "cov.cuh"
 #include "gemm.cuh"
@@ -792,8 +790,7 @@ extern "C" int mfgp_svgp_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const do
         // step is not capturable the loop falls back to eager launches.
         rc = one_step();
         int done = 1;
-        static const bool use_graph = [] { const char* e = getenv("MFGP_SVGP_GRAPH"); return !(e && e[0] == '0'); }();
-        if (rc == 0 && nsteps > 2 && use_graph) {
+        if (rc == 0 && nsteps > 2) {
             cudaGraph_t graph = nullptr;
             cudaGraphExec_t exec = nullptr;
             wsg.fix();  // no allocation nodes in the graph (if the arena cannot be had the capture still works, see below)

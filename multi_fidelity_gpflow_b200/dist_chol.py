@@ -22,7 +22,6 @@ lives in tests/, the product path has no CPU fallback."""
 from __future__ import annotations
 
 import math
-import os
 
 import numpy as np
 
@@ -117,8 +116,6 @@ class GpuOps:
     def peer_buffers(self, count, nb, group):
         """`count` symmetric nb x nb blocks (torch symmetric memory: every rank's allocation is mapped into every peer
         over NVLink).  Returns (local [count, nb, nb], handle, [peer views]) or None when peer memory is unavailable."""
-        if os.environ.get("MFGP_DIST_P2P") == "0":
-            return None
         try:
             import torch.distributed as dist
             import torch.distributed._symmetric_memory as symm
@@ -292,20 +289,12 @@ def distributed_gpr_nlml(handle_or_ops, X, Y, theta, noise, nbd=1024, group=None
         cache["Xrow"] = torch.empty(nb, N, dtype=torch.float64, device=dev)
         cache["tmpb"] = torch.empty(nb, nb, dtype=torch.float64, device=dev)
     if lookahead:
-        s_main, s_pan, s_crit = cache["s_main"], cache["s_pan"], cache["s_crit"]
         # One communicator: NCCL executes its collectives in issue order (W_k, blk_k, panel k, W_k+1, ...), which is also
         # the dependency order.  A second communicator for the small broadcasts was measured 10x SLOWER on 4 GPUs (two NCCL
-        # kernels of different communicators spin against each other); MFGP_DIST_TWO_COMMS=1 re-enables it for experiments.
-        if os.environ.get("MFGP_DIST_TWO_COMMS") == "1":
-            if cache.get("crit_group") is None:
-                ranks = dist.get_process_group_ranks(group if group is not None else dist.group.WORLD)
-                cache["crit_group"] = dist.new_group(ranks=ranks)
-            crit_group = cache["crit_group"]
-        else:
-            crit_group = group
-    else:  # reference schedule: the same steps, one stream, one communicator
+        # kernels of different communicators spin against each other).
+        s_main, s_pan, s_crit = cache["s_main"], cache["s_pan"], cache["s_crit"]
+    else:  # reference schedule: the same steps, one stream
         s_main = s_pan = s_crit = cache["s_main"]
-        crit_group = group
 
     # ---- assembly (no communication) -------------------------------------------------------------------
     cols = cache["cols"]
@@ -389,7 +378,7 @@ def distributed_gpr_nlml(handle_or_ops, X, Y, theta, noise, nbd=1024, group=None
                 else:
                     ops.peer_wait(p2p["W"][1], rank_of(k, k), 0)
             else:
-                dist.broadcast(Wk, src=rank_of(k, k), group=crit_group)
+                dist.broadcast(Wk, src=rank_of(k, k), group=group)
         ev_W[k] = ops.record(s_crit, f"W{k}") if hasattr(ops, "timeline") else ops.record(s_crit)
         if k + 1 >= nblk:
             return
@@ -407,7 +396,7 @@ def distributed_gpr_nlml(handle_or_ops, X, Y, theta, noise, nbd=1024, group=None
                 else:
                     ops.peer_wait(p2p["B"][1], src, 1)
             else:
-                dist.broadcast(blk, src=src, group=crit_group)
+                dist.broadcast(blk, src=src, group=group)
             ev_blk[k] = ops.record(s_crit, f"blk{k}") if hasattr(ops, "timeline") else ops.record(s_crit)
             if rank == rank_of(k + 1, k + 1):
                 D = cols[k + 1][:nb]

@@ -25,7 +25,7 @@ def timed(steps):
 steps = 20
 long_steps = int(sys.argv[2]) if len(sys.argv) > 2 else 0
 t20 = timed(steps)
-print(f"{which}: {t20 / steps * 1e3:.3f} ms per step  (MFGP_GEMM_CFG={os.environ.get('MFGP_GEMM_CFG')})  loss {mdl.loss_history[-1]:.6f}")
+print(f"{which}: {t20 / steps * 1e3:.3f} ms per step  loss {mdl.loss_history[-1]:.6f}")
 if long_steps > steps:
     # the per-call cost (parameters + Adam moments host<->device, the eager first step, graph capture) is the same for
     # both lengths: the difference isolates the replayed step

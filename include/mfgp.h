@@ -214,6 +214,16 @@ int mfgp_svgp_posterior_create(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const d
                                mfgp_svgp_posterior** out);
 int mfgp_svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns,
                                 double* mean, double* var);
+/* mfgp_svgp_posterior_predict_grad: mean [Ns, P] and var [Ns, P] as mfgp_svgp_posterior_predict, and their gradients
+ * with respect to the d continuous coordinates of each test point, dmean [Ns, P, d] = d mean / d Xs[s, j] and
+ * dvar [Ns, P, d] = d var / d Xs[s, j] (the fidelity column has no gradient).  All four outputs are required.  A test row
+ * with fidelity not in {0, 1} has zero gradients, dead inducing points contribute nothing, and a failed latent gives NaN
+ * in its outputs (with W in all of them).  Pointers, async mode, the device check and Ns == 0 as for _predict.  The
+ * fused route (M <= 64, d <= 16) is one kernel, svgp_posterior_predict_grad_kernel, plus the two mixes when W is given;
+ * the blocked route adds R = V - Lq U and beta = Wm^T R (two batched GEMMs), alpha = Wm^T q_mu and posterior_dx_kernel to
+ * the _predict pipeline.  A point's results do not depend on the other points of the call. */
+int mfgp_svgp_posterior_predict_grad(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns,
+                                     double* mean, double* var, double* dmean, double* dvar);
 int mfgp_svgp_posterior_destroy(mfgp_svgp_posterior* post);
 
 /* Training loop on the device for the SVGP models (SURVEY 8(f) rank 1): the optimize() loops of mfgpflow/singlebin_svgp.py:

@@ -63,6 +63,7 @@ def _load():
         "mfgp_svgp_predict": ([vp, vp, vp, i, vp, vp, vp, vp, vp, vp, vp], i),
         "mfgp_svgp_posterior_create": ([vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(vp)], i),
         "mfgp_svgp_posterior_predict": ([vp, vp, vp, i, vp, vp], i),
+        "mfgp_svgp_posterior_predict_grad": ([vp, vp, vp, i, vp, vp, vp, vp], i),
         "mfgp_svgp_posterior_destroy": ([vp], i),
         "mfgp_svgp_adam": ([vp, vp, vp, vp, i, vp, vp, vp, vp, vp, d, d, d, i, vp, vp], i),
         "mfgp_svgp_flat_size": ([vp, i], l),
@@ -93,7 +94,8 @@ EXPORTED_SYMBOLS = [
     "mfgp_gpr_posterior_create", "mfgp_gpr_posterior_predict", "mfgp_gpr_posterior_predict_grad",
     "mfgp_gpr_posterior_destroy",
     "mfgp_graph_nparams", "mfgp_graph_cov", "mfgp_graph_cov_diag", "mfgp_graph_gpr_nlml_grad", "mfgp_svgp_elbo_grad", "mfgp_svgp_elbo_grad_v", "mfgp_svgp_predict",
-    "mfgp_svgp_posterior_create", "mfgp_svgp_posterior_predict", "mfgp_svgp_posterior_destroy", "mfgp_svgp_adam",
+    "mfgp_svgp_posterior_create", "mfgp_svgp_posterior_predict", "mfgp_svgp_posterior_predict_grad",
+    "mfgp_svgp_posterior_destroy", "mfgp_svgp_adam",
     "mfgp_svgp_flat_size", "mfgp_svgp_constrain", "mfgp_svgp_elbo_grad_flat", "mfgp_svgp_adam_update", "mfgp_gemm",
     "mfgp_potrf", "mfgp_potrf_inv", "mfgp_tall_skinny_update", "mfgp_peer_store", "mfgp_graph_mem_trim", "mfgp_workspace", "mfgp_fp64_peak",
 ]
@@ -598,6 +600,20 @@ class SvgpPosterior(_Posterior):
         self.handle._check(_lib.mfgp_svgp_posterior_predict(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean), _ptr(var)),
                            "mfgp_svgp_posterior_predict")
         return mean, var
+
+    def predict_grad(self, Xs, mean=None, var=None, dmean=None, dvar=None):
+        """predict() plus the gradients with respect to the d continuous coordinates of each test point:
+        (mean [Ns, P], var [Ns, P], dmean [Ns, P, d], dvar [Ns, P, d]).  Host arrays or device tensors."""
+        Xs = self._xs(Xs)
+        Ns = Xs.shape[0]
+        mean = np.empty((Ns, self.P)) if mean is None else mean
+        var = np.empty((Ns, self.P)) if var is None else var
+        dmean = np.empty((Ns, self.P, self.d)) if dmean is None else dmean
+        dvar = np.empty((Ns, self.P, self.d)) if dvar is None else dvar
+        self.handle._check(_lib.mfgp_svgp_posterior_predict_grad(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean),
+                                                                 _ptr(var), _ptr(dmean), _ptr(dvar)),
+                           "mfgp_svgp_posterior_predict_grad")
+        return mean, var, dmean, dvar
 
 
 _default = {}

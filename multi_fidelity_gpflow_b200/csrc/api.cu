@@ -553,31 +553,57 @@ int mfgp_svgp_posterior_create(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const d
     return publish_posterior(h, rc, info, mem, SvgpPosteriorData{L, M, P, d, ld, dZ, dT, dW, dWm, dLq, dQ}, out);
 }
 
-int mfgp_svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns, double* mean,
-                                double* var) {
-    if (const int rc = posterior_predict_prologue(h, post, Xs, Ns, mean, var, "mfgp_svgp_posterior_predict"); rc <= 0)
-        return rc;
+}  // extern "C"
+
+namespace {
+// mfgp_svgp_posterior_predict and _predict_grad: one body, the gradients when dmean != NULL.  With W the fused route
+// writes the latents to [L][Ns] (and [L][Ns][d]) scratch and the mix kernels form the outputs.
+int svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns, double* mean,
+                           double* var, double* dmean, double* dvar, const char* name) {
+    if (const int rc = posterior_predict_prologue(h, post, Xs, Ns, mean, var, name); rc <= 0) return rc;
     const SvgpPosteriorData& q = post->q;
     Scope sc(h);
     const double* dXs = sc.in(Xs, (size_t)Ns * (q.d + 1));
     double* dm = sc.out(mean, (size_t)Ns * q.P);
     double* dv = sc.out(var, (size_t)Ns * q.P);
+    double* ddm = dmean ? sc.out(dmean, (size_t)Ns * q.P * q.d) : nullptr;
+    double* ddv = dmean ? sc.out(dvar, (size_t)Ns * q.P * q.d) : nullptr;
     if (!sc.ok) return sc.finish();
     if (svgp_posterior_fused_ok(q.L, q.M, q.d)) {
         if (!q.W) {
-            if (svgp_posterior_predict_fused(h->stream, q, dXs, Ns, dm, dv, 1, q.P))
-                return mfgp_fail(h, MFGP_ERR_CUDA, "mfgp_svgp_posterior_predict: fused kernel launch failed");
+            if (svgp_posterior_predict_fused(h->stream, q, dXs, Ns, dm, dv, 1, q.P, ddm, ddv))
+                return mfgp_fail(h, MFGP_ERR_CUDA, "%s: fused kernel launch failed", name);
         } else {
-            double* g = sc.alloc<double>((size_t)2 * q.L * Ns);  // latent marginals [L][Ns], mean then var
+            const size_t lat = (size_t)q.L * Ns;
+            double* g = sc.alloc<double>(2 * lat);  // latent marginals [L][Ns], mean then var
+            double* gd = dmean ? sc.alloc<double>(2 * lat * q.d) : nullptr;  // latent gradients [L][Ns][d], mean then var
             if (!sc.ok) return sc.finish();
-            if (svgp_posterior_predict_fused(h->stream, q, dXs, Ns, g, g + (size_t)q.L * Ns, Ns, 1) ||
-                launch_svgp_mix(h->stream, g, g + (size_t)q.L * Ns, q.L, Ns, q.P, q.W, dm, dv))
-                return mfgp_fail(h, MFGP_ERR_CUDA, "mfgp_svgp_posterior_predict: fused kernel launch failed");
+            if (svgp_posterior_predict_fused(h->stream, q, dXs, Ns, g, g + lat, Ns, 1, gd, dmean ? gd + lat * q.d : nullptr) ||
+                launch_svgp_mix(h->stream, g, g + lat, q.L, Ns, q.P, q.W, dm, dv) ||
+                (dmean && launch_svgp_grad_mix(h->stream, gd, gd + lat * q.d, q.L, Ns, q.P, q.d, q.W, ddm, ddv)))
+                return mfgp_fail(h, MFGP_ERR_CUDA, "%s: fused kernel launch failed", name);
         }
     } else {
-        MFGP_TRY(svgp_posterior_predict_blocked(h, q, dXs, Ns, dm, dv));
+        MFGP_TRY(svgp_posterior_predict_blocked(h, q, dXs, Ns, dm, dv, ddm, ddv));
     }
     return sc.finish();
+}
+}  // namespace
+
+extern "C" {
+
+int mfgp_svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns, double* mean,
+                                double* var) {
+    return svgp_posterior_predict(h, post, Xs, Ns, mean, var, nullptr, nullptr, "mfgp_svgp_posterior_predict");
+}
+
+int mfgp_svgp_posterior_predict_grad(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns,
+                                     double* mean, double* var, double* dmean, double* dvar) {
+    if (!dmean || !dvar) {
+        CHECK_H(h);
+        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_posterior_predict_grad: bad argument (dmean and dvar are required)");
+    }
+    return svgp_posterior_predict(h, post, Xs, Ns, mean, var, dmean, dvar, "mfgp_svgp_posterior_predict_grad");
 }
 
 int mfgp_svgp_posterior_destroy(mfgp_svgp_posterior* post) {

@@ -32,6 +32,12 @@
 // svgp_posterior_predict_kernel (mfgp_svgp_posterior_predict): the inducing points Z in the place of X, one latent per
 // blockIdx.y, W = Wm.  U = Lq^T V (upper_tri_product with F = Lq) never leaves the accumulators: sum U^2 is lane-local.
 // var = k_ss - sum V^2 + sum U^2, mean = V^T q_mu.
+//
+// svgp_posterior_predict_grad_kernel (mfgp_svgp_posterior_predict_grad): predict's values, computed as predict computes
+// them, plus the input gradients.  d var / dx*_j = -2 beta . gk with beta = Wm^T (V - Lq U): U stays in a fragment row,
+// Lq U runs over the tiles m <= n reading predict's Lt staging in the other direction (lower_tri_product), and beta is
+// upper_tri_product with F = Wm.  d mean / dx*_j = alpha . gk with alpha = Wm^T q_mu, formed once per CTA.  gk as in the
+// exact grad kernel.
 #include <cmath>
 #include <type_traits>
 
@@ -65,6 +71,10 @@ struct SvgpFusedArgs {
     double* var;
     long ls, ns;  // output of (latent l, point n) at l * ls + n * ns
 };
+struct SvgpFusedGradArgs : SvgpFusedArgs {
+    double* dmean;  // gradients of (latent l, point n) at (l * ls + n * ns) * d + j
+    double* dvar;
+};
 
 // Shared-memory pitches (doubles).  W rows: WP = NP + 4 (= 4 or 12 mod 16) puts the B-fragment loads W[8i+g][4k+t] of a
 // half-warp into 16 different bank pairs; a rows: AP = round_up(P, 8) + 2 (2 mod 8) does the same for a[8i+2t+e][8j+g].
@@ -88,6 +98,11 @@ size_t fused_grad_smem_bytes(int NT, int d, int P) {
 size_t svgp_fused_smem_bytes(int NT, int d) {
     const int NP = 8 * NT;
     return sizeof(double) * (2 * (size_t)NP * w_pitch(NP) + NP + (size_t)(2 * d + 4) * NP + (size_t)PW * 8 * rec_len(d));
+}
+// SVGP grad kernel: a third factor copy (Wm transposed), alpha next to q_mu, and the 2d inverse lengthscales
+size_t svgp_fused_grad_smem_bytes(int NT, int d) {
+    const int NP = 8 * NT;
+    return svgp_fused_smem_bytes(NT, d) + sizeof(double) * ((size_t)NP * w_pitch(NP) + NP + 2 * d);
 }
 
 // C-fragment order of the training index: slot 4k + t (k-step k, lane t) holds
@@ -165,6 +180,21 @@ __device__ __forceinline__ void upper_tri_product(double& c0, double& c1, const 
     for (int i2 = i; i2 < NT; ++i2) {
         dmma(c0, c1, v[2 * i2], fr[8 * i2]);
         dmma(c0, c1, v[2 * i2 + 1], fr[8 * i2 + 4]);
+    }
+}
+
+// (c0, c1) = slots 2i, 2i + 1 of F u = u^T F^T over the tiles i2 <= i, from the same Ft staging as upper_tri_product read
+// in the other direction: F[n][m] = Ft[m][perm_slot(n)], so one staged copy serves F^T u and F u.
+template <int NT>
+__device__ __forceinline__ void lower_tri_product(double& c0, double& c1, const double (&u)[2 * NT], const double* Ft, int i,
+                                                  int g, int t) {
+    constexpr int WP = w_pitch(8 * NT);
+    c0 = c1 = 0.0;
+    const double* fr = Ft + (2 * t) * WP + perm_slot(8 * i + g);
+#pragma unroll
+    for (int i2 = 0; i2 <= i; ++i2) {
+        dmma(c0, c1, u[2 * i2], fr[(8 * i2) * WP]);
+        dmma(c0, c1, u[2 * i2 + 1], fr[(8 * i2 + 1) * WP]);
     }
 }
 
@@ -609,6 +639,210 @@ __global__ void __launch_bounds__(PW * 32) svgp_posterior_predict_kernel(SvgpFus
     }
 }
 
+template <int NT>
+__global__ void __launch_bounds__(PW * 32, 1) svgp_posterior_predict_grad_kernel(SvgpFusedGradArgs p) {
+    constexpr int NP = 8 * NT, WP = w_pitch(NP);
+    extern __shared__ __align__(16) double sm[];
+    __shared__ __align__(16) double etab[512];
+    const SvgpPosteriorData& q = p.q;
+    const int M = q.M, d = q.d, S1 = rec_len(d);
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
+    const long l = blockIdx.y;
+    const double* __restrict__ th = q.theta + l * (2 * d + 3);
+    double* Ws = sm;                            // [NP][WP]  Wm, as svgp_posterior_predict_kernel stages it
+    double* Lt = Ws + NP * WP;                  // [NP][WP]  Lt[c][slot] = Lq[perm_n(slot)][c], as predict
+    double* Wt = Lt + NP * WP;                  // [NP][WP]  Wt[c][slot] = Wm[perm_n(slot)][c]
+    double* Qs = Wt + NP * WP;                  // [NP]      q_mu[:, l]
+    double* Al = Qs + NP;                       // [NP]      alpha = Wm^T q_mu[:, l]
+    double* Xt = Al + NP;                       // [2d+4][NP]  inducing points, k-major
+    double* Il = Xt + (2 * d + 4) * NP;         // [2d]  -1/ls_L, -1/ls_delta
+    double* Xw = Il + 2 * d + warp * 8 * S1;    // [8][S1]  this warp's test points
+    fexp512_table_fill(etab, tid, blockDim.x);
+    const double hlL = 0.5 * log(th[1 + d]), hlD = 0.5 * log(th[2 + 2 * d]);
+
+    // ---- stage the latent: Wm (twice), Lq^T (lower triangles; zero elsewhere), q_mu, scaled inducing points; then alpha
+    {
+        const double* __restrict__ Wg = q.Wm + l * M * q.ld;
+        const double* __restrict__ Lg = q.Lq + l * M * q.ld;
+        for (int idx = tid; idx < NP * NP; idx += blockDim.x) {
+            const int r = idx / NP, c = idx - r * NP, m = perm_n(c);
+            Ws[r * WP + c] = (r < M && c <= r) ? Wg[(long)r * q.ld + c] : 0.0;
+            Lt[r * WP + c] = (m < M && r <= m) ? Lg[(long)m * q.ld + r] : 0.0;
+            Wt[r * WP + c] = (m < M && r <= m) ? Wg[(long)m * q.ld + r] : 0.0;
+        }
+        for (int m = tid; m < NP; m += blockDim.x) Qs[m] = m < M ? q.q_mu[(long)m * q.L + l] : 0.0;
+        for (int n = tid; n < NP; n += blockDim.x) prescale_point(q.Z + (long)n * (d + 1), n < M, d, th, hlL, hlD, Xt + n, NP);
+        for (int k = tid; k < d; k += blockDim.x) {
+            Il[k] = -1.0 / th[1 + k];
+            Il[d + k] = -1.0 / th[2 + d + k];
+        }
+    }
+    __syncthreads();
+    for (int n = tid; n < NP; n += blockDim.x) {
+        double s = 0.0;
+        for (int m = n; m < M; ++m) s = fma(Ws[m * WP + n], Qs[m], s);
+        Al[n] = s;
+    }
+    __syncthreads();
+    const double rho = th[0], vL = th[1 + d], vD = th[2 + 2 * d];
+    const double kss_hf = __dadd_rn(__dmul_rn(vL, __dmul_rn(rho, rho)), vD);  // K_diag at fidelity 1, as cov_diag_kernel
+
+    for (int grp = warp; grp < p.gpc; grp += PW) {
+        const long pt0 = ((long)blockIdx.x * p.gpc + grp) * 8;
+        if (pt0 >= p.Ns) break;
+        if (lane < 8) {
+            const long pt = pt0 + lane;
+            const bool exists = pt < p.Ns;
+            double* rec = Xw + lane * S1;
+            prescale_point(p.Xs + (exists ? pt : 0) * (d + 1), exists, d, th, hlL, hlD, rec, 1);
+            rec[2 * d + 4] = rec[2 * d + 3] != 0.0 ? kss_hf : (rec[2 * d + 2] != 0.0 ? vL : 0.0);
+        }
+        __syncwarp();
+        const double* xg = Xw + g * S1;
+        const double sg = xg[2 * d + 2], hg = xg[2 * d + 3];
+        const bool anyh = __any_sync(0xffffffffu, hg != 0.0);
+
+        // ---- the two parts of K_s^T in predict's A-fragment layout: kL[k], kD[k] at m = 4k + t
+        double kL[2 * NT], kD[2 * NT];
+        {
+            const double* xe = Xt + 2 * d * NP + t;
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) kL[k] = xe[4 * k] + xg[2 * d];
+            for (int c = 0; c < d; ++c) {
+                const double xc = xg[c];
+                const double* xr = Xt + c * NP + t;
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k) kL[k] = fma(xr[4 * k], xc, kL[k]);
+            }
+            const double* sr = Xt + (2 * d + 2) * NP + t;
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) kL[k] = fexp512(kL[k], etab) * (sr[4 * k] * sg);
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) kD[k] = 0.0;
+            if (anyh) {
+                const double* xf = Xt + (2 * d + 1) * NP + t;
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k) kD[k] = xf[4 * k] + xg[2 * d + 1];
+                for (int c = 0; c < d; ++c) {
+                    const double xc = xg[d + c];
+                    const double* xr = Xt + (d + c) * NP + t;
+#pragma unroll
+                    for (int k = 0; k < 2 * NT; ++k) kD[k] = fma(xr[4 * k], xc, kD[k]);
+                }
+                const double* hr = Xt + (2 * d + 3) * NP + t;
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k) kD[k] = hr[4 * k] * hg != 0.0 ? fexp512(kD[k], etab) : 0.0;
+            }
+        }
+
+        // ---- V^T = K_s^T Wm^T over the lower-triangular tiles: v[2i + e] = V^T[g][8i + 2t + e]
+        double v[2 * NT];
+        {
+            double ks[2 * NT];
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) ks[k] = __dadd_rn(kL[k], kD[k]);  // predict's K_s, not contracted
+            lower_tri_v<NT>(v, ks, Ws, g, t);
+        }
+
+        // ---- U^T = V^T Lq over the tiles m >= n; var = k_ss - sum V^2 + sum U^2, mean = V^T q_mu  (as predict)
+        double u[2 * NT];
+        double ss = sum_sq<NT>(v);
+        double su = 0.0;
+#pragma unroll
+        for (int i = 0; i < NT; ++i) {
+            upper_tri_product<NT>(u[2 * i], u[2 * i + 1], v, Lt, i, g, t);
+            su = fma(u[2 * i + 1], u[2 * i + 1], fma(u[2 * i], u[2 * i], su));
+        }
+        ss = quad_sum(ss);
+        su = quad_sum(su);
+        double m = 0.0;
+        {
+            const double* qr = Qs + 2 * t;
+#pragma unroll
+            for (int i = 0; i < NT; ++i) m = fma(v[2 * i + 1], qr[8 * i + 1], fma(v[2 * i], qr[8 * i], m));
+        }
+        m = quad_sum(m);
+        const long ptg = pt0 + g;
+        const bool live = ptg < p.Ns;
+        if (t == 0 && live) {
+            const long o = l * p.ls + ptg * p.ns;
+            p.mean[o] = m;
+            p.var[o] = xg[2 * d + 4] - ss + su;
+        }
+
+        // ---- r = V - Lq U over the tiles m <= n (Lt read transposed), then beta^T = r^T Wm over the tiles m >= n:
+        //      be[2i + e] = beta[8i + 2t + e]
+        {
+            double r[2 * NT];
+#pragma unroll
+            for (int i = 0; i < NT; ++i) {
+                double c0, c1;
+                lower_tri_product<NT>(c0, c1, u, Lt, i, g, t);
+                r[2 * i] = v[2 * i] - c0;
+                r[2 * i + 1] = v[2 * i + 1] - c1;
+            }
+#pragma unroll
+            for (int i = 0; i < NT; ++i) upper_tri_product<NT>(v[2 * i], v[2 * i + 1], r, Wt, i, g, t);
+        }
+        const double(&be)[2 * NT] = v;
+
+        // ---- kL, kD to the C-fragment order: slot 2i + e of lane t <- m = 8i + 2t + e, which lane (2t + e) & 3 of the
+        //      quad holds in slot 2i + t / 2
+        {
+            const int src0 = (lane & ~3) | ((2 * t) & 3), src1 = (lane & ~3) | ((2 * t + 1) & 3);
+            const bool hi = t >= 2;
+#pragma unroll
+            for (int i = 0; i < NT; ++i) {
+                const double a0 = __shfl_sync(0xffffffffu, kL[2 * i], src0), b0 = __shfl_sync(0xffffffffu, kL[2 * i + 1], src0);
+                const double a1 = __shfl_sync(0xffffffffu, kL[2 * i], src1), b1 = __shfl_sync(0xffffffffu, kL[2 * i + 1], src1);
+                kL[2 * i] = hi ? b0 : a0;
+                kL[2 * i + 1] = hi ? b1 : a1;
+            }
+            if (anyh) {
+#pragma unroll
+                for (int i = 0; i < NT; ++i) {
+                    const double a0 = __shfl_sync(0xffffffffu, kD[2 * i], src0), b0 = __shfl_sync(0xffffffffu, kD[2 * i + 1], src0);
+                    const double a1 = __shfl_sync(0xffffffffu, kD[2 * i], src1), b1 = __shfl_sync(0xffffffffu, kD[2 * i + 1], src1);
+                    kD[2 * i] = hi ? b0 : a0;
+                    kD[2 * i + 1] = hi ? b1 : a1;
+                }
+            }
+        }
+
+        // ---- per coordinate j: gk = dk_s/dx*_j, dvar_j = -2 beta . gk, dmean_j = alpha . gk
+        const double* ar = Al + 2 * t;
+        const long od = (l * p.ls + ptg * p.ns) * d;
+        for (int j = 0; j < d; ++j) {
+            double gk[2 * NT];
+            {
+                const double uj = xg[j], cL = Il[j];
+                const double* ur = Xt + j * NP + 2 * t;
+#pragma unroll
+                for (int k = 0; k < 2 * NT; ++k) gk[k] = kL[k] * (uj - ur[slot_off(k)]) * cL;
+                if (anyh) {
+                    const double wj = xg[d + j], cD = Il[d + j];
+                    const double* wr = Xt + (d + j) * NP + 2 * t;
+#pragma unroll
+                    for (int k = 0; k < 2 * NT; ++k) gk[k] = fma(kD[k] * (wj - wr[slot_off(k)]), cD, gk[k]);
+                }
+            }
+            double sv = 0.0, sa = 0.0;
+#pragma unroll
+            for (int i = 0; i < NT; ++i) {
+                sv = fma(be[2 * i + 1], gk[2 * i + 1], fma(be[2 * i], gk[2 * i], sv));
+                sa = fma(gk[2 * i + 1], ar[8 * i + 1], fma(gk[2 * i], ar[8 * i], sa));
+            }
+            sv = quad_sum(sv);
+            sa = quad_sum(sa);
+            if (t == 0 && live) {
+                p.dmean[od + j] = sa;
+                p.dvar[od + j] = -2.0 * sv;
+            }
+        }
+        __syncwarp();
+    }
+}
+
 // Input gradient of the blocked route (launch_posterior_dx): one CTA per (tile of TS test points, chunk of PC columns,
 // problem), walking the training points in tiles of TN.  Per tile it evaluates kL and kD from the scaled inputs (as K5
 // recomputes dK: nothing N x Ns is stored), forms G[j][s][n] = dk_sn/dx_sj in shared memory and adds G alpha (thread =
@@ -808,12 +1042,19 @@ bool svgp_posterior_fused_ok(int L, int M, int d) {
 }
 
 int svgp_posterior_predict_fused(cudaStream_t s, const SvgpPosteriorData& q, const double* Xs, int Ns, double* mean,
-                                 double* var, long ls, long ns) {
+                                 double* var, long ls, long ns, double* dmean, double* dvar) {
     if (!svgp_posterior_fused_ok(q.L, q.M, q.d)) return -1;
     if (Ns <= 0) return 0;
     const int NT = (q.M + 7) / 8;
-    const size_t smem = svgp_fused_smem_bytes(NT, q.d);
     const SvgpFusedArgs a{q, Xs, Ns, groups_per_cta(Ns, q.L), mean, var, ls, ns};
+    if (dmean) {
+        const SvgpFusedGradArgs ag{a, dmean, dvar};
+        return with_nt(NT, [&](auto nt) {
+            return launch_fused<svgp_posterior_predict_grad_kernel<decltype(nt)::value>>(s, ag, q.L,
+                                                                                        svgp_fused_grad_smem_bytes(NT, q.d));
+        });
+    }
+    const size_t smem = svgp_fused_smem_bytes(NT, q.d);
     return with_nt(NT, [&](auto nt) {
         return launch_fused<svgp_posterior_predict_kernel<decltype(nt)::value>>(s, a, q.L, smem);
     });

@@ -21,6 +21,7 @@
 #include "chol.cuh"
 #include "cov.cuh"
 #include "gemm.cuh"
+#include "gpr.cuh"
 
 namespace {
 
@@ -134,6 +135,46 @@ __global__ void mix_ve_kernel(int mode, const double* __restrict__ g_mean, const
             part[2 * blockIdx.x + 1] = b;
         }
     }
+}
+
+// dmean[n][p][j] = sum_l W[p][l] gm[l][n][j], dvar[n][p][j] = sum_l W[p][l]^2 gv[l][n][j] (l ascending, as mix_ve_kernel);
+// without W output p is latent p.  One thread per (n, p, j).
+__global__ void mix_grad_kernel(const double* __restrict__ gm, const double* __restrict__ gv, int L, int B, int P, int d,
+                                const double* __restrict__ W, double* __restrict__ dmean, double* __restrict__ dvar) {
+    const long idx = blockIdx.x * (long)blockDim.x + threadIdx.x;
+    if (idx >= (long)B * P * d) return;
+    const int j = (int)(idx % d), p = (int)((idx / d) % P);
+    const long n = idx / ((long)d * P);
+    double fm, fv;
+    if (W) {
+        fm = 0.0;
+        fv = 0.0;
+        for (int l = 0; l < L; ++l) {
+            const double w = W[(long)p * L + l];
+            const long o = ((long)l * B + n) * d + j;
+            fm = fma(gm[o], w, fm);
+            fv = fma(gv[o], w * w, fv);
+        }
+    } else {
+        const long o = ((long)p * B + n) * d + j;
+        fm = gm[o];
+        fv = gv[o];
+    }
+    dmean[idx] = fm;
+    dvar[idx] = fv;
+}
+
+// alpha[l][n][0] = sum_{m >= n} Wm[l][m][n] q_mu[m][l] (Wm lower triangular), alpha[l][n][1] = 0: the [L][M][2] table
+// posterior_dx_kernel reads as a with P = 1, Pp = 2.
+__global__ void svgp_alpha_kernel(const double* __restrict__ Wm, long ldM, const double* __restrict__ q_mu, int M, int L,
+                                  double* __restrict__ alpha) {
+    const int l = blockIdx.y, n = blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= M) return;
+    const double* W = Wm + (long)l * M * ldM;
+    double s = 0.0;
+    for (int m = n; m < M; ++m) s = fma(W[(long)m * ldM + n], q_mu[(long)m * L + l], s);
+    alpha[((long)l * M + n) * 2] = s;
+    alpha[((long)l * M + n) * 2 + 1] = 0.0;
 }
 
 // glik[p] = scale * sum_n lbuf[p][n]   (per-output likelihood variances; one block per output, fixed summation order)
@@ -404,12 +445,33 @@ int launch_svgp_mix(cudaStream_t s, const double* g_mean, const double* g_var, i
     return cudaGetLastError() == cudaSuccess ? 0 : MFGP_ERR_CUDA;
 }
 
+int launch_svgp_grad_mix(cudaStream_t s, const double* gm, const double* gv, int L, int B, int P, int d, const double* W,
+                         double* dmean, double* dvar) {
+    const long tot = (long)B * P * d;
+    if (tot == 0) return 0;
+    mix_grad_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(gm, gv, L, B, P, d, W, dmean, dvar);
+    return cudaGetLastError() == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+}
+
 // Cached-posterior prediction for any M, d: per chunk of test points svgp_conditional from the cached Wm and Lq, then the
-// mix.  Chunked so that the chunk's Kmn, A and C take at most half of the free device memory.  The same kernels on the
-// same factors as mfgp_svgp_predict.
+// mix.  Chunked so that the chunk's Kmn, A and C (and the latent gradients) take at most half of the free device memory.
+// The same kernels on the same factors as mfgp_svgp_predict.  With dmean / dvar the chunk goes on from V = f.A and
+// U = f.C: R = V - Lq U (into f.A), beta = Wm^T R (into f.Kmn, free by then), and posterior_dx_kernel contracts
+// dK_s/dx* with beta and alpha = Wm^T q_mu (formed once per call), one latent per problem; then the gradient mix.
 int svgp_posterior_predict_blocked(mfgp_handle* h, const SvgpPosteriorData& q, const double* Xs, int Ns, double* mean,
-                                   double* var) {
-    const long chunk = chunk_by_free_memory(((size_t)3 * q.L * q.M + (size_t)3 * q.L) * sizeof(double), 2, LONG_MAX);
+                                   double* var, double* dmean, double* dvar) {
+    cudaStream_t s = h->stream;
+    Scope outer(h);
+    double* alpha = nullptr;
+    if (dmean) {
+        alpha = outer.alloc<double>((size_t)q.L * q.M * 2);
+        if (!outer.ok) return outer.finish();
+        svgp_alpha_kernel<<<dim3((q.M + 127) / 128, q.L), 128, 0, s>>>(q.Wm, q.ld, q.q_mu, q.M, q.L, alpha);
+    }
+    // the latents as posterior_dx_kernel's problems: inducing points in the place of X, one column of alpha
+    const GprPosteriorData ql{q.M, q.d, 1, 2, q.L, q.ld, q.Z, q.theta, nullptr, nullptr, nullptr};
+    const size_t per = ((size_t)3 * q.L * q.M + (size_t)3 * q.L + (dmean ? (size_t)2 * q.L * q.d : 0)) * sizeof(double);
+    const long chunk = chunk_by_free_memory(per, 2, LONG_MAX);
     for (long n0 = 0; n0 < Ns; n0 += chunk) {
         const int nb = (int)((Ns - n0) < chunk ? (Ns - n0) : chunk);
         Scope inner(h);
@@ -418,9 +480,33 @@ int svgp_posterior_predict_blocked(mfgp_handle* h, const SvgpPosteriorData& q, c
         f.Lq = const_cast<double*>(q.Lq);
         f.ldM = q.ld;
         f.sMM = (long)q.M * q.ld;
-        MFGP_TRY(svgp_conditional(h, inner, q.L, q.M, nb, q.d, Xs + n0 * (q.d + 1), q.Z, q.theta, q.q_mu, f));
-        if (launch_svgp_mix(h->stream, f.g_mean, f.g_var, q.L, nb, q.P, q.W, mean + n0 * q.P, var + n0 * q.P))
+        const double* Xc = Xs + n0 * (q.d + 1);
+        MFGP_TRY(svgp_conditional(h, inner, q.L, q.M, nb, q.d, Xc, q.Z, q.theta, q.q_mu, f));
+        if (launch_svgp_mix(s, f.g_mean, f.g_var, q.L, nb, q.P, q.W, mean + n0 * q.P, var + n0 * q.P))
             return mfgp_fail(h, MFGP_ERR_CUDA, "svgp posterior: mix launch failed");
+        if (!dmean) continue;
+        double* gm = inner.alloc<double>((size_t)2 * q.L * nb * q.d);  // latent gradients [L][nb][d], mean then var
+        if (!inner.ok) return inner.finish();
+        double* gv = gm + (size_t)q.L * nb * q.d;
+        GemmArgs r;  // R = V - Lq U, in place of V
+        r.M = q.M; r.N = nb; r.K = q.M;
+        r.alpha = -1.0; r.beta = 1.0;
+        r.A = f.Lq; r.lda = f.ldM; r.strideA = f.sMM;
+        r.B = f.C; r.ldb = f.ldB; r.strideB = f.sMB;
+        r.C = f.A; r.ldc = f.ldB; r.strideC = f.sMB;
+        r.batch = q.L; r.krange = KR_HI_I;
+        if (launch_gemm(s, r)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp posterior: gemm (R) failed");
+        GemmArgs bt;  // beta = Wm^T R, into the K_s buffer
+        bt.transA = true;
+        bt.M = q.M; bt.N = nb; bt.K = q.M;
+        bt.A = f.Wm; bt.lda = f.ldM; bt.strideA = f.sMM;
+        bt.B = f.A; bt.ldb = f.ldB; bt.strideB = f.sMB;
+        bt.C = f.Kmn; bt.ldc = f.ldB; bt.strideC = f.sMB;
+        bt.batch = q.L; bt.krange = KR_LO_I;
+        if (launch_gemm(s, bt)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp posterior: gemm (beta) failed");
+        if (launch_posterior_dx(s, ql, q.L, Xc, nb, alpha, f.Kmn, f.ldB, gm, gv) ||
+            launch_svgp_grad_mix(s, gm, gv, q.L, nb, q.P, q.d, q.W, dmean + n0 * q.P * q.d, dvar + n0 * q.P * q.d))
+            return mfgp_fail(h, MFGP_ERR_CUDA, "svgp posterior: gradient launch failed");
     }
     return 0;
 }

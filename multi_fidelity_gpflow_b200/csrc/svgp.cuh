@@ -39,11 +39,16 @@ struct SvgpPosteriorData {
 };
 // Fused route (posterior.cu): one kernel for M <= 64, d <= 16.  Writes the latent marginals of point n and latent l
 // to mean[l * ls + n * ns] and var[l * ls + n * ns]: (ls, ns) = (1, P) is the [Ns][P] output itself when W == NULL,
-// (Ns, 1) the [L][Ns] input of launch_svgp_mix.
+// (Ns, 1) the [L][Ns] input of launch_svgp_mix.  With dmean / dvar (both or neither; svgp_posterior_predict_grad_kernel)
+// also the latent input gradients d mean / dx*_j and d var / dx*_j at (l * ls + n * ns) * d + j.
 bool svgp_posterior_fused_ok(int L, int M, int d);
 int svgp_posterior_predict_fused(cudaStream_t s, const SvgpPosteriorData& q, const double* Xs, int Ns, double* mean,
-                                 double* var, long ls, long ns);
+                                 double* var, long ls, long ns, double* dmean = nullptr, double* dvar = nullptr);
 // Blocked route (svgp.cu): any size, svgp_conditional and the mix from the cached factors, chunked over Ns.
-// mean / var [Ns][P].
+// mean / var [Ns][P]; with dmean / dvar [Ns][P][d] (both or neither) also the input gradients.
 int svgp_posterior_predict_blocked(mfgp_handle* h, const SvgpPosteriorData& q, const double* Xs, int Ns, double* mean,
-                                   double* var);
+                                   double* var, double* dmean = nullptr, double* dvar = nullptr);
+// dmean / dvar [B][P][d] from the latent gradients gm / gv [L][B][d] as launch_svgp_mix mixes the marginals:
+// dmean = sum_l W_pl gm_l, dvar = sum_l W_pl^2 gv_l in a fixed l order, or the gather of latent p when W == NULL.
+int launch_svgp_grad_mix(cudaStream_t s, const double* gm, const double* gv, int L, int B, int P, int d, const double* W,
+                         double* dmean, double* dvar);

@@ -242,7 +242,8 @@ class SVGPBase:
 
 
 class SVGPPosterior:
-    """What SVGPBase.posterior() returns: predict_f(Xnew) -> mean, var [N*, P] from the cached factors."""
+    """What SVGPBase.posterior() returns: predict_f(Xnew) -> mean, var [N*, P] from the cached factors, and
+    predict_f_grad(Xnew) with their input gradients."""
 
     def __init__(self, post):
         self.post = post
@@ -251,3 +252,11 @@ class SVGPPosterior:
         if full_cov or full_output_cov:
             raise NotImplementedError("the reference only calls predict_f(Xnew) (marginal variances)")
         return self.post.predict(_lib.as_f64(Xnew))
+
+    def predict_f_grad(self, Xnew):
+        """predict_f and its gradient with respect to Xnew: mean, var [N*, P] and dmean_dx, dvar_dx [N*, P, d+1]
+        (d value[s, p] / d Xnew[s, j]).  The last (fidelity) column is exactly 0, as tape.gradient gives it in the
+        reference."""
+        mean, var, dmean, dvar = self.post.predict_grad(_lib.as_f64(Xnew))
+        pad = lambda g: np.concatenate([g, np.zeros(g.shape[:-1] + (1,))], axis=-1)
+        return mean, var, pad(dmean), pad(dvar)

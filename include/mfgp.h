@@ -117,6 +117,30 @@ int mfgp_gpr_posterior_predict(mfgp_handle* h, const mfgp_gpr_posterior* post, c
  * results do not depend on the other points or problems of the call. */
 int mfgp_gpr_posterior_predict_grad(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns,
                                     double* mean, double* var, double* dmean, double* dvar);
+/* Joint posterior over the Ns test points (GPflow GPR.predict_f(full_cov=True) and predict_f_samples):
+ * Sigma_b = K(Xs, Xs) - V^T V with V = W K(X, Xs), the same for every output column of problem b.
+ * mfgp_gpr_posterior_predict_cov: mean [B, Ns, P] and the joint covariance cov [B, Ns, Ns] (both triangles, exactly
+ * symmetric).  mean is _predict's mean bit for bit and the diagonal of cov is _predict's var bit for bit.
+ * mfgp_gpr_posterior_sample: samples[b, i, k, c] = mean[b, i, c] + sum_j L_b[i, j] z[b, j, k, c] with
+ * L_b L_b^T = Sigma_b + jitter I, Sigma_b exactly the matrix _predict_cov returns (GPflow sample_mvn, full_cov=True).
+ * z and samples are [B, Ns, S, P]: each test point's S * P draws are contiguous, and z and samples must not overlap.
+ *  - Failures: info[b] (info [B] or NULL) is the 1-based first pivot of Sigma_b + jitter I that is not > 0 (NaN counts),
+ *    so a problem whose factorisation failed at creation reports 1.  All samples of a failing problem are NaN.  The call
+ *    returns the first failure's pivot with or without info; with info that is the problem's status.  _predict_cov gives
+ *    NaN mean and cov for a problem that failed at creation, as _predict does, and returns 0.
+ *  - A test row with fidelity not in {0, 1} has a zero row and column in cov and a zero mean.  With jitter > 0 its row of
+ *    L is sqrt(jitter) e_i, so its samples are sqrt(jitter) z; with jitter == 0 it is a failed pivot.
+ *  - jitter finite and >= 0, S >= 0, no NULL pointer except info: otherwise -1.  Ns == 0 or S == 0 returns 0.  Pointers,
+ *    async mode (a non-PD status then reaches mfgp_sync) and the device check as for _predict.
+ *  - A problem's results do not depend on the other problems of the call, and a sample column's values do not depend on S
+ *    or on how the work is split.  Indices are 64-bit: B * Ns * S * P may exceed 2^31.
+ *  - Routes as for _predict.  N <= 64, d <= 16, P <= 64 and Ns <= 64 run ONE kernel (gpr_posterior_joint_kernel: each CTA
+ *    rebuilds Sigma on DMMA, factors it in shared memory and streams its chunk of z); anything else extends the blocked
+ *    route with K1 for K(Xs, Xs), one GEMM for Sigma, potrf and one GEMM for L Z. */
+int mfgp_gpr_posterior_predict_cov(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns,
+                                   double* mean, double* cov);
+int mfgp_gpr_posterior_sample(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns, int S,
+                              double jitter, const double* z, double* samples, int* info);
 int mfgp_gpr_posterior_destroy(mfgp_gpr_posterior* post);
 
 /* Training loop on the device (SURVEY 8(f) rank 1): the Adam branch of MultiFidelityGPModel.optimize (mfgpflow/linear.py:

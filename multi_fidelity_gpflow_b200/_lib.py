@@ -53,6 +53,8 @@ def _load():
         "mfgp_gpr_posterior_create": ([vp, vp, i, i, vp, l, i, i, i, vp, vp, vp, C.POINTER(vp)], i),
         "mfgp_gpr_posterior_predict": ([vp, vp, vp, i, vp, vp], i),
         "mfgp_gpr_posterior_predict_grad": ([vp, vp, vp, i, vp, vp, vp, vp], i),
+        "mfgp_gpr_posterior_predict_cov": ([vp, vp, vp, i, vp, vp], i),
+        "mfgp_gpr_posterior_sample": ([vp, vp, vp, i, i, d, vp, vp, vp], i),
         "mfgp_gpr_posterior_destroy": ([vp], i),
         "mfgp_graph_nparams": ([i, i], i),
         "mfgp_graph_cov": ([vp, vp, i, i, i, vp, vp, l], i),
@@ -92,7 +94,7 @@ EXPORTED_SYMBOLS = [
     "mfgp_last_error", "mfgp_sm_count", "mfgp_cov", "mfgp_cov_diag", "mfgp_cov_grad", "mfgp_gpr_nlml", "mfgp_gpr_nlml_grad",
     "mfgp_gpr_predict", "mfgp_gpr_batched_nlml_grad", "mfgp_gpr_batched_adam",
     "mfgp_gpr_posterior_create", "mfgp_gpr_posterior_predict", "mfgp_gpr_posterior_predict_grad",
-    "mfgp_gpr_posterior_destroy",
+    "mfgp_gpr_posterior_predict_cov", "mfgp_gpr_posterior_sample", "mfgp_gpr_posterior_destroy",
     "mfgp_graph_nparams", "mfgp_graph_cov", "mfgp_graph_cov_diag", "mfgp_graph_gpr_nlml_grad", "mfgp_svgp_elbo_grad", "mfgp_svgp_elbo_grad_v", "mfgp_svgp_predict",
     "mfgp_svgp_posterior_create", "mfgp_svgp_posterior_predict", "mfgp_svgp_posterior_predict_grad",
     "mfgp_svgp_posterior_destroy", "mfgp_svgp_adam",
@@ -579,6 +581,49 @@ class GprPosterior(_Posterior):
         self.handle._check(_lib.mfgp_gpr_posterior_predict_grad(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean), _ptr(var),
                                                                 _ptr(dmean), _ptr(dvar)), "mfgp_gpr_posterior_predict_grad")
         return mean, var, dmean, dvar
+
+    def predict_cov(self, Xs, mean=None, cov=None):
+        """Mean [B, Ns, P] and the joint covariance [B, Ns, Ns] over the test points (the same for every column of a
+        problem).  mean is predict()'s mean and diag(cov) predict()'s var, bit for bit.  Host arrays or device tensors."""
+        Xs = self._xs(Xs)
+        Ns = Xs.shape[0]
+        mean = np.empty((self.B, Ns, self.P)) if mean is None else mean
+        cov = np.empty((self.B, Ns, Ns)) if cov is None else cov
+        self.handle._check(_lib.mfgp_gpr_posterior_predict_cov(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean), _ptr(cov)),
+                           "mfgp_gpr_posterior_predict_cov")
+        return mean, cov
+
+    def sample(self, Xs, z, jitter=1e-6, samples=None, info=None):
+        """Joint draws [B, Ns, S, P]: samples[b] = mean[b] + L_b z[b] over the test-point axis, L_b L_b^T = cov[b] +
+        jitter I, for standard normals z [B, Ns, S, P].  A problem whose factor fails raises NotPositiveDefiniteError
+        unless a per-problem `info` array (int32 [B]) is passed: then info[b] holds its 1-based pivot (0 = ok) and its
+        samples are NaN.  Host arrays or device tensors."""
+        Xs = self._xs(Xs)
+        Ns = Xs.shape[0]
+        z = as_f64(z)
+        if tuple(z.shape[:2]) != (self.B, Ns) or len(z.shape) != 4 or z.shape[3] != self.P:
+            raise ValueError(f"z must be [B={self.B}, Ns={Ns}, S, P={self.P}]")
+        S = int(z.shape[2])
+        samples = np.empty((self.B, Ns, S, self.P)) if samples is None else samples
+        rc = _lib.mfgp_gpr_posterior_sample(self.handle._h, self._p, _ptr(Xs), Ns, S, float(jitter), _ptr(z), _ptr(samples),
+                                            _ptr(info))
+        if not (rc > 0 and info is not None):
+            self.handle._check(rc, "mfgp_gpr_posterior_sample")
+        return samples
+
+    def draw_f(self, Xs, num_samples=None, full_cov=True, full_output_cov=False, seed=None, info=None):
+        """GPflow's predict_f_samples over every problem: [B, Ns, S, P] (S = 1 when num_samples is None), from
+        z = np.random.default_rng(seed).standard_normal((B, Ns, S, P)).  full_cov=True: sample() with GPflow's default
+        jitter 1e-6; full_cov=False: mean + sqrt(var) z from predict(), without jitter."""
+        if full_output_cov:
+            raise NotImplementedError("full_output_cov: the outputs of an exact GP are independent given its kernel")
+        Xs = self._xs(Xs)
+        S = 1 if num_samples is None else int(num_samples)
+        z = np.random.default_rng(seed).standard_normal((self.B, Xs.shape[0], S, self.P))
+        if full_cov:
+            return self.sample(Xs, z, jitter=1e-6, info=info)
+        mean, var = self.predict(Xs)
+        return mean[:, :, None, :] + np.sqrt(var)[:, :, None, None] * z
 
 
 class SvgpPosterior(_Posterior):

@@ -1,6 +1,7 @@
 // api.cu -- extern "C" entry points of libmfgp.so (see include/mfgp.h for the contract).
 #include <cuda_runtime.h>
 
+#include <cmath>
 #include <vector>
 
 #include "chol.cuh"
@@ -498,6 +499,72 @@ int mfgp_gpr_posterior_predict_grad(mfgp_handle* h, const mfgp_gpr_posterior* po
         return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_gpr_posterior_predict_grad: bad argument (dmean and dvar are required)");
     }
     return posterior_predict(h, post, Xs, Ns, mean, var, dmean, dvar, "mfgp_gpr_posterior_predict_grad");
+}
+
+}  // extern "C"
+
+namespace {
+// mfgp_gpr_posterior_predict_cov and _sample: one body, the samples when `sample`.
+int posterior_joint(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns, double* mean, double* cov,
+                    bool sample, int S, double jitter, const double* z, double* samples, int* info, const char* name) {
+    CHECK_H(h);
+    if (!post || !Xs || Ns < 0 ||
+        (sample ? (!z || !samples || S < 0 || !std::isfinite(jitter) || jitter < 0.0) : (!mean || !cov)))
+        return mfgp_fail(h, MFGP_ERR_ARG, "%s: bad argument", name);
+    if (post->m.device != h->device)
+        return mfgp_fail(h, MFGP_ERR_ARG, "%s: the posterior lives on device %d, the handle on %d", name, post->m.device,
+                         h->device);
+    const GprPosteriorData& q = post->q;
+    const long SP = sample ? (long)S * q.P : 0;
+    if (sample) {
+        const size_t bytes = (size_t)q.B * Ns * SP * sizeof(double);
+        const char *zc = reinterpret_cast<const char*>(z), *sc = reinterpret_cast<const char*>(samples);
+        if (zc < sc + bytes && sc < zc + bytes && bytes) return mfgp_fail(h, MFGP_ERR_ARG, "%s: z and samples overlap", name);
+    }
+    if (Ns == 0 || (sample && S == 0)) return 0;
+    cudaSetDevice(h->device);
+    Scope sc(h);
+    const double* dXs = sc.in(Xs, (size_t)Ns * (q.d + 1));
+    double* dm = sample ? sc.alloc<double>((size_t)q.B * Ns * q.P) : sc.out(mean, (size_t)q.B * Ns * q.P);
+    GprJointOut j{};
+    j.SP = SP;
+    j.jitter = jitter;
+    if (sample) {
+        j.z = sc.in(z, (size_t)q.B * Ns * SP);
+        j.samples = sc.out(samples, (size_t)q.B * Ns * SP);
+        j.info = info ? sc.out(info, q.B, true) : sc.alloc<int>(q.B, true);
+    } else {
+        j.cov = sc.out(cov, (size_t)q.B * Ns * Ns);
+    }
+    if (!sc.ok) return sc.finish();
+    if (gpr_posterior_joint_fused_ok(q.N, q.d, q.P, Ns)) {
+        if (gpr_posterior_joint_fused(h->stream, q, dXs, Ns, dm, j, h->d_info))
+            return mfgp_fail(h, MFGP_ERR_CUDA, "%s: fused kernel launch failed", name);
+    } else {
+        double* dv = sc.alloc<double>((size_t)q.B * Ns);
+        if (!sc.ok) return sc.finish();
+        // mean and diag(cov) are _predict's bits: when _predict runs the fused kernel (N <= 64 with Ns > 64), so do they
+        j.mean_var_given = gpr_posterior_fused_ok(q.N, q.d, q.P);
+        if (j.mean_var_given && gpr_posterior_predict_fused(h->stream, q, dXs, Ns, dm, dv))
+            return mfgp_fail(h, MFGP_ERR_CUDA, "%s: fused kernel launch failed", name);
+        MFGP_TRY(gpr_posterior_predict_blocked(h, q, dXs, Ns, dm, dv, nullptr, nullptr, &j));
+    }
+    return sc.finish();
+}
+}  // namespace
+
+extern "C" {
+
+int mfgp_gpr_posterior_predict_cov(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns, double* mean,
+                                   double* cov) {
+    return posterior_joint(h, post, Xs, Ns, mean, cov, false, 0, 0.0, nullptr, nullptr, nullptr,
+                           "mfgp_gpr_posterior_predict_cov");
+}
+
+int mfgp_gpr_posterior_sample(mfgp_handle* h, const mfgp_gpr_posterior* post, const double* Xs, int Ns, int S,
+                              double jitter, const double* z, double* samples, int* info) {
+    return posterior_joint(h, post, Xs, Ns, nullptr, nullptr, true, S, jitter, z, samples, info,
+                           "mfgp_gpr_posterior_sample");
 }
 
 int mfgp_gpr_posterior_destroy(mfgp_gpr_posterior* post) {

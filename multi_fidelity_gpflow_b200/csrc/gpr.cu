@@ -68,6 +68,99 @@ __global__ void predict_var_kernel(const double* __restrict__ As, int N, int Ns,
     var[b * Ns + j] = kss[b * Ns + j] - s;
 }
 
+// Sigma's diagonal <- var (+ jitter for the factorisation); with cov, the whole matrix out: the lower triangle, mirrored.
+__global__ void joint_diag_kernel(double* __restrict__ Sg, int Ns, long lds, const double* __restrict__ var, double jitter,
+                                  double* __restrict__ cov) {
+    const long b = blockIdx.y;
+    double* S = Sg + b * Ns * lds;
+    const double* v = var + b * Ns;
+    if (!cov) {
+        for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < Ns; i += gridDim.x * blockDim.x) S[(long)i * lds + i] = v[i] + jitter;
+        return;
+    }
+    double* c = cov + b * Ns * Ns;
+    for (long idx = blockIdx.x * (long)blockDim.x + threadIdx.x; idx < (long)Ns * Ns; idx += (long)gridDim.x * blockDim.x) {
+        const long i = idx / Ns, j = idx - i * Ns;
+        c[idx] = i == j ? v[i] : (i > j ? S[i * lds + j] : S[j * lds + i]);
+    }
+}
+
+// samples [nb][Ns][SP] (holding L z) += mean [nb][Ns][P] broadcast over the S draws; NaN for a problem whose factor failed.
+__global__ void joint_sample_epilogue_kernel(double* __restrict__ out, int Ns, long SP, int P, const double* __restrict__ mean,
+                                             const int* __restrict__ info) {
+    const long b = blockIdx.y, per = (long)Ns * SP;
+    const bool bad = info[b] != 0;
+    const double qnan = __longlong_as_double(0x7ff8000000000000ll);
+    double* o = out + b * per;
+    const double* m = mean + b * Ns * P;
+    for (long idx = blockIdx.x * (long)blockDim.x + threadIdx.x; idx < per; idx += (long)gridDim.x * blockDim.x) {
+        const long i = idx / SP, col = idx - i * SP;
+        o[idx] = bad ? qnan : o[idx] + m[i * P + col % P];
+    }
+}
+
+// The joint outputs of nb problems (from b0) of the blocked route, from the chunk's A_s = W K_s [nb][N][lds], var and mean:
+// K_ss (K1, symmetric), Sigma = K_ss - A_s^T A_s (lower tiles), diag <- var.  _predict_cov mirrors Sigma into cov;
+// _sample adds the jitter, factors with potrf and forms samples = L Z + mean.
+int joint_chunk(mfgp_handle* h, Scope& sc, const GprPosteriorData& q, long b0, int nb, const double* Xs, int Ns,
+                const double* th, const double* As, long lds, const double* var, const double* mean, const GprJointOut& j) {
+    cudaStream_t s = h->stream;
+    const int np = 2 * q.d + 3, N = q.N;
+    double* Sg = sc.alloc<double>((size_t)nb * Ns * lds, true);
+    if (!sc.ok) return sc.finish();
+    CovArgs k{};
+    k.Xa = Xs; k.Na = Ns; k.Xb = Xs; k.Nb = Ns; k.d = q.d;
+    k.theta = th; k.theta_stride = np;
+    k.K = Sg; k.ldk = lds; k.strideK = (long)Ns * lds;
+    k.symmetric = 1;
+    k.batch = nb; k.route_batch = q.B;
+    if (launch_cov(s, k)) return mfgp_fail(h, MFGP_ERR_CUDA, "cov launch (K_ss) failed");
+    GemmArgs g;  // Sigma = K_ss - A_s^T A_s
+    g.transA = true;
+    g.M = Ns; g.N = Ns; g.K = N;
+    g.alpha = -1.0; g.beta = 1.0;
+    g.A = As; g.lda = lds; g.strideA = (long)N * lds;
+    g.B = As; g.ldb = lds; g.strideB = (long)N * lds;
+    g.C = Sg; g.ldc = lds; g.strideC = (long)Ns * lds;
+    g.batch = nb;
+    g.lower_only = 1;
+    if (launch_gemm(s, g)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (Sigma) failed");
+    const long work = j.SP ? Ns : (long)Ns * Ns;
+    const dim3 dgrid((unsigned)((work + 255) / 256 < 64 ? (work + 255) / 256 : 64), (unsigned)nb);
+    joint_diag_kernel<<<dgrid, 256, 0, s>>>(Sg, Ns, lds, var, j.SP ? j.jitter : 0.0, j.SP ? nullptr : j.cov + b0 * Ns * Ns);
+    if (!j.SP) return cudaGetLastError() == cudaSuccess ? 0 : mfgp_fail(h, MFGP_ERR_CUDA, "joint_diag_kernel launch failed");
+
+    CholArgs ch{};
+    ch.A = Sg; ch.N = Ns; ch.lda = lds; ch.strideA = (long)Ns * lds; ch.batch = nb;
+    ch.dinv = sc.alloc<double>((size_t)chol_dinv_count(Ns, nb));
+    ch.logd = sc.alloc<double>((size_t)nb * Ns);
+    const long ldz = round_up(j.SP, 2);
+    double* Zw = sc.alloc<double>((size_t)nb * Ns * ldz);
+    if (!sc.ok) return sc.finish();
+    ch.d_info = h->d_info; ch.aux = h->aux_stream; ch.ev = h->ev; ch.info_vec = j.info + b0;
+    if (launch_potrf(s, ch)) return mfgp_fail(h, MFGP_ERR_CUDA, "potrf launch (Sigma) failed");
+    // the GEMM's TMA operands need an even leading dimension: stage z with ld = round_up(S P, 2)
+    CUDA_TRY(h, cudaMemcpy2DAsync(Zw, ldz * sizeof(double), j.z + b0 * Ns * j.SP, j.SP * sizeof(double),
+                                  j.SP * sizeof(double), (size_t)nb * Ns, cudaMemcpyDeviceToDevice, s));
+    double* out = j.samples + b0 * Ns * j.SP;
+    constexpr long MAX_COLS = 1L << 30;  // GemmArgs::N is an int
+    for (long c0 = 0; c0 < j.SP; c0 += MAX_COLS) {
+        GemmArgs lz;  // samples = L Z (L lower triangular)
+        lz.M = Ns; lz.N = (int)(j.SP - c0 < MAX_COLS ? j.SP - c0 : MAX_COLS); lz.K = Ns;
+        lz.A = Sg; lz.lda = lds; lz.strideA = (long)Ns * lds;
+        lz.B = Zw + c0; lz.ldb = ldz; lz.strideB = (long)Ns * ldz;
+        lz.C = out + c0; lz.ldc = j.SP; lz.strideC = (long)Ns * j.SP;
+        lz.batch = nb;
+        lz.krange = KR_HI_I;
+        lz.small_tiles = 1;  // one tile shape whatever S * P: a column's value does not depend on S
+        if (launch_gemm(s, lz)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (L Z) failed");
+    }
+    const long per = (long)Ns * j.SP;
+    const unsigned ex = (unsigned)((per + 255) / 256 < 1024 ? (per + 255) / 256 : 1024);
+    joint_sample_epilogue_kernel<<<dim3(ex, (unsigned)nb), 256, 0, s>>>(out, Ns, j.SP, q.P, mean, j.info + b0);
+    return cudaGetLastError() == cudaSuccess ? 0 : mfgp_fail(h, MFGP_ERR_CUDA, "joint_sample_epilogue_kernel launch failed");
+}
+
 }  // namespace
 
 using Factor = GprFactor;
@@ -278,11 +371,14 @@ int gpr_predict_device(mfgp_handle* h, Scope& sc, const double* X, const double*
 // the free device memory.  With dmean / dvar the chunk goes on from the same A_s: beta = W^T A_s = K^-1 K_s (into the
 // K_s buffer, which is free by then), alpha = W^T a, and posterior_dx_kernel contracts dK_s/dx* with both.
 int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
-                                  double* var, double* dmean, double* dvar) {
+                                  double* var, double* dmean, double* dvar, const GprJointOut* joint) {
     cudaStream_t s = h->stream;
     const int np = 2 * q.d + 3, N = q.N;
     const long lds = round_up(Ns, 2);
-    const size_t per = ((size_t)2 * N * lds + Ns + (dmean ? (size_t)N * q.Pp : 0)) * sizeof(double);
+    size_t per = ((size_t)2 * N * lds + Ns + (dmean ? (size_t)N * q.Pp : 0)) * sizeof(double);
+    if (joint)  // Sigma, and for _sample potrf's workspaces and the staged z
+        per += ((size_t)Ns * lds + (joint->SP ? (size_t)chol_dinv_count(Ns, 1) + Ns + (size_t)Ns * round_up(joint->SP, 2) : 0)) *
+               sizeof(double);
     const long chunk = chunk_by_free_memory(per, 1, 16384);  // 16384: grid z of the batched kernels
     for (long b0 = 0; b0 < q.B; b0 += chunk) {
         const int nb = (int)((q.B - b0) < chunk ? (q.B - b0) : chunk);
@@ -308,7 +404,6 @@ int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, con
         g.batch = nb;
         g.krange = KR_HI_I;
         if (launch_gemm(s, g)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (As) failed");
-        predict_var_kernel<<<dim3((Ns + 127) / 128, nb), 128, 0, s>>>(As, N, Ns, lds, kss, var + b0 * Ns, (long)N * lds);
         GemmArgs m;  // mean = A_s^T a
         m.transA = true;
         m.M = Ns; m.N = q.P; m.K = N;
@@ -316,7 +411,14 @@ int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, con
         m.B = q.a + b0 * N * q.Pp; m.ldb = q.Pp; m.strideB = (long)N * q.Pp;
         m.C = mean + b0 * Ns * q.P; m.ldc = q.P; m.strideC = (long)Ns * q.P;
         m.batch = nb;
-        if (launch_gemm(s, m)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (mean) failed");
+        if (!(joint && joint->mean_var_given)) {
+            predict_var_kernel<<<dim3((Ns + 127) / 128, nb), 128, 0, s>>>(As, N, Ns, lds, kss, var + b0 * Ns, (long)N * lds);
+            if (launch_gemm(s, m)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (mean) failed");
+        }
+        if (joint) {
+            MFGP_TRY(joint_chunk(h, inner, q, b0, nb, Xs, Ns, th, As, lds, var + b0 * Ns, m.C, *joint));
+            continue;
+        }
         if (!dmean) continue;
         GemmArgs bt;  // beta = W^T A_s, into the K_s buffer
         bt.transA = true;

@@ -57,9 +57,27 @@ struct GprPosteriorData {
 bool gpr_posterior_fused_ok(int N, int d, int P);
 int gpr_posterior_predict_fused(cudaStream_t s, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
                                 double* var, double* dmean = nullptr, double* dvar = nullptr);
-// Blocked route (gpr.cu): any size, built from K1 / cov_diag / the batched GEMM, chunked over problems.
+// Joint outputs (mfgp_gpr_posterior_predict_cov / _sample), device pointers.  SP == 0: cov [B][Ns][Ns].  SP = S * P > 0:
+// samples [B][Ns][SP] = mean + L z with L L^T = Sigma + jitter I, z [B][Ns][SP], info [B] zeroed by the caller.
+struct GprJointOut {
+    double* cov;
+    long SP;
+    double jitter;
+    const double* z;
+    double* samples;
+    int* info;
+    bool mean_var_given;  // mean and var were computed by _predict's own route (the fused kernel): the chunks only read them
+};
+// Fused joint route (posterior.cu): gpr_posterior_fused_ok and Ns <= 64, one kernel.  mean [B][Ns][P] is written for
+// _predict_cov only; a failed factor is also CAS'ed into d_info.
+bool gpr_posterior_joint_fused_ok(int N, int d, int P, int Ns);
+int gpr_posterior_joint_fused(cudaStream_t s, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
+                              const GprJointOut& j, int* d_info);
+// Blocked route (gpr.cu): any size, built from K1 / cov_diag / the batched GEMM, chunked over problems.  With `joint` the
+// chunk goes on to the joint outputs; mean and var are then required, full-size workspaces or outputs.
 int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
-                                  double* var, double* dmean = nullptr, double* dvar = nullptr);
+                                  double* var, double* dmean = nullptr, double* dvar = nullptr,
+                                  const GprJointOut* joint = nullptr);
 // The input-gradient contraction of the blocked route (posterior.cu) for nb problems of q (theta from q.theta):
 // dmean[b][s][p][j] = sum_n alpha[b][n][p] dk_sn/dx_sj, dvar[b][s][j] = -2 sum_n beta[b][n][s] dk_sn/dx_sj, with
 // alpha [nb][N][q.Pp] = W^T a and beta [nb][N][ldb] = K^-1 K_s.

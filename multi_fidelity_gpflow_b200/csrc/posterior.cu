@@ -29,6 +29,11 @@
 // (differences, never the expanded form), dvar_j = -2 sum_n beta_n gk_n (lane-local, then the quad), dmean_:j = alpha^T gk
 // (contract_table with gk in the place of V).
 //
+// gpr_posterior_joint_kernel (mfgp_gpr_posterior_predict_cov / _sample, Ns <= 64): predict's K_s, V, var and mean per
+// 8-point group (so mean and diag(Sigma) are predict's bits), V^T to shared memory, then Sigma = K_ss - V^T V on the lower
+// 8x8 tiles (DMMA over the training index, K_ss from the point records) with var on the diagonal, mirrored.  _sample goes
+// on: L L^T = Sigma + jitter I in shared memory, and samples = mean + L z over the CTA's chunk of the S * P columns.
+//
 // svgp_posterior_predict_kernel (mfgp_svgp_posterior_predict): the inducing points Z in the place of X, one latent per
 // blockIdx.y, W = Wm.  U = Lq^T V (upper_tri_product with F = Lq) never leaves the accumulators: sum U^2 is lane-local.
 // var = k_ss - sum V^2 + sum U^2, mean = V^T q_mu.
@@ -146,6 +151,42 @@ __device__ __forceinline__ void prescale_point(const double* __restrict__ x, boo
 
 // ---- building blocks of the fused kernels.  A fragment row `double f[2 * NT]` holds one value per training index of
 //      the lane's point, in the C-fragment order of the file comment (slot 2i + e <-> n = 8i + 2t + e) unless noted.
+
+// K_s^T fragment in the A-fragment order: ks[k] = k(x_n, xs_g), n = 4k + t, from the training points Xt [2d+4][NP]
+// (k-major) and the point record xg (prescale_point, K1's expanded-square form).  The same operations in the same order as
+// the K_s block of gpr_posterior_predict_kernel, which keeps its own copy so that its SASS does not move.
+template <int NT>
+__device__ __forceinline__ void ks_fragment(double (&ks)[2 * NT], const double* Xt, const double* xg, int d, int t,
+                                            const double* etab) {
+    constexpr int NP = 8 * NT;
+    const double sg = xg[2 * d + 2], hg = xg[2 * d + 3];
+    double e[2 * NT];
+#pragma unroll
+    for (int k = 0; k < 2 * NT; ++k) e[k] = Xt[2 * d * NP + 4 * k + t] + xg[2 * d];
+    for (int c = 0; c < d; ++c) {
+        const double xc = xg[c];
+        const double* xr = Xt + c * NP + t;
+#pragma unroll
+        for (int k = 0; k < 2 * NT; ++k) e[k] = fma(xr[4 * k], xc, e[k]);
+    }
+    const double* sr = Xt + (2 * d + 2) * NP + t;
+#pragma unroll
+    for (int k = 0; k < 2 * NT; ++k) ks[k] = fexp512(e[k], etab) * (sr[4 * k] * sg);
+    if (__any_sync(0xffffffffu, hg != 0.0)) {  // some HF test point: discrepancy GP on the HF x HF pairs
+#pragma unroll
+        for (int k = 0; k < 2 * NT; ++k) e[k] = Xt[(2 * d + 1) * NP + 4 * k + t] + xg[2 * d + 1];
+        for (int c = 0; c < d; ++c) {
+            const double xc = xg[d + c];
+            const double* xr = Xt + (d + c) * NP + t;
+#pragma unroll
+            for (int k = 0; k < 2 * NT; ++k) e[k] = fma(xr[4 * k], xc, e[k]);
+        }
+        const double* hr = Xt + (2 * d + 3) * NP + t;
+#pragma unroll
+        for (int k = 0; k < 2 * NT; ++k)
+            if (hr[4 * k] * hg != 0.0) ks[k] += fexp512(e[k], etab);
+    }
+}
 
 // V^T = K_s^T W^T over the lower-triangular tiles of Ws [NP][WP] (zero above the diagonal): ks in the A-fragment order, v in the C order.
 template <int NT>
@@ -843,6 +884,259 @@ __global__ void __launch_bounds__(PW * 32, 1) svgp_posterior_predict_grad_kernel
     }
 }
 
+// ---- joint posterior (mfgp_gpr_posterior_predict_cov / _sample), Ns <= 64 test points.  One CTA per (chunk of sample
+//      columns, problem); every CTA of a problem rebuilds Sigma and its factor the same way, so no result depends on the
+//      chunking.  Shared memory (doubles), regions reused once their first tenant is dead:
+//        RA  W [NP][WP]                       -> Sigma, then L  [NSP][SPp]
+//        As  a [NP][AP]     Xt [2d+4][NP]     Xr  records of all test points [NSP][S1]
+//        RB  V^T [NSP][WP]                    -> z tile [NSP][JZP]   (_sample)
+//        Dg  predict's var, then diag(L) [NSP]     Lc  column of L being formed [NSP]     Ms  mean [NSP][P] (_sample)
+constexpr int JZC = 64;        // z columns per shared-memory tile
+constexpr int JZP = JZC + 4;   // its pitch: 4 mod 16 keeps the B-fragment loads Zs[4k + t][8j + g] free of bank conflicts
+constexpr int JL = 8;          // z loads in flight per thread
+constexpr int JOINT_MAX_NS = 64;
+constexpr long JOINT_MIN_COLS = 256;  // sample columns per CTA at least: the CTA's rebuild of Sigma and L stays small
+__host__ __device__ constexpr int s_pitch(int NSP) { return NSP + 4; }
+
+struct JointSmem {
+    int ra, as, xt, xr, rb, dg, lc, ms, total;  // offsets in doubles
+    __host__ __device__ JointSmem(int NT, int NST, int d, int P, bool sample) {
+        const int NP = 8 * NT, NSP = 8 * NST;
+        const int wsz = NP * w_pitch(NP), ssz = NSP * s_pitch(NSP), vsz = NSP * w_pitch(NP), zsz = sample ? NSP * JZP : 0;
+        int o = 0;
+        ra = o; o += wsz > ssz ? wsz : ssz;
+        as = o; o += NP * a_pitch(P);
+        xt = o; o += (2 * d + 4) * NP;
+        xr = o; o += NSP * rec_len(d);
+        rb = o; o += vsz > zsz ? vsz : zsz;
+        dg = o; o += NSP;
+        lc = o; o += NSP;
+        ms = o; o += sample ? NSP * P : 0;
+        total = o;
+    }
+};
+
+struct JointArgs {
+    GprPosteriorData q;
+    const double* Xs;
+    int Ns;
+    long SP;       // S * P sample columns per test point; 0: _predict_cov
+    long cpc;      // sample columns per CTA (a multiple of JZC)
+    double jitter;
+    const double* z;  // [B][Ns][SP]
+    double* samples;  // [B][Ns][SP]
+    int* info;        // [B]
+    int* d_info;
+    double* mean;     // _predict_cov: [B][Ns][P]
+    double* cov;      //               [B][Ns][Ns]
+};
+
+// k(x_i, x_j) from two point records in K1's expanded-square form (the form ks_fragment evaluates).
+__device__ __forceinline__ double kss_pair(const double* xi, const double* xj, int d, const double* etab) {
+    double e = xj[2 * d] + xi[2 * d];
+    for (int c = 0; c < d; ++c) e = fma(xj[c], xi[c], e);
+    double k = fexp512(e, etab) * (xj[2 * d + 2] * xi[2 * d + 2]);
+    if (xj[2 * d + 3] * xi[2 * d + 3] != 0.0) {
+        double e2 = xj[2 * d + 1] + xi[2 * d + 1];
+        for (int c = 0; c < d; ++c) e2 = fma(xj[d + c], xi[d + c], e2);
+        k += fexp512(e2, etab);
+    }
+    return k;
+}
+
+template <int NT>
+__global__ void __launch_bounds__(PW * 32) gpr_posterior_joint_kernel(JointArgs p) {
+    constexpr int NP = 8 * NT, WP = w_pitch(NP);
+    extern __shared__ __align__(16) double sm[];
+    __shared__ __align__(16) double etab[512];
+    __shared__ int fail;
+    const GprPosteriorData& q = p.q;
+    const int N = q.N, d = q.d, P = q.P, AP = a_pitch(P), S1 = rec_len(d), Ns = p.Ns;
+    const int NST = (Ns + 7) / 8, NSP = 8 * NST, SPp = s_pitch(NSP);
+    const bool sample = p.SP > 0;
+    const JointSmem lay(NT, NST, d, P, sample);
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
+    const long b = blockIdx.y;
+    const double* __restrict__ th = q.theta + b * (2 * d + 3);
+    double* Ws = sm + lay.ra;
+    double* Sg = Ws;  // Sigma, then L, once W is dead
+    double* As = sm + lay.as;
+    double* Xt = sm + lay.xt;
+    double* Xr = sm + lay.xr;
+    double* Vt = sm + lay.rb;
+    double* Zs = Vt;  // z tiles, once V is dead
+    double* Dg = sm + lay.dg;
+    double* Lc = sm + lay.lc;
+    double* Ms = sm + lay.ms;
+    fexp512_table_fill(etab, tid, blockDim.x);
+    const double hlL = 0.5 * log(th[1 + d]), hlD = 0.5 * log(th[2 + 2 * d]);
+    const double rho = th[0], vL = th[1 + d], vD = th[2 + 2 * d];
+    const double kss_hf = __dadd_rn(__dmul_rn(vL, __dmul_rn(rho, rho)), vD);  // as gpr_posterior_predict_kernel
+
+    // ---- stage the problem as gpr_posterior_predict_kernel does, and the records of every test point (padding: dead)
+    {
+        const double* __restrict__ Wg = q.W + b * N * q.ld;
+        for (int idx = tid; idx < NP * NP; idx += blockDim.x) {
+            const int r = idx / NP, c = idx - r * NP;
+            Ws[r * WP + c] = (r < N && c <= r) ? Wg[(long)r * q.ld + c] : 0.0;
+        }
+        const double* __restrict__ ag = q.a + b * N * q.Pp;
+        for (int idx = tid; idx < NP * AP; idx += blockDim.x) {
+            const int r = idx / AP, c = idx - r * AP;
+            As[idx] = (r < N && c < P) ? ag[(long)r * q.Pp + c] : 0.0;
+        }
+        for (int n = tid; n < NP; n += blockDim.x) prescale_point(q.X + (long)n * (d + 1), n < N, d, th, hlL, hlD, Xt + n, NP);
+        for (int i = tid; i < NSP; i += blockDim.x) {
+            const bool exists = i < Ns;
+            double* rec = Xr + i * S1;
+            prescale_point(p.Xs + (long)(exists ? i : 0) * (d + 1), exists, d, th, hlL, hlD, rec, 1);
+            rec[2 * d + 4] = rec[2 * d + 3] != 0.0 ? kss_hf : (rec[2 * d + 2] != 0.0 ? vL : 0.0);
+        }
+    }
+    __syncthreads();
+
+    // ---- per 8-point group: K_s, V, var and mean with predict's code (so mean and diag(Sigma) are predict's bits); V^T
+    //      to shared memory
+    for (int grp = warp; grp < NST; grp += PW) {
+        const int i = 8 * grp + g;
+        const double* xg = Xr + i * S1;
+        double ks[2 * NT];
+        ks_fragment<NT>(ks, Xt, xg, d, t, etab);
+        double v[2 * NT];
+        lower_tri_v<NT>(v, ks, Ws, g, t);
+        double ss = sum_sq<NT>(v);
+        ss = quad_sum(ss);
+        if (t == 0) Dg[i] = xg[2 * d + 4] - ss;
+#pragma unroll
+        for (int k = 0; k < NT; ++k) {
+            Vt[i * WP + 8 * k + 2 * t] = v[2 * k];
+            Vt[i * WP + 8 * k + 2 * t + 1] = v[2 * k + 1];
+        }
+        const bool live = i < Ns;
+        if (sample) {
+            contract_table<NT>(v, As, AP, P, g, t, live, [&](int c, double m) { Ms[i * P + c] = m; });
+        } else {
+            double* mrow = p.mean + (b * Ns + i) * P;
+            contract_table<NT>(v, As, AP, P, g, t, live, [&](int c, double m) { mrow[c] = m; });
+        }
+    }
+    __syncthreads();
+
+    // ---- Sigma = K_ss - V^T V on the lower 8x8 tiles (DMMA over the NP training indices), predict's var on the diagonal,
+    //      each entry also stored mirrored: Sigma is exactly symmetric.  Padding rows and columns: identity.
+    for (int tt = warp; tt < NST * (NST + 1) / 2; tt += PW) {
+        int I = 0;
+        while ((I + 1) * (I + 2) / 2 <= tt) ++I;
+        const int J = tt - I * (I + 1) / 2;
+        double c0 = 0.0, c1 = 0.0;
+        const double* ar = Vt + (8 * I + g) * WP + t;
+        const double* br = Vt + (8 * J + g) * WP + t;
+#pragma unroll
+        for (int k = 0; k < 2 * NT; ++k) dmma(c0, c1, ar[4 * k], br[4 * k]);
+        const int i = 8 * I + g;
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            const int j = 8 * J + 2 * t + e;
+            if (j > i) continue;
+            double s;
+            if (i >= Ns || j >= Ns) s = i == j ? 1.0 : 0.0;
+            else if (i == j) s = Dg[i];
+            else s = kss_pair(Xr + i * S1, Xr + j * S1, d, etab) - (e ? c1 : c0);
+            Sg[i * SPp + j] = s;
+            Sg[j * SPp + i] = s;
+        }
+    }
+    __syncthreads();
+
+    if (!sample) {
+        double* cb = p.cov + b * Ns * Ns;
+        for (long idx = tid; idx < (long)Ns * Ns; idx += blockDim.x) {
+            const int i = (int)(idx / Ns), j = (int)(idx - (long)i * Ns);
+            cb[idx] = Sg[i * SPp + j];
+        }
+        return;
+    }
+
+    // ---- L L^T = Sigma + jitter I in place, one column per step (right-looking).  Every thread reads the same pivot, so
+    //      the exit at a pivot that is not > 0 (NaN included) is uniform.  diag(L) goes to Dg, the column to Lc.
+    if (tid == 0) fail = 0;
+    for (int i = tid; i < Ns; i += blockDim.x) Sg[i * SPp + i] += p.jitter;
+    __syncthreads();
+    for (int j = 0; j < Ns; ++j) {
+        const double piv = Sg[j * SPp + j];
+        if (!(piv > 0.0)) {
+            if (tid == 0) fail = j + 1;
+            break;
+        }
+        const double ljj = sqrt(piv);
+        for (int i = j + 1 + tid; i < Ns; i += blockDim.x) {
+            const double l = Sg[i * SPp + j] / ljj;
+            Lc[i] = l;
+            Sg[i * SPp + j] = l;
+        }
+        if (tid == 0) Dg[j] = ljj;
+        __syncthreads();
+        for (int i = j + 1 + warp; i < Ns; i += PW) {
+            const double li = Lc[i];
+            for (int k = j + 1 + lane; k <= i; k += 32) Sg[i * SPp + k] = fma(-li, Lc[k], Sg[i * SPp + k]);
+        }
+        __syncthreads();
+    }
+    __syncthreads();
+    const int bad = fail;
+    for (int idx = tid; idx < NSP * NSP; idx += blockDim.x) {  // L: diagonal from Dg, zero above it
+        const int i = idx / NSP, k = idx - i * NSP;
+        if (k > i) Sg[i * SPp + k] = 0.0;
+        else if (k == i && i < Ns) Sg[i * SPp + k] = Dg[i];
+    }
+    if (blockIdx.x == 0 && tid == 0) {
+        p.info[b] = bad;
+        if (bad) atomicCAS(p.d_info, 0, bad);
+    }
+    __syncthreads();
+
+    // ---- samples = mean + L z over this CTA's columns, JZC at a time: z rows through shared memory (coalesced along the
+    //      S * P axis), L's lower tiles on DMMA (k-steps 0 .. 2I + 1 for row tile I), stores 64 contiguous bytes per row
+    const double qnan = __longlong_as_double(0x7ff8000000000000ll);
+    const long c_beg = blockIdx.x * p.cpc, c_end = c_beg + p.cpc < p.SP ? c_beg + p.cpc : p.SP;
+    const double* __restrict__ zb = p.z + b * Ns * p.SP;
+    double* __restrict__ ob = p.samples + b * Ns * p.SP;
+    for (long c0 = c_beg; c0 < c_end; c0 += JZC) {
+        const int nc = c_end - c0 < JZC ? (int)(c_end - c0) : JZC;
+        if (!bad)  // JL independent loads in flight per thread before the stores
+            for (int base = tid; base < NSP * JZC; base += JL * PW * 32) {
+                double zv[JL];
+#pragma unroll
+                for (int u = 0; u < JL; ++u) {
+                    const int idx = base + u * PW * 32, r = idx / JZC, cc = idx % JZC;
+                    zv[u] = (idx < NSP * JZC && r < Ns && cc < nc) ? zb[(long)r * p.SP + c0 + cc] : 0.0;
+                }
+#pragma unroll
+                for (int u = 0; u < JL; ++u) {
+                    const int idx = base + u * PW * 32;
+                    if (idx < NSP * JZC) Zs[(idx / JZC) * JZP + idx % JZC] = zv[u];
+                }
+            }
+        __syncthreads();
+        for (int tt = warp; tt < NST * (JZC / 8); tt += PW) {
+            const int I = tt / (JZC / 8), Jc = tt % (JZC / 8);
+            double c0v = 0.0, c1v = 0.0;
+            if (!bad) {
+                const double* lr = Sg + (8 * I + g) * SPp + t;
+                const double* zr = Zs + t * JZP + 8 * Jc + g;
+                for (int k = 0; k <= 2 * I + 1; ++k) dmma(c0v, c1v, lr[4 * k], zr[4 * k * JZP]);
+            }
+            const int i = 8 * I + g, cc = 8 * Jc + 2 * t;
+            if (i < Ns) {
+                double* orow = ob + (long)i * p.SP + c0;
+                if (cc < nc) orow[cc] = bad ? qnan : Ms[i * P + (int)((c0 + cc) % P)] + c0v;
+                if (cc + 1 < nc) orow[cc + 1] = bad ? qnan : Ms[i * P + (int)((c0 + cc + 1) % P)] + c1v;
+            }
+        }
+        __syncthreads();
+    }
+}
+
 // Input gradient of the blocked route (launch_posterior_dx): one CTA per (tile of TS test points, chunk of PC columns,
 // problem), walking the training points in tiles of TN.  Per tile it evaluates kL and kD from the scaled inputs (as K5
 // recomputes dK: nothing N x Ns is stored), forms G[j][s][n] = dk_sn/dx_sj in shared memory and adds G alpha (thread =
@@ -1021,6 +1315,56 @@ int gpr_posterior_predict_fused(cudaStream_t s, const GprPosteriorData& q, const
             constexpr int K = decltype(nt)::value;
             return grad ? launch_fused<gpr_posterior_predict_grad_kernel<K>>(s, a, nb, smem)
                         : launch_fused<gpr_posterior_predict_kernel<K>>(s, a, nb, smem);
+        });
+        if (rc) return rc;
+    }
+    return 0;
+}
+
+bool gpr_posterior_joint_fused_ok(int N, int d, int P, int Ns) { return gpr_posterior_fused_ok(N, d, P) && Ns <= JOINT_MAX_NS; }
+
+int gpr_posterior_joint_fused(cudaStream_t s, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
+                              const GprJointOut& j, int* d_info) {
+    if (!gpr_posterior_joint_fused_ok(q.N, q.d, q.P, Ns)) return -1;
+    if (Ns <= 0 || q.B <= 0) return 0;
+    const bool sample = j.SP > 0;
+    const int NT = (q.N + 7) / 8, NST = (Ns + 7) / 8;
+    const size_t smem = sizeof(double) * (size_t)JointSmem(NT, NST, q.d, q.P, sample).total;
+    // sample columns per CTA: about 4 CTAs per SM over the whole call, at least JOINT_MIN_COLS (a multiple of JZC)
+    long cpc = 0, chunks = 1;
+    if (sample) {
+        const long target = (long)mfgp_current_dev_info().sms * 4;
+        const long tot = (long)q.B * j.SP;
+        cpc = round_up((tot + target - 1) / target, JZC);
+        if (cpc < JOINT_MIN_COLS) cpc = JOINT_MIN_COLS;
+        if (cpc > round_up(j.SP, JZC)) cpc = round_up(j.SP, JZC);
+        chunks = (j.SP + cpc - 1) / cpc;
+    }
+    constexpr int MAX_GRID_Y = 65535;
+    for (int b0 = 0; b0 < q.B; b0 += MAX_GRID_Y) {
+        const int nb = q.B - b0 < MAX_GRID_Y ? q.B - b0 : MAX_GRID_Y;
+        JointArgs a{};
+        a.q = q;
+        a.q.B = nb;
+        a.q.theta = q.theta + (long)b0 * (2 * q.d + 3);
+        a.q.noise = q.noise + b0;
+        a.q.W = q.W + (long)b0 * q.N * q.ld;
+        a.q.a = q.a + (long)b0 * q.N * q.Pp;
+        a.Xs = Xs; a.Ns = Ns; a.SP = j.SP; a.cpc = cpc; a.jitter = j.jitter; a.d_info = d_info;
+        if (sample) {
+            a.z = j.z + (long)b0 * Ns * j.SP;
+            a.samples = j.samples + (long)b0 * Ns * j.SP;
+            a.info = j.info + b0;
+        } else {
+            a.mean = mean + (long)b0 * Ns * q.P;
+            a.cov = j.cov + (long)b0 * Ns * Ns;
+        }
+        const int rc = with_nt(NT, [&](auto nt) {
+            constexpr auto K = gpr_posterior_joint_kernel<decltype(nt)::value>;
+            static SmemOptIn optin;
+            if (!optin.ensure(K, smem)) return -2;
+            K<<<dim3((unsigned)chunks, (unsigned)nb), PW * 32, smem, s>>>(a);
+            return cudaGetLastError() == cudaSuccess ? 0 : -2;
         });
         if (rc) return rc;
     }

@@ -86,6 +86,15 @@ class MultiFidelityGPModel:
         post = self.handle.gpr_posterior(X, Y, np.ascontiguousarray(theta)[None, :], np.array([noise]), P=Y.shape[1])
         return MultiFidelityGPPosterior(post, noise)
 
+    def predict_f_samples(self, Xnew, num_samples=None, full_cov=True, full_output_cov=False, seed=None):
+        """GPflow's GPModel.predict_f_samples: [S, N*, P] ([N*, P] when num_samples is None), from a cached posterior made
+        and freed by this call (MultiFidelityGPPosterior.predict_f_samples)."""
+        post = self.posterior()
+        try:
+            return post.predict_f_samples(Xnew, num_samples, full_cov, full_output_cov, seed)
+        finally:
+            post.close()
+
     # ---- training loops (linear.py:190-234) ----------------------------------------------------
     def optimize(self, max_iters=1000, learning_rate=0.01, use_adam=True, unfix_noise_after=500, verbose=True):
         self.loss_history = []
@@ -132,6 +141,20 @@ class MultiFidelityGPPosterior:
     def predict_y(self, Xnew):
         mean, var = self.predict_f(Xnew)
         return mean, var + self.noise
+
+    def predict_f_full_cov(self, Xnew):
+        """GPflow's predict_f(Xnew, full_cov=True): mean [N*, P] and cov [P, N*, N*], the P slices one read-only matrix
+        (every output column shares the kernel)."""
+        mean, cov = self._post.predict_cov(np.ascontiguousarray(Xnew, dtype=np.float64))
+        return mean[0], np.broadcast_to(cov[0], (mean.shape[2],) + cov.shape[1:])
+
+    def predict_f_samples(self, Xnew, num_samples=None, full_cov=True, full_output_cov=False, seed=None):
+        """GPflow's predict_f_samples: [S, N*, P] ([N*, P] when num_samples is None).  full_cov=True draws jointly over
+        the N* points with jitter 1e-6, full_cov=False independently per point.  The normals are
+        np.random.default_rng(seed).standard_normal((1, N*, S, P))."""
+        f = self._post.draw_f(np.ascontiguousarray(Xnew, dtype=np.float64), num_samples, full_cov, full_output_cov, seed)
+        f = np.swapaxes(f[0], 0, 1)  # [S, N*, P]
+        return np.ascontiguousarray(f[0] if num_samples is None else f)
 
     def predict_f_grad(self, Xnew):
         """predict_f and its gradient with respect to Xnew: mean [N*, P], var [N*, P], dmean_dx [N*, P, d+1] and

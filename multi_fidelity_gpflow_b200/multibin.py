@@ -100,6 +100,15 @@ class MultiBinMFGP:
             mean[:, p], var[:, p] = mu[:, 0], s2
         return mean, var
 
+    def predict_f_samples(self, Xnew, num_samples=None, full_cov=True, full_output_cov=False, seed=None):
+        """GPflow's GPModel.predict_f_samples for every bin at its best restart: [S, N*, P] ([N*, P] when num_samples is
+        None), from a cached posterior made and freed by this call (MultiBinPosterior.predict_f_samples)."""
+        post = self.posterior("best")
+        try:
+            return post.predict_f_samples(Xnew, num_samples, full_cov, full_output_cov, seed)
+        finally:
+            post.close()
+
     def posterior(self, restarts="best"):
         """Cached posterior of the bins at the current hyper-parameters (a snapshot: later training does not change it).
         restarts="best": each bin at its best restart, predict_f(Xnew) -> [N*, P] (equal to predict_f);
@@ -153,6 +162,31 @@ class MultiBinPosterior:
         if self.noises.ndim == 1:
             return tuple(np.ascontiguousarray(a[0]) for a in out)
         return tuple(np.ascontiguousarray(a) for a in out)
+
+    def predict_f_full_cov(self, Xnew):
+        """GPflow's predict_f(Xnew, full_cov=True): mean [N*, P] and the joint covariance [P, N*, N*] of each bin ("best"),
+        or the same with a leading restart axis R ("all"; NaN for a failed restart)."""
+        mean, cov = self._post.predict_cov(np.ascontiguousarray(Xnew, dtype=np.float64))  # [B, N*, 1], [B, N*, N*]
+        P, Ns = self.noises.shape[-1], mean.shape[1]
+        mean = np.swapaxes(mean[:, :, 0].reshape(-1, P, Ns), 1, 2)  # [R, N*, P], problem b = r * P + p
+        cov = cov.reshape(-1, P, Ns, Ns)
+        if self.noises.ndim == 1:
+            return np.ascontiguousarray(mean[0]), cov[0]
+        return np.ascontiguousarray(mean), cov
+
+    def predict_f_samples(self, Xnew, num_samples=None, full_cov=True, full_output_cov=False, seed=None):
+        """GPflow's predict_f_samples: draws [S, N*, P] of every bin ([N*, P] when num_samples is None), with a leading
+        restart axis R for "all" (NaN for a restart whose joint covariance cannot be factored; "best" raises
+        NotPositiveDefiniteError instead).  full_cov=True draws jointly over the N* points with jitter 1e-6, full_cov=False
+        independently per point.  The normals are np.random.default_rng(seed).standard_normal((R * P, N*, S, 1))."""
+        info = None if self.failed is None else np.zeros(self.failed.size, dtype=np.int32)
+        f = self._post.draw_f(np.ascontiguousarray(Xnew, dtype=np.float64), num_samples, full_cov, full_output_cov, seed,
+                              info)  # [B, N*, S, 1]
+        P, Ns, S = self.noises.shape[-1], f.shape[1], f.shape[2]
+        f = f[..., 0].reshape(-1, P, Ns, S).transpose(0, 3, 2, 1)  # [R, S, N*, P]
+        if num_samples is None:
+            f = f[:, 0]
+        return np.ascontiguousarray(f[0] if self.noises.ndim == 1 else f)
 
     def predict_y(self, Xnew):
         """predict_f plus each problem's likelihood noise on the variance."""

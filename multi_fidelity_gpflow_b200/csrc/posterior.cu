@@ -2,9 +2,9 @@
 // mfgp_svgp_posterior_predict) for the small problems of the per-bin emulators (N or M <= 64, d <= 16): one launch serves
 // every problem (or latent) and test point.  Also the input-gradient kernel of the exact posterior's blocked route.
 //
-// The three fused kernels share one decomposition.  One CTA per (problem, chunk of test points) stages the problem's
-// factor W = L^-1 (lower triangle) and its scaled training inputs in shared memory once; each warp then takes 8 test
-// points at a time:
+// The five fused kernels are built from one set of device pieces (the building blocks below) on one decomposition.  One
+// CTA per (problem, chunk of test points) stages the problem's factor W = L^-1 (lower triangle) and its scaled training
+// inputs in shared memory once; each warp then takes 8 test points at a time:
 //   K_s^T [8 x N]    built directly in the DMMA A-fragment layout: lane (g, t) evaluates k(x_n, xs_g) for n = 4k + t, so
 //                    every lane computes N / 4 distinct entries and K_s never needs a shared-memory round trip
 //   V^T = K_s^T W^T  mma.sync.m8n8k4.f64 over the lower-triangular tiles of W only (k-steps 0 .. 2i+1 for row tile i);
@@ -149,12 +149,68 @@ __device__ __forceinline__ void prescale_point(const double* __restrict__ x, boo
     out[(2 * d + 3) * stride] = h;
 }
 
+// ---- staging of the fused kernels: one problem's (or latent's) hyperparameters, points and factors in shared memory.
+
+// What the point records of one problem need from its theta th: log(var_L) / 2 and log(var_delta) / 2 (prescale_point),
+// and k_ss at fidelity 0 (var_L) and 1 (K_diag at fidelity 1, as cov_diag_kernel).
+struct RecordParams {
+    const double* th;
+    double hlL, hlD, vL, kss_hf;
+};
+__device__ __forceinline__ RecordParams record_params(const double* th, int d) {
+    const double rho = th[0], vL = th[1 + d], vD = th[2 + 2 * d];
+    return {th, 0.5 * log(vL), 0.5 * log(vD), vL, __dadd_rn(__dmul_rn(vL, __dmul_rn(rho, rho)), vD)};
+}
+
+// Record of test point pt of Xs [Ns][d+1] (rec_len(d) doubles): prescale_point, then k_ss.  pt >= Ns gives a dead
+// record: K_s = 0, and the kernels never store its results.
+__device__ __forceinline__ void point_record(double* rec, const double* Xs, long pt, long Ns, int d,
+                                             const RecordParams& rp) {
+    const bool exists = pt < Ns;
+    prescale_point(Xs + (exists ? pt : 0) * (d + 1), exists, d, rp.th, rp.hlL, rp.hlD, rec, 1);
+    rec[2 * d + 4] = rec[2 * d + 3] != 0.0 ? rp.kss_hf : (rec[2 * d + 2] != 0.0 ? rp.vL : 0.0);
+}
+
+// The N training (or inducing) points X [N][d+1] scaled into Xt [2d+4][NP], k-major; the NP - N padding columns are dead.
+__device__ __forceinline__ void stage_points(double* Xt, const double* X, int N, int NP, int d, const RecordParams& rp,
+                                             int tid) {
+    for (int n = tid; n < NP; n += blockDim.x)
+        prescale_point(X + (long)n * (d + 1), n < N, d, rp.th, rp.hlL, rp.hlD, Xt + n, NP);
+}
+
+// Entry (r, c) of the two staged layouts [NP][WP] of an n x n lower-triangular factor F (leading dimension ld), zero
+// outside the triangle and in the padding.  lower_entry: F itself (lower_tri_v).  transposed_entry: F^T with its columns
+// in the C-fragment order, Ft[c][slot] = F[perm_n(slot)][c] (upper_tri_product, lower_tri_product).  The kernels stage
+// all their copies in one pass over (r, c).
+__device__ __forceinline__ double lower_entry(const double* F, long ld, int n, int r, int c) {
+    return (r < n && c <= r) ? F[(long)r * ld + c] : 0.0;
+}
+__device__ __forceinline__ double transposed_entry(const double* F, long ld, int n, int r, int c) {
+    const int m = perm_n(c);
+    return (m < n && r <= m) ? F[(long)m * ld + r] : 0.0;
+}
+
+// Table T [n][P] (leading dimension ld) into Ts [NP][AP] (contract_table's layout), zero in the padding.
+__device__ __forceinline__ void stage_table(double* Ts, const double* T, long ld, int n, int P, int AP, int NP, int tid) {
+    for (int idx = tid; idx < NP * AP; idx += blockDim.x) {
+        const int r = idx / AP, c = idx - r * AP;
+        Ts[idx] = (r < n && c < P) ? T[(long)r * ld + c] : 0.0;
+    }
+}
+
+// Il [2d] = -1/ls_L, -1/ls_delta: the factors of gk_fragment.
+__device__ __forceinline__ void stage_inv_ls(double* Il, const double* th, int d, int tid) {
+    for (int k = tid; k < d; k += blockDim.x) {
+        Il[k] = -1.0 / th[1 + k];
+        Il[d + k] = -1.0 / th[2 + d + k];
+    }
+}
+
 // ---- building blocks of the fused kernels.  A fragment row `double f[2 * NT]` holds one value per training index of
 //      the lane's point, in the C-fragment order of the file comment (slot 2i + e <-> n = 8i + 2t + e) unless noted.
 
 // K_s^T fragment in the A-fragment order: ks[k] = k(x_n, xs_g), n = 4k + t, from the training points Xt [2d+4][NP]
-// (k-major) and the point record xg (prescale_point, K1's expanded-square form).  The same operations in the same order as
-// the K_s block of gpr_posterior_predict_kernel, which keeps its own copy so that its SASS does not move.
+// (k-major) and the point record xg (point_record, K1's expanded-square form).
 template <int NT>
 __device__ __forceinline__ void ks_fragment(double (&ks)[2 * NT], const double* Xt, const double* xg, int d, int t,
                                             const double* etab) {
@@ -185,6 +241,40 @@ __device__ __forceinline__ void ks_fragment(double (&ks)[2 * NT], const double* 
 #pragma unroll
         for (int k = 0; k < 2 * NT; ++k)
             if (hr[4 * k] * hg != 0.0) ks[k] += fexp512(e[k], etab);
+    }
+}
+
+// A fragment row from the A-fragment order (n = 4k + t) to the C-fragment order, within the quad: slot 2i + e of lane t
+// takes n = 8i + 2t + e, which lane (2t + e) & 3 holds in slot 2i + t / 2.
+template <int NT>
+__device__ __forceinline__ void to_c_order(double (&f)[2 * NT], int lane, int t) {
+    const int src0 = (lane & ~3) | ((2 * t) & 3), src1 = (lane & ~3) | ((2 * t + 1) & 3);
+    const bool hi = t >= 2;
+#pragma unroll
+    for (int i = 0; i < NT; ++i) {
+        const double a0 = __shfl_sync(0xffffffffu, f[2 * i], src0), b0 = __shfl_sync(0xffffffffu, f[2 * i + 1], src0);
+        const double a1 = __shfl_sync(0xffffffffu, f[2 * i], src1), b1 = __shfl_sync(0xffffffffu, f[2 * i + 1], src1);
+        f[2 * i] = hi ? b0 : a0;
+        f[2 * i + 1] = hi ? b1 : a1;
+    }
+}
+
+// gk = dk_s/dx*_j in the C-fragment order, from kL and kD in that order (to_c_order) and Il (stage_inv_ls):
+// gk_n = -kL_n (u*_j - u_nj) / ls_Lj - kD_n (w*_j - w_nj) / ls_dj, differences formed directly.
+template <int NT>
+__device__ __forceinline__ void gk_fragment(double (&gk)[2 * NT], const double (&kL)[2 * NT], const double (&kD)[2 * NT],
+                                            const double* Xt, const double* xg, const double* Il, int d, int j, int t,
+                                            bool anyh) {
+    constexpr int NP = 8 * NT;
+    const double uj = xg[j], cL = Il[j];
+    const double* ur = Xt + j * NP + 2 * t;
+#pragma unroll
+    for (int k = 0; k < 2 * NT; ++k) gk[k] = kL[k] * (uj - ur[slot_off(k)]) * cL;
+    if (anyh) {
+        const double wj = xg[d + j], cD = Il[d + j];
+        const double* wr = Xt + (d + j) * NP + 2 * t;
+#pragma unroll
+        for (int k = 0; k < 2 * NT; ++k) gk[k] = fma(kD[k] * (wj - wr[slot_off(k)]), cD, gk[k]);
     }
 }
 
@@ -286,71 +376,31 @@ __global__ void __launch_bounds__(PW * 32) gpr_posterior_predict_kernel(FusedArg
     double* Xt = As + NP * AP;                        // [2d+4][NP]  training points, k-major
     double* Xw = Xt + (2 * d + 4) * NP + warp * 8 * S1;  // [8][S1]  this warp's test points
     fexp512_table_fill(etab, tid, blockDim.x);
-    const double hlL = 0.5 * log(th[1 + d]), hlD = 0.5 * log(th[2 + 2 * d]);
+    const RecordParams rp = record_params(th, d);
 
     // ---- stage the problem: W (lower triangle; zero above it and in the padding), a, scaled training inputs
     {
         const double* __restrict__ Wg = q.W + b * N * q.ld;
         for (int idx = tid; idx < NP * NP; idx += blockDim.x) {
             const int r = idx / NP, c = idx - r * NP;
-            Ws[r * WP + c] = (r < N && c <= r) ? Wg[(long)r * q.ld + c] : 0.0;
+            Ws[r * WP + c] = lower_entry(Wg, q.ld, N, r, c);
         }
-        const double* __restrict__ ag = q.a + b * N * q.Pp;
-        for (int idx = tid; idx < NP * AP; idx += blockDim.x) {
-            const int r = idx / AP, c = idx - r * AP;
-            As[idx] = (r < N && c < P) ? ag[(long)r * q.Pp + c] : 0.0;
-        }
-        for (int n = tid; n < NP; n += blockDim.x) prescale_point(q.X + (long)n * (d + 1), n < N, d, th, hlL, hlD, Xt + n, NP);
+        stage_table(As, q.a + b * N * q.Pp, q.Pp, N, P, AP, NP, tid);
+        stage_points(Xt, q.X, N, NP, d, rp, tid);
     }
     __syncthreads();
-    const double rho = th[0], vL = th[1 + d], vD = th[2 + 2 * d];
-    const double kss_hf = __dadd_rn(__dmul_rn(vL, __dmul_rn(rho, rho)), vD);  // K_diag at fidelity 1, as cov_diag_kernel
 
     for (int grp = warp; grp < p.gpc; grp += PW) {
         const long pt0 = ((long)blockIdx.x * p.gpc + grp) * 8;
         if (pt0 >= p.Ns) break;
         // ---- this group's 8 test points (padding points beyond Ns are dead: K_s = 0, never stored)
-        if (lane < 8) {
-            const long pt = pt0 + lane;
-            const bool exists = pt < p.Ns;
-            double* rec = Xw + lane * S1;
-            prescale_point(p.Xs + (exists ? pt : 0) * (d + 1), exists, d, th, hlL, hlD, rec, 1);
-            rec[2 * d + 4] = rec[2 * d + 3] != 0.0 ? kss_hf : (rec[2 * d + 2] != 0.0 ? vL : 0.0);
-        }
+        if (lane < 8) point_record(Xw + lane * S1, p.Xs, pt0 + lane, p.Ns, d, rp);
         __syncwarp();
         const double* xg = Xw + g * S1;
-        const double sg = xg[2 * d + 2], hg = xg[2 * d + 3];
 
         // ---- K_s^T fragment: ks[k] = k(x_n, xs_g), n = 4k + t
         double ks[2 * NT];
-        {
-            double e[2 * NT];
-#pragma unroll
-            for (int k = 0; k < 2 * NT; ++k) e[k] = Xt[2 * d * NP + 4 * k + t] + xg[2 * d];
-            for (int c = 0; c < d; ++c) {
-                const double xc = xg[c];
-                const double* xr = Xt + c * NP + t;
-#pragma unroll
-                for (int k = 0; k < 2 * NT; ++k) e[k] = fma(xr[4 * k], xc, e[k]);
-            }
-            const double* sr = Xt + (2 * d + 2) * NP + t;
-#pragma unroll
-            for (int k = 0; k < 2 * NT; ++k) ks[k] = fexp512(e[k], etab) * (sr[4 * k] * sg);
-            if (__any_sync(0xffffffffu, hg != 0.0)) {  // some HF test point: discrepancy GP on the HF x HF pairs
-#pragma unroll
-                for (int k = 0; k < 2 * NT; ++k) e[k] = Xt[(2 * d + 1) * NP + 4 * k + t] + xg[2 * d + 1];
-                for (int c = 0; c < d; ++c) {
-                    const double xc = xg[d + c];
-                    const double* xr = Xt + (d + c) * NP + t;
-#pragma unroll
-                    for (int k = 0; k < 2 * NT; ++k) e[k] = fma(xr[4 * k], xc, e[k]);
-                }
-                const double* hr = Xt + (2 * d + 3) * NP + t;
-#pragma unroll
-                for (int k = 0; k < 2 * NT; ++k)
-                    if (hr[4 * k] * hg != 0.0) ks[k] += fexp512(e[k], etab);
-            }
-        }
+        ks_fragment<NT>(ks, Xt, xg, d, t, etab);
 
         // ---- V^T = K_s^T W^T over the lower-triangular tiles: v[2i + e] = V^T[g][8i + 2t + e]
         double v[2 * NT];
@@ -387,26 +437,19 @@ __global__ void __launch_bounds__(PW * 32) gpr_posterior_predict_grad_kernel(Fus
     double* Il = Xt + (2 * d + 4) * NP;         // [2d]  -1/ls_L, -1/ls_delta
     double* Xw = Il + 2 * d + warp * 8 * S1;    // [8][S1]  this warp's test points
     fexp512_table_fill(etab, tid, blockDim.x);
-    const double hlL = 0.5 * log(th[1 + d]), hlD = 0.5 * log(th[2 + 2 * d]);
+    const RecordParams rp = record_params(th, d);
 
     // ---- stage the problem: W twice (lower triangle, zero elsewhere), a, scaled training inputs; then alpha = W^T a
     {
         const double* __restrict__ Wg = q.W + b * N * q.ld;
         for (int idx = tid; idx < NP * NP; idx += blockDim.x) {
-            const int r = idx / NP, c = idx - r * NP, m = perm_n(c);
-            Ws[r * WP + c] = (r < N && c <= r) ? Wg[(long)r * q.ld + c] : 0.0;
-            Wt[r * WP + c] = (m < N && r <= m) ? Wg[(long)m * q.ld + r] : 0.0;
+            const int r = idx / NP, c = idx - r * NP;
+            Ws[r * WP + c] = lower_entry(Wg, q.ld, N, r, c);
+            Wt[r * WP + c] = transposed_entry(Wg, q.ld, N, r, c);
         }
-        const double* __restrict__ ag = q.a + b * N * q.Pp;
-        for (int idx = tid; idx < NP * AP; idx += blockDim.x) {
-            const int r = idx / AP, c = idx - r * AP;
-            As[idx] = (r < N && c < P) ? ag[(long)r * q.Pp + c] : 0.0;
-        }
-        for (int n = tid; n < NP; n += blockDim.x) prescale_point(q.X + (long)n * (d + 1), n < N, d, th, hlL, hlD, Xt + n, NP);
-        for (int k = tid; k < d; k += blockDim.x) {
-            Il[k] = -1.0 / th[1 + k];
-            Il[d + k] = -1.0 / th[2 + d + k];
-        }
+        stage_table(As, q.a + b * N * q.Pp, q.Pp, N, P, AP, NP, tid);
+        stage_points(Xt, q.X, N, NP, d, rp, tid);
+        stage_inv_ls(Il, th, d, tid);
     }
     __syncthreads();
     for (int idx = tid; idx < NP * AP; idx += blockDim.x) {
@@ -417,19 +460,11 @@ __global__ void __launch_bounds__(PW * 32) gpr_posterior_predict_grad_kernel(Fus
         Al[idx] = s;
     }
     __syncthreads();
-    const double rho = th[0], vL = th[1 + d], vD = th[2 + 2 * d];
-    const double kss_hf = __dadd_rn(__dmul_rn(vL, __dmul_rn(rho, rho)), vD);
 
     for (int grp = warp; grp < p.gpc; grp += PW) {
         const long pt0 = ((long)blockIdx.x * p.gpc + grp) * 8;
         if (pt0 >= p.Ns) break;
-        if (lane < 8) {
-            const long pt = pt0 + lane;
-            const bool exists = pt < p.Ns;
-            double* rec = Xw + lane * S1;
-            prescale_point(p.Xs + (exists ? pt : 0) * (d + 1), exists, d, th, hlL, hlD, rec, 1);
-            rec[2 * d + 4] = rec[2 * d + 3] != 0.0 ? kss_hf : (rec[2 * d + 2] != 0.0 ? vL : 0.0);
-        }
+        if (lane < 8) point_record(Xw + lane * S1, p.Xs, pt0 + lane, p.Ns, d, rp);
         __syncwarp();
         const double* xg = Xw + g * S1;
         const double sg = xg[2 * d + 2], hg = xg[2 * d + 3];
@@ -486,28 +521,9 @@ __global__ void __launch_bounds__(PW * 32) gpr_posterior_predict_grad_kernel(Fus
         double* mrow = p.mean + (b * p.Ns + ptg) * P;
         contract_table<NT>(v, As, AP, P, g, t, live, [&](int c, double m) { mrow[c] = m; });
 
-        // ---- kL, kD to the C-fragment order: slot 2i + e of lane t <- n = 8i + 2t + e, which lane (2t + e) & 3 of the
-        //      quad holds in slot 2i + t / 2
-        {
-            const int src0 = (lane & ~3) | ((2 * t) & 3), src1 = (lane & ~3) | ((2 * t + 1) & 3);
-            const bool hi = t >= 2;
-#pragma unroll
-            for (int i = 0; i < NT; ++i) {
-                const double a0 = __shfl_sync(0xffffffffu, kL[2 * i], src0), b0 = __shfl_sync(0xffffffffu, kL[2 * i + 1], src0);
-                const double a1 = __shfl_sync(0xffffffffu, kL[2 * i], src1), b1 = __shfl_sync(0xffffffffu, kL[2 * i + 1], src1);
-                kL[2 * i] = hi ? b0 : a0;
-                kL[2 * i + 1] = hi ? b1 : a1;
-            }
-            if (anyh) {
-#pragma unroll
-                for (int i = 0; i < NT; ++i) {
-                    const double a0 = __shfl_sync(0xffffffffu, kD[2 * i], src0), b0 = __shfl_sync(0xffffffffu, kD[2 * i + 1], src0);
-                    const double a1 = __shfl_sync(0xffffffffu, kD[2 * i], src1), b1 = __shfl_sync(0xffffffffu, kD[2 * i + 1], src1);
-                    kD[2 * i] = hi ? b0 : a0;
-                    kD[2 * i + 1] = hi ? b1 : a1;
-                }
-            }
-        }
+        // ---- kL, kD to the C-fragment order
+        to_c_order<NT>(kL, lane, t);
+        if (anyh) to_c_order<NT>(kD, lane, t);
 
         // ---- beta^T = V^T W over the tiles m >= n: be[2i + e] = beta[8i + 2t + e], the n of kL[2i + e] / kD[2i + e]
         double be[2 * NT];
@@ -518,49 +534,13 @@ __global__ void __launch_bounds__(PW * 32) gpr_posterior_predict_grad_kernel(Fus
         double* dmrow = p.dmean + (b * p.Ns + ptg) * P * d;
         for (int j = 0; j < d; ++j) {
             double gk[2 * NT];
-            {
-                const double uj = xg[j], cL = Il[j];
-                const double* ur = Xt + j * NP + 2 * t;
-#pragma unroll
-                for (int k = 0; k < 2 * NT; ++k) gk[k] = kL[k] * (uj - ur[slot_off(k)]) * cL;
-                if (anyh) {
-                    const double wj = xg[d + j], cD = Il[d + j];
-                    const double* wr = Xt + (d + j) * NP + 2 * t;
-#pragma unroll
-                    for (int k = 0; k < 2 * NT; ++k) gk[k] = fma(kD[k] * (wj - wr[slot_off(k)]), cD, gk[k]);
-                }
-            }
+            gk_fragment<NT>(gk, kL, kD, Xt, xg, Il, d, j, t, anyh);
             double sv = 0.0;
 #pragma unroll
             for (int k = 0; k < 2 * NT; ++k) sv = fma(be[k], gk[k], sv);
             sv = quad_sum(sv);
             if (t == 0 && live) p.dvar[(b * p.Ns + ptg) * d + j] = -2.0 * sv;
-            if (P >= 8) {
-                for (int jj = 0; jj < (P + 7) / 8; ++jj) {
-                    double c0 = 0.0, c1 = 0.0;
-                    const double* ar = Al + (2 * t) * AP + 8 * jj + g;
-#pragma unroll
-                    for (int i = 0; i < NT; ++i) {
-                        dmma(c0, c1, gk[2 * i], ar[(8 * i) * AP]);
-                        dmma(c0, c1, gk[2 * i + 1], ar[(8 * i + 1) * AP]);
-                    }
-                    const int col = 8 * jj + 2 * t;
-                    if (live) {
-                        if (col < P) dmrow[col * d + j] = c0;
-                        if (col + 1 < P) dmrow[(col + 1) * d + j] = c1;
-                    }
-                }
-            } else {
-                for (int c = 0; c < P; ++c) {
-                    const double* ar = Al + (2 * t) * AP + c;
-                    double m = 0.0;
-#pragma unroll
-                    for (int i = 0; i < NT; ++i)
-                        m = fma(gk[2 * i + 1], ar[(8 * i + 1) * AP], fma(gk[2 * i], ar[(8 * i) * AP], m));
-                    m = quad_sum(m);
-                    if (t == 0 && live) dmrow[c * d + j] = m;
-                }
-            }
+            contract_table<NT>(gk, Al, AP, P, g, t, live, [&](int c, double m) { dmrow[c * d + j] = m; });
         }
         __syncwarp();
     }
@@ -582,69 +562,33 @@ __global__ void __launch_bounds__(PW * 32) svgp_posterior_predict_kernel(SvgpFus
     double* Xt = Qs + NP;                             // [2d+4][NP]  inducing points, k-major
     double* Xw = Xt + (2 * d + 4) * NP + warp * 8 * S1;  // [8][S1]  this warp's test points
     fexp512_table_fill(etab, tid, blockDim.x);
-    const double hlL = 0.5 * log(th[1 + d]), hlD = 0.5 * log(th[2 + 2 * d]);
+    const RecordParams rp = record_params(th, d);
 
     // ---- stage the latent: Wm and Lq^T (lower triangles; zero elsewhere), q_mu, scaled inducing points
     {
         const double* __restrict__ Wg = q.Wm + l * M * q.ld;
         const double* __restrict__ Lg = q.Lq + l * M * q.ld;
         for (int idx = tid; idx < NP * NP; idx += blockDim.x) {
-            const int r = idx / NP, c = idx - r * NP, m = perm_n(c);
-            Ws[r * WP + c] = (r < M && c <= r) ? Wg[(long)r * q.ld + c] : 0.0;
-            Lt[r * WP + c] = (m < M && r <= m) ? Lg[(long)m * q.ld + r] : 0.0;
+            const int r = idx / NP, c = idx - r * NP;
+            Ws[r * WP + c] = lower_entry(Wg, q.ld, M, r, c);
+            Lt[r * WP + c] = transposed_entry(Lg, q.ld, M, r, c);
         }
-        for (int m = tid; m < NP; m += blockDim.x) Qs[m] = m < M ? q.q_mu[(long)m * q.L + l] : 0.0;
-        for (int n = tid; n < NP; n += blockDim.x) prescale_point(q.Z + (long)n * (d + 1), n < M, d, th, hlL, hlD, Xt + n, NP);
+        stage_table(Qs, q.q_mu + l, q.L, M, 1, 1, NP, tid);
+        stage_points(Xt, q.Z, M, NP, d, rp, tid);
     }
     __syncthreads();
-    const double rho = th[0], vL = th[1 + d], vD = th[2 + 2 * d];
-    const double kss_hf = __dadd_rn(__dmul_rn(vL, __dmul_rn(rho, rho)), vD);  // K_diag at fidelity 1, as cov_diag_kernel
 
     for (int grp = warp; grp < p.gpc; grp += PW) {
         const long pt0 = ((long)blockIdx.x * p.gpc + grp) * 8;
         if (pt0 >= p.Ns) break;
         // ---- this group's 8 test points (padding points beyond Ns are dead: K_s = 0, never stored)
-        if (lane < 8) {
-            const long pt = pt0 + lane;
-            const bool exists = pt < p.Ns;
-            double* rec = Xw + lane * S1;
-            prescale_point(p.Xs + (exists ? pt : 0) * (d + 1), exists, d, th, hlL, hlD, rec, 1);
-            rec[2 * d + 4] = rec[2 * d + 3] != 0.0 ? kss_hf : (rec[2 * d + 2] != 0.0 ? vL : 0.0);
-        }
+        if (lane < 8) point_record(Xw + lane * S1, p.Xs, pt0 + lane, p.Ns, d, rp);
         __syncwarp();
         const double* xg = Xw + g * S1;
-        const double sg = xg[2 * d + 2], hg = xg[2 * d + 3];
 
         // ---- K_s^T fragment: ks[k] = k(z_m, xs_g), m = 4k + t
         double ks[2 * NT];
-        {
-            double e[2 * NT];
-#pragma unroll
-            for (int k = 0; k < 2 * NT; ++k) e[k] = Xt[2 * d * NP + 4 * k + t] + xg[2 * d];
-            for (int c = 0; c < d; ++c) {
-                const double xc = xg[c];
-                const double* xr = Xt + c * NP + t;
-#pragma unroll
-                for (int k = 0; k < 2 * NT; ++k) e[k] = fma(xr[4 * k], xc, e[k]);
-            }
-            const double* sr = Xt + (2 * d + 2) * NP + t;
-#pragma unroll
-            for (int k = 0; k < 2 * NT; ++k) ks[k] = fexp512(e[k], etab) * (sr[4 * k] * sg);
-            if (__any_sync(0xffffffffu, hg != 0.0)) {  // some HF test point: discrepancy GP on the HF x HF pairs
-#pragma unroll
-                for (int k = 0; k < 2 * NT; ++k) e[k] = Xt[(2 * d + 1) * NP + 4 * k + t] + xg[2 * d + 1];
-                for (int c = 0; c < d; ++c) {
-                    const double xc = xg[d + c];
-                    const double* xr = Xt + (d + c) * NP + t;
-#pragma unroll
-                    for (int k = 0; k < 2 * NT; ++k) e[k] = fma(xr[4 * k], xc, e[k]);
-                }
-                const double* hr = Xt + (2 * d + 3) * NP + t;
-#pragma unroll
-                for (int k = 0; k < 2 * NT; ++k)
-                    if (hr[4 * k] * hg != 0.0) ks[k] += fexp512(e[k], etab);
-            }
-        }
+        ks_fragment<NT>(ks, Xt, xg, d, t, etab);
 
         // ---- V^T = K_s^T Wm^T over the lower-triangular tiles: v[2i + e] = V^T[g][8i + 2t + e]
         double v[2 * NT];
@@ -661,21 +605,13 @@ __global__ void __launch_bounds__(PW * 32) svgp_posterior_predict_kernel(SvgpFus
         }
         ss = quad_sum(ss);
         su = quad_sum(su);
-
-        // ---- mean = V^T q_mu
-        double m = 0.0;
-        {
-            const double* qr = Qs + 2 * t;
-#pragma unroll
-            for (int i = 0; i < NT; ++i) m = fma(v[2 * i + 1], qr[8 * i + 1], fma(v[2 * i], qr[8 * i], m));
-        }
-        m = quad_sum(m);
         const long ptg = pt0 + g;
-        if (t == 0 && ptg < p.Ns) {
-            const long o = l * p.ls + ptg * p.ns;
-            p.mean[o] = m;
-            p.var[o] = xg[2 * d + 4] - ss + su;
-        }
+        const bool live = ptg < p.Ns;
+        const long o = l * p.ls + ptg * p.ns;
+        if (t == 0 && live) p.var[o] = xg[2 * d + 4] - ss + su;
+
+        // ---- mean = V^T q_mu: q_mu as a table with one column
+        contract_table<NT>(v, Qs, 1, 1, g, t, live, [&](int, double m) { p.mean[o] = m; });
         __syncwarp();  // the group's records are read by every lane before lanes 0-7 overwrite them
     }
 }
@@ -699,24 +635,21 @@ __global__ void __launch_bounds__(PW * 32, 1) svgp_posterior_predict_grad_kernel
     double* Il = Xt + (2 * d + 4) * NP;         // [2d]  -1/ls_L, -1/ls_delta
     double* Xw = Il + 2 * d + warp * 8 * S1;    // [8][S1]  this warp's test points
     fexp512_table_fill(etab, tid, blockDim.x);
-    const double hlL = 0.5 * log(th[1 + d]), hlD = 0.5 * log(th[2 + 2 * d]);
+    const RecordParams rp = record_params(th, d);
 
     // ---- stage the latent: Wm (twice), Lq^T (lower triangles; zero elsewhere), q_mu, scaled inducing points; then alpha
     {
         const double* __restrict__ Wg = q.Wm + l * M * q.ld;
         const double* __restrict__ Lg = q.Lq + l * M * q.ld;
         for (int idx = tid; idx < NP * NP; idx += blockDim.x) {
-            const int r = idx / NP, c = idx - r * NP, m = perm_n(c);
-            Ws[r * WP + c] = (r < M && c <= r) ? Wg[(long)r * q.ld + c] : 0.0;
-            Lt[r * WP + c] = (m < M && r <= m) ? Lg[(long)m * q.ld + r] : 0.0;
-            Wt[r * WP + c] = (m < M && r <= m) ? Wg[(long)m * q.ld + r] : 0.0;
+            const int r = idx / NP, c = idx - r * NP;
+            Ws[r * WP + c] = lower_entry(Wg, q.ld, M, r, c);
+            Lt[r * WP + c] = transposed_entry(Lg, q.ld, M, r, c);
+            Wt[r * WP + c] = transposed_entry(Wg, q.ld, M, r, c);
         }
-        for (int m = tid; m < NP; m += blockDim.x) Qs[m] = m < M ? q.q_mu[(long)m * q.L + l] : 0.0;
-        for (int n = tid; n < NP; n += blockDim.x) prescale_point(q.Z + (long)n * (d + 1), n < M, d, th, hlL, hlD, Xt + n, NP);
-        for (int k = tid; k < d; k += blockDim.x) {
-            Il[k] = -1.0 / th[1 + k];
-            Il[d + k] = -1.0 / th[2 + d + k];
-        }
+        stage_table(Qs, q.q_mu + l, q.L, M, 1, 1, NP, tid);
+        stage_points(Xt, q.Z, M, NP, d, rp, tid);
+        stage_inv_ls(Il, th, d, tid);
     }
     __syncthreads();
     for (int n = tid; n < NP; n += blockDim.x) {
@@ -725,19 +658,11 @@ __global__ void __launch_bounds__(PW * 32, 1) svgp_posterior_predict_grad_kernel
         Al[n] = s;
     }
     __syncthreads();
-    const double rho = th[0], vL = th[1 + d], vD = th[2 + 2 * d];
-    const double kss_hf = __dadd_rn(__dmul_rn(vL, __dmul_rn(rho, rho)), vD);  // K_diag at fidelity 1, as cov_diag_kernel
 
     for (int grp = warp; grp < p.gpc; grp += PW) {
         const long pt0 = ((long)blockIdx.x * p.gpc + grp) * 8;
         if (pt0 >= p.Ns) break;
-        if (lane < 8) {
-            const long pt = pt0 + lane;
-            const bool exists = pt < p.Ns;
-            double* rec = Xw + lane * S1;
-            prescale_point(p.Xs + (exists ? pt : 0) * (d + 1), exists, d, th, hlL, hlD, rec, 1);
-            rec[2 * d + 4] = rec[2 * d + 3] != 0.0 ? kss_hf : (rec[2 * d + 2] != 0.0 ? vL : 0.0);
-        }
+        if (lane < 8) point_record(Xw + lane * S1, p.Xs, pt0 + lane, p.Ns, d, rp);
         __syncwarp();
         const double* xg = Xw + g * S1;
         const double sg = xg[2 * d + 2], hg = xg[2 * d + 3];
@@ -796,20 +721,11 @@ __global__ void __launch_bounds__(PW * 32, 1) svgp_posterior_predict_grad_kernel
         }
         ss = quad_sum(ss);
         su = quad_sum(su);
-        double m = 0.0;
-        {
-            const double* qr = Qs + 2 * t;
-#pragma unroll
-            for (int i = 0; i < NT; ++i) m = fma(v[2 * i + 1], qr[8 * i + 1], fma(v[2 * i], qr[8 * i], m));
-        }
-        m = quad_sum(m);
         const long ptg = pt0 + g;
         const bool live = ptg < p.Ns;
-        if (t == 0 && live) {
-            const long o = l * p.ls + ptg * p.ns;
-            p.mean[o] = m;
-            p.var[o] = xg[2 * d + 4] - ss + su;
-        }
+        const long o = l * p.ls + ptg * p.ns;
+        if (t == 0 && live) p.var[o] = xg[2 * d + 4] - ss + su;
+        contract_table<NT>(v, Qs, 1, 1, g, t, live, [&](int, double m) { p.mean[o] = m; });
 
         // ---- r = V - Lq U over the tiles m <= n (Lt read transposed), then beta^T = r^T Wm over the tiles m >= n:
         //      be[2i + e] = beta[8i + 2t + e]
@@ -827,46 +743,16 @@ __global__ void __launch_bounds__(PW * 32, 1) svgp_posterior_predict_grad_kernel
         }
         const double(&be)[2 * NT] = v;
 
-        // ---- kL, kD to the C-fragment order: slot 2i + e of lane t <- m = 8i + 2t + e, which lane (2t + e) & 3 of the
-        //      quad holds in slot 2i + t / 2
-        {
-            const int src0 = (lane & ~3) | ((2 * t) & 3), src1 = (lane & ~3) | ((2 * t + 1) & 3);
-            const bool hi = t >= 2;
-#pragma unroll
-            for (int i = 0; i < NT; ++i) {
-                const double a0 = __shfl_sync(0xffffffffu, kL[2 * i], src0), b0 = __shfl_sync(0xffffffffu, kL[2 * i + 1], src0);
-                const double a1 = __shfl_sync(0xffffffffu, kL[2 * i], src1), b1 = __shfl_sync(0xffffffffu, kL[2 * i + 1], src1);
-                kL[2 * i] = hi ? b0 : a0;
-                kL[2 * i + 1] = hi ? b1 : a1;
-            }
-            if (anyh) {
-#pragma unroll
-                for (int i = 0; i < NT; ++i) {
-                    const double a0 = __shfl_sync(0xffffffffu, kD[2 * i], src0), b0 = __shfl_sync(0xffffffffu, kD[2 * i + 1], src0);
-                    const double a1 = __shfl_sync(0xffffffffu, kD[2 * i], src1), b1 = __shfl_sync(0xffffffffu, kD[2 * i + 1], src1);
-                    kD[2 * i] = hi ? b0 : a0;
-                    kD[2 * i + 1] = hi ? b1 : a1;
-                }
-            }
-        }
+        // ---- kL, kD to the C-fragment order
+        to_c_order<NT>(kL, lane, t);
+        if (anyh) to_c_order<NT>(kD, lane, t);
 
         // ---- per coordinate j: gk = dk_s/dx*_j, dvar_j = -2 beta . gk, dmean_j = alpha . gk
         const double* ar = Al + 2 * t;
-        const long od = (l * p.ls + ptg * p.ns) * d;
+        const long od = o * d;
         for (int j = 0; j < d; ++j) {
             double gk[2 * NT];
-            {
-                const double uj = xg[j], cL = Il[j];
-                const double* ur = Xt + j * NP + 2 * t;
-#pragma unroll
-                for (int k = 0; k < 2 * NT; ++k) gk[k] = kL[k] * (uj - ur[slot_off(k)]) * cL;
-                if (anyh) {
-                    const double wj = xg[d + j], cD = Il[d + j];
-                    const double* wr = Xt + (d + j) * NP + 2 * t;
-#pragma unroll
-                    for (int k = 0; k < 2 * NT; ++k) gk[k] = fma(kD[k] * (wj - wr[slot_off(k)]), cD, gk[k]);
-                }
-            }
+            gk_fragment<NT>(gk, kL, kD, Xt, xg, Il, d, j, t, anyh);
             double sv = 0.0, sa = 0.0;
 #pragma unroll
             for (int i = 0; i < NT; ++i) {
@@ -969,29 +855,18 @@ __global__ void __launch_bounds__(PW * 32) gpr_posterior_joint_kernel(JointArgs 
     double* Lc = sm + lay.lc;
     double* Ms = sm + lay.ms;
     fexp512_table_fill(etab, tid, blockDim.x);
-    const double hlL = 0.5 * log(th[1 + d]), hlD = 0.5 * log(th[2 + 2 * d]);
-    const double rho = th[0], vL = th[1 + d], vD = th[2 + 2 * d];
-    const double kss_hf = __dadd_rn(__dmul_rn(vL, __dmul_rn(rho, rho)), vD);  // as gpr_posterior_predict_kernel
+    const RecordParams rp = record_params(th, d);
 
     // ---- stage the problem as gpr_posterior_predict_kernel does, and the records of every test point (padding: dead)
     {
         const double* __restrict__ Wg = q.W + b * N * q.ld;
         for (int idx = tid; idx < NP * NP; idx += blockDim.x) {
             const int r = idx / NP, c = idx - r * NP;
-            Ws[r * WP + c] = (r < N && c <= r) ? Wg[(long)r * q.ld + c] : 0.0;
+            Ws[r * WP + c] = lower_entry(Wg, q.ld, N, r, c);
         }
-        const double* __restrict__ ag = q.a + b * N * q.Pp;
-        for (int idx = tid; idx < NP * AP; idx += blockDim.x) {
-            const int r = idx / AP, c = idx - r * AP;
-            As[idx] = (r < N && c < P) ? ag[(long)r * q.Pp + c] : 0.0;
-        }
-        for (int n = tid; n < NP; n += blockDim.x) prescale_point(q.X + (long)n * (d + 1), n < N, d, th, hlL, hlD, Xt + n, NP);
-        for (int i = tid; i < NSP; i += blockDim.x) {
-            const bool exists = i < Ns;
-            double* rec = Xr + i * S1;
-            prescale_point(p.Xs + (long)(exists ? i : 0) * (d + 1), exists, d, th, hlL, hlD, rec, 1);
-            rec[2 * d + 4] = rec[2 * d + 3] != 0.0 ? kss_hf : (rec[2 * d + 2] != 0.0 ? vL : 0.0);
-        }
+        stage_table(As, q.a + b * N * q.Pp, q.Pp, N, P, AP, NP, tid);
+        stage_points(Xt, q.X, N, NP, d, rp, tid);
+        for (int i = tid; i < NSP; i += blockDim.x) point_record(Xr + i * S1, p.Xs, i, Ns, d, rp);
     }
     __syncthreads();
 
@@ -1269,15 +1144,37 @@ int with_nt(int NT, F f) {
     }
 }
 
-// One launch of a fused kernel over `batch` problems (grid y) and the 8-point groups of a.Ns (grid x, a.gpc per CTA).
+// CTAs along grid x of a predict kernel: the 8-point groups of Ns, gpc per CTA.
+long point_chunks(int Ns, int gpc) {
+    const long G = (Ns + 7) / 8;
+    return (G + gpc - 1) / gpc;
+}
+
+// One launch of a fused kernel over `batch` problems (grid y) and gx CTAs along grid x.
 template <auto Kernel, class Args>
-int launch_fused(cudaStream_t s, const Args& a, int batch, size_t smem) {
+int launch_fused(cudaStream_t s, const Args& a, long gx, int batch, size_t smem) {
     static SmemOptIn optin;
     if (!optin.ensure(Kernel, smem)) return -2;
-    const long G = (a.Ns + 7) / 8;
-    dim3 grid((unsigned)((G + a.gpc - 1) / a.gpc), (unsigned)batch);
-    Kernel<<<grid, PW * 32, smem, s>>>(a);
+    Kernel<<<dim3((unsigned)gx, (unsigned)batch), PW * 32, smem, s>>>(a);
     return cudaGetLastError() == cudaSuccess ? 0 : -2;
+}
+
+// f(qs, b0) for the problems of q in slices of at most 65 535 (the grid-y limit): qs describes problems b0 .. b0 + qs.B - 1
+// as a batch of their own.  Stops at the first nonzero return.
+template <class F>
+int for_batch_slices(const GprPosteriorData& q, F f) {
+    constexpr int MAX_GRID_Y = 65535;
+    for (int b0 = 0; b0 < q.B; b0 += MAX_GRID_Y) {
+        GprPosteriorData qs = q;
+        qs.B = q.B - b0 < MAX_GRID_Y ? q.B - b0 : MAX_GRID_Y;
+        qs.theta = q.theta + (long)b0 * (2 * q.d + 3);
+        qs.noise = q.noise + b0;
+        qs.W = q.W + (long)b0 * q.N * q.ld;
+        qs.a = q.a + (long)b0 * q.N * q.Pp;
+        const int rc = f(qs, (long)b0);
+        if (rc) return rc;
+    }
+    return 0;
 }
 
 }  // namespace
@@ -1294,31 +1191,23 @@ int gpr_posterior_predict_fused(cudaStream_t s, const GprPosteriorData& q, const
     const int NT = (q.N + 7) / 8;
     const size_t smem = grad ? fused_grad_smem_bytes(NT, q.d, q.P) : fused_smem_bytes(NT, q.d, q.P);
     const int gpc = groups_per_cta(Ns, q.B);
-    constexpr int MAX_GRID_Y = 65535;
-    for (int b0 = 0; b0 < q.B; b0 += MAX_GRID_Y) {
-        const int nb = q.B - b0 < MAX_GRID_Y ? q.B - b0 : MAX_GRID_Y;
+    const long gx = point_chunks(Ns, gpc);
+    return for_batch_slices(q, [&](const GprPosteriorData& qs, long b0) {
         FusedArgs a{};
-        a.q = q;
-        a.q.B = nb;
-        a.q.theta = q.theta + (long)b0 * (2 * q.d + 3);
-        a.q.noise = q.noise + b0;
-        a.q.W = q.W + (long)b0 * q.N * q.ld;
-        a.q.a = q.a + (long)b0 * q.N * q.Pp;
+        a.q = qs;
         a.Xs = Xs; a.Ns = Ns; a.gpc = gpc;
-        a.mean = mean + (long)b0 * Ns * q.P;
-        a.var = var + (long)b0 * Ns;
+        a.mean = mean + b0 * Ns * q.P;
+        a.var = var + b0 * Ns;
         if (grad) {
-            a.dmean = dmean + (long)b0 * Ns * q.P * q.d;
-            a.dvar = dvar + (long)b0 * Ns * q.d;
+            a.dmean = dmean + b0 * Ns * q.P * q.d;
+            a.dvar = dvar + b0 * Ns * q.d;
         }
-        const int rc = with_nt(NT, [&](auto nt) {
+        return with_nt(NT, [&](auto nt) {
             constexpr int K = decltype(nt)::value;
-            return grad ? launch_fused<gpr_posterior_predict_grad_kernel<K>>(s, a, nb, smem)
-                        : launch_fused<gpr_posterior_predict_kernel<K>>(s, a, nb, smem);
+            return grad ? launch_fused<gpr_posterior_predict_grad_kernel<K>>(s, a, gx, qs.B, smem)
+                        : launch_fused<gpr_posterior_predict_kernel<K>>(s, a, gx, qs.B, smem);
         });
-        if (rc) return rc;
-    }
-    return 0;
+    });
 }
 
 bool gpr_posterior_joint_fused_ok(int N, int d, int P, int Ns) { return gpr_posterior_fused_ok(N, d, P) && Ns <= JOINT_MAX_NS; }
@@ -1340,35 +1229,22 @@ int gpr_posterior_joint_fused(cudaStream_t s, const GprPosteriorData& q, const d
         if (cpc > round_up(j.SP, JZC)) cpc = round_up(j.SP, JZC);
         chunks = (j.SP + cpc - 1) / cpc;
     }
-    constexpr int MAX_GRID_Y = 65535;
-    for (int b0 = 0; b0 < q.B; b0 += MAX_GRID_Y) {
-        const int nb = q.B - b0 < MAX_GRID_Y ? q.B - b0 : MAX_GRID_Y;
+    return for_batch_slices(q, [&](const GprPosteriorData& qs, long b0) {
         JointArgs a{};
-        a.q = q;
-        a.q.B = nb;
-        a.q.theta = q.theta + (long)b0 * (2 * q.d + 3);
-        a.q.noise = q.noise + b0;
-        a.q.W = q.W + (long)b0 * q.N * q.ld;
-        a.q.a = q.a + (long)b0 * q.N * q.Pp;
+        a.q = qs;
         a.Xs = Xs; a.Ns = Ns; a.SP = j.SP; a.cpc = cpc; a.jitter = j.jitter; a.d_info = d_info;
         if (sample) {
-            a.z = j.z + (long)b0 * Ns * j.SP;
-            a.samples = j.samples + (long)b0 * Ns * j.SP;
+            a.z = j.z + b0 * Ns * j.SP;
+            a.samples = j.samples + b0 * Ns * j.SP;
             a.info = j.info + b0;
         } else {
-            a.mean = mean + (long)b0 * Ns * q.P;
-            a.cov = j.cov + (long)b0 * Ns * Ns;
+            a.mean = mean + b0 * Ns * q.P;
+            a.cov = j.cov + b0 * Ns * Ns;
         }
-        const int rc = with_nt(NT, [&](auto nt) {
-            constexpr auto K = gpr_posterior_joint_kernel<decltype(nt)::value>;
-            static SmemOptIn optin;
-            if (!optin.ensure(K, smem)) return -2;
-            K<<<dim3((unsigned)chunks, (unsigned)nb), PW * 32, smem, s>>>(a);
-            return cudaGetLastError() == cudaSuccess ? 0 : -2;
+        return with_nt(NT, [&](auto nt) {
+            return launch_fused<gpr_posterior_joint_kernel<decltype(nt)::value>>(s, a, chunks, qs.B, smem);
         });
-        if (rc) return rc;
-    }
-    return 0;
+    });
 }
 
 int launch_posterior_dx(cudaStream_t s, const GprPosteriorData& q, int nb, const double* Xs, int Ns, const double* alpha,
@@ -1391,15 +1267,16 @@ int svgp_posterior_predict_fused(cudaStream_t s, const SvgpPosteriorData& q, con
     if (Ns <= 0) return 0;
     const int NT = (q.M + 7) / 8;
     const SvgpFusedArgs a{q, Xs, Ns, groups_per_cta(Ns, q.L), mean, var, ls, ns};
+    const long gx = point_chunks(Ns, a.gpc);
     if (dmean) {
         const SvgpFusedGradArgs ag{a, dmean, dvar};
+        const size_t smem = svgp_fused_grad_smem_bytes(NT, q.d);
         return with_nt(NT, [&](auto nt) {
-            return launch_fused<svgp_posterior_predict_grad_kernel<decltype(nt)::value>>(s, ag, q.L,
-                                                                                        svgp_fused_grad_smem_bytes(NT, q.d));
+            return launch_fused<svgp_posterior_predict_grad_kernel<decltype(nt)::value>>(s, ag, gx, q.L, smem);
         });
     }
     const size_t smem = svgp_fused_smem_bytes(NT, q.d);
     return with_nt(NT, [&](auto nt) {
-        return launch_fused<svgp_posterior_predict_kernel<decltype(nt)::value>>(s, a, q.L, smem);
+        return launch_fused<svgp_posterior_predict_kernel<decltype(nt)::value>>(s, a, gx, q.L, smem);
     });
 }

@@ -96,7 +96,8 @@ int mfgp_gpr_batched_nlml_grad(mfgp_handle* h, const double* X, int N, int d, co
  *    destroyed before or after the handle that created it.
  *  - info [B] or NULL.  With info, a non-PD problem is that problem's status (1-based pivot in info[b]), it predicts NaN,
  *    *out is set and the call returns the first failure's pivot like the other batched calls.  Without info, a non-PD
- *    problem makes the call return its pivot with *out = NULL.  Creation always synchronises (it decides what is returned).
+ *    problem makes the call return its pivot with *out = NULL.  Creation always synchronises (it decides what is returned;
+ *    mfgp_gpr_batched_lbfgs does too, because when it ends depends on the data).
  *  - Cost: the blocked batched factorisation (K1 -> potrf -> trtri -> a = W Y), chunked over B by free memory.
  * mfgp_gpr_posterior_predict: mean [B, Ns, P], var [B, Ns] (the same for every column, like mfgp_gpr_predict); host or
  * device pointers, async mode as for every call.  N <= 64, d <= 16, P <= 64 run ONE fused kernel for all problems and
@@ -156,6 +157,42 @@ int mfgp_gpr_posterior_destroy(mfgp_gpr_posterior* post);
 int mfgp_gpr_batched_adam(mfgp_handle* h, const double* X, int N, int d, const double* Y, long ldy, int ycols, int B,
                           double* u, double* m, double* v, const double* noise, const double* lr_t, double beta1,
                           double beta2, double eps, int fix_rho, int nsteps, double* loss_hist, double* theta_out, int* info);
+
+/* Multi-start L-BFGS on the device: the SciPy branch of MultiFidelityGPModel.optimize (mfgpflow/linear.py:222-234,
+ * gpflow.optimizers.Scipy -> scipy.optimize.minimize(method="L-BFGS-B")) for B independent per-bin GPs in one loop.
+ * Problem indexing, Y, X and the limits (N <= 64, d <= 16) are those of mfgp_gpr_batched_nlml_grad (b = r * bins + p).
+ *  - Variables: u [B, 2d+3] in/out, theta = softplus(u) as in mfgp_gpr_batched_adam.  fix_rho != 0 keeps rho out of the
+ *    variable vector (u[b, 0] is left bit for bit).  train_noise == 0 uses noise [B] exactly as passed (then the objective
+ *    is Adam's, bit for bit); train_noise != 0 adds the variable v, noise = 1e-6 + softplus(v) (gpflow Gaussian's lower
+ *    bound), started at v = softplus^-1(noise - 1e-6) and written back to noise at the end.
+ *  - Algorithm: SciPy's L-BFGS-B on unbounded variables, written out: two-loop direction over the last m pairs, MINPACK-2
+ *    dcsrch line search (ftol 1e-3, gtol 0.9, xtol 0.1), stp = min(1/||d||, 1e10) on iteration 0.  After an accepted step
+ *    the tests run in SciPy's order: nit >= maxiter, nfev > maxfun, ||g||_inf <= gtol, relative reduction of f <= ftol.
+ *    One deliberate deviation: a trial point whose covariance is not positive definite, or whose objective or gradient is
+ *    not finite, fails that problem's trial only (GPflow's closure would abort the whole minimize).  It counts as an
+ *    evaluation and against maxls, and the search restarts from its base point with stp = 0.1 x the failed step and
+ *    stpmax = 0.5 x the failed step.
+ *  - opts NULL = SciPy's defaults {m 10, maxiter 15000, maxfun 15000, maxls 20, ftol 2.220446049250313e-09, gtol 1e-5};
+ *    1 <= m <= MFGP_LBFGS_MAX_M, maxiter, maxfun, maxls >= 1, ftol, gtol >= 0.
+ *  - Outputs [B]: f (final loss, NaN for MFGP_LBFGS_NOT_PD), nit, nfev, status (MFGP_LBFGS_*), info or NULL.  A problem
+ *    whose START point fails stops with MFGP_LBFGS_NOT_PD, its 1-based pivot in info[b] (0 when the factor exists but the
+ *    objective is not finite) and its u and noise unchanged.  The call returns the pivot of the lowest-index such
+ *    problem: with info that is the problems' status, without info the call's error, as for the other batched calls.
+ *  - Cost: one round = one K6 launch over all B problems at their current trial points + one lbfgs_step_kernel.  Finished
+ *    problems stay in the K6 launch at their last point.  The host reads the number of active problems every 16 rounds.
+ *  - A problem's results do not depend on the other problems of the call.  Host or device pointers.  The call always
+ *    synchronises: when it ends depends on the data (as for mfgp_gpr_posterior_create). */
+#define MFGP_LBFGS_PGTOL 1    /* ||g||_inf <= gtol */
+#define MFGP_LBFGS_FTOL 2     /* (f_old - f) <= ftol * max(|f_old|, |f|, 1) */
+#define MFGP_LBFGS_MAXITER 3  /* nit reached maxiter */
+#define MFGP_LBFGS_MAXFUN 4   /* nfev exceeded maxfun */
+#define MFGP_LBFGS_ABNORMAL 5 /* the line search failed with an empty memory ("ABNORMAL_TERMINATION_IN_LNSRCH") */
+#define MFGP_LBFGS_NOT_PD 6   /* the start point is not positive definite or not finite */
+#define MFGP_LBFGS_MAX_M 32
+typedef struct { int m, maxiter, maxfun, maxls; double ftol, gtol; } mfgp_lbfgs_opts;
+int mfgp_gpr_batched_lbfgs(mfgp_handle* h, const double* X, int N, int d, const double* Y, long ldy, int ycols, int B,
+                           double* u, double* noise, int fix_rho, int train_noise, const mfgp_lbfgs_opts* opts,
+                           double* f, int* nit, int* nfev, int* status, int* info);
 
 /* ---- Graph-structured multi-fidelity kernel (SURVEY 8(f) rank 3) ---------------------------------------------------
  * replaces GraphMultiFidelityKernel.K / K_diag (mfgpflow/graph.py:39-93, :96-115) and, for GraphMultiFidelityGPModel

@@ -50,6 +50,7 @@ def _load():
         "mfgp_gpr_predict": ([vp, vp, vp, i, i, i, vp, i, vp, d, vp, vp], i),
         "mfgp_gpr_batched_nlml_grad": ([vp, vp, i, i, vp, l, i, i, vp, vp, vp, vp, vp], i),
         "mfgp_gpr_batched_adam": ([vp, vp, i, i, vp, l, i, i, vp, vp, vp, vp, vp, d, d, d, i, i, vp, vp, vp], i),
+        "mfgp_gpr_batched_lbfgs": ([vp, vp, i, i, vp, l, i, i, vp, vp, i, i, vp, vp, vp, vp, vp, vp], i),
         "mfgp_gpr_posterior_create": ([vp, vp, i, i, vp, l, i, i, i, vp, vp, vp, C.POINTER(vp)], i),
         "mfgp_gpr_posterior_predict": ([vp, vp, vp, i, vp, vp], i),
         "mfgp_gpr_posterior_predict_grad": ([vp, vp, vp, i, vp, vp, vp, vp], i),
@@ -92,7 +93,7 @@ _lib = _load()
 EXPORTED_SYMBOLS = [
     "mfgp_version", "mfgp_create", "mfgp_destroy", "mfgp_set_stream", "mfgp_reset_stream", "mfgp_set_async", "mfgp_sync",
     "mfgp_last_error", "mfgp_sm_count", "mfgp_cov", "mfgp_cov_diag", "mfgp_cov_grad", "mfgp_gpr_nlml", "mfgp_gpr_nlml_grad",
-    "mfgp_gpr_predict", "mfgp_gpr_batched_nlml_grad", "mfgp_gpr_batched_adam",
+    "mfgp_gpr_predict", "mfgp_gpr_batched_nlml_grad", "mfgp_gpr_batched_adam", "mfgp_gpr_batched_lbfgs",
     "mfgp_gpr_posterior_create", "mfgp_gpr_posterior_predict", "mfgp_gpr_posterior_predict_grad",
     "mfgp_gpr_posterior_predict_cov", "mfgp_gpr_posterior_sample", "mfgp_gpr_posterior_destroy",
     "mfgp_graph_nparams", "mfgp_graph_cov", "mfgp_graph_cov_diag", "mfgp_graph_gpr_nlml_grad", "mfgp_svgp_elbo_grad", "mfgp_svgp_elbo_grad_v", "mfgp_svgp_predict",
@@ -109,6 +110,16 @@ class SvgpCfg(C.Structure):
         ("scale", C.c_double), ("kl_mult", C.c_double), ("jitter", C.c_double), ("lik_lower", C.c_double),
         ("masked", C.c_int), ("lik_per_output", C.c_int),
     ]
+
+
+class LbfgsOpts(C.Structure):
+    _fields_ = [("m", C.c_int), ("maxiter", C.c_int), ("maxfun", C.c_int), ("maxls", C.c_int), ("ftol", C.c_double),
+                ("gtol", C.c_double)]
+
+
+# status codes of mfgp_gpr_batched_lbfgs (include/mfgp.h: MFGP_LBFGS_*)
+LBFGS_STATUS = {1: "pgtol", 2: "ftol", 3: "maxiter", 4: "maxfun", 5: "abnormal", 6: "not_pd"}
+LBFGS_NOT_PD = 6
 
 
 # ---- DLPack consumer (dlpack.h, DLManagedTensor ABI v0) -------------------------------------------------------
@@ -375,6 +386,36 @@ class Handle:
         if not (rc > 0 and info is not None):  # per-problem status in info[]: the other problems' steps stand
             self._check(rc, "mfgp_gpr_batched_adam")
         return loss_hist, theta_out
+
+    def gpr_batched_lbfgs(self, X, Y, u, noises, fix_rho=False, train_noise=False, m=10, maxiter=15000, maxfun=15000,
+                          maxls=20, ftol=2.220446049250313e-09, gtol=1e-5, f=None, nit=None, nfev=None, status=None,
+                          info=None):
+        """SciPy's L-BFGS-B for B = u.shape[0] per-bin GPs on the device (include/mfgp.h: mfgp_gpr_batched_lbfgs); the
+        defaults are scipy.optimize.minimize's.  u [B, 2d+3] (theta = softplus(u)) is updated in place, and so is
+        noises [B] when train_noise (noise = 1e-6 + softplus(v)).  Returns (f, nit, nfev, status) [B]; status holds
+        MFGP_LBFGS_* codes (LBFGS_STATUS names them).  A start point that is not positive definite raises
+        NotPositiveDefiniteError unless a per-problem `info` array (int32 [B]) is passed: then that problem's status is
+        not_pd, info[b] its pivot, and the others run on.  Host arrays or device tensors."""
+        X, Y = as_f64(X), as_f64(Y)
+        if not train_noise:
+            noises = as_f64(noises)
+        N, d = X.shape[0], X.shape[1] - 1
+        ycols = ldy = Y.shape[1]
+        B = u.shape[0]
+        for a in (u, noises) if train_noise else (u,):
+            if isinstance(a, np.ndarray) and not (a.dtype == np.float64 and a.flags.c_contiguous):
+                raise ValueError("u (and noises when train_noise) must be C-contiguous float64: they are updated in place")
+        f = np.empty(B) if f is None else f
+        nit = np.empty(B, dtype=np.int32) if nit is None else nit
+        nfev = np.empty(B, dtype=np.int32) if nfev is None else nfev
+        status = np.empty(B, dtype=np.int32) if status is None else status
+        opts = LbfgsOpts(int(m), int(maxiter), int(maxfun), int(maxls), float(ftol), float(gtol))
+        rc = _lib.mfgp_gpr_batched_lbfgs(self._h, _ptr(X), N, d, _ptr(Y), ldy, ycols, B, _ptr(u), _ptr(noises),
+                                         int(bool(fix_rho)), int(bool(train_noise)), C.byref(opts), _ptr(f), _ptr(nit),
+                                         _ptr(nfev), _ptr(status), _ptr(info))
+        if not (rc > 0 and info is not None):  # with info a failed start point is that problem's status
+            self._check(rc, "mfgp_gpr_batched_lbfgs")
+        return f, nit, nfev, status
 
     # -- graph-structured multi-fidelity kernel (reference mfgpflow/graph.py) -------------------------------
     def graph_cov(self, X, num_lf, gtheta):

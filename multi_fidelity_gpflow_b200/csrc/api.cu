@@ -712,9 +712,6 @@ int mfgp_cov_grad(mfgp_handle* h, const double* X, int N, int d, const double* t
 // ---------------------------------------------------------------------------------------------
 // Device-resident Adam loop for the batched per-bin GPs (SURVEY 8(f) rank 1; reference loop mfgpflow/linear.py:190-221).
 namespace {
-__device__ __forceinline__ double softplus_fwd(double u) {  // gpflow.utilities.positive(): tfp Softplus, lower = 0
-    return u > 0.0 ? u + log1p(exp(-u)) : log1p(exp(u));
-}
 __global__ void adam_softplus_kernel(const double* __restrict__ u, double* __restrict__ theta, long n) {
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) theta[i] = softplus_fwd(u[i]);

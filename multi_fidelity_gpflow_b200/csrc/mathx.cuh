@@ -89,6 +89,12 @@ __device__ __forceinline__ double fexp512(double x, const double* tab) {
     return __hiloint2double(__double2hiint(v) + ((n >> 9) << 20), __double2loint(v));
 }
 
+// gpflow.utilities.positive(): tfp Softplus, lower = 0.  The device training loops (Adam, L-BFGS) share it, so that they
+// optimise the same objective bit for bit.
+__device__ __forceinline__ double softplus_fwd(double u) {
+    return u > 0.0 ? u + log1p(exp(-u)) : log1p(exp(u));
+}
+
 // 1/sqrt(x) for positive normal x: hardware seed (rsqrt.approx.ftz.f64, ~2^-22) + two Newton steps (8 instructions
 // against 13 for the CUDA library call, no special-case branch: x <= 0 / NaN give NaN or inf, which the caller detects).
 __device__ __forceinline__ double frsqrt(double x) {

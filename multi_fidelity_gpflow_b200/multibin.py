@@ -30,6 +30,7 @@ class MultiBinMFGP:
             raise ValueError("MultiBinMFGP runs the small-matrix kernel (N <= 64); use MultiFidelityGPModel for larger problems")
         self.handle = handle if handle is not None else _lib.default_handle()
         self.noise = float(noise)
+        self.noises = np.full((self.R, self.P), self.noise)  # likelihood variance of every (restart, bin)
         self.use_rho = bool(use_rho)
         self._tf = positive()
         np_ = 2 * self.d + 3
@@ -43,6 +44,7 @@ class MultiBinMFGP:
         self.iterations = 0
         self.loss_history = np.zeros((0, self.R, self.P))
         self.failed = np.zeros((self.R, self.P), dtype=np.int32)  # first failing Cholesky pivot per (restart, bin), 0 = healthy
+        self.lbfgs_result = []  # per phase of the last optimize_lbfgs call
 
     # ---- parameters --------------------------------------------------------------------------------
     @property
@@ -54,7 +56,7 @@ class MultiBinMFGP:
         """NLML of every (restart, bin): [R, P]; NaN where that problem's covariance is not positive definite."""
         B = self.R * self.P
         info = np.zeros(B, dtype=np.int32)
-        nlml, _ = self.handle.gpr_batched_nlml_grad(self.X, self.Y, self.thetas.reshape(B, -1), np.full(B, self.noise),
+        nlml, _ = self.handle.gpr_batched_nlml_grad(self.X, self.Y, self.thetas.reshape(B, -1), self.noises.reshape(B),
                                                     info=info, want_grad=False)
         return np.where(info == 0, nlml, np.nan).reshape(self.R, self.P)
 
@@ -72,12 +74,37 @@ class MultiBinMFGP:
         B = self.R * self.P
         hist = np.empty((max_iters, B))
         info = np.zeros(B, dtype=np.int32)
-        self.handle.gpr_batched_adam(self.X, self.Y, self.u, self.m, self.v, np.full(B, self.noise), lr_t, b1, b2, epsilon,
+        self.handle.gpr_batched_adam(self.X, self.Y, self.u, self.m, self.v, self.noises.reshape(B), lr_t, b1, b2, epsilon,
                                      fix_rho=not self.use_rho, loss_hist=hist, info=info)
         self.iterations += max_iters
         self.loss_history = np.concatenate([self.loss_history, hist.reshape(max_iters, self.R, self.P)])
         new = info.reshape(self.R, self.P)
         self.failed = np.where(self.failed != 0, self.failed, new)
+        return self
+
+    def optimize_lbfgs(self, max_iters=1000, fix_noise_first=True):
+        """The SciPy L-BFGS-B branch of the reference's optimize (linear.py:222-234, MultiFidelityGPModel.optimize with
+        use_adam=False) for all R * P problems in one device loop (Handle.gpr_batched_lbfgs, SciPy's default options):
+        phase 1 with every problem's noise fixed, then phase 2 with the noise trained as well (noise = 1e-6 +
+        softplus(v), gpflow Gaussian's bound), maxiter=max_iters each.  fix_noise_first=False runs phase 2 only.
+        Updates u and `noises`; `lbfgs_result` holds one dict per phase (train_noise, f, nit, nfev, status [R, P], status
+        names from _lib.LBFGS_STATUS).  A restart whose start point is not positive definite stops with status "not_pd"
+        and is recorded in `failed` as optimize does; the others run on.  L-BFGS leaves the Adam state alone: the moments
+        m and v, `iterations` and `loss_history` are not touched."""
+        B = self.R * self.P
+        self.lbfgs_result = []
+        for train_noise in ((False, True) if fix_noise_first else (True,)):
+            noises = np.ascontiguousarray(self.noises.reshape(B))
+            info = np.zeros(B, dtype=np.int32)
+            f, nit, nfev, status = self.handle.gpr_batched_lbfgs(self.X, self.Y, self.u, noises, fix_rho=not self.use_rho,
+                                                                 train_noise=train_noise, maxiter=max_iters, info=info)
+            self.noises = noises.reshape(self.R, self.P)
+            shape = (self.R, self.P)
+            self.lbfgs_result.append(dict(train_noise=train_noise, f=np.asarray(f).reshape(shape),
+                                          nit=np.asarray(nit).reshape(shape), nfev=np.asarray(nfev).reshape(shape),
+                                          status=np.vectorize(_lib.LBFGS_STATUS.get)(np.asarray(status).reshape(shape))))
+            new = info.reshape(shape)
+            self.failed = np.where(self.failed != 0, self.failed, new)
         return self
 
     # ---- model selection and prediction ----------------------------------------------------------------
@@ -87,16 +114,20 @@ class MultiBinMFGP:
         return np.argmin(np.where(np.isfinite(loss), loss, np.inf), axis=0)
 
     def best_thetas(self):
+        return self._best()[0]
+
+    def _best(self):
+        """(thetas [P, 2d+3], noises [P]) of every bin at its best restart."""
         r = self.best_restart()
-        return self.thetas[r, np.arange(self.P)]
+        return self.thetas[r, np.arange(self.P)], self.noises[r, np.arange(self.P)]
 
     def predict_f(self, Xnew):
         """Posterior mean / variance [N*, P] of every bin at its best restart (GPR.predict_f per bin)."""
         Xnew = np.ascontiguousarray(Xnew, dtype=np.float64)
-        th = self.best_thetas()
+        th, nz = self._best()
         mean, var = np.empty((Xnew.shape[0], self.P)), np.empty((Xnew.shape[0], self.P))
         for p in range(self.P):
-            mu, s2 = self.handle.gpr_predict(self.X, np.ascontiguousarray(self.Y[:, p:p + 1]), Xnew, th[p], self.noise)
+            mu, s2 = self.handle.gpr_predict(self.X, np.ascontiguousarray(self.Y[:, p:p + 1]), Xnew, th[p], nz[p])
             mean[:, p], var[:, p] = mu[:, 0], s2
         return mean, var
 
@@ -115,15 +146,15 @@ class MultiBinMFGP:
         "all": every (restart, bin), predict_f -> [R, N*, P], NaN for a restart whose covariance is not positive
         definite.  One cached factorisation per problem b = r * P + p; every prediction is one library call."""
         if restarts == "best":
-            th = self.best_thetas()
-            post = self.handle.gpr_posterior(self.X, self.Y, np.ascontiguousarray(th), np.full(self.P, self.noise))
-            return MultiBinPosterior(post, np.full(self.P, self.noise), None)
+            th, nz = self._best()
+            post = self.handle.gpr_posterior(self.X, self.Y, np.ascontiguousarray(th), np.ascontiguousarray(nz))
+            return MultiBinPosterior(post, nz, None)
         if restarts == "all":
             B = self.R * self.P
             info = np.zeros(B, dtype=np.int32)
             post = self.handle.gpr_posterior(self.X, self.Y, np.ascontiguousarray(self.thetas.reshape(B, -1)),
-                                             np.full(B, self.noise), info=info)
-            return MultiBinPosterior(post, np.full(B, self.noise).reshape(self.R, self.P), info.reshape(self.R, self.P))
+                                             np.ascontiguousarray(self.noises.reshape(B)), info=info)
+            return MultiBinPosterior(post, self.noises.copy(), info.reshape(self.R, self.P))
         raise ValueError('restarts must be "best" or "all"')
 
 

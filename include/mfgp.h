@@ -300,6 +300,39 @@ int mfgp_svgp_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* X, co
                    double* m, double* v, const unsigned char* mask, const double* lr_t, double beta1, double beta2,
                    double eps, int nsteps, double* loss_hist, double* kl_hist);
 
+/* Minibatch stream: the rows the minibatch SVGP loops train on, one endless sequence of shuffled epochs over a data set of
+ * N rows, defined by an integer-only stateless rule (the GPU evaluates it inside a captured graph from the device step
+ * counter; every rank of a data-parallel run computes its slice of the same global batch without communicating).
+ *  - Stream position p >= 0 (64-bit) is epoch e = p / N, offset i = p mod N, row pi_{seed,e}(i).
+ *  - pi_{seed,e} is a balanced Feistel network on 2k-bit values, k the smallest integer with 4^k >= N, cycle-walked (the
+ *    network is applied again until the value is below N).  A value x splits into l = x >> k, r = x & (2^k - 1); each of
+ *    8 rounds j = 0..7 does (l, r) <- (r, l ^ (mix32(r ^ key_j) & (2^k - 1))); x = (l << k) | r.
+ *  - key_j = low 32 bits of splitmix64(splitmix64(splitmix64(seed) ^ e) ^ j), all arithmetic modulo 2^64.
+ *    splitmix64(z): z += 0x9E3779B97F4A7C15; z = (z ^ z >> 30) * 0xBF58476D1CE4E5B9; z = (z ^ z >> 27) * 0x94D049BB133111EB;
+ *    z ^ z >> 31.  mix32(x) (32-bit): x ^= x >> 16; x *= 0x7FEB352D; x ^= x >> 15; x *= 0x846CA68B; x ^ x >> 16.
+ *  - Step t of a loop that starts at position pos0 with batch size B reads positions pos0 + t B ... pos0 + t B + B - 1:
+ *    batches cross epoch boundaries and B need not divide N.
+ * The rule is fixed: changing any constant above changes every minibatch trajectory.
+ *
+ * mfgp_svgp_adam_minibatch: mfgp_svgp_adam on minibatches of that stream.  X [N, d+1] and Y [N, ycols] are the whole data
+ * set (copied to the device once per call when they are host memory); cfg->B is the batch size, 1 <= B <= N, and
+ * cfg->scale what the caller wants (num_data / B).  Each step gathers its B rows (minibatch_gather_kernel) and then runs
+ * the step of mfgp_svgp_adam on them; loss_hist / kl_hist receive each step's minibatch estimate.  The batch buffers are
+ * allocated before the step is captured, so the graph has no allocation nodes.  pos0 >= 0; otherwise -1.
+ *
+ * mfgp_minibatch_gather: Xb [count, xcols] and Yb [count, ycols] <- rows X[row], Y[row] of positions
+ * pos0 + (*step) B + lo + j, j < count, with 1 <= B <= N, 0 <= lo, lo + count <= B.  step is an int (host or device), or
+ * NULL for 0; Y and Yb may both be NULL.  A data-parallel rank r gathers lo, count = its shard of each global batch of B
+ * rows, reading the step counter mfgp_svgp_adam_update advances.  Host or device pointers; NaN entries are copied as they
+ * are. */
+int mfgp_svgp_adam_minibatch(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* X, const double* Y, int N,
+                             unsigned long long seed, long long pos0, int has_W, double* u, double* m, double* v,
+                             const unsigned char* mask, const double* lr_t, double beta1, double beta2, double eps,
+                             int nsteps, double* loss_hist, double* kl_hist);
+int mfgp_minibatch_gather(mfgp_handle* h, const double* X, int xcols, const double* Y, int ycols, int N,
+                          unsigned long long seed, long long pos0, const int* step, int B, int lo, int count, double* Xb,
+                          double* Yb);
+
 /* Data-parallel SVGP training step on device memory only (SURVEY 8(e) row 2: rows of the minibatch shard across one
  * process per GPU, ONE all-reduce of the flat gradient; reference loops singlebin_svgp.py:79-85, linear_svgp.py:181-190).
  * Per step every rank runs, on the handle's stream and without any host synchronisation:

@@ -32,6 +32,7 @@ def _load():
         )
     lib = C.CDLL(LIB_PATH)
     vp, i, l, d = C.c_void_p, C.c_int, C.c_long, C.c_double
+    i64, u64 = C.c_longlong, C.c_ulonglong
     sig = {
         "mfgp_version": ([], i),
         "mfgp_create": ([i, C.POINTER(vp)], i),
@@ -69,6 +70,8 @@ def _load():
         "mfgp_svgp_posterior_predict_grad": ([vp, vp, vp, i, vp, vp, vp, vp], i),
         "mfgp_svgp_posterior_destroy": ([vp], i),
         "mfgp_svgp_adam": ([vp, vp, vp, vp, i, vp, vp, vp, vp, vp, d, d, d, i, vp, vp], i),
+        "mfgp_svgp_adam_minibatch": ([vp, vp, vp, vp, i, u64, i64, i, vp, vp, vp, vp, vp, d, d, d, i, vp, vp], i),
+        "mfgp_minibatch_gather": ([vp, vp, i, vp, i, i, u64, i64, vp, i, i, i, vp, vp], i),
         "mfgp_svgp_flat_size": ([vp, i], l),
         "mfgp_svgp_constrain": ([vp, vp, i, vp, vp], i),
         "mfgp_svgp_elbo_grad_flat": ([vp, vp, vp, vp, i, vp, i, vp], i),
@@ -98,7 +101,7 @@ EXPORTED_SYMBOLS = [
     "mfgp_gpr_posterior_predict_cov", "mfgp_gpr_posterior_sample", "mfgp_gpr_posterior_destroy",
     "mfgp_graph_nparams", "mfgp_graph_cov", "mfgp_graph_cov_diag", "mfgp_graph_gpr_nlml_grad", "mfgp_svgp_elbo_grad", "mfgp_svgp_elbo_grad_v", "mfgp_svgp_predict",
     "mfgp_svgp_posterior_create", "mfgp_svgp_posterior_predict", "mfgp_svgp_posterior_predict_grad",
-    "mfgp_svgp_posterior_destroy", "mfgp_svgp_adam",
+    "mfgp_svgp_posterior_destroy", "mfgp_svgp_adam", "mfgp_svgp_adam_minibatch", "mfgp_minibatch_gather",
     "mfgp_svgp_flat_size", "mfgp_svgp_constrain", "mfgp_svgp_elbo_grad_flat", "mfgp_svgp_adam_update", "mfgp_gemm",
     "mfgp_potrf", "mfgp_potrf_inv", "mfgp_tall_skinny_update", "mfgp_peer_store", "mfgp_graph_mem_trim", "mfgp_workspace", "mfgp_fp64_peak",
 ]
@@ -197,6 +200,14 @@ def _ptr(x):
         p._dlpack_owner = cap  # keeps the exporter's memory alive for as long as the pointer object lives (the call)
         return p
     raise TypeError(f"unsupported buffer type {type(x)}")
+
+
+def _seed(seed):
+    """A minibatch stream seed: an integer in [0, 2^64)."""
+    seed = int(seed)
+    if not 0 <= seed < 1 << 64:
+        raise ValueError(f"seed must be an integer in [0, 2**64), got {seed}")
+    return seed
 
 
 def as_f64(x):
@@ -368,6 +379,45 @@ class Handle:
                                  float(eps), n, _ptr(loss), _ptr(kl))
         self._check(rc, "mfgp_svgp_adam")
         return loss, kl
+
+    def svgp_adam_minibatch(self, X, Y, L, M, P, has_W, u, m, v, mask, lr_t, beta1, beta2, eps=1e-7, batch_size=None, seed=0,
+                            pos0=0, scale=1.0, kl_mult=1.0, hetero=False, jitter=1e-6, lik_lower=1e-6, masked=False,
+                            lik_per_output=False):
+        """len(lr_t) Adam steps on minibatches of `batch_size` rows of the shuffled stream over the N rows of X, Y (include/
+        mfgp.h: minibatch stream), starting at stream position pos0; otherwise as svgp_adam.  scale is the caller's
+        (num_data / batch_size).  Returns (loss_hist, kl_hist), each step's minibatch estimate."""
+        X, Y, lr_t = as_f64(X), as_f64(Y), as_f64(lr_t)
+        N, d = X.shape[0], X.shape[1] - 1
+        cfg = SvgpCfg(L, M, P, int(batch_size), d, int(hetero), float(scale), float(kl_mult), float(jitter), float(lik_lower),
+                      int(masked), int(lik_per_output))
+        n = int(lr_t.shape[0])
+        loss, kl = np.empty(n), np.empty(n)
+        mk = None if mask is None else np.ascontiguousarray(mask, dtype=np.uint8)
+        rc = _lib.mfgp_svgp_adam_minibatch(self._h, C.byref(cfg), _ptr(X), _ptr(Y), N, _seed(seed), int(pos0), int(bool(has_W)),
+                                           _ptr(u), _ptr(m), _ptr(v), None if mk is None else C.c_void_p(mk.ctypes.data),
+                                           _ptr(lr_t), float(beta1), float(beta2), float(eps), n, _ptr(loss), _ptr(kl))
+        self._check(rc, "mfgp_svgp_adam_minibatch")
+        return loss, kl
+
+    def minibatch_gather(self, X, Y, seed, pos0, batch_size, lo=0, count=None, step=None, Xb=None, Yb=None):
+        """Rows of stream positions pos0 + step * batch_size + lo + j, j < count (default batch_size - lo), of the shuffled
+        stream over the N rows of X (and Y, or None): (Xb [count, xcols], Yb [count, ycols] or None).  step: an int32
+        device tensor holding the step (the data-parallel loop's counter), a host int, or None for 0.  Host arrays or
+        device tensors."""
+        X = as_f64(X)
+        Y = None if Y is None else as_f64(Y)
+        N, xcols = X.shape[0], X.shape[1]
+        ycols = 0 if Y is None else Y.shape[1]
+        count = int(batch_size) - int(lo) if count is None else int(count)
+        Xb = np.empty((count, xcols)) if Xb is None else Xb
+        if Y is not None and Yb is None:
+            Yb = np.empty((count, ycols))
+        if step is not None and not hasattr(step, "data_ptr"):
+            step = np.array([int(step)], dtype=np.int32)
+        rc = _lib.mfgp_minibatch_gather(self._h, _ptr(X), xcols, _ptr(Y), ycols, N, _seed(seed), int(pos0), _ptr(step),
+                                        int(batch_size), int(lo), count, _ptr(Xb), _ptr(Yb) if Y is not None else None)
+        self._check(rc, "mfgp_minibatch_gather")
+        return Xb, Yb
 
     def gpr_batched_adam(self, X, Y, u, m, v, noises, lr_t, beta1, beta2, eps=1e-7, fix_rho=False, loss_hist=None,
                          theta_out=None, info=None):

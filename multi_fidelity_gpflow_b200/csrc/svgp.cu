@@ -825,15 +825,19 @@ struct AsyncGuard {  // nested library calls only enqueue; the caller's mode com
 };
 }  // namespace
 
-extern "C" int mfgp_svgp_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* X, const double* Y, int has_W, double* u,
-                              double* m, double* v, const unsigned char* mask, const double* lr_t, double beta1, double beta2,
-                              double eps, int nsteps, double* loss_hist, double* kl_hist) {
+namespace {
+// The loop of mfgp_svgp_adam and mfgp_svgp_adam_minibatch.  Without a stream (mb == nullptr) every step evaluates the cfg->B
+// rows of X, Y; with one, X, Y hold the N = mb->N rows of the data set and each step first gathers its cfg->B rows of the
+// shuffled stream into batch buffers (positions mb->pos0 + step * B ...), reading the device step counter.
+int svgp_adam_loop(mfgp_handle* h, const char* who, const mfgp_svgp_cfg* cfg, const double* X, const double* Y,
+                   const MinibatchStream* mb, int has_W, double* u, double* m, double* v, const unsigned char* mask,
+                   const double* lr_t, double beta1, double beta2, double eps, int nsteps, double* loss_hist, double* kl_hist) {
     if (!h) return MFGP_ERR_ARG;
-    if (!cfg || !X || !Y || !u || !m || !v || !lr_t || nsteps < 0)
-        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_adam: NULL argument");
+    if (!cfg || !X || !Y || !u || !m || !v || !lr_t || nsteps < 0) return mfgp_fail(h, MFGP_ERR_ARG, "%s: NULL argument", who);
     const int L = cfg->L, M = cfg->M, P = cfg->P, B = cfg->B, d = cfg->d;
     if (L < 1 || M < 1 || P < 1 || B < 1 || d < 1 || d > MFGP_MAX_D || (!has_W && L != P))
-        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_adam: bad configuration");
+        return mfgp_fail(h, MFGP_ERR_ARG, "%s: bad configuration", who);
+    if (mb && (mb->N < B || mb->pos0 < 0)) return mfgp_fail(h, MFGP_ERR_ARG, "%s: need 1 <= B <= N and pos0 >= 0", who);
     if (nsteps == 0) return 0;
     cudaSetDevice(h->device);
     cudaStream_t s = h->stream;
@@ -843,8 +847,11 @@ extern "C" int mfgp_svgp_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const do
     const int ycols = cfg->hetero ? 2 * P : P;
     int rc = 0;
     Scope sc(h);
-    const double* dX = sc.in(X, (size_t)B * (d + 1));
-    const double* dY = sc.in(Y, (size_t)B * ycols);
+    const size_t rows = mb ? (size_t)mb->N : (size_t)B;
+    const double* dX = sc.in(X, rows * (d + 1));
+    const double* dY = sc.in(Y, rows * ycols);
+    double* Xb = mb ? sc.alloc<double>((size_t)B * (d + 1)) : nullptr;  // the step's batch, filled by the gather
+    double* Yb = mb ? sc.alloc<double>((size_t)B * ycols) : nullptr;
     const double* dlr = sc.in(lr_t, nsteps);
     const unsigned char* dmask = mask ? sc.in(mask, (size_t)n) : nullptr;
     double* du = sc.inout(u, (size_t)n);
@@ -862,10 +869,14 @@ extern "C" int mfgp_svgp_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const do
     {
         AsyncGuard guard(h);  // the nested evaluations only enqueue: all their pointers are device memory
         WorkspaceGuard wsg(h);  // step 0 measures the step's temporaries; the captured step takes them from one arena
+        const MinibatchStream ds = mb ? MinibatchStream{dX, d + 1, dY, ycols, mb->N, mb->seed, mb->pos0} : MinibatchStream{};
         auto one_step = [&]() -> int {
+            if (mb && launch_minibatch_gather(s, ds, dstep, B, 0, B, Xb, Yb))
+                return mfgp_fail(h, MFGP_ERR_CUDA, "%s: gather launch failed", who);
             svgp_constrain_kernel<<<gb, tb, 0, s>>>(du, c, n, n_theta, o_lv, cfg->lik_lower);
-            int r = mfgp_svgp_elbo_grad_v(h, cfg, dX, dY, c + o_Z, c, has_W ? c + o_W : nullptr, c + o_qm, c + o_qs, c + o_lv, ek,
-                                          ek + 1, g + o_Z, g, has_W ? g + o_W : nullptr, g + o_qm, g + o_qs, g + o_lv);
+            int r = mfgp_svgp_elbo_grad_v(h, cfg, mb ? Xb : dX, mb ? Yb : dY, c + o_Z, c, has_W ? c + o_W : nullptr, c + o_qm,
+                                          c + o_qs, c + o_lv, ek, ek + 1, g + o_Z, g, has_W ? g + o_W : nullptr, g + o_qm,
+                                          g + o_qs, g + o_lv);
             svgp_adam_kernel<<<gb, tb, 0, s>>>(du, dm, dv, c, g, dmask, n, n_theta, o_lv, cfg->lik_lower, dlr, dstep, beta1, beta2,
                                                eps, ek, cfg->kl_mult, dl, dk);
             svgp_step_inc_kernel<<<1, 1, 0, s>>>(dstep);
@@ -888,7 +899,7 @@ extern "C" int mfgp_svgp_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const do
             if (ok) ok = cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess;
             if (ok) {
                 for (; done < nsteps && ok; ++done) ok = cudaGraphLaunch(exec, s) == cudaSuccess;
-                if (!ok) rc = mfgp_fail(h, MFGP_ERR_CUDA, "mfgp_svgp_adam: graph launch failed");
+                if (!ok) rc = mfgp_fail(h, MFGP_ERR_CUDA, "%s: graph launch failed", who);
             } else {
                 cudaGetLastError();  // capture not possible: clear the error, run eagerly
             }
@@ -906,6 +917,26 @@ extern "C" int mfgp_svgp_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const do
     }
     if (rc) return rc;
     return sc.finish();
+}
+}  // namespace
+
+extern "C" int mfgp_svgp_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* X, const double* Y, int has_W, double* u,
+                              double* m, double* v, const unsigned char* mask, const double* lr_t, double beta1, double beta2,
+                              double eps, int nsteps, double* loss_hist, double* kl_hist) {
+    return svgp_adam_loop(h, "mfgp_svgp_adam", cfg, X, Y, nullptr, has_W, u, m, v, mask, lr_t, beta1, beta2, eps, nsteps,
+                          loss_hist, kl_hist);
+}
+
+extern "C" int mfgp_svgp_adam_minibatch(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* X, const double* Y, int N,
+                                        unsigned long long seed, long long pos0, int has_W, double* u, double* m, double* v,
+                                        const unsigned char* mask, const double* lr_t, double beta1, double beta2, double eps,
+                                        int nsteps, double* loss_hist, double* kl_hist) {
+    MinibatchStream mb{};  // the stream's data pointers and column counts are the loop's device copies of X and Y
+    mb.N = N;
+    mb.seed = seed;
+    mb.pos0 = pos0;
+    return svgp_adam_loop(h, "mfgp_svgp_adam_minibatch", cfg, X, Y, &mb, has_W, u, m, v, mask, lr_t, beta1, beta2, eps, nsteps,
+                          loss_hist, kl_hist);
 }
 
 // ---------------------------------------------------------------------------------------------

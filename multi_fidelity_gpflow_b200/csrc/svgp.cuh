@@ -52,3 +52,18 @@ int svgp_posterior_predict_blocked(mfgp_handle* h, const SvgpPosteriorData& q, c
 // dmean = sum_l W_pl gm_l, dvar = sum_l W_pl^2 gv_l in a fixed l order, or the gather of latent p when W == NULL.
 int launch_svgp_grad_mix(cudaStream_t s, const double* gm, const double* gv, int L, int B, int P, int d, const double* W,
                          double* dmean, double* dvar);
+
+// The shuffled-epoch row stream over a device-resident data set (include/mfgp.h: minibatch stream): X [N][xcols],
+// Y [N][ycols] or nullptr.
+struct MinibatchStream {
+    const double* X;
+    int xcols;
+    const double* Y;
+    int ycols;
+    long long N;
+    unsigned long long seed;
+    long long pos0;
+};
+// minibatch.cu: Xb [count][xcols] (and Yb) <- the rows of positions pos0 + (*step) B + lo + j, j < count (step nullptr: 0).
+int launch_minibatch_gather(cudaStream_t s, const MinibatchStream& ms, const int* step, int B, int lo, int count, double* Xb,
+                            double* Yb);

@@ -128,6 +128,9 @@ class SvgpDeviceOps:
         self._chk(self.L.mfgp_svgp_elbo_grad_flat(self.h._h, C.byref(cfg), p(X), p(Y), int(has_W), p(c), int(nranks), p(eg)),
                   "mfgp_svgp_elbo_grad_flat")
 
+    def gather(self, X, Y, seed, pos0, step, B, lo, Xb, Yb):
+        self.h.minibatch_gather(X, Y, seed, pos0, B, lo=lo, count=Xb.shape[0], step=step, Xb=Xb, Yb=Yb)
+
     def adam_update(self, cfg, has_W, u, m, v, mask, c, eg, lr_t, step, b1, b2, eps, loss_hist, kl_hist, scratch):
         import ctypes as C
 
@@ -138,10 +141,14 @@ class SvgpDeviceOps:
 
 
 def dp_svgp_adam(handle_or_ops, X, Y, shape, u, mask, lr_t, beta1, beta2, eps=1e-7, num_data=None, kl_mult=1.0,
-                 group=None, timing=None, use_graph=None):
+                 group=None, timing=None, use_graph=None, minibatch=None):
     """len(lr_t) data-parallel Adam steps.  Every rank passes the same GLOBAL (mini)batch X [B, d+1], Y, the same flat
     unconstrained parameter vector `u` (layout of mfgp_svgp_adam), trainable mask and per-step factors `lr_t`
     (optimizers.adam_step_factors); rank r evaluates rows shard_range(B, r, world).
+    minibatch=(B, seed, pos0): X, Y are the whole data set instead, held by every rank, and step t's global batch is the B
+    rows at positions pos0 + t B ... of the shuffled stream (include/mfgp.h: minibatch stream); rank r gathers its rows
+    shard_range(B, r, world) of it at the start of each step, reading the device step counter (ops.gather), and the ELBO
+    scale is num_data / B.
 
     shape: dict(L, M, P, d, has_W, hetero, masked, lik_per_output, lik_lower).
     Returns (u_final, loss_hist, kl_hist) as NumPy arrays, identical on every rank (same reduced gradient, same update).
@@ -160,6 +167,8 @@ def dp_svgp_adam(handle_or_ops, X, Y, shape, u, mask, lr_t, beta1, beta2, eps=1e
     X = np.ascontiguousarray(X, dtype=np.float64)
     Y = np.ascontiguousarray(Y, dtype=np.float64)
     B, d = X.shape[0], X.shape[1] - 1
+    if minibatch is not None:
+        B, seed, pos0 = minibatch
     if B < world:
         raise ValueError(f"batch of {B} rows cannot be sharded over {world} ranks")
     lo, hi = shard_range(B, rank, world)
@@ -169,7 +178,11 @@ def dp_svgp_adam(handle_or_ops, X, Y, shape, u, mask, lr_t, beta1, beta2, eps=1e
     has_W = bool(shape["has_W"])
     n, nsteps = int(np.size(u)), int(len(lr_t))
     f64 = dict(dtype=torch.float64, device=dev)
-    Xd, Yd = torch.from_numpy(X[lo:hi].copy()).to(dev), torch.from_numpy(Y[lo:hi].copy()).to(dev)
+    if minibatch is None:
+        Xd, Yd = torch.from_numpy(X[lo:hi].copy()).to(dev), torch.from_numpy(Y[lo:hi].copy()).to(dev)
+    else:  # the whole data set stays on the device; Xd, Yd receive this rank's rows of each step's batch
+        Xall, Yall = torch.from_numpy(X).to(dev), torch.from_numpy(Y).to(dev)
+        Xd, Yd = torch.empty((hi - lo, d + 1), **f64), torch.empty((hi - lo, Y.shape[1]), **f64)
     ud = torch.from_numpy(np.ascontiguousarray(u, dtype=np.float64).ravel().copy()).to(dev)
     md, vd, c = torch.zeros(n, **f64), torch.zeros(n, **f64), torch.empty(n, **f64)
     eg = torch.zeros(n + 2, **f64)
@@ -192,6 +205,8 @@ def dp_svgp_adam(handle_or_ops, X, Y, shape, u, mask, lr_t, beta1, beta2, eps=1e
             e0.record()
 
         def one_step():
+            if minibatch is not None:
+                ops.gather(Xall, Yall, seed, pos0, step, B, lo, Xd, Yd)
             ops.constrain(cfg, has_W, ud, c)
             ops.elbo_grad_flat(cfg, Xd, Yd, has_W, c, world, eg)
             if world > 1:

@@ -152,21 +152,35 @@ class SVGPBase:
             mask[sl] = 1 if par.trainable else 0
         return items, u, mask
 
-    def _device_loop(self, data, max_iters, initial_lr, kl_multiplier, run):
+    def _device_loop(self, data, max_iters, initial_lr, kl_multiplier, run, minibatch_size=None, seed=0):
         """Shared by optimize_on_device / optimize_data_parallel: history semantics of the reference loops, flat packing,
-        per-step factors; `run(X, Y, shape, u, mask, lr_t, b1, b2, scale)` -> (u_final, loss_hist, kl_hist)."""
+        per-step factors, the minibatch stream position; `run(X, Y, shape, u, mask, lr_t, b1, b2, batch)` -> (u_final,
+        loss_hist, kl_hist), with batch None (full batch) or (minibatch_size, seed, pos0)."""
         from .optimizers import adam_step_factors
 
         X, Y = data
         X = np.ascontiguousarray(X, dtype=np.float64)
         Y = np.ascontiguousarray(Y, dtype=np.float64)
         d = X.shape[1] - 1
+        if minibatch_size is not None:
+            N, B = X.shape[0], int(minibatch_size)
+            if not 1 <= B <= N:
+                raise ValueError(f"minibatch_size must be in [1, {N}] (the number of rows), got {minibatch_size}")
+            if self.num_data is None and B < N:
+                raise ValueError("minibatches need the model's num_data (the ELBO scale num_data / minibatch_size): this "
+                                 "model has num_data=None, which scales the ELBO by 1 and would bias the estimate; set "
+                                 "model.num_data = N")
         resumable = hasattr(self, "kl_history")
         if not resumable:
             self.loss_history = []
         nsteps = int(max_iters) - (len(self.loss_history) if resumable else 0)
         if nsteps <= 0:
             return self
+        batch = None
+        if minibatch_size is not None:
+            # a resumable model continues the stream where its last minibatch call stopped (counted in rows, so that the
+            # batch size may change between calls); a model that restarts its loop restarts the stream too
+            batch = (B, int(seed), getattr(self, "minibatch_position", 0) if resumable else 0)
         items, u, mask = self._flat_pack(d)
         lr_t, b1, b2 = adam_step_factors(initial_lr, nsteps, cosine_decay_steps=int(max_iters))
         M, L = self.q_mu.shape
@@ -175,44 +189,62 @@ class SVGPBase:
         shape = dict(L=L, M=M, P=L if W is None else W.shape[0], d=d, has_W=W is not None, hetero=lik.heteroscedastic,
                      masked=lik.masked, lik_per_output=int(np.size(lik.variance.unconstrained)) > 1,
                      lik_lower=lik.variance.transform.lower)
-        u, loss, kl = run(X, Y, shape, u, mask, lr_t, b1, b2)
+        u, loss, kl = run(X, Y, shape, u, mask, lr_t, b1, b2, batch)
         for par, sl in items:
             par.unconstrained = u[sl].reshape(np.shape(par.unconstrained)).copy()
         self.loss_history = list(self.loss_history) + list(loss)
         if resumable:
             self.kl_history = list(self.kl_history) + list(kl)
+            if batch is not None:
+                self.minibatch_position = batch[2] + nsteps * batch[0]
         return self
 
-    def optimize_on_device(self, data, max_iters, initial_lr, kl_multiplier=1.0):
+    def optimize_on_device(self, data, max_iters, initial_lr, kl_multiplier=1.0, minibatch_size=None, seed=0):
         """The model's optimize() loop -- full-batch Adam with CosineDecay(initial_lr, max_iters) on the unconstrained
         trainable variables, loss = -ELBO + (kl_multiplier - 1) KL -- run by mfgp_svgp_adam without a host round trip per
         step.  Same trajectory and the same history semantics as the model's optimize() (tests/test_svgp_device_loop.py):
         a model with a `kl_history` (LatentMFCoregionalizationSVGP, linear_svgp.py:194) runs the REMAINING steps
         range(len(loss_history), max_iters) and appends; SingleBinSVGP (singlebin_svgp.py:79) resets loss_history and runs
-        max_iters steps.  Like the reference, every call starts a fresh optimizer (Adam moments zero, iteration 0)."""
+        max_iters steps.  Like the reference, every call starts a fresh optimizer (Adam moments zero, iteration 0).
 
-        def run(X, Y, shape, u, mask, lr_t, b1, b2):
-            scale = 1.0 if self.num_data is None else float(self.num_data) / X.shape[0]
+        minibatch_size=B trains on shuffled minibatches instead (GPflow's Dataset.shuffle(N).repeat().batch(B) feeding
+        training_loss): step t uses the B rows at positions pos0 + t B ... of the stream of shuffled epochs over the N rows
+        of `data` drawn with `seed` (include/mfgp.h: minibatch stream), gathered on the GPU inside the captured step by
+        mfgp_svgp_adam_minibatch, with ELBO scale num_data / B.  loss_history receives each step's minibatch estimate.  A
+        resumable model continues the stream at `minibatch_position` (rows drawn so far); SingleBinSVGP starts at 0.
+        A model with num_data=None (SingleBinSVGP's default) accepts only B = N: set num_data to train on minibatches."""
+
+        def run(X, Y, shape, u, mask, lr_t, b1, b2, batch):
             m, v = np.zeros_like(u), np.zeros_like(u)
-            loss, kl = self.handle.svgp_adam(X, Y, shape["L"], shape["M"], shape["P"], shape["has_W"], u, m, v, mask, lr_t, b1, b2,
-                                             1e-7, scale=scale, kl_mult=kl_multiplier, hetero=shape["hetero"],
-                                             lik_lower=shape["lik_lower"], masked=shape["masked"],
-                                             lik_per_output=shape["lik_per_output"])
+            kw = dict(kl_mult=kl_multiplier, hetero=shape["hetero"], lik_lower=shape["lik_lower"], masked=shape["masked"],
+                      lik_per_output=shape["lik_per_output"])
+            args = (X, Y, shape["L"], shape["M"], shape["P"], shape["has_W"], u, m, v, mask, lr_t, b1, b2, 1e-7)
+            if batch is None:
+                scale = 1.0 if self.num_data is None else float(self.num_data) / X.shape[0]
+                loss, kl = self.handle.svgp_adam(*args, scale=scale, **kw)
+            else:
+                B, seed_, pos0 = batch
+                scale = float(X.shape[0] if self.num_data is None else self.num_data) / B
+                loss, kl = self.handle.svgp_adam_minibatch(*args, batch_size=B, seed=seed_, pos0=pos0, scale=scale, **kw)
             return u, loss, kl
 
-        return self._device_loop(data, max_iters, initial_lr, kl_multiplier, run)
+        return self._device_loop(data, max_iters, initial_lr, kl_multiplier, run, minibatch_size, seed)
 
-    def optimize_data_parallel(self, data, max_iters, initial_lr, kl_multiplier=1.0, group=None, timing=None):
+    def optimize_data_parallel(self, data, max_iters, initial_lr, kl_multiplier=1.0, group=None, timing=None,
+                               minibatch_size=None, seed=0):
         """optimize_on_device across the ranks of a torch.distributed group (one process per GPU, NCCL): the rows of the
         batch shard across ranks, one in-place all-reduce of the flat device gradient per step (dist.dp_svgp_adam); every
-        rank ends with the same parameters and histories."""
+        rank ends with the same parameters and histories.  With minibatch_size=B every rank holds the whole data set and
+        draws its shard_range slice of each global batch of B rows of optimize_on_device's stream inside the captured
+        step, so the run follows the single-GPU minibatch trajectory (ELBO scale num_data / B)."""
         from .dist import dp_svgp_adam
 
-        def run(X, Y, shape, u, mask, lr_t, b1, b2):
-            return dp_svgp_adam(self.handle, X, Y, shape, u, mask, lr_t, b1, b2, 1e-7, num_data=self.num_data,
-                                kl_mult=kl_multiplier, group=group, timing=timing)
+        def run(X, Y, shape, u, mask, lr_t, b1, b2, batch):
+            num_data = self.num_data if batch is None or self.num_data is not None else X.shape[0]
+            return dp_svgp_adam(self.handle, X, Y, shape, u, mask, lr_t, b1, b2, 1e-7, num_data=num_data,
+                                kl_mult=kl_multiplier, group=group, timing=timing, minibatch=batch)
 
-        return self._device_loop(data, max_iters, initial_lr, kl_multiplier, run)
+        return self._device_loop(data, max_iters, initial_lr, kl_multiplier, run, minibatch_size, seed)
 
     def predict_f(self, Xnew, full_cov=False, full_output_cov=False):
         if full_cov or full_output_cov:

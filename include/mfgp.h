@@ -333,6 +333,43 @@ int mfgp_minibatch_gather(mfgp_handle* h, const double* X, int xcols, const doub
                           unsigned long long seed, long long pos0, const int* step, int B, int lo, int count, double* Xb,
                           double* Yb);
 
+/* Natural-gradient step on the variational distributions (GPflow 2.9 NaturalGradient with the default XiNat, as
+ * natgrad.minimize(loss, [(q_mu, q_sqrt)]) applies it) for all L latents in one call.  Per latent l, with m = q_mu[:, l],
+ * Lq = tril(q_sqrt[l]) (any signs on the diagonal), gm = g_q_mu[:, l], G = tril(g_q_sqrt[l]) the loss gradients
+ * mfgp_svgp_elbo_grad returns, and S = Lq Lq^T:
+ *   g_S = (X + X^T) / 2,  X = Lq^-T Phi(Lq^T G) Lq^-1  (Phi: lower triangle, halved diagonal): dL/d eta2 of the
+ *   expectation parameters eta1 = m, eta2 = S + m m^T, and dL/d eta1 = gm - 2 g_S m;
+ *   Lam = S^-1,  theta1' = Lam m - gamma dL/d eta1,  Lam' = Lam + 2 gamma g_S;
+ *   R = chol(Lam'),  S' = R^-T R^-1,  m' = S' theta1',  Lq' = chol(S') with its strictly upper part zero.
+ * m' and Lq' are written back in place.  Deliberate deviation from GPflow, which raises when a Cholesky fails: a latent
+ * whose R or Lq' factorisation fails keeps its m and Lq bit for bit and gets the 1-based pivot of the first failed
+ * factorisation (R first) in info[l]; the other latents are unaffected.  A latent's result does not depend on the other
+ * latents of the call.
+ *  - q_mu [M, L] and q_sqrt [L, M, M] (in/out), g_q_mu [M, L], g_q_sqrt [L, M, M]: the q_mu and q_sqrt blocks of the flat
+ *    layout below.  Only the lower triangles of q_sqrt and g_q_sqrt are read.  info [L] or NULL.  cfg supplies L and M;
+ *    its other fields are ignored.
+ *  - Returns the first failing pivot like the other batched calls (with info that is the latents' status); host or device
+ *    pointers, async mode as for every call (a failure then reaches mfgp_sync).
+ *  - Cost: about 3 M^3 flop per latent: batched trtri of Lq (its diagonal blocks inverted by tri_block_inv_kernel), five
+ *    DMMA GEMMs on triangular k-ranges, two batched potrf and one trtri, and four streaming kernels. */
+int mfgp_svgp_natgrad(mfgp_handle* h, const mfgp_svgp_cfg* cfg, double gamma, double* q_mu, double* q_sqrt,
+                      const double* g_q_mu, const double* g_q_sqrt, int* info);
+/* mfgp_svgp_natgrad_adam: the device loop of mfgp_svgp_adam with GPflow's natural-gradient recipe.  Step t is
+ * natgrad.minimize(loss, [(q_mu, q_sqrt)]); adam.minimize(loss, other_vars), in that order:
+ *   (a) evaluate the loss and gradients at the current parameters (loss_hist[t], kl_hist[t] come from this evaluation);
+ *   mfgp_svgp_natgrad with gamma = gamma_t[t] on the q_mu and q_sqrt blocks of u;
+ *   (b) evaluate again and apply the Adam update of mfgp_svgp_adam to every entry except the q blocks (their m and v are
+ *   never touched, whatever mask says).
+ * N == 0: every evaluation uses the cfg->B rows of X, Y.  N > 0: X [N, d+1], Y [N, ycols] are the data set and the two
+ * evaluations of step t read the minibatch stream positions pos0 + 2 t B ... + B - 1 and pos0 + (2 t + 1) B ... (GPflow's
+ * training_loss_closure(iter(dataset)) draws a new batch for each optimiser), 1 <= B = cfg->B <= N.  gamma_t [nsteps];
+ * info [L] (required) receives each latent's first natgrad failure as mfgp_svgp_natgrad reports it; the call then returns
+ * a pivot > 0 after writing u, m, v and the histories back.  The rest as mfgp_svgp_adam_minibatch. */
+int mfgp_svgp_natgrad_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* X, const double* Y, int N,
+                           unsigned long long seed, long long pos0, int has_W, double* u, double* m, double* v,
+                           const unsigned char* mask, const double* lr_t, const double* gamma_t, double beta1, double beta2,
+                           double eps, int nsteps, double* loss_hist, double* kl_hist, int* info);
+
 /* Data-parallel SVGP training step on device memory only (SURVEY 8(e) row 2: rows of the minibatch shard across one
  * process per GPU, ONE all-reduce of the flat gradient; reference loops singlebin_svgp.py:79-85, linear_svgp.py:181-190).
  * Per step every rank runs, on the handle's stream and without any host synchronisation:

@@ -72,6 +72,8 @@ def _load():
         "mfgp_svgp_adam": ([vp, vp, vp, vp, i, vp, vp, vp, vp, vp, d, d, d, i, vp, vp], i),
         "mfgp_svgp_adam_minibatch": ([vp, vp, vp, vp, i, u64, i64, i, vp, vp, vp, vp, vp, d, d, d, i, vp, vp], i),
         "mfgp_minibatch_gather": ([vp, vp, i, vp, i, i, u64, i64, vp, i, i, i, vp, vp], i),
+        "mfgp_svgp_natgrad": ([vp, vp, d, vp, vp, vp, vp, vp], i),
+        "mfgp_svgp_natgrad_adam": ([vp, vp, vp, vp, i, u64, i64, i, vp, vp, vp, vp, vp, vp, d, d, d, i, vp, vp, vp], i),
         "mfgp_svgp_flat_size": ([vp, i], l),
         "mfgp_svgp_constrain": ([vp, vp, i, vp, vp], i),
         "mfgp_svgp_elbo_grad_flat": ([vp, vp, vp, vp, i, vp, i, vp], i),
@@ -102,6 +104,7 @@ EXPORTED_SYMBOLS = [
     "mfgp_graph_nparams", "mfgp_graph_cov", "mfgp_graph_cov_diag", "mfgp_graph_gpr_nlml_grad", "mfgp_svgp_elbo_grad", "mfgp_svgp_elbo_grad_v", "mfgp_svgp_predict",
     "mfgp_svgp_posterior_create", "mfgp_svgp_posterior_predict", "mfgp_svgp_posterior_predict_grad",
     "mfgp_svgp_posterior_destroy", "mfgp_svgp_adam", "mfgp_svgp_adam_minibatch", "mfgp_minibatch_gather",
+    "mfgp_svgp_natgrad", "mfgp_svgp_natgrad_adam",
     "mfgp_svgp_flat_size", "mfgp_svgp_constrain", "mfgp_svgp_elbo_grad_flat", "mfgp_svgp_adam_update", "mfgp_gemm",
     "mfgp_potrf", "mfgp_potrf_inv", "mfgp_tall_skinny_update", "mfgp_peer_store", "mfgp_graph_mem_trim", "mfgp_workspace", "mfgp_fp64_peak",
 ]
@@ -208,6 +211,11 @@ def _seed(seed):
     if not 0 <= seed < 1 << 64:
         raise ValueError(f"seed must be an integer in [0, 2**64), got {seed}")
     return seed
+
+
+def _any_nonzero(a):
+    """Whether a host array or device tensor holds a nonzero entry."""
+    return bool((a != 0).any())
 
 
 def as_f64(x):
@@ -398,6 +406,54 @@ class Handle:
                                            _ptr(lr_t), float(beta1), float(beta2), float(eps), n, _ptr(loss), _ptr(kl))
         self._check(rc, "mfgp_svgp_adam_minibatch")
         return loss, kl
+
+    def svgp_natgrad_adam(self, X, Y, L, M, P, has_W, u, m, v, mask, lr_t, gamma_t, beta1, beta2, eps=1e-7, batch_size=None,
+                          seed=0, pos0=0, scale=1.0, kl_mult=1.0, hetero=False, jitter=1e-6, lik_lower=1e-6, masked=False,
+                          lik_per_output=False, info=None):
+        """len(lr_t) steps of GPflow's natural-gradient recipe on the device (include/mfgp.h: mfgp_svgp_natgrad_adam): a
+        natural-gradient step with gamma_t[t] on q_mu and q_sqrt, then Adam on every other entry.  batch_size None: every
+        evaluation uses all rows of X, Y; otherwise the two evaluations of step t read stream positions pos0 + 2 t B ...
+        and pos0 + (2 t + 1) B ....  u, m, v are updated in place as in svgp_adam.  A latent whose natural-gradient step
+        fails raises NotPositiveDefiniteError unless a per-latent `info` array (int32 [L]) is passed: then info[l] holds
+        its first failure's pivot (0 = ok) and the call returns normally.  Returns (loss_hist, kl_hist)."""
+        X, Y, lr_t, gamma_t = as_f64(X), as_f64(Y), as_f64(lr_t), as_f64(gamma_t)
+        n = int(lr_t.shape[0])
+        if tuple(gamma_t.shape) != (n,):
+            raise ValueError(f"gamma_t must hold one step size per step ({n}), got shape {tuple(gamma_t.shape)}")
+        N, d = X.shape[0], X.shape[1] - 1
+        B = N if batch_size is None else int(batch_size)
+        cfg = SvgpCfg(L, M, P, B, d, int(hetero), float(scale), float(kl_mult), float(jitter), float(lik_lower), int(masked),
+                      int(lik_per_output))
+        loss, kl = np.empty(n), np.empty(n)
+        mk = None if mask is None else np.ascontiguousarray(mask, dtype=np.uint8)
+        inf = np.zeros(L, dtype=np.int32) if info is None else info
+        rc = _lib.mfgp_svgp_natgrad_adam(self._h, C.byref(cfg), _ptr(X), _ptr(Y), 0 if batch_size is None else N, _seed(seed),
+                                         int(pos0), int(bool(has_W)), _ptr(u), _ptr(m), _ptr(v),
+                                         None if mk is None else C.c_void_p(mk.ctypes.data), _ptr(lr_t), _ptr(gamma_t),
+                                         float(beta1), float(beta2), float(eps), n, _ptr(loss), _ptr(kl), _ptr(inf))
+        if not (rc > 0 and info is not None and _any_nonzero(info)):  # natgrad failures are the latents' status with info
+            self._check(rc, "mfgp_svgp_natgrad_adam")
+        return loss, kl
+
+    def svgp_natgrad(self, q_mu, q_sqrt, g_q_mu, g_q_sqrt, gamma, info=None):
+        """One natural-gradient step (include/mfgp.h: mfgp_svgp_natgrad) for all L = q_mu.shape[1] latents: q_mu [M, L] and
+        q_sqrt [L, M, M] are updated in place (C-contiguous float64 arrays or device tensors); only the lower triangles of
+        q_sqrt and g_q_sqrt are read.  A latent whose step fails raises NotPositiveDefiniteError unless a per-latent
+        `info` array (int32 [L]) is passed: then info[l] holds its pivot (0 = ok), that latent keeps its values bit for
+        bit and the call returns normally.  Returns info."""
+        for a in (q_mu, q_sqrt):
+            if isinstance(a, np.ndarray) and not (a.dtype == np.float64 and a.flags.c_contiguous):
+                raise ValueError("q_mu and q_sqrt must be C-contiguous float64: they are updated in place")
+        g_q_mu, g_q_sqrt = as_f64(g_q_mu), as_f64(g_q_sqrt)
+        M, L = q_mu.shape
+        if tuple(q_sqrt.shape) != (L, M, M) or tuple(g_q_mu.shape) != (M, L) or tuple(g_q_sqrt.shape) != (L, M, M):
+            raise ValueError(f"need q_mu, g_q_mu [M, L] and q_sqrt, g_q_sqrt [L, M, M] with M={M}, L={L}")
+        cfg = SvgpCfg(L, M, L, 0, 1, 0, 1.0, 1.0, 0.0, 0.0, 0, 0)
+        rc = _lib.mfgp_svgp_natgrad(self._h, C.byref(cfg), float(gamma), _ptr(q_mu), _ptr(q_sqrt), _ptr(g_q_mu), _ptr(g_q_sqrt),
+                                    _ptr(info))
+        if not (rc > 0 and info is not None):
+            self._check(rc, "mfgp_svgp_natgrad")
+        return info
 
     def minibatch_gather(self, X, Y, seed, pos0, batch_size, lo=0, count=None, step=None, Xb=None, Yb=None):
         """Rows of stream positions pos0 + step * batch_size + lo + j, j < count (default batch_size - lo), of the shuffled

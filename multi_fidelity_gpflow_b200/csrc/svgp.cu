@@ -43,6 +43,8 @@ __device__ inline double block_sum256(double v, double* sh) {  // result valid o
     return t;
 }
 
+}  // namespace
+
 // Lq[l][i][j] = tril(q_sqrt[l])  (ld = ldM, zero padded)
 __global__ void tril_copy_kernel(const double* __restrict__ q, int M, long ldM, double* __restrict__ Lq) {
     const int l = blockIdx.y;
@@ -52,6 +54,8 @@ __global__ void tril_copy_kernel(const double* __restrict__ q, int M, long ldM, 
         Lq[(long)l * tot + idx] = (j <= i && j < M) ? q[((long)l * M + i) * M + j] : 0.0;
     }
 }
+
+namespace {
 
 // g_mean[l][n] = sum_m A[m][n] q_mu[m][l];  g_var[l][n] = knn - sum A^2 + sum C^2
 __global__ void col_reduce_kernel(const double* __restrict__ A, const double* __restrict__ Cm, int M, int B, long ldB,
@@ -276,6 +280,8 @@ __global__ void qsqrt_grad_kernel(const double* __restrict__ S1, const double* _
     }
 }
 
+}  // namespace
+
 // mode 0: S <- -tril(S);  mode 1: S <- Phi(S) (lower, halved diagonal)
 __global__ void tri_mask_kernel(double* __restrict__ S, int M, long ldM, int mode) {
     const int l = blockIdx.y;
@@ -302,6 +308,8 @@ __global__ void symmetrize_kernel(const double* __restrict__ T, int M, long ldM,
         if (j < M) Gs[(long)l * tot + idx] = 0.5 * (T[(long)l * tot + idx] + T[(long)l * tot + (long)j * ldM + i]);
     }
 }
+
+namespace {
 
 // theta gradient through K_diag(X): knn = [f=0] vL + [f=1] (rho^2 vL + vD)
 __global__ void knn_grad_kernel(const double* __restrict__ X, int B, int d, const double* __restrict__ theta,
@@ -826,12 +834,16 @@ struct AsyncGuard {  // nested library calls only enqueue; the caller's mode com
 }  // namespace
 
 namespace {
-// The loop of mfgp_svgp_adam and mfgp_svgp_adam_minibatch.  Without a stream (mb == nullptr) every step evaluates the cfg->B
-// rows of X, Y; with one, X, Y hold the N = mb->N rows of the data set and each step first gathers its cfg->B rows of the
-// shuffled stream into batch buffers (positions mb->pos0 + step * B ...), reading the device step counter.
+// The loop of mfgp_svgp_adam, mfgp_svgp_adam_minibatch and mfgp_svgp_natgrad_adam.  Without a stream (mb == nullptr) every
+// step evaluates the cfg->B rows of X, Y; with one, X, Y hold the N = mb->N rows of the data set and each step first gathers
+// its cfg->B rows of the shuffled stream into batch buffers (positions mb->pos0 + step * B ...), reading the device step
+// counter.  With gamma_t the step is GPflow's natgrad.minimize(loss, [(q_mu, q_sqrt)]); adam.minimize(loss, other_vars):
+// evaluate, natural-gradient step on the q blocks of u (status in info [L]), evaluate again, Adam on every other entry;
+// with a stream the two evaluations read the two halves of a global batch of 2B rows (positions pos0 + 2 step B ...).
 int svgp_adam_loop(mfgp_handle* h, const char* who, const mfgp_svgp_cfg* cfg, const double* X, const double* Y,
                    const MinibatchStream* mb, int has_W, double* u, double* m, double* v, const unsigned char* mask,
-                   const double* lr_t, double beta1, double beta2, double eps, int nsteps, double* loss_hist, double* kl_hist) {
+                   const double* lr_t, const double* gamma_t, double beta1, double beta2, double eps, int nsteps,
+                   double* loss_hist, double* kl_hist, int* info) {
     if (!h) return MFGP_ERR_ARG;
     if (!cfg || !X || !Y || !u || !m || !v || !lr_t || nsteps < 0) return mfgp_fail(h, MFGP_ERR_ARG, "%s: NULL argument", who);
     const int L = cfg->L, M = cfg->M, P = cfg->P, B = cfg->B, d = cfg->d;
@@ -861,8 +873,17 @@ int svgp_adam_loop(mfgp_handle* h, const char* who, const mfgp_svgp_cfg* cfg, co
     double* dk = kl_hist ? sc.out(kl_hist, nsteps) : nullptr;
     double* c = sc.alloc<double>((size_t)n);
     double* g = sc.alloc<double>((size_t)n, true);
-    double* ek = sc.alloc<double>(2);
+    double* ek = sc.alloc<double>(gamma_t ? 4 : 2);  // natgrad: [elbo, kl] of the first evaluation, then of the second
     int* dstep = sc.alloc<int>(1, true);
+    const double* dgam = gamma_t ? sc.in(gamma_t, nsteps) : nullptr;
+    int* dinfo = gamma_t ? sc.out(info, (size_t)L, true) : nullptr;
+    unsigned char* qmask = nullptr;  // natgrad: the Adam mask with the q blocks frozen
+    if (gamma_t) {
+        qmask = sc.alloc<unsigned char>((size_t)n);
+        if (qmask && dmask) cudaMemcpyAsync(qmask, dmask, (size_t)n, cudaMemcpyDeviceToDevice, s);
+        else if (qmask) cudaMemsetAsync(qmask, 1, (size_t)n, s);
+        if (qmask) cudaMemsetAsync(qmask + o_qm, 0, (size_t)(n_qm + n_qs), s);
+    }
     if (!sc.ok) return sc.finish();
     const int tb = 256;
     const unsigned gb = (unsigned)((n + tb - 1) / tb);
@@ -870,7 +891,27 @@ int svgp_adam_loop(mfgp_handle* h, const char* who, const mfgp_svgp_cfg* cfg, co
         AsyncGuard guard(h);  // the nested evaluations only enqueue: all their pointers are device memory
         WorkspaceGuard wsg(h);  // step 0 measures the step's temporaries; the captured step takes them from one arena
         const MinibatchStream ds = mb ? MinibatchStream{dX, d + 1, dY, ycols, mb->N, mb->seed, mb->pos0} : MinibatchStream{};
+        auto natgrad_step = [&]() -> int {
+            if (mb && launch_minibatch_gather(s, ds, dstep, 2 * B, 0, B, Xb, Yb))
+                return mfgp_fail(h, MFGP_ERR_CUDA, "%s: gather launch failed", who);
+            svgp_constrain_kernel<<<gb, tb, 0, s>>>(du, c, n, n_theta, o_lv, cfg->lik_lower);
+            MFGP_TRY(mfgp_svgp_elbo_grad_v(h, cfg, mb ? Xb : dX, mb ? Yb : dY, c + o_Z, c, has_W ? c + o_W : nullptr, c + o_qm,
+                                           c + o_qs, c + o_lv, ek, ek + 1, g + o_Z, g, has_W ? g + o_W : nullptr, g + o_qm,
+                                           g + o_qs, g + o_lv));
+            MFGP_TRY(svgp_natgrad_step(h, L, M, du + o_qm, du + o_qs, g + o_qm, g + o_qs, 0.0, dgam, dstep, dinfo));
+            if (mb && launch_minibatch_gather(s, ds, dstep, 2 * B, B, B, Xb, Yb))
+                return mfgp_fail(h, MFGP_ERR_CUDA, "%s: gather launch failed", who);
+            svgp_constrain_kernel<<<gb, tb, 0, s>>>(du, c, n, n_theta, o_lv, cfg->lik_lower);
+            int r = mfgp_svgp_elbo_grad_v(h, cfg, mb ? Xb : dX, mb ? Yb : dY, c + o_Z, c, has_W ? c + o_W : nullptr, c + o_qm,
+                                          c + o_qs, c + o_lv, ek + 2, ek + 3, g + o_Z, g, has_W ? g + o_W : nullptr, g + o_qm,
+                                          g + o_qs, g + o_lv);
+            svgp_adam_kernel<<<gb, tb, 0, s>>>(du, dm, dv, c, g, qmask, n, n_theta, o_lv, cfg->lik_lower, dlr, dstep, beta1, beta2,
+                                               eps, ek, cfg->kl_mult, dl, dk);  // histories from the first evaluation
+            svgp_step_inc_kernel<<<1, 1, 0, s>>>(dstep);
+            return r;
+        };
         auto one_step = [&]() -> int {
+            if (gamma_t) return natgrad_step();
             if (mb && launch_minibatch_gather(s, ds, dstep, B, 0, B, Xb, Yb))
                 return mfgp_fail(h, MFGP_ERR_CUDA, "%s: gather launch failed", who);
             svgp_constrain_kernel<<<gb, tb, 0, s>>>(du, c, n, n_theta, o_lv, cfg->lik_lower);
@@ -923,8 +964,8 @@ int svgp_adam_loop(mfgp_handle* h, const char* who, const mfgp_svgp_cfg* cfg, co
 extern "C" int mfgp_svgp_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* X, const double* Y, int has_W, double* u,
                               double* m, double* v, const unsigned char* mask, const double* lr_t, double beta1, double beta2,
                               double eps, int nsteps, double* loss_hist, double* kl_hist) {
-    return svgp_adam_loop(h, "mfgp_svgp_adam", cfg, X, Y, nullptr, has_W, u, m, v, mask, lr_t, beta1, beta2, eps, nsteps,
-                          loss_hist, kl_hist);
+    return svgp_adam_loop(h, "mfgp_svgp_adam", cfg, X, Y, nullptr, has_W, u, m, v, mask, lr_t, nullptr, beta1, beta2, eps,
+                          nsteps, loss_hist, kl_hist, nullptr);
 }
 
 extern "C" int mfgp_svgp_adam_minibatch(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* X, const double* Y, int N,
@@ -935,8 +976,22 @@ extern "C" int mfgp_svgp_adam_minibatch(mfgp_handle* h, const mfgp_svgp_cfg* cfg
     mb.N = N;
     mb.seed = seed;
     mb.pos0 = pos0;
-    return svgp_adam_loop(h, "mfgp_svgp_adam_minibatch", cfg, X, Y, &mb, has_W, u, m, v, mask, lr_t, beta1, beta2, eps, nsteps,
-                          loss_hist, kl_hist);
+    return svgp_adam_loop(h, "mfgp_svgp_adam_minibatch", cfg, X, Y, &mb, has_W, u, m, v, mask, lr_t, nullptr, beta1, beta2, eps,
+                          nsteps, loss_hist, kl_hist, nullptr);
+}
+
+extern "C" int mfgp_svgp_natgrad_adam(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* X, const double* Y, int N,
+                                      unsigned long long seed, long long pos0, int has_W, double* u, double* m, double* v,
+                                      const unsigned char* mask, const double* lr_t, const double* gamma_t, double beta1,
+                                      double beta2, double eps, int nsteps, double* loss_hist, double* kl_hist, int* info) {
+    if (!h) return MFGP_ERR_ARG;
+    if (!gamma_t || !info || N < 0) return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_natgrad_adam: NULL gamma_t / info or N < 0");
+    MinibatchStream mb{};
+    mb.N = N;
+    mb.seed = seed;
+    mb.pos0 = pos0;
+    return svgp_adam_loop(h, "mfgp_svgp_natgrad_adam", cfg, X, Y, N ? &mb : nullptr, has_W, u, m, v, mask, lr_t, gamma_t, beta1,
+                          beta2, eps, nsteps, loss_hist, kl_hist, info);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -53,6 +53,21 @@ int svgp_posterior_predict_blocked(mfgp_handle* h, const SvgpPosteriorData& q, c
 int launch_svgp_grad_mix(cudaStream_t s, const double* gm, const double* gv, int L, int B, int P, int d, const double* W,
                          double* dmean, double* dvar);
 
+// Streaming helpers of K7's backward pass, shared with the natural-gradient step (natgrad.cu).  All [L][M][ldM] with the
+// latent in blockIdx.y.  tril_copy_kernel: Lq = tril(q) from a dense [L][M][M] q, zero above the diagonal and in the
+// padding.  tri_mask_kernel: mode 0 S <- -tril(S), mode 1 S <- Phi(S) (lower triangle, halved diagonal).
+// symmetrize_kernel: Gs = (T + T^T) / 2.
+__global__ void tril_copy_kernel(const double* __restrict__ q, int M, long ldM, double* __restrict__ Lq);
+__global__ void tri_mask_kernel(double* __restrict__ S, int M, long ldM, int mode);
+__global__ void symmetrize_kernel(const double* __restrict__ T, int M, long ldM, double* __restrict__ Gs);
+
+// natgrad.cu: one natural-gradient step (include/mfgp.h: mfgp_svgp_natgrad) on device memory, enqueued on h->stream with
+// temporaries from a Scope of its own.  q_mu [M][L] and q_sqrt [L][M][M] in place, g_q_mu / g_q_sqrt alike.  The step size
+// is gamma_t[*step] when gamma_t is given, else gamma.  info [L]: a latent whose step fails gets its 1-based pivot unless it
+// already holds a failure, and keeps q_mu[:, l] and q_sqrt[l] bit for bit; failures also reach h->d_info.
+int svgp_natgrad_step(mfgp_handle* h, int L, int M, double* q_mu, double* q_sqrt, const double* g_q_mu, const double* g_q_sqrt,
+                      double gamma, const double* gamma_t, const int* step, int* info);
+
 // The shuffled-epoch row stream over a device-resident data set (include/mfgp.h: minibatch stream): X [N][xcols],
 // Y [N][ycols] or nullptr.
 struct MinibatchStream {

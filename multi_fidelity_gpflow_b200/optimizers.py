@@ -1,6 +1,6 @@
 """Optimisers as the reference's training loops drive them (linear.py:201-234,
 singlebin_svgp.py:77, linear_svgp.py:169): tf.optimizers.Adam with optional
-tf.keras CosineDecay, and gpflow.optimizers.Scipy (L-BFGS-B)."""
+tf.keras CosineDecay, gpflow.optimizers.Scipy (L-BFGS-B) and gpflow.optimizers.NaturalGradient."""
 from __future__ import annotations
 
 import math
@@ -95,3 +95,38 @@ class Scipy:
         res = scipy.optimize.minimize(fun, x0, jac=True, method=method, options=options or {})
         unpack(res.x)
         return res
+
+
+class NaturalGradient:
+    """gpflow.optimizers.NaturalGradient(gamma) with its default XiNat: minimize(value_and_grad, var_list=[(q_mu, q_sqrt)])
+    takes one natural-gradient step on each (q_mu, q_sqrt) pair.  value_and_grad() returns the loss and, LAST, the list of
+    loss gradients of the pairs' parameters in var_list order ([g_q_mu, g_q_sqrt, ...]), for example
+    ``lambda: model.value_and_grad(data, [model.q_mu, model.q_sqrt])``.  The step runs on the GPU
+    (Handle.svgp_natgrad, include/mfgp.h: mfgp_svgp_natgrad).  Unlike GPflow, a latent whose Cholesky factorisation fails
+    does not abort the others: they are updated, it keeps its values, and NotPositiveDefiniteError names it afterwards."""
+
+    def __init__(self, gamma, handle=None):
+        self.gamma = float(gamma)
+        self.handle = handle
+
+    def minimize(self, value_and_grad, var_list):
+        from . import _lib
+
+        h = self.handle or _lib.default_handle()
+        out = value_and_grad()
+        loss, grads = out[0], out[-1]
+        if len(grads) != 2 * len(var_list):
+            raise ValueError(f"value_and_grad returned {len(grads)} gradients for {len(var_list)} (q_mu, q_sqrt) pairs")
+        failed = []
+        for k, (q_mu, q_sqrt) in enumerate(var_list):
+            m = np.array(q_mu.unconstrained, dtype=np.float64, order="C")
+            S = np.ascontiguousarray(np.tril(q_sqrt.unconstrained), dtype=np.float64)
+            info = np.zeros(m.shape[1], dtype=np.int32)
+            h.svgp_natgrad(m, S, grads[2 * k], grads[2 * k + 1], self.gamma, info=info)
+            q_mu.unconstrained = m
+            q_sqrt.unconstrained = S
+            failed += [(k, int(l), int(info[l])) for l in np.flatnonzero(info)]
+        if failed:
+            raise _lib.NotPositiveDefiniteError(
+                "natural-gradient step: Cholesky decomposition was not successful for (pair, latent, pivot) " + str(failed))
+        return loss

@@ -152,10 +152,11 @@ class SVGPBase:
             mask[sl] = 1 if par.trainable else 0
         return items, u, mask
 
-    def _device_loop(self, data, max_iters, initial_lr, kl_multiplier, run, minibatch_size=None, seed=0):
+    def _device_loop(self, data, max_iters, initial_lr, kl_multiplier, run, minibatch_size=None, seed=0, batches_per_step=1):
         """Shared by optimize_on_device / optimize_data_parallel: history semantics of the reference loops, flat packing,
         per-step factors, the minibatch stream position; `run(X, Y, shape, u, mask, lr_t, b1, b2, batch)` -> (u_final,
-        loss_hist, kl_hist), with batch None (full batch) or (minibatch_size, seed, pos0)."""
+        loss_hist, kl_hist), with batch None (full batch) or (minibatch_size, seed, pos0).  Each step draws
+        batches_per_step minibatches from the stream."""
         from .optimizers import adam_step_factors
 
         X, Y = data
@@ -196,10 +197,11 @@ class SVGPBase:
         if resumable:
             self.kl_history = list(self.kl_history) + list(kl)
             if batch is not None:
-                self.minibatch_position = batch[2] + nsteps * batch[0]
+                self.minibatch_position = batch[2] + nsteps * batches_per_step * batch[0]
         return self
 
-    def optimize_on_device(self, data, max_iters, initial_lr, kl_multiplier=1.0, minibatch_size=None, seed=0):
+    def optimize_on_device(self, data, max_iters, initial_lr, kl_multiplier=1.0, minibatch_size=None, seed=0,
+                           natgrad_gamma=None):
         """The model's optimize() loop -- full-batch Adam with CosineDecay(initial_lr, max_iters) on the unconstrained
         trainable variables, loss = -ELBO + (kl_multiplier - 1) KL -- run by mfgp_svgp_adam without a host round trip per
         step.  Same trajectory and the same history semantics as the model's optimize() (tests/test_svgp_device_loop.py):
@@ -212,13 +214,35 @@ class SVGPBase:
         of `data` drawn with `seed` (include/mfgp.h: minibatch stream), gathered on the GPU inside the captured step by
         mfgp_svgp_adam_minibatch, with ELBO scale num_data / B.  loss_history receives each step's minibatch estimate.  A
         resumable model continues the stream at `minibatch_position` (rows drawn so far); SingleBinSVGP starts at 0.
-        A model with num_data=None (SingleBinSVGP's default) accepts only B = N: set num_data to train on minibatches."""
+        A model with num_data=None (SingleBinSVGP's default) accepts only B = N: set num_data to train on minibatches.
+
+        natgrad_gamma (a float, or one value per step this call runs) trains q_mu and q_sqrt with natural gradients
+        instead, as GPflow's natural-gradient recipe does: every step is NaturalGradient(gamma).minimize on
+        [(q_mu, q_sqrt)] and then Adam on the other trainable variables, each on a fresh evaluation of the loss
+        (mfgp_svgp_natgrad_adam).  loss_history receives the loss before the natural-gradient step.  With minibatch_size
+        each of the two evaluations draws its own batch, so minibatch_position advances 2 B per step.  A latent whose
+        natural-gradient step fails keeps its q(u); the parameters and histories are written back and then
+        NotPositiveDefiniteError names the latents."""
+        failed = []
 
         def run(X, Y, shape, u, mask, lr_t, b1, b2, batch):
             m, v = np.zeros_like(u), np.zeros_like(u)
             kw = dict(kl_mult=kl_multiplier, hetero=shape["hetero"], lik_lower=shape["lik_lower"], masked=shape["masked"],
                       lik_per_output=shape["lik_per_output"])
             args = (X, Y, shape["L"], shape["M"], shape["P"], shape["has_W"], u, m, v, mask, lr_t, b1, b2, 1e-7)
+            if natgrad_gamma is not None:
+                n = len(lr_t)
+                gamma_t = np.ascontiguousarray(np.broadcast_to(np.asarray(natgrad_gamma, dtype=np.float64), (n,)))
+                info = np.zeros(shape["L"], dtype=np.int32)
+                gkw = dict(scale=1.0 if self.num_data is None else float(self.num_data) / X.shape[0])
+                if batch is not None:
+                    B, seed_, pos0 = batch
+                    gkw = dict(batch_size=B, seed=seed_, pos0=pos0,
+                               scale=float(X.shape[0] if self.num_data is None else self.num_data) / B)
+                args = args[:11] + (gamma_t,) + args[11:]
+                loss, kl = self.handle.svgp_natgrad_adam(*args, info=info, **gkw, **kw)
+                failed.extend((int(l), int(info[l])) for l in np.flatnonzero(info))
+                return u, loss, kl
             if batch is None:
                 scale = 1.0 if self.num_data is None else float(self.num_data) / X.shape[0]
                 loss, kl = self.handle.svgp_adam(*args, scale=scale, **kw)
@@ -228,7 +252,15 @@ class SVGPBase:
                 loss, kl = self.handle.svgp_adam_minibatch(*args, batch_size=B, seed=seed_, pos0=pos0, scale=scale, **kw)
             return u, loss, kl
 
-        return self._device_loop(data, max_iters, initial_lr, kl_multiplier, run, minibatch_size, seed)
+        if natgrad_gamma is not None and np.ndim(natgrad_gamma) not in (0, 1):
+            raise ValueError("natgrad_gamma must be a float or one value per step")
+        self._device_loop(data, max_iters, initial_lr, kl_multiplier, run, minibatch_size, seed,
+                          batches_per_step=1 if natgrad_gamma is None else 2)
+        if failed:
+            raise _lib.NotPositiveDefiniteError(
+                "natural-gradient step: Cholesky decomposition was not successful for (latent, pivot) " + str(failed)
+                + "; those latents kept their q(u), the other parameters and the histories were written back")
+        return self
 
     def optimize_data_parallel(self, data, max_iters, initial_lr, kl_multiplier=1.0, group=None, timing=None,
                                minibatch_size=None, seed=0):

@@ -257,6 +257,8 @@ int mfgp_svgp_predict(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const double* Xs
  * every latent in one launch, with the results of mfgp_svgp_predict.
  *  - cfg supplies L, M, P, d and jitter as for mfgp_svgp_predict; B and the likelihood fields are ignored.  W [P, L] or
  *    NULL (SeparateIndependent, L == P).  Only the lower triangle of q_sqrt [L, M, M] is read; q_mu is [M, L].
+ *    L <= 65 535: the factorisation launches its batched kernels with the latent index on grid y or z, whose limit that
+ *    is, so a larger L is a bad argument (-1).
  *  - Snapshot: the posterior owns device copies of Z, theta, W, q_mu, Wm = Lm^-1 of K_l(Z,Z) + jitter I and
  *    Lq = tril(q_sqrt) (the factors mfgp_svgp_predict computes); later changes to the caller's buffers do not reach it.
  *  - Memory: one plain cudaMalloc block on the handle's device, owned by the device (not the handle): any handle on that

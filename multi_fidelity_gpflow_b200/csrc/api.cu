@@ -586,6 +586,11 @@ int mfgp_svgp_posterior_create(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const d
     const int L = cfg->L, M = cfg->M, P = cfg->P, d = cfg->d;
     if (L < 1 || M < 1 || P < 1 || d < 1 || d > MFGP_MAX_D || (!W && L != P))
         return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_posterior_create: bad configuration");
+    // svgp_factor puts the latent index on grid y (K1's prescale, tril_copy) or grid z (K1's tile kernel)
+    constexpr int MAX_L = 65535;
+    if (L > MAX_L)
+        return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_posterior_create: L = %d latents, at most %d (the CUDA grid-y/z limit)", L,
+                         MAX_L);
     cudaSetDevice(h->device);
     const int np = 2 * d + 3;
     const long ld = round_up(M, 2);

@@ -287,6 +287,33 @@ int mfgp_svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post,
  * the _predict pipeline.  A point's results do not depend on the other points of the call. */
 int mfgp_svgp_posterior_predict_grad(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns,
                                      double* mean, double* var, double* dmean, double* dvar);
+/* Joint posterior over the Ns test points (GPflow 2.9 SVGP.predict_f(full_cov=True) and predict_f_samples with
+ * full_output_cov=False), per latent l:  Sigma_l = K_l(Xs, Xs) - V^T V + U^T U, V = Wm K_l(Z, Xs), U = Lq^T V;  per output
+ * p:  Sigma_p = sum_l W_pl^2 Sigma_l with W (mix_latent_gp), Sigma_p = Sigma_p's own latent without W (L == P).
+ * mfgp_svgp_posterior_predict_cov: mean [Ns, P] and cov [P, Ns, Ns] (both triangles, exactly symmetric).  mean is
+ * _predict's mean bit for bit and diag(cov[p]) is _predict's var[:, p] bit for bit.
+ * mfgp_svgp_posterior_sample: samples[p, i, k] = mean[i, p] + sum_j L_p[i, j] z[p, j, k] with L_p L_p^T = Sigma_p +
+ * jitter I, Sigma_p exactly the matrix _predict_cov returns (GPflow sample_mvn per output: no draw is correlated across
+ * outputs).  z and samples are [P, Ns, S] and must not overlap.
+ *  - Failures: info[p] (info [P] or NULL) is the 1-based first pivot of Sigma_p + jitter I that is not > 0 (NaN counts),
+ *    so an output reached by a latent whose factorisation failed at creation reports 1, and all of its samples are NaN.
+ *    The call returns the first failure's pivot with or without info.  _predict_cov gives NaN for such outputs and
+ *    returns 0.
+ *  - A test row with fidelity not in {0, 1} has a zero row and column in cov and a zero mean.  With jitter > 0 its samples
+ *    are sqrt(jitter) z; with jitter == 0 it is a failed pivot.
+ *  - jitter finite and >= 0, S >= 0, no NULL pointer except info: otherwise -1.  P > 65 535 outputs: -1 (the outputs are
+ *    the problems of batched launches; _predict accepts any P).  Ns == 0 or S == 0 returns 0.  Pointers, async mode and
+ *    the device check as for _predict.  Indices are 64-bit: P * Ns * S and P * Ns^2 may exceed 2^31.
+ *  - A sample column's values do not depend on S or on how the work is split.
+ *  - Routes: mean and var run _predict's own route.  M <= 64, d <= 16 and Ns <= 64 form every Sigma_l in ONE kernel
+ *    (svgp_posterior_joint_kernel, one CTA per latent); anything else runs svgp_conditional on all Ns points, K1 for
+ *    K_l(Xs, Xs) and two lower-only batched GEMMs, not chunked (an out-of-memory error gives the workspace size).  Then
+ *    the mix (with W), and the exact GP's blocked tail with one problem per output: the diagonal <- var (+ jitter), and
+ *    cov, or potrf and the L Z GEMM. */
+int mfgp_svgp_posterior_predict_cov(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns,
+                                    double* mean, double* cov);
+int mfgp_svgp_posterior_sample(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns, int S,
+                               double jitter, const double* z, double* samples, int* info);
 int mfgp_svgp_posterior_destroy(mfgp_svgp_posterior* post);
 
 /* Training loop on the device for the SVGP models (SURVEY 8(f) rank 1): the optimize() loops of mfgpflow/singlebin_svgp.py:

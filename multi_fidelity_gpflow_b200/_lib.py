@@ -68,6 +68,8 @@ def _load():
         "mfgp_svgp_posterior_create": ([vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(vp)], i),
         "mfgp_svgp_posterior_predict": ([vp, vp, vp, i, vp, vp], i),
         "mfgp_svgp_posterior_predict_grad": ([vp, vp, vp, i, vp, vp, vp, vp], i),
+        "mfgp_svgp_posterior_predict_cov": ([vp, vp, vp, i, vp, vp], i),
+        "mfgp_svgp_posterior_sample": ([vp, vp, vp, i, i, d, vp, vp, vp], i),
         "mfgp_svgp_posterior_destroy": ([vp], i),
         "mfgp_svgp_adam": ([vp, vp, vp, vp, i, vp, vp, vp, vp, vp, d, d, d, i, vp, vp], i),
         "mfgp_svgp_adam_minibatch": ([vp, vp, vp, vp, i, u64, i64, i, vp, vp, vp, vp, vp, d, d, d, i, vp, vp], i),
@@ -103,7 +105,7 @@ EXPORTED_SYMBOLS = [
     "mfgp_gpr_posterior_predict_cov", "mfgp_gpr_posterior_sample", "mfgp_gpr_posterior_destroy",
     "mfgp_graph_nparams", "mfgp_graph_cov", "mfgp_graph_cov_diag", "mfgp_graph_gpr_nlml_grad", "mfgp_svgp_elbo_grad", "mfgp_svgp_elbo_grad_v", "mfgp_svgp_predict",
     "mfgp_svgp_posterior_create", "mfgp_svgp_posterior_predict", "mfgp_svgp_posterior_predict_grad",
-    "mfgp_svgp_posterior_destroy", "mfgp_svgp_adam", "mfgp_svgp_adam_minibatch", "mfgp_minibatch_gather",
+    "mfgp_svgp_posterior_predict_cov", "mfgp_svgp_posterior_sample", "mfgp_svgp_posterior_destroy", "mfgp_svgp_adam", "mfgp_svgp_adam_minibatch", "mfgp_minibatch_gather",
     "mfgp_svgp_natgrad", "mfgp_svgp_natgrad_adam",
     "mfgp_svgp_flat_size", "mfgp_svgp_constrain", "mfgp_svgp_elbo_grad_flat", "mfgp_svgp_adam_update", "mfgp_gemm",
     "mfgp_potrf", "mfgp_potrf_inv", "mfgp_tall_skinny_update", "mfgp_peer_store", "mfgp_graph_mem_trim", "mfgp_workspace", "mfgp_fp64_peak",
@@ -806,6 +808,50 @@ class SvgpPosterior(_Posterior):
                                                                  _ptr(var), _ptr(dmean), _ptr(dvar)),
                            "mfgp_svgp_posterior_predict_grad")
         return mean, var, dmean, dvar
+
+    def predict_cov(self, Xs, mean=None, cov=None):
+        """Mean [Ns, P] and each output's joint covariance cov [P, Ns, Ns] over the test points (GPflow
+        SVGP.predict_f(full_cov=True)).  mean is predict()'s mean and diag(cov[p]) predict()'s var[:, p], bit for bit.
+        Host arrays or device tensors."""
+        Xs = self._xs(Xs)
+        Ns = Xs.shape[0]
+        mean = np.empty((Ns, self.P)) if mean is None else mean
+        cov = np.empty((self.P, Ns, Ns)) if cov is None else cov
+        self.handle._check(_lib.mfgp_svgp_posterior_predict_cov(self.handle._h, self._p, _ptr(Xs), Ns, _ptr(mean), _ptr(cov)),
+                           "mfgp_svgp_posterior_predict_cov")
+        return mean, cov
+
+    def sample(self, Xs, z, jitter=1e-6, samples=None, info=None):
+        """Draws [P, Ns, S], each output on its own: samples[p] = mean[:, p] + L_p z[p] over the test-point axis,
+        L_p L_p^T = cov[p] + jitter I, for standard normals z [P, Ns, S].  An output whose factor fails raises
+        NotPositiveDefiniteError unless a per-output `info` array (int32 [P]) is passed: then info[p] holds its 1-based
+        pivot (0 = ok) and its samples are NaN.  Host arrays or device tensors."""
+        Xs = self._xs(Xs)
+        Ns = Xs.shape[0]
+        z = as_f64(z)
+        if len(z.shape) != 3 or tuple(z.shape[:2]) != (self.P, Ns):
+            raise ValueError(f"z must be [P={self.P}, Ns={Ns}, S]")
+        S = int(z.shape[2])
+        samples = np.empty((self.P, Ns, S)) if samples is None else samples
+        rc = _lib.mfgp_svgp_posterior_sample(self.handle._h, self._p, _ptr(Xs), Ns, S, float(jitter), _ptr(z), _ptr(samples),
+                                             _ptr(info))
+        if not (rc > 0 and info is not None):
+            self.handle._check(rc, "mfgp_svgp_posterior_sample")
+        return samples
+
+    def draw_f(self, Xs, num_samples=None, full_cov=True, full_output_cov=False, seed=None, info=None):
+        """GPflow's predict_f_samples with full_output_cov=False: [P, Ns, S] (S = 1 when num_samples is None), from
+        z = np.random.default_rng(seed).standard_normal((P, Ns, S)).  full_cov=True: sample() with GPflow's default
+        jitter 1e-6; full_cov=False: mean + sqrt(var) z from predict(), without jitter."""
+        if full_output_cov:
+            raise NotImplementedError("full_output_cov: draws correlated across the outputs through W are not supported")
+        Xs = self._xs(Xs)
+        S = 1 if num_samples is None else int(num_samples)
+        z = np.random.default_rng(seed).standard_normal((self.P, Xs.shape[0], S))
+        if full_cov:
+            return self.sample(Xs, z, jitter=1e-6, info=info)
+        mean, var = self.predict(Xs)
+        return mean.T[:, :, None] + np.sqrt(var).T[:, :, None] * z
 
 
 _default = {}

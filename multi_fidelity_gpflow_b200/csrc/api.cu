@@ -628,8 +628,30 @@ int mfgp_svgp_posterior_create(mfgp_handle* h, const mfgp_svgp_cfg* cfg, const d
 }  // extern "C"
 
 namespace {
-// mfgp_svgp_posterior_predict and _predict_grad: one body, the gradients when dmean != NULL.  With W the fused route
-// writes the latents to [L][Ns] (and [L][Ns][d]) scratch and the mix kernels form the outputs.
+// _predict's route on device buffers: the fused kernel for M <= 64, d <= 16 (with W into [L][Ns] (and [L][Ns][d])
+// scratch, then the mix kernels), the blocked route otherwise.  mean / var [Ns][P], dmean / dvar [Ns][P][d] or NULL.
+int svgp_predict_device(mfgp_handle* h, Scope& sc, const SvgpPosteriorData& q, const double* dXs, int Ns, double* dm,
+                        double* dv, double* ddm, double* ddv, const char* name) {
+    if (svgp_posterior_fused_ok(q.L, q.M, q.d)) {
+        if (!q.W) {
+            if (svgp_posterior_predict_fused(h->stream, q, dXs, Ns, dm, dv, 1, q.P, ddm, ddv))
+                return mfgp_fail(h, MFGP_ERR_CUDA, "%s: fused kernel launch failed", name);
+        } else {
+            const size_t lat = (size_t)q.L * Ns;
+            double* g = sc.alloc<double>(2 * lat);  // latent marginals [L][Ns], mean then var
+            double* gd = ddm ? sc.alloc<double>(2 * lat * q.d) : nullptr;  // latent gradients [L][Ns][d], mean then var
+            if (!sc.ok) return sc.finish();
+            if (svgp_posterior_predict_fused(h->stream, q, dXs, Ns, g, g + lat, Ns, 1, gd, ddm ? gd + lat * q.d : nullptr) ||
+                launch_svgp_mix(h->stream, g, g + lat, q.L, Ns, q.P, q.W, dm, dv) ||
+                (ddm && launch_svgp_grad_mix(h->stream, gd, gd + lat * q.d, q.L, Ns, q.P, q.d, q.W, ddm, ddv)))
+                return mfgp_fail(h, MFGP_ERR_CUDA, "%s: fused kernel launch failed", name);
+        }
+        return 0;
+    }
+    return svgp_posterior_predict_blocked(h, q, dXs, Ns, dm, dv, ddm, ddv);
+}
+
+// mfgp_svgp_posterior_predict and _predict_grad: one body, the gradients when dmean != NULL.
 int svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns, double* mean,
                            double* var, double* dmean, double* dvar, const char* name) {
     if (const int rc = posterior_predict_prologue(h, post, Xs, Ns, mean, var, name); rc <= 0) return rc;
@@ -641,23 +663,78 @@ int svgp_posterior_predict(mfgp_handle* h, const mfgp_svgp_posterior* post, cons
     double* ddm = dmean ? sc.out(dmean, (size_t)Ns * q.P * q.d) : nullptr;
     double* ddv = dmean ? sc.out(dvar, (size_t)Ns * q.P * q.d) : nullptr;
     if (!sc.ok) return sc.finish();
-    if (svgp_posterior_fused_ok(q.L, q.M, q.d)) {
-        if (!q.W) {
-            if (svgp_posterior_predict_fused(h->stream, q, dXs, Ns, dm, dv, 1, q.P, ddm, ddv))
-                return mfgp_fail(h, MFGP_ERR_CUDA, "%s: fused kernel launch failed", name);
-        } else {
-            const size_t lat = (size_t)q.L * Ns;
-            double* g = sc.alloc<double>(2 * lat);  // latent marginals [L][Ns], mean then var
-            double* gd = dmean ? sc.alloc<double>(2 * lat * q.d) : nullptr;  // latent gradients [L][Ns][d], mean then var
-            if (!sc.ok) return sc.finish();
-            if (svgp_posterior_predict_fused(h->stream, q, dXs, Ns, g, g + lat, Ns, 1, gd, dmean ? gd + lat * q.d : nullptr) ||
-                launch_svgp_mix(h->stream, g, g + lat, q.L, Ns, q.P, q.W, dm, dv) ||
-                (dmean && launch_svgp_grad_mix(h->stream, gd, gd + lat * q.d, q.L, Ns, q.P, q.d, q.W, ddm, ddv)))
-                return mfgp_fail(h, MFGP_ERR_CUDA, "%s: fused kernel launch failed", name);
-        }
-    } else {
-        MFGP_TRY(svgp_posterior_predict_blocked(h, q, dXs, Ns, dm, dv, ddm, ddv));
+    MFGP_TRY(svgp_predict_device(h, sc, q, dXs, Ns, dm, dv, ddm, ddv, name));
+    return sc.finish();
+}
+
+// mfgp_svgp_posterior_predict_cov and _sample: one body, the samples when `sample`.  mean and var come from _predict's own
+// route; Sigma_l from the fused kernel or the blocked route; with W the mix to Sigma_p; then the exact GP's blocked tail
+// with the P outputs as its problems (one column each): the diagonal <- var, and cov out or the samples.
+int svgp_posterior_joint(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns, double* mean, double* cov,
+                         bool sample, int S, double jitter, const double* z, double* samples, int* info, const char* name) {
+    CHECK_H(h);
+    if (!post || !Xs || Ns < 0 ||
+        (sample ? (!z || !samples || S < 0 || !std::isfinite(jitter) || jitter < 0.0) : (!mean || !cov)))
+        return mfgp_fail(h, MFGP_ERR_ARG, "%s: bad argument", name);
+    if (post->m.device != h->device)
+        return mfgp_fail(h, MFGP_ERR_ARG, "%s: the posterior lives on device %d, the handle on %d", name, post->m.device,
+                         h->device);
+    const SvgpPosteriorData& q = post->q;
+    constexpr int MAX_P = 65535;  // the outputs are the problems of the batched factorisation and GEMMs (grid y / z)
+    if (q.P > MAX_P)
+        return mfgp_fail(h, MFGP_ERR_ARG, "%s: P = %d outputs, at most %d (the CUDA grid-y/z limit)", name, q.P, MAX_P);
+    if (sample) {
+        const size_t bytes = (size_t)q.P * Ns * S * sizeof(double);
+        const char *zc = reinterpret_cast<const char*>(z), *sc = reinterpret_cast<const char*>(samples);
+        if (zc < sc + bytes && sc < zc + bytes && bytes) return mfgp_fail(h, MFGP_ERR_ARG, "%s: z and samples overlap", name);
     }
+    if (Ns == 0 || (sample && S == 0)) return 0;
+    cudaSetDevice(h->device);
+    const long lds = round_up(Ns, 2);
+    const bool fused = svgp_posterior_joint_fused_ok(q.L, q.M, q.d, Ns);
+    {  // the covariances couple every pair of points, so nothing is chunked: check the workspace up front
+        const size_t sig = (size_t)q.L * Ns * lds + (q.W ? (size_t)q.P * Ns * lds : 0);
+        const size_t cond = fused ? 0 : (size_t)3 * q.L * q.M * lds + (size_t)3 * q.L * Ns;
+        const size_t tail = sample ? (size_t)chol_dinv_count(Ns, q.P) + (size_t)q.P * Ns * (1 + round_up(S, 2)) : 0;
+        const size_t need = (sig + cond + tail + (size_t)4 * q.P * Ns) * sizeof(double);
+        size_t freeb = 0, totb = 0;
+        cudaMemGetInfo(&freeb, &totb);
+        if (need > freeb)
+            return mfgp_fail(h, MFGP_ERR_CUDA, "%s: out of memory: the joint covariance of %d latents and %d outputs over %d "
+                             "points needs %zu bytes of workspace, %zu are free", name, q.L, q.P, Ns, need, freeb);
+    }
+    Scope sc(h);
+    cudaStream_t s = h->stream;
+    const double* dXs = sc.in(Xs, (size_t)Ns * (q.d + 1));
+    double* dm = sample ? sc.alloc<double>((size_t)Ns * q.P) : sc.out(mean, (size_t)Ns * q.P);
+    double* dv = sc.alloc<double>((size_t)Ns * q.P);
+    double* vt = sc.alloc<double>((size_t)q.P * Ns);  // var, then mean as [P][Ns]
+    double* mt = sample ? sc.alloc<double>((size_t)q.P * Ns) : nullptr;
+    double* Sl = sc.alloc<double>((size_t)q.L * Ns * lds);
+    double* Sp = q.W ? sc.alloc<double>((size_t)q.P * Ns * lds) : Sl;
+    if (!sc.ok) return sc.finish();
+    MFGP_TRY(svgp_predict_device(h, sc, q, dXs, Ns, dm, dv, nullptr, nullptr, name));
+    if (fused) {
+        if (svgp_posterior_cov_fused(s, q, dXs, Ns, Sl, lds))
+            return mfgp_fail(h, MFGP_ERR_CUDA, "%s: fused kernel launch failed", name);
+    } else {
+        MFGP_TRY(svgp_posterior_cov_blocked(h, sc, q, dXs, Ns, Sl, lds));
+    }
+    if ((q.W && launch_svgp_cov_mix(s, Sl, q.L, Ns, lds, q.P, q.W, Sp)) || launch_outputs_major(s, dv, Ns, q.P, vt) ||
+        (sample && launch_outputs_major(s, dm, Ns, q.P, mt)))
+        return mfgp_fail(h, MFGP_ERR_CUDA, "%s: mix launch failed", name);
+    if (!sample) {
+        double* dc = sc.out(cov, (size_t)q.P * Ns * Ns);
+        if (!sc.ok) return sc.finish();
+        if (launch_joint_diag(s, Sp, Ns, lds, q.P, vt, 0.0, dc))
+            return mfgp_fail(h, MFGP_ERR_CUDA, "%s: joint_diag_kernel launch failed", name);
+        return sc.finish();
+    }
+    const double* dz = sc.in(z, (size_t)q.P * Ns * S);
+    double* ds = sc.out(samples, (size_t)q.P * Ns * S);
+    int* di = info ? sc.out(info, q.P, true) : sc.alloc<int>(q.P, true);
+    if (!sc.ok) return sc.finish();
+    MFGP_TRY(gpr_joint_sample(h, sc, Sp, Ns, lds, q.P, vt, jitter, dz, S, 1, mt, ds, di));
     return sc.finish();
 }
 }  // namespace
@@ -676,6 +753,18 @@ int mfgp_svgp_posterior_predict_grad(mfgp_handle* h, const mfgp_svgp_posterior* 
         return mfgp_fail(h, MFGP_ERR_ARG, "mfgp_svgp_posterior_predict_grad: bad argument (dmean and dvar are required)");
     }
     return svgp_posterior_predict(h, post, Xs, Ns, mean, var, dmean, dvar, "mfgp_svgp_posterior_predict_grad");
+}
+
+int mfgp_svgp_posterior_predict_cov(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns, double* mean,
+                                    double* cov) {
+    return svgp_posterior_joint(h, post, Xs, Ns, mean, cov, false, 0, 0.0, nullptr, nullptr, nullptr,
+                                "mfgp_svgp_posterior_predict_cov");
+}
+
+int mfgp_svgp_posterior_sample(mfgp_handle* h, const mfgp_svgp_posterior* post, const double* Xs, int Ns, int S,
+                               double jitter, const double* z, double* samples, int* info) {
+    return svgp_posterior_joint(h, post, Xs, Ns, nullptr, nullptr, true, S, jitter, z, samples, info,
+                                "mfgp_svgp_posterior_sample");
 }
 
 int mfgp_svgp_posterior_destroy(mfgp_svgp_posterior* post) {

@@ -101,12 +101,11 @@ __global__ void joint_sample_epilogue_kernel(double* __restrict__ out, int Ns, l
 
 // The joint outputs of nb problems (from b0) of the blocked route, from the chunk's A_s = W K_s [nb][N][lds], var and mean:
 // K_ss (K1, symmetric), Sigma = K_ss - A_s^T A_s (lower tiles), diag <- var.  _predict_cov mirrors Sigma into cov;
-// _sample adds the jitter, factors with potrf and forms samples = L Z + mean.
+// _sample goes on in gpr_joint_sample.
 int joint_chunk(mfgp_handle* h, Scope& sc, const GprPosteriorData& q, long b0, int nb, const double* Xs, int Ns,
                 const double* th, const double* As, long lds, const double* var, const double* mean, const GprJointOut& j) {
     cudaStream_t s = h->stream;
-    const int np = 2 * q.d + 3, N = q.N;
-    double* Sg = sc.alloc<double>((size_t)nb * Ns * lds, true);
+    const int np = 2 * q.d + 3, N = q.N;    double* Sg = sc.alloc<double>((size_t)nb * Ns * lds, true);
     if (!sc.ok) return sc.finish();
     CovArgs k{};
     k.Xa = Xs; k.Na = Ns; k.Xb = Xs; k.Nb = Ns; k.d = q.d;
@@ -125,43 +124,58 @@ int joint_chunk(mfgp_handle* h, Scope& sc, const GprPosteriorData& q, long b0, i
     g.batch = nb;
     g.lower_only = 1;
     if (launch_gemm(s, g)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (Sigma) failed");
-    const long work = j.SP ? Ns : (long)Ns * Ns;
-    const dim3 dgrid((unsigned)((work + 255) / 256 < 64 ? (work + 255) / 256 : 64), (unsigned)nb);
-    joint_diag_kernel<<<dgrid, 256, 0, s>>>(Sg, Ns, lds, var, j.SP ? j.jitter : 0.0, j.SP ? nullptr : j.cov + b0 * Ns * Ns);
-    if (!j.SP) return cudaGetLastError() == cudaSuccess ? 0 : mfgp_fail(h, MFGP_ERR_CUDA, "joint_diag_kernel launch failed");
+    if (!j.SP) {
+        if (launch_joint_diag(s, Sg, Ns, lds, nb, var, 0.0, j.cov + b0 * Ns * Ns))
+            return mfgp_fail(h, MFGP_ERR_CUDA, "joint_diag_kernel launch failed");
+        return 0;
+    }
+    return gpr_joint_sample(h, sc, Sg, Ns, lds, nb, var, j.jitter, j.z + b0 * Ns * j.SP, j.SP, q.P, mean,
+                            j.samples + b0 * Ns * j.SP, j.info + b0);
+}
 
+}  // namespace
+
+int launch_joint_diag(cudaStream_t s, double* Sg, int Ns, long lds, int nb, const double* var, double jitter, double* cov) {
+    const long work = cov ? (long)Ns * Ns : Ns;
+    const dim3 dgrid((unsigned)((work + 255) / 256 < 64 ? (work + 255) / 256 : 64), (unsigned)nb);
+    joint_diag_kernel<<<dgrid, 256, 0, s>>>(Sg, Ns, lds, var, jitter, cov);
+    return cudaGetLastError() == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+}
+
+int gpr_joint_sample(mfgp_handle* h, Scope& sc, double* Sg, int Ns, long lds, int nb, const double* var, double jitter,
+                     const double* z, long SP, int P, const double* mean, double* samples, int* info) {
+    cudaStream_t s = h->stream;
+    if (launch_joint_diag(s, Sg, Ns, lds, nb, var, jitter, nullptr))
+        return mfgp_fail(h, MFGP_ERR_CUDA, "joint_diag_kernel launch failed");
     CholArgs ch{};
     ch.A = Sg; ch.N = Ns; ch.lda = lds; ch.strideA = (long)Ns * lds; ch.batch = nb;
     ch.dinv = sc.alloc<double>((size_t)chol_dinv_count(Ns, nb));
     ch.logd = sc.alloc<double>((size_t)nb * Ns);
-    const long ldz = round_up(j.SP, 2);
+    const long ldz = round_up(SP, 2);
     double* Zw = sc.alloc<double>((size_t)nb * Ns * ldz);
     if (!sc.ok) return sc.finish();
-    ch.d_info = h->d_info; ch.aux = h->aux_stream; ch.ev = h->ev; ch.info_vec = j.info + b0;
+    ch.d_info = h->d_info; ch.aux = h->aux_stream; ch.ev = h->ev; ch.info_vec = info;
     if (launch_potrf(s, ch)) return mfgp_fail(h, MFGP_ERR_CUDA, "potrf launch (Sigma) failed");
-    // the GEMM's TMA operands need an even leading dimension: stage z with ld = round_up(S P, 2)
-    CUDA_TRY(h, cudaMemcpy2DAsync(Zw, ldz * sizeof(double), j.z + b0 * Ns * j.SP, j.SP * sizeof(double),
-                                  j.SP * sizeof(double), (size_t)nb * Ns, cudaMemcpyDeviceToDevice, s));
-    double* out = j.samples + b0 * Ns * j.SP;
+    // the GEMM's TMA operands need an even leading dimension: stage z with ld = round_up(SP, 2)
+    CUDA_TRY(h, cudaMemcpy2DAsync(Zw, ldz * sizeof(double), z, SP * sizeof(double), SP * sizeof(double), (size_t)nb * Ns,
+                                  cudaMemcpyDeviceToDevice, s));
     constexpr long MAX_COLS = 1L << 30;  // GemmArgs::N is an int
-    for (long c0 = 0; c0 < j.SP; c0 += MAX_COLS) {
+    for (long c0 = 0; c0 < SP; c0 += MAX_COLS) {
         GemmArgs lz;  // samples = L Z (L lower triangular)
-        lz.M = Ns; lz.N = (int)(j.SP - c0 < MAX_COLS ? j.SP - c0 : MAX_COLS); lz.K = Ns;
+        lz.M = Ns; lz.N = (int)(SP - c0 < MAX_COLS ? SP - c0 : MAX_COLS); lz.K = Ns;
         lz.A = Sg; lz.lda = lds; lz.strideA = (long)Ns * lds;
         lz.B = Zw + c0; lz.ldb = ldz; lz.strideB = (long)Ns * ldz;
-        lz.C = out + c0; lz.ldc = j.SP; lz.strideC = (long)Ns * j.SP;
+        lz.C = samples + c0; lz.ldc = SP; lz.strideC = (long)Ns * SP;
         lz.batch = nb;
         lz.krange = KR_HI_I;
-        lz.small_tiles = 1;  // one tile shape whatever S * P: a column's value does not depend on S
+        lz.small_tiles = 1;  // one tile shape whatever SP: a column's value does not depend on S
         if (launch_gemm(s, lz)) return mfgp_fail(h, MFGP_ERR_CUDA, "gemm (L Z) failed");
     }
-    const long per = (long)Ns * j.SP;
+    const long per = (long)Ns * SP;
     const unsigned ex = (unsigned)((per + 255) / 256 < 1024 ? (per + 255) / 256 : 1024);
-    joint_sample_epilogue_kernel<<<dim3(ex, (unsigned)nb), 256, 0, s>>>(out, Ns, j.SP, q.P, mean, j.info + b0);
+    joint_sample_epilogue_kernel<<<dim3(ex, (unsigned)nb), 256, 0, s>>>(samples, Ns, SP, P, mean, info);
     return cudaGetLastError() == cudaSuccess ? 0 : mfgp_fail(h, MFGP_ERR_CUDA, "joint_sample_epilogue_kernel launch failed");
 }
-
-}  // namespace
 
 using Factor = GprFactor;
 

@@ -78,6 +78,15 @@ int gpr_posterior_joint_fused(cudaStream_t s, const GprPosteriorData& q, const d
 int gpr_posterior_predict_blocked(mfgp_handle* h, const GprPosteriorData& q, const double* Xs, int Ns, double* mean,
                                   double* var, double* dmean = nullptr, double* dvar = nullptr,
                                   const GprJointOut* joint = nullptr);
+// The tail of the blocked joint route, shared with the SVGP posterior (api.cu), for nb problems of Sigma [nb][Ns][lds]
+// whose lower triangle is valid off the diagonal.  launch_joint_diag: the diagonal <- var [nb][Ns] + jitter; with cov
+// [nb][Ns][Ns], cov <- Sigma with var on the diagonal, the lower triangle mirrored (Sigma itself keeps its diagonal).
+// gpr_joint_sample: the diagonal <- var + jitter, L L^T = Sigma (potrf, in place), samples [nb][Ns][SP] = L z + mean for
+// z [nb][Ns][SP] and mean [nb][Ns][P] (column c takes mean column c % P).  info [nb], zeroed by the caller, gets each
+// problem's 1-based failed pivot, whose samples are then NaN; the first failure also reaches h->d_info.
+int launch_joint_diag(cudaStream_t s, double* Sg, int Ns, long lds, int nb, const double* var, double jitter, double* cov);
+int gpr_joint_sample(mfgp_handle* h, Scope& sc, double* Sg, int Ns, long lds, int nb, const double* var, double jitter,
+                     const double* z, long SP, int P, const double* mean, double* samples, int* info);
 // The input-gradient contraction of the blocked route (posterior.cu) for nb problems of q (theta from q.theta):
 // dmean[b][s][p][j] = sum_n alpha[b][n][p] dk_sn/dx_sj, dvar[b][s][j] = -2 sum_n beta[b][n][s] dk_sn/dx_sj, with
 // alpha [nb][N][q.Pp] = W^T a and beta [nb][N][ldb] = K^-1 K_s.

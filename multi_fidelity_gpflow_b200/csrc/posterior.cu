@@ -2,7 +2,7 @@
 // mfgp_svgp_posterior_predict) for the small problems of the per-bin emulators (N or M <= 64, d <= 16): one launch serves
 // every problem (or latent) and test point.  Also the input-gradient kernel of the exact posterior's blocked route.
 //
-// The five fused kernels are built from one set of device pieces (the building blocks below) on one decomposition.  One
+// The six fused kernels are built from one set of device pieces (the building blocks below) on one decomposition.  One
 // CTA per (problem, chunk of test points) stages the problem's factor W = L^-1 (lower triangle) and its scaled training
 // inputs in shared memory once; each warp then takes 8 test points at a time:
 //   K_s^T [8 x N]    built directly in the DMMA A-fragment layout: lane (g, t) evaluates k(x_n, xs_g) for n = 4k + t, so
@@ -37,6 +37,10 @@
 // svgp_posterior_predict_kernel (mfgp_svgp_posterior_predict): the inducing points Z in the place of X, one latent per
 // blockIdx.y, W = Wm.  U = Lq^T V (upper_tri_product with F = Lq) never leaves the accumulators: sum U^2 is lane-local.
 // var = k_ss - sum V^2 + sum U^2, mean = V^T q_mu.
+//
+// svgp_posterior_joint_kernel (mfgp_svgp_posterior_predict_cov / _sample, Ns <= 64): one CTA per latent; predict's K_s, V
+// and U per 8-point group, V^T and U^T to shared memory, then Sigma_l = K_ss - V^T V + U^T U on the lower 8x8 tiles as the
+// exact joint kernel forms K_ss - V^T V, mirrored.  The outputs' mix, diagonal and sampling tail run after it (api.cu).
 //
 // svgp_posterior_predict_grad_kernel (mfgp_svgp_posterior_predict_grad): predict's values, computed as predict computes
 // them, plus the input gradients.  d var / dx*_j = -2 beta . gk with beta = Wm^T (V - Lq U): U stays in a fragment row,
@@ -1012,6 +1016,103 @@ __global__ void __launch_bounds__(PW * 32) gpr_posterior_joint_kernel(JointArgs 
     }
 }
 
+// ---- joint covariance of the SVGP latents (mfgp_svgp_posterior_predict_cov / _sample), Ns <= 64 test points.  One CTA
+//      per latent, all latents in one launch: predict's staging of Wm, Lq^T and Z, the records of every test point, then
+//      per 8-point group predict's K_s, V and U with V^T and U^T to shared memory, then Sigma_l = K_ss - V^T V + U^T U on
+//      the lower 8x8 tiles (DMMA over the inducing index, K_ss from the point records), each entry also stored mirrored.
+//      The diagonal is written too; the caller replaces it with predict's var.
+size_t svgp_joint_smem_bytes(int NT, int NST, int d) {
+    const int NP = 8 * NT, NSP = 8 * NST;
+    return sizeof(double) * (2 * (size_t)NP * w_pitch(NP) + (size_t)(2 * d + 4) * NP + (size_t)NSP * rec_len(d) +
+                             2 * (size_t)NSP * w_pitch(NP));
+}
+
+struct SvgpJointArgs {
+    SvgpPosteriorData q;
+    const double* Xs;
+    int Ns;
+    double* Sl;  // [L][Ns][lds]
+    long lds;
+};
+
+template <int NT>
+__global__ void __launch_bounds__(PW * 32, 1) svgp_posterior_joint_kernel(SvgpJointArgs p) {
+    constexpr int NP = 8 * NT, WP = w_pitch(NP);
+    extern __shared__ __align__(16) double sm[];
+    __shared__ __align__(16) double etab[512];
+    const SvgpPosteriorData& q = p.q;
+    const int M = q.M, d = q.d, S1 = rec_len(d), Ns = p.Ns, NST = (Ns + 7) / 8, NSP = 8 * NST;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
+    const long l = blockIdx.y;
+    const double* __restrict__ th = q.theta + l * (2 * d + 3);
+    double* Ws = sm;                     // [NP][WP]    Wm, as svgp_posterior_predict_kernel stages it
+    double* Lt = Ws + NP * WP;           // [NP][WP]    Lt[c][slot] = Lq[perm_n(slot)][c], as predict
+    double* Xt = Lt + NP * WP;           // [2d+4][NP]  inducing points, k-major
+    double* Xr = Xt + (2 * d + 4) * NP;  // [NSP][S1]   records of all test points (padding: dead)
+    double* Vt = Xr + NSP * S1;          // [NSP][WP]   V^T
+    double* Ut = Vt + NSP * WP;          // [NSP][WP]   U^T
+    fexp512_table_fill(etab, tid, blockDim.x);
+
+    {
+        const RecordParams rp = record_params(th, d);
+        const double* __restrict__ Wg = q.Wm + l * M * q.ld;
+        const double* __restrict__ Lg = q.Lq + l * M * q.ld;
+        for (int idx = tid; idx < NP * NP; idx += blockDim.x) {
+            const int r = idx / NP, c = idx - r * NP;
+            Ws[r * WP + c] = lower_entry(Wg, q.ld, M, r, c);
+            Lt[r * WP + c] = transposed_entry(Lg, q.ld, M, r, c);
+        }
+        stage_points(Xt, q.Z, M, NP, d, rp, tid);
+        for (int i = tid; i < NSP; i += blockDim.x) point_record(Xr + i * S1, p.Xs, i, Ns, d, rp);
+    }
+    __syncthreads();
+
+    // ---- per 8-point group: K_s, V^T = K_s^T Wm^T and U^T = V^T Lq as predict forms them, to shared memory in the
+    //      natural inducing order (slot 2k + e of lane t is m = 8k + 2t + e)
+    for (int grp = warp; grp < NST; grp += PW) {
+        const int i = 8 * grp + g;
+        double ks[2 * NT];
+        ks_fragment<NT>(ks, Xt, Xr + i * S1, d, t, etab);
+        double v[2 * NT];
+        lower_tri_v<NT>(v, ks, Ws, g, t);
+#pragma unroll
+        for (int k = 0; k < NT; ++k) {
+            Vt[i * WP + 8 * k + 2 * t] = v[2 * k];
+            Vt[i * WP + 8 * k + 2 * t + 1] = v[2 * k + 1];
+        }
+#pragma unroll
+        for (int k = 0; k < NT; ++k) upper_tri_product<NT>(Ut[i * WP + 8 * k + 2 * t], Ut[i * WP + 8 * k + 2 * t + 1], v, Lt, k, g, t);
+    }
+    __syncthreads();
+
+    // ---- Sigma_l on the lower 8x8 tiles, as gpr_posterior_joint_kernel forms K_ss - V^T V, plus U^T U
+    double* __restrict__ So = p.Sl + l * Ns * p.lds;
+    for (int tt = warp; tt < NST * (NST + 1) / 2; tt += PW) {
+        int I = 0;
+        while ((I + 1) * (I + 2) / 2 <= tt) ++I;
+        const int J = tt - I * (I + 1) / 2;
+        double c0 = 0.0, c1 = 0.0, e0 = 0.0, e1 = 0.0;
+        const double* va = Vt + (8 * I + g) * WP + t;
+        const double* vb = Vt + (8 * J + g) * WP + t;
+        const double* ua = Ut + (8 * I + g) * WP + t;
+        const double* ub = Ut + (8 * J + g) * WP + t;
+#pragma unroll
+        for (int k = 0; k < 2 * NT; ++k) {
+            dmma(c0, c1, va[4 * k], vb[4 * k]);
+            dmma(e0, e1, ua[4 * k], ub[4 * k]);
+        }
+        const int i = 8 * I + g;
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            const int j = 8 * J + 2 * t + e;
+            if (j > i || i >= Ns) continue;
+            const double s = kss_pair(Xr + i * S1, Xr + j * S1, d, etab) - (e ? c1 : c0) + (e ? e1 : e0);
+            So[(long)i * p.lds + j] = s;
+            So[(long)j * p.lds + i] = s;
+        }
+    }
+}
+
 // Input gradient of the blocked route (launch_posterior_dx): one CTA per (tile of TS test points, chunk of PC columns,
 // problem), walking the training points in tiles of TN.  Per tile it evaluates kL and kD from the scaled inputs (as K5
 // recomputes dK: nothing N x Ns is stored), forms G[j][s][n] = dk_sn/dx_sj in shared memory and adds G alpha (thread =
@@ -1278,5 +1379,18 @@ int svgp_posterior_predict_fused(cudaStream_t s, const SvgpPosteriorData& q, con
     const size_t smem = svgp_fused_smem_bytes(NT, q.d);
     return with_nt(NT, [&](auto nt) {
         return launch_fused<svgp_posterior_predict_kernel<decltype(nt)::value>>(s, a, gx, q.L, smem);
+    });
+}
+
+bool svgp_posterior_joint_fused_ok(int L, int M, int d, int Ns) { return svgp_posterior_fused_ok(L, M, d) && Ns <= JOINT_MAX_NS; }
+
+int svgp_posterior_cov_fused(cudaStream_t s, const SvgpPosteriorData& q, const double* Xs, int Ns, double* Sl, long lds) {
+    if (!svgp_posterior_joint_fused_ok(q.L, q.M, q.d, Ns)) return -1;
+    if (Ns <= 0) return 0;
+    const int NT = (q.M + 7) / 8;
+    const size_t smem = svgp_joint_smem_bytes(NT, (Ns + 7) / 8, q.d);
+    const SvgpJointArgs a{q, Xs, Ns, Sl, lds};
+    return with_nt(NT, [&](auto nt) {
+        return launch_fused<svgp_posterior_joint_kernel<decltype(nt)::value>>(s, a, 1, q.L, smem);
     });
 }

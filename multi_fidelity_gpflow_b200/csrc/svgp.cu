@@ -168,6 +168,32 @@ __global__ void mix_grad_kernel(const double* __restrict__ gm, const double* __r
     dvar[idx] = fv;
 }
 
+// Sp[p][i][j] = sum_l W[p][l]^2 Sl[l][i][j] on the lower triangle (l ascending, as mix_ve_kernel), mirrored: the joint
+// covariance of output p (mix_latent_gp with full_cov).  [.][Ns][lds] layouts; one thread per (p, i, j), j <= i working.
+__global__ void mix_cov_kernel(const double* __restrict__ Sl, int L, int Ns, long lds, int P, const double* __restrict__ W,
+                               double* __restrict__ Sp) {
+    const long per = (long)Ns * Ns, sl = (long)Ns * lds;
+    for (long idx = blockIdx.x * (long)blockDim.x + threadIdx.x; idx < (long)P * per; idx += (long)gridDim.x * blockDim.x) {
+        const long p = idx / per, r = idx - p * per, i = r / Ns, j = r - i * Ns;
+        if (j > i) continue;
+        double s = 0.0;
+        for (int l = 0; l < L; ++l) {
+            const double w = W[p * L + l];
+            s = fma(Sl[l * sl + i * lds + j], w * w, s);
+        }
+        Sp[p * sl + i * lds + j] = s;
+        Sp[p * sl + j * lds + i] = s;
+    }
+}
+
+// out[p][n] = in[n][P]: mean / var of _predict ([Ns][P]) as the per-output problems of the joint tail.
+__global__ void outputs_major_kernel(const double* __restrict__ in, int Ns, int P, double* __restrict__ out) {
+    for (long idx = blockIdx.x * (long)blockDim.x + threadIdx.x; idx < (long)Ns * P; idx += (long)gridDim.x * blockDim.x) {
+        const long p = idx / Ns, n = idx - p * Ns;
+        out[idx] = in[n * P + p];
+    }
+}
+
 // alpha[l][n][0] = sum_{m >= n} Wm[l][m][n] q_mu[m][l] (Wm lower triangular), alpha[l][n][1] = 0: the [L][M][2] table
 // posterior_dx_kernel reads as a with P = 1, Pp = 2.
 __global__ void svgp_alpha_kernel(const double* __restrict__ Wm, long ldM, const double* __restrict__ q_mu, int M, int L,
@@ -459,6 +485,55 @@ int launch_svgp_grad_mix(cudaStream_t s, const double* gm, const double* gv, int
     if (tot == 0) return 0;
     mix_grad_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(gm, gv, L, B, P, d, W, dmean, dvar);
     return cudaGetLastError() == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+}
+
+int launch_svgp_cov_mix(cudaStream_t s, const double* Sl, int L, int Ns, long lds, int P, const double* W, double* Sp) {
+    const long tot = (long)P * Ns * Ns;
+    const long nblk = (tot + 255) / 256 < 65536 ? (tot + 255) / 256 : 65536;
+    mix_cov_kernel<<<(unsigned)nblk, 256, 0, s>>>(Sl, L, Ns, lds, P, W, Sp);
+    return cudaGetLastError() == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+}
+
+int launch_outputs_major(cudaStream_t s, const double* in, int Ns, int P, double* out) {
+    const long tot = (long)Ns * P;
+    const long nblk = (tot + 255) / 256 < 65536 ? (tot + 255) / 256 : 65536;
+    outputs_major_kernel<<<(unsigned)nblk, 256, 0, s>>>(in, Ns, P, out);
+    return cudaGetLastError() == cudaSuccess ? 0 : MFGP_ERR_CUDA;
+}
+
+// Sigma_l = K_l(Xs, Xs) - V^T V + U^T U for every latent: V = f.A and U = f.C of svgp_conditional on all Ns points (not
+// chunked: Sigma couples every pair of points), K_ss from K1 (symmetric, batched over the latents with their theta
+// stride), then two lower-only batched GEMMs.
+int svgp_posterior_cov_blocked(mfgp_handle* h, Scope& sc, const SvgpPosteriorData& q, const double* Xs, int Ns, double* Sl,
+                               long lds) {
+    cudaStream_t s = h->stream;
+    Fwd f{};
+    f.Wm = const_cast<double*>(q.Wm);  // read only: svgp_conditional does not write the factors
+    f.Lq = const_cast<double*>(q.Lq);
+    f.ldM = q.ld;
+    f.sMM = (long)q.M * q.ld;
+    MFGP_TRY(svgp_conditional(h, sc, q.L, q.M, Ns, q.d, Xs, q.Z, q.theta, q.q_mu, f));
+    CovArgs k{};
+    k.Xa = Xs; k.Na = Ns; k.Xb = Xs; k.Nb = Ns; k.d = q.d;
+    k.theta = q.theta; k.theta_stride = 2 * q.d + 3;
+    k.K = Sl; k.ldk = lds; k.strideK = (long)Ns * lds;
+    k.symmetric = 1;
+    k.batch = q.L;
+    if (launch_cov(s, k)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp posterior: cov launch (K_ss) failed");
+    for (int pass = 0; pass < 2; ++pass) {  // Sigma -= V^T V, then Sigma += U^T U
+        const double* F = pass ? f.C : f.A;
+        GemmArgs g;
+        g.transA = true;
+        g.M = Ns; g.N = Ns; g.K = q.M;
+        g.alpha = pass ? 1.0 : -1.0; g.beta = 1.0;
+        g.A = F; g.lda = f.ldB; g.strideA = f.sMB;
+        g.B = F; g.ldb = f.ldB; g.strideB = f.sMB;
+        g.C = Sl; g.ldc = lds; g.strideC = (long)Ns * lds;
+        g.batch = q.L;
+        g.lower_only = 1;
+        if (launch_gemm(s, g)) return mfgp_fail(h, MFGP_ERR_CUDA, "svgp posterior: gemm (Sigma) failed");
+    }
+    return 0;
 }
 
 // Cached-posterior prediction for any M, d: per chunk of test points svgp_conditional from the cached Wm and Lq, then the

@@ -48,6 +48,18 @@ int svgp_posterior_predict_fused(cudaStream_t s, const SvgpPosteriorData& q, con
 // mean / var [Ns][P]; with dmean / dvar [Ns][P][d] (both or neither) also the input gradients.
 int svgp_posterior_predict_blocked(mfgp_handle* h, const SvgpPosteriorData& q, const double* Xs, int Ns, double* mean,
                                    double* var, double* dmean = nullptr, double* dvar = nullptr);
+// Joint covariance of every latent over Ns test points (mfgp_svgp_posterior_predict_cov / _sample), Sigma_l = K_l(Xs, Xs)
+// - V^T V + U^T U into Sl [L][Ns][lds] (lds even; the lower triangle and its mirror; the diagonal is the caller's to set).
+// Fused route (posterior.cu): one kernel for svgp_posterior_fused_ok and Ns <= 64.  Blocked route (svgp.cu): any size,
+// svgp_conditional on all Ns points with buffers from sc.
+bool svgp_posterior_joint_fused_ok(int L, int M, int d, int Ns);
+int svgp_posterior_cov_fused(cudaStream_t s, const SvgpPosteriorData& q, const double* Xs, int Ns, double* Sl, long lds);
+int svgp_posterior_cov_blocked(mfgp_handle* h, Scope& sc, const SvgpPosteriorData& q, const double* Xs, int Ns, double* Sl,
+                               long lds);
+// Sp [P][Ns][lds] = sum_l W_pl^2 Sl on the lower triangle in a fixed l order, mirrored.
+int launch_svgp_cov_mix(cudaStream_t s, const double* Sl, int L, int Ns, long lds, int P, const double* W, double* Sp);
+// out [P][Ns] <- in [Ns][P].
+int launch_outputs_major(cudaStream_t s, const double* in, int Ns, int P, double* out);
 // dmean / dvar [B][P][d] from the latent gradients gm / gv [L][B][d] as launch_svgp_mix mixes the marginals:
 // dmean = sum_l W_pl gm_l, dvar = sum_l W_pl^2 gv_l in a fixed l order, or the gather of latent p when W == NULL.
 int launch_svgp_grad_mix(cudaStream_t s, const double* gm, const double* gv, int L, int B, int P, int d, const double* W,

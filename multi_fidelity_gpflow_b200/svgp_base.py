@@ -294,6 +294,15 @@ class SVGPBase:
         return SVGPPosterior(self.handle.svgp_posterior(Z, self._thetas(d), self._W(), self.q_mu.numpy(),
                                                         np.tril(self.q_sqrt.numpy())))
 
+    def predict_f_samples(self, Xnew, num_samples=None, full_cov=True, full_output_cov=False, seed=None):
+        """GPflow's GPModel.predict_f_samples: [S, N*, P] ([N*, P] when num_samples is None), from a cached posterior made
+        and freed by this call (SVGPPosterior.predict_f_samples)."""
+        post = self.posterior()
+        try:
+            return post.predict_f_samples(Xnew, num_samples, full_cov, full_output_cov, seed)
+        finally:
+            post.close()
+
     # ---- checkpoint (pickle of gpflow.utilities.parameter_dict-style names) ------------------------
     def save_model(self, filename):
         with open(filename, "wb") as f:
@@ -306,8 +315,9 @@ class SVGPBase:
 
 
 class SVGPPosterior:
-    """What SVGPBase.posterior() returns: predict_f(Xnew) -> mean, var [N*, P] from the cached factors, and
-    predict_f_grad(Xnew) with their input gradients."""
+    """What SVGPBase.posterior() returns: predict_f(Xnew) -> mean, var [N*, P] from the cached factors,
+    predict_f_grad(Xnew) with their input gradients, and the joint posterior over the N* points, predict_f_full_cov and
+    predict_f_samples."""
 
     def __init__(self, post):
         self.post = post
@@ -316,6 +326,22 @@ class SVGPPosterior:
         if full_cov or full_output_cov:
             raise NotImplementedError("the reference only calls predict_f(Xnew) (marginal variances)")
         return self.post.predict(_lib.as_f64(Xnew))
+
+    def predict_f_full_cov(self, Xnew):
+        """SVGP.predict_f(Xnew, full_cov=True): mean [N*, P] and each output's covariance over the N* points, cov
+        [P, N*, N*].  mean and the diagonals are predict_f's, bit for bit."""
+        return self.post.predict_cov(_lib.as_f64(Xnew))
+
+    def predict_f_samples(self, Xnew, num_samples=None, full_cov=True, full_output_cov=False, seed=None):
+        """GPflow's predict_f_samples with full_output_cov=False: [S, N*, P] ([N*, P] when num_samples is None), each
+        output drawn on its own.  full_cov=True draws jointly over the N* points with jitter 1e-6, full_cov=False
+        independently per point.  The normals are np.random.default_rng(seed).standard_normal((P, N*, S))."""
+        f = self.post.draw_f(_lib.as_f64(Xnew), num_samples, full_cov, full_output_cov, seed)
+        f = np.transpose(f, (2, 1, 0))  # [S, N*, P]
+        return np.ascontiguousarray(f[0] if num_samples is None else f)
+
+    def close(self):
+        self.post.close()
 
     def predict_f_grad(self, Xnew):
         """predict_f and its gradient with respect to Xnew: mean, var [N*, P] and dmean_dx, dvar_dx [N*, P, d+1]
